@@ -524,6 +524,16 @@ def c3_sweep_block(rank, world, dev, steps=3):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+def dump_outputs(out_dir, res, prefix=""):
+    """The arrays a caller of the timed path receives (Pipeline.result(): rows windowKLD/GC/PI/SI/CRI, row status bits,
+    background tables, window coordinates, totalLen/exMax/nnTotal), all of them, as float64: counts and coordinates stay
+    below 2**53, so the conversion is exact.  About 2 MB per GPU for C2."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"rows": res.rows, "status": res.status, "tables": res.tables, "coords": res.coords, "meta": np.array(res.meta)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -594,12 +604,14 @@ def run_gpu(args):
     stage = np.array([[m[i].elapsed_time(m[i + 1]) for i in range(3)] for m in marks_all])   # ms
     step_ms = np.array([m[0].elapsed_time(m[3]) for m in marks_all])
     total_ms = float(step_ms.sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pipe.result(names=False), "" if world == 1 else "rank%d_" % rank)
 
     # ---- end to end through ONE C-ABI call from pinned host buffers; H2D of planes + window list and D2H of the rows
     # ---- inside the timer.  No cross-rank host barrier between steps (a pipeline has none): the ranks meet inside the call.
     out = engine.HostOutputs(n_win, PARAMS["kmax"])
     wins = pipe.wins
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
 
     def e2e_once():
         if world == 1:
@@ -835,7 +847,11 @@ def main():
     ap.add_argument("--profile", action="store_true", help="kernels only: skip the e2e, extra-block and CPU-baseline legs (for ncu)")
     ap.add_argument("--quick", action="store_true", help="skip the parity / strong / c5 / c3_sweep blocks")
     ap.add_argument("--c5", action="store_true", help="N = 1: run the c5 block too (1.75 Gbp from FASTA text)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step to DIR/<name>.npy "
+                                                          "(float64), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,6 +3,8 @@ C-ABI surface.  No compute kernels are called (there is no GPU here and no CPU f
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -26,14 +28,20 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_fails_loudly_without_a_gpu():
-    if _lib.device_count() > 0:
-        pytest.skip("a GPU is present")
-    g = engine.PackedGenome.from_scaffolds(synth.make("edge"))
-    with pytest.raises(_lib.FriskError) as ei:
-        engine.run(g)
-    assert ei.value.code == _lib.E_NO_DEVICE
-    with pytest.raises(_lib.FriskError):
-        engine.run_host(g)
+    """Runs in a child process that sees no CUDA device, so the check holds on machines with a GPU too."""
+    code = ("import pytest\n"
+            "from frisk_b200 import _lib, engine, synth\n"
+            "assert _lib.device_count() == 0\n"
+            "g = engine.PackedGenome.from_scaffolds(synth.make('edge'))\n"
+            "with pytest.raises(_lib.FriskError) as ei:\n"
+            "    engine.run(g)\n"
+            "assert ei.value.code == _lib.E_NO_DEVICE\n"
+            "with pytest.raises(_lib.FriskError):\n"
+            "    engine.run_host(g)\n"
+            "print('no device: refused')\n")
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT, env=env, timeout=600)
+    assert out.returncode == 0 and "no device: refused" in out.stdout, out.stdout[-1000:] + out.stderr[-3000:]
 
 
 def _unpack(g, s):
