@@ -65,6 +65,13 @@ PROTOTYPES = {
                                   C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _p]),
     "frisk_b200_windows_device": (_i, [_p, _p, _u64, _i, _i, _i, _u64, _p, _p, _p, _p, _p]),
     "frisk_b200_fasta_info": (_i, [_p, C.POINTER(_u64), C.POINTER(_u64), _p]),
+    "frisk_b200_bgzf_blocks": (_i, [_p, _u64, _u64, _p, _p, _p, _p, C.POINTER(_u64), C.POINTER(_u64)]),
+    "frisk_b200_bgzf_inflate": (_i, [_p, _p, _p, _p, _p, _u64, _u64, _p, _p, _p]),
+    "frisk_b200_bgzf_inflate_host": (_i, [_p, _p, _p, _p, _p, _u64, _u64, _p, _p, _p]),
+    "frisk_b200_fasta_open_bgzf": (_i, [_p, _u64, _p, C.POINTER(C.c_void_p), C.POINTER(_u64), C.POINTER(_u64), _p]),
+    "frisk_b200_run_fasta_bgzf": (_i, [_p, _u64, _p, _u64, _i, _i, _i, _i, _i, _i, _i, _u64, _p, _p, _p, _p, C.POINTER(_u64),
+                                       C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _p]),
+    "frisk_b200_fasta_name_text": (_i, [_p, C.POINTER(C.c_void_p), C.POINTER(_u64)]),
     "frisk_b200_fasta_planes": (_i, [_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     "frisk_b200_last_run_timing": (_i, [C.POINTER(C.c_float), _i, C.POINTER(_i)]),
     "frisk_b200_score_sweep": (_i, [_p, _p, _p, _p, _p, _u64, C.c_uint32, _p, _i, _i, _p, _p, _p]),
@@ -92,7 +99,7 @@ class FriskError(RuntimeError):
 def build(force: bool = False) -> str:
     """Compile the shared library in-tree (nvcc, sm_100a).  Cross-compiles without a GPU."""
     src_dir = os.path.join(HERE, "csrc")
-    srcs = [os.path.join(src_dir, f) for f in ("frisk_kernels.cu", "frisk_direct.cu", "frisk_device.cuh", "frisk_general.cu", "frisk_ingest.cu", "frisk_features.cu", "frisk_host.cpp", "frisk_internal.h", "Makefile")]
+    srcs = [os.path.join(src_dir, f) for f in ("frisk_kernels.cu", "frisk_direct.cu", "frisk_device.cuh", "frisk_general.cu", "frisk_ingest.cu", "frisk_bgzf.cu", "frisk_features.cu", "frisk_host.cpp", "frisk_internal.h", "Makefile")]
     srcs.append(os.path.join(os.path.dirname(HERE), "include", "frisk_b200.h"))
     stale = not os.path.exists(SO_PATH) or any(os.path.getmtime(s) > os.path.getmtime(SO_PATH) for s in srcs)
     if force or stale:

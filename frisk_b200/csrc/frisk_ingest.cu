@@ -21,6 +21,8 @@
 // the state between chunks in device memory.  Record table and planes are sized by a guess so that the host synchronises
 // once; a text that does not fit the guesses, or a line decision that needs a byte of a later chunk, is redone in one piece
 // with exact sizes (open_any).  The planes belong to the handle.
+// A BGZF source (frisk_b200_fasta_open_bgzf, frisk_b200_run_fasta_bgzf) shares all of it: the compressed bytes go up on the
+// upload lane, frisk_bgzf.cu inflates them into the text buffer, and the passes wait on that instead of on the text's copy.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -627,6 +629,40 @@ fasta_pack_kernel(const uint8_t* __restrict__ t, uint64_t n, uint64_t tile0, uin
     }
 }
 
+// ---- names of a BGZF open: the text stays on the device, so the header lines are gathered into one buffer ----------------
+// line_len[r]: bytes of record r's header line from hdr_pos[r], its newline included (none at the end of the text)
+__global__ void header_len_kernel(const uint8_t* __restrict__ t, uint64_t n, const unsigned long long* __restrict__ hdr_pos,
+                                  uint64_t n_rec, unsigned long long* __restrict__ line_len) {
+    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rec) return;
+    uint64_t i = hdr_pos[r];
+    while (i < n && t[i] != '\n') ++i;
+    line_len[r] = (i < n ? i + 1 : n) - hdr_pos[r];
+}
+
+// in place: line_len[0..n_rec) -> exclusive prefix sum, line_len[n_rec] = total (one CTA of kST threads)
+__global__ void __launch_bounds__(kST) header_scan_kernel(unsigned long long* __restrict__ v, uint64_t n_rec) {
+    __shared__ unsigned long long sm[64];
+    unsigned long long carry = 0;
+    for (uint64_t b0 = 0; b0 < n_rec; b0 += kST) {
+        const uint64_t i = b0 + threadIdx.x;
+        const unsigned long long x = i < n_rec ? v[i] : 0ull;
+        unsigned long long total;
+        const unsigned long long e = block_excl_sum<unsigned long long>(x, sm, &total);
+        if (i < n_rec) v[i] = carry + e;
+        carry += total;
+    }
+    if (threadIdx.x == 0) v[n_rec] = carry;
+}
+
+__global__ void header_gather_kernel(const uint8_t* __restrict__ t, const unsigned long long* __restrict__ hdr_pos,
+                                     const unsigned long long* __restrict__ line_off, uint64_t n_rec, uint8_t* __restrict__ out) {
+    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_rec) return;
+    const uint64_t a = hdr_pos[r], o = line_off[r], len = line_off[r + 1] - o;
+    for (uint64_t k = 0; k < len; ++k) out[o + k] = t[a + k];
+}
+
 }  // namespace
 
 struct frisk_b200_fasta {
@@ -641,16 +677,19 @@ struct frisk_b200_fasta {
     void *d_scan_slab = nullptr, *d_out_slab = nullptr;                  // what the pointers above (but d_text) are carved from
     uint64_t rec_cap = 0;                                                // entries of the device record table
     bool streamed = false;                                               // opened on the chunked, speculatively sized path
+    bool bgzf = false;                                                   // opened from BGZF: names index name_text
+    void* d_gz_slab = nullptr;                                           // BGZF: compressed bytes, block table, status words
     std::vector<uint64_t> name_off, seq_len, scaf_off, hdr_pos;
     std::vector<uint32_t> name_len;
+    std::vector<char> name_text;                                         // BGZF: the header lines, one after the other
 };
 
 namespace {
 int free_all(frisk_b200_fasta* h, cudaStream_t st) {
-    void* ptrs[] = {h->d_text, h->d_scan_slab, h->d_out_slab};
+    void* ptrs[] = {h->d_text, h->d_scan_slab, h->d_out_slab, h->d_gz_slab};
     for (void* p : ptrs)
         if (p) FRISK_CK(cudaFreeAsync(p, st));
-    h->d_text = nullptr; h->d_scan_slab = h->d_out_slab = nullptr;
+    h->d_text = nullptr; h->d_scan_slab = h->d_out_slab = h->d_gz_slab = nullptr;
     h->d_nhdr = h->d_head = h->d_pre = h->d_post = h->d_inner = h->d_rec_base = nullptr;
     h->d_key = h->d_carry = nullptr;
     h->d_base_in = h->d_open_off = h->d_hdr_pos = h->d_len = h->d_scaf_off = h->d_counters = nullptr;
@@ -691,9 +730,90 @@ int upload_lane(UploadLane** out) {
         FRISK_CK(cudaStreamCreateWithFlags(&l.copy, cudaStreamNonBlocking));
         FRISK_CK(cudaEventCreateWithFlags(&l.ready, cudaEventDisableTiming));
         for (auto& e : l.done) FRISK_CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        FRISK_CK(cudaHostAlloc((void**)&l.stage, (2 * kFirstFetch + kCtrCount) * 8, cudaHostAllocDefault));
+        FRISK_CK(cudaHostAlloc((void**)&l.stage, (2 * kFirstFetch + kCtrCount + 1) * 8, cudaHostAllocDefault));
     }
     *out = &l;
+    return FRISK_OK;
+}
+
+// What an open reads: a host text, or a BGZF buffer with its block table (the text is inflated on the device).
+struct Source {
+    const char* text = nullptr;           // host text (nullptr for BGZF)
+    uint64_t n = 0;                       // text bytes (BGZF: inflated)
+    bool bgzf = false;
+    const uint8_t* gz = nullptr;
+    uint64_t gz_n = 0, n_blocks = 0;
+    std::vector<uint64_t> table;          // per block: comp_off, text_off (8 bytes each), comp_len, crc (4 bytes each)
+    uint8_t* d_ready = nullptr;           // the exact re-open: the text the first attempt inflated (the handle takes it)
+};
+
+int make_source(const char* text, uint64_t n, bool bgzf, Source* src) {
+    if (!bgzf) { src->text = text; src->n = n; return FRISK_OK; }
+    src->bgzf = true;
+    src->gz = reinterpret_cast<const uint8_t*>(text);
+    src->gz_n = n;
+    uint64_t nb = 0, tl = 0;
+    int rc = frisk_b200_bgzf_blocks(src->gz, n, 0, nullptr, nullptr, nullptr, nullptr, &nb, &tl);
+    if (rc) return rc;
+    src->table.assign(nb * 3, 0);
+    uint64_t* const t = src->table.data();
+    uint32_t* const t32 = reinterpret_cast<uint32_t*>(t + 2 * nb);
+    if ((rc = frisk_b200_bgzf_blocks(src->gz, n, nb, t, t32, t32 + nb, t + nb, &nb, &tl))) return rc;
+    src->n_blocks = nb;
+    src->n = tl;
+    return FRISK_OK;
+}
+
+// BGZF: compressed bytes and block table up on `copy`, every member inflated into h->d_text behind them.  The status words
+// and the "some member failed" word stay in h->d_gz_slab until the open has read that word back.
+int bgzf_upload_inflate(frisk_b200_fasta* h, const Source& src, cudaStream_t alloc_st, cudaStream_t copy, unsigned int** d_any_bad) {
+    const uint64_t nb = src.n_blocks;
+    const uint64_t gz_bytes = (src.gz_n + 255) & ~255ull, tab_bytes = nb * 24;
+    FRISK_CK(cudaMallocAsync(&h->d_gz_slab, gz_bytes + tab_bytes + nb * 4 + 256, alloc_st));
+    char* const base = (char*)h->d_gz_slab;
+    const uint64_t* const tab = (const uint64_t*)(base + gz_bytes);
+    uint32_t* const status = (uint32_t*)(base + gz_bytes + tab_bytes);
+    *d_any_bad = (unsigned int*)(status + nb);
+    FRISK_CK(cudaMemsetAsync(*d_any_bad, 0, 4, alloc_st));
+    cudaEvent_t ready;                                                  // (the slab exists in stream order)
+    FRISK_CK(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
+    FRISK_CK(cudaEventRecord(ready, alloc_st));
+    FRISK_CK(cudaStreamWaitEvent(copy, ready, 0));
+    FRISK_CK(cudaEventDestroy(ready));
+    FRISK_CK(cudaMemcpyAsync(base, src.gz, src.gz_n, cudaMemcpyHostToDevice, copy));
+    FRISK_CK(cudaMemcpyAsync((void*)tab, src.table.data(), tab_bytes, cudaMemcpyHostToDevice, copy));
+    const uint32_t* const t32 = (const uint32_t*)(tab + 2 * nb);
+    return frisk_internal::bgzf_inflate((const uint8_t*)base, tab, t32, t32 + nb, tab + nb, nb, src.n, h->d_text, status, *d_any_bad, copy);
+}
+
+// The names of a BGZF handle: the header lines (hdr_pos[r] to their newline) are gathered on the device into one buffer that
+// comes back in one copy; parse_header_name then reads it exactly as it reads the text of a text open.
+int gather_names(frisk_b200_fasta* h, cudaStream_t st) {
+    const uint64_t R = h->n_rec;
+    h->name_text.clear();
+    if (!R) return FRISK_OK;
+    unsigned long long* d_off = nullptr;
+    FRISK_CK(cudaMallocAsync((void**)&d_off, (R + 1) * 8, st));
+    const unsigned grid = (unsigned)((R + 255) / 256);
+    header_len_kernel<<<grid, 256, 0, st>>>(h->d_text, h->n, h->d_hdr_pos, R, d_off);
+    header_scan_kernel<<<1, kST, 0, st>>>(d_off, R);
+    FRISK_CK(cudaGetLastError());
+    std::vector<uint64_t> off(R + 1);
+    FRISK_CK(cudaMemcpyAsync(off.data(), d_off, (R + 1) * 8, cudaMemcpyDeviceToHost, st));
+    FRISK_CK(cudaStreamSynchronize(st));
+    const uint64_t total = off[R];
+    uint8_t* d_lines = nullptr;
+    FRISK_CK(cudaMallocAsync((void**)&d_lines, total + 1, st));
+    header_gather_kernel<<<grid, 256, 0, st>>>(h->d_text, h->d_hdr_pos, d_off, R, d_lines);
+    FRISK_CK(cudaGetLastError());
+    h->name_text.resize(total);
+    FRISK_CK(cudaMemcpyAsync(h->name_text.data(), d_lines, total, cudaMemcpyDeviceToHost, st));
+    FRISK_CK(cudaFreeAsync(d_lines, st));
+    FRISK_CK(cudaFreeAsync(d_off, st));
+    FRISK_CK(cudaStreamSynchronize(st));
+    const unsigned char* const t = reinterpret_cast<const unsigned char*>(h->name_text.data());
+    for (uint64_t r = 0; r < R; ++r)
+        if (!frisk_internal::parse_header_name(t, total, off[r], &h->name_off[r], &h->name_len[r])) return FRISK_E_FORMAT;
     return FRISK_OK;
 }
 
@@ -706,11 +826,18 @@ int upload_lane(UploadLane** out) {
 // exact = true: one copy; summary + tile scan give the record count and the layout's length, the host reads them (one more
 //   synchronisation), allocates exactly and runs the pack pass.  Cannot fail that way.
 // sink (nullable, !exact only): sink->on_range is handed the plane words that became final with every chunk.
-int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st, bool exact, frisk_internal::IngestSink* sink) {
+// BGZF source: the compressed bytes go up on the upload lane in one copy and one inflate launch fills the text buffer; the
+// passes of every chunk wait on it (the whole text is there, so no line decision needs a later chunk), and the text is one
+// chunk unless ingest_chunk_tiles asks for more.  The exact re-open takes over the text the first attempt inflated.
+int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exact, frisk_internal::IngestSink* sink) {
     int rc = frisk_internal::pool_ready();
     if (rc) return rc;
     if (exact) sink = nullptr;
+    const char* const text = src.text;
+    const uint64_t n = src.n;
     h->n = n;
+    h->bgzf = src.bgzf;
+    unsigned int* d_any_bad = nullptr;                                  // BGZF: some member failed to inflate
     h->n_tiles = n ? (n + kTile - 1) / kTile : 0;
     if (h->n_tiles > 0x7fffffffull) return FRISK_E_UNSUPPORTED;         // 8 TB of text per call
     const uint64_t T = h->n_tiles;
@@ -748,10 +875,22 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         if ((rc = alloc_out(1, 128))) return rc;
         FRISK_CK(cudaMemsetAsync(h->d_inv, 0xff, 128 / 8, st));
         h->padded_len = 128;
+        if (src.n_blocks) {                                             // empty members only: still checked
+            if ((rc = bgzf_upload_inflate(h, src, st, st, &d_any_bad))) return rc;
+            if (sink && sink->uploaded_mark) FRISK_CK(cudaEventRecord(sink->uploaded_mark, st));
+            unsigned int bad = 0;
+            FRISK_CK(cudaMemcpyAsync(&bad, d_any_bad, 4, cudaMemcpyDeviceToHost, st));
+            FRISK_CK(cudaStreamSynchronize(st));
+            if (bad) return FRISK_E_FORMAT;
+        }
     } else {
         const uint64_t padded_text = T * kTile + 16;
-        FRISK_CK(cudaMallocAsync((void**)&h->d_text, padded_text, st));
-        FRISK_CK(cudaMemsetAsync(h->d_text + n, '\n', padded_text - n, st));
+        if (src.d_ready) {
+            h->d_text = src.d_ready;                                    // (its padding is in place)
+        } else {
+            FRISK_CK(cudaMallocAsync((void**)&h->d_text, padded_text, st));
+            FRISK_CK(cudaMemsetAsync(h->d_text + n, '\n', padded_text - n, st));
+        }
         // Chunk plan (tile bounds, multiples of kSP): equal chunks of >= 1400 tiles (5.6 MiB; ingest_chunk_tiles overrides), at most
         // kMaxChunks.  Measured on C2 (40.8 MB, 52 GB/s over PCIe): beside a running H2D copy the three passes + count of a
         // chunk take about as long as the chunk's copy, and every launch of a short chunk costs ~10 us whatever its size, so
@@ -765,7 +904,8 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         if (!exact) {
             auto round_sp = [](uint64_t v) { return (v + kSP - 1) / kSP * kSP; };
             const uint64_t min_tiles = frisk_internal::g_ingest_chunk_tiles > 0 ? (uint64_t)frisk_internal::g_ingest_chunk_tiles : kMinChunkTiles;
-            const uint64_t want = std::max<uint64_t>(1, std::min<uint64_t>(kMaxChunks, T / min_tiles));
+            const uint64_t want = src.bgzf && frisk_internal::g_ingest_chunk_tiles <= 0
+                                      ? 1 : std::max<uint64_t>(1, std::min<uint64_t>(kMaxChunks, T / min_tiles));
             const uint64_t per = round_sp((T + want - 1) / want);
             n_chunks = 0;
             for (uint64_t t0 = 0; t0 < T; t0 += per) bound[++n_chunks] = std::min<uint64_t>(t0 + per, T);
@@ -786,6 +926,7 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         };
         tmark(st);
         auto issue_copy = [&](int c) -> int {
+            if (src.bgzf) return FRISK_OK;                              // (uploaded and inflated below, all chunks at once)
             const uint64_t b0 = bound[c] * kTile, b1 = std::min<uint64_t>(bound[c + 1] * kTile, n);
             FRISK_CK(cudaMemcpyAsync(h->d_text + b0, text + b0, b1 - b0, cudaMemcpyHostToDevice, lane->copy));
             FRISK_CK(cudaEventRecord(lane->done[c], lane->copy));
@@ -795,8 +936,13 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         // page-locked text: every copy is queued before anything else is set up (the first byte leaves ~20 us earlier);
         // pageable text: a copy returns when its chunk is staged, so each one is issued just before its chunk's passes
         cudaPointerAttributes pa{};
-        const bool pinned = cudaPointerGetAttributes(&pa, text) == cudaSuccess && pa.type == cudaMemoryTypeHost;
+        const bool pinned = !src.bgzf && cudaPointerGetAttributes(&pa, text) == cudaSuccess && pa.type == cudaMemoryTypeHost;
         cudaGetLastError();
+        if (src.bgzf) {
+            if (!src.d_ready && (rc = bgzf_upload_inflate(h, src, st, lane->copy, &d_any_bad))) return rc;
+            for (int c = 0; c <= last_chunk; ++c) FRISK_CK(cudaEventRecord(lane->done[c], lane->copy));
+            if (sink && sink->uploaded_mark) FRISK_CK(cudaEventRecord(sink->uploaded_mark, lane->copy));
+        }
         if (pinned && !trace)
             for (int c = 0; c <= last_chunk; ++c)
                 if ((rc = issue_copy(c))) return rc;
@@ -811,6 +957,7 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         for (int c = 0; c <= last_chunk; ++c) {
             const uint64_t t0 = bound[c], t1 = bound[c + 1];
             const uint64_t b1 = std::min<uint64_t>(t1 * kTile, n);
+            const uint64_t avail = src.bgzf ? n : b1;                   // bytes on the device when the chunk's passes run
             const bool final = c == last_chunk;
             if (!pinned || trace) {
                 if ((rc = issue_copy(c))) return rc;
@@ -819,13 +966,13 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
             FRISK_CK(cudaStreamWaitEvent(st, lane->done[c], 0));
             unsigned long long* const d_range = h->d_counters + kCtrCount + (size_t)kRangeSlots * c;
             const bool count_now = sink && sink->on_range && count_at[c];
-            fasta_summary_kernel<<<(unsigned)(t1 - t0), kTT, 0, st>>>(h->d_text, n, t0, b1, h->d_counters, h->d_nhdr, h->d_key, h->d_head,
+            fasta_summary_kernel<<<(unsigned)(t1 - t0), kTT, 0, st>>>(h->d_text, n, t0, avail, h->d_counters, h->d_nhdr, h->d_key, h->d_head,
                                                                        h->d_pre, h->d_post, h->d_inner);
             fasta_tilescan_kernel<<<1, kST, 0, st>>>(h->d_nhdr, h->d_key, h->d_head, h->d_pre, h->d_post, h->d_inner, t0, t1, h->d_rec_base,
                                                      h->d_carry, h->d_base_in, h->d_open_off, h->d_counters, d_range,
                                                      exact ? ~0ull : rec_cap, exact ? ~0ull : plane_cap, (int)count_now, (int)final);
             tmark(st);
-            if (!exact) pack_pass(t0, t1, b1, final);
+            if (!exact) pack_pass(t0, t1, avail, final);
             tmark(st);
             FRISK_CK(cudaGetLastError());
             if (final && !exact) {                                      // the record table is complete: the host can have it now,
@@ -865,8 +1012,11 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
         FRISK_CK(cudaMemcpyAsync(sg, h->d_len, first * 8, cudaMemcpyDeviceToHost, back));
         FRISK_CK(cudaMemcpyAsync(sg + kFirstFetch, h->d_hdr_pos, first * 8, cudaMemcpyDeviceToHost, back));
         FRISK_CK(cudaMemcpyAsync(sg + 2 * kFirstFetch, h->d_counters, kCtrCount * 8, cudaMemcpyDeviceToHost, back));
+        sg[2 * kFirstFetch + kCtrCount] = 0;
+        if (d_any_bad) FRISK_CK(cudaMemcpyAsync(sg + 2 * kFirstFetch + kCtrCount, d_any_bad, 4, cudaMemcpyDeviceToHost, back));
         FRISK_CK(cudaStreamSynchronize(back));
         memcpy(ctr, sg + 2 * kFirstFetch, kCtrCount * 8);
+        if (sg[2 * kFirstFetch + kCtrCount]) return FRISK_E_FORMAT;    // a BGZF member is not valid deflate or fails its CRC
         if (!exact && (ctr[kCtrAmbig] || ctr[kCtrOverflow])) return kRetryExact;
         if (ctr[kCtrWhitespace]) return FRISK_E_FORMAT;                // whitespace inside a sequence line
         const uint64_t n_rec = ctr[kCtrRecords];
@@ -887,12 +1037,18 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
     // names (F:156) and the 128-base aligned layout
     const uint64_t R = h->n_rec;
     h->name_off.resize(R); h->name_len.resize(R); h->scaf_off.resize(R);
-    const unsigned char* tt = reinterpret_cast<const unsigned char*>(text);
-    uint64_t total = 0;
-    for (uint64_t r = 0; r < R; ++r) {
-        if (!frisk_internal::parse_header_name(tt, n, h->hdr_pos[r], &h->name_off[r], &h->name_len[r])) return FRISK_E_FORMAT;
-        total += h->seq_len[r];
+    if (src.bgzf) {
+        if (h->d_gz_slab) FRISK_CK(cudaFreeAsync(h->d_gz_slab, st));    // (the inflate is behind the synchronisation above)
+        h->d_gz_slab = nullptr;
+        // beside the tail run_fasta may have queued on `st`: on the upload lane, which follows the last chunk's pack
+        if ((rc = gather_names(h, exact || !T ? st : lane->copy))) return rc;
+    } else {
+        const unsigned char* tt = reinterpret_cast<const unsigned char*>(text);
+        for (uint64_t r = 0; r < R; ++r)
+            if (!frisk_internal::parse_header_name(tt, n, h->hdr_pos[r], &h->name_off[r], &h->name_len[r])) return FRISK_E_FORMAT;
     }
+    uint64_t total = 0;
+    for (uint64_t r = 0; r < R; ++r) total += h->seq_len[r];
     h->stats[0] = total;
     const uint64_t device_padded = h->padded_len;
     rc = frisk_b200_pack_layout(h->seq_len.data(), R, h->scaf_off.data(), &h->padded_len);
@@ -904,43 +1060,36 @@ int open_impl(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st
 }
 
 // open with retry
-int open_any(frisk_b200_fasta* h, const char* text, uint64_t n, cudaStream_t st, frisk_internal::IngestSink* sink) {
+int open_any(frisk_b200_fasta* h, Source& src, cudaStream_t st, frisk_internal::IngestSink* sink) {
     const bool exact = frisk_internal::g_ingest_exact != 0;
     if (sink) sink->counted = false;
-    int rc = open_impl(h, text, n, st, exact, sink);
+    int rc = open_impl(h, src, st, exact, sink);
     if (rc == FRISK_OK && !exact) g_open_stats[0].fetch_add(1);
     if (rc == kRetryExact) {
         g_open_stats[1].fetch_add(1);
         FRISK_CK(cudaStreamSynchronize(st));                            // (the abandoned attempt's work targets what is freed next)
         if (sink && sink->abandon && (rc = sink->abandon(st))) return rc;
+        if (src.bgzf) { src.d_ready = h->d_text; h->d_text = nullptr; }  // inflated once: the re-open keeps the text
         if ((rc = free_all(h, st))) return rc;
         *h = frisk_b200_fasta();
-        rc = open_impl(h, text, n, st, true, nullptr);
+        rc = open_impl(h, src, st, true, nullptr);
+        if (src.bgzf && !h->d_text && src.d_ready) FRISK_CK(cudaFreeAsync(src.d_ready, st));   // (not taken over)
+        src.d_ready = nullptr;
         if (sink) sink->counted = false;
     }
     return rc;
 }
-}  // namespace
 
-bool frisk_internal::fasta_open_was_streamed(const frisk_b200_fasta* h) { return h && h->streamed; }
-
-int frisk_internal::fasta_device_table(const frisk_b200_fasta* h, const unsigned long long** d_len, const unsigned long long** d_scaf_off,
-                                       const unsigned long long** d_counters, uint64_t* rec_cap, const uint32_t** d_codes,
-                                       const uint32_t** d_inv, const uint32_t** d_low) {
-    if (!h || !h->d_counters || !h->d_len || !h->d_codes) return FRISK_E_INVALID;
-    *d_len = h->d_len; *d_scaf_off = h->d_scaf_off; *d_counters = h->d_counters; *rec_cap = h->rec_cap;
-    *d_codes = h->d_codes; *d_inv = h->d_inv; *d_low = h->d_low;
-    return FRISK_OK;
-}
-
-int frisk_internal::fasta_open_planes(const char* text, uint64_t n, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out) {
-    if (!out || !sink || (!text && n)) return FRISK_E_INVALID;
+// the public opens and the one-call path: block table (BGZF), open with retry; no handle on failure
+int open_handle(const char* text, uint64_t n, bool bgzf, cudaStream_t st, frisk_internal::IngestSink* sink, frisk_b200_fasta** out) {
     *out = nullptr;
     frisk_b200_fasta* h = new (std::nothrow) frisk_b200_fasta();
     if (!h) return FRISK_E_INVALID;
     int rc;
-    try {
-        rc = open_any(h, text, n, st, sink);
+    try {                                                 // std::bad_alloc of the record table: nothing crosses the ABI
+        Source src;
+        rc = make_source(text, n, bgzf, &src);
+        if (!rc) rc = open_any(h, src, st, sink);
     } catch (...) {
         rc = FRISK_E_CAPACITY;
     }
@@ -950,6 +1099,39 @@ int frisk_internal::fasta_open_planes(const char* text, uint64_t n, cudaStream_t
         return rc;
     }
     *out = h;
+    return FRISK_OK;
+}
+
+// frisk_b200_fasta_open and frisk_b200_fasta_open_bgzf
+int open_public(const char* text, uint64_t n, bool bgzf, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
+                uint64_t* padded_len, uint64_t stats[3]) {
+    if (!out || (!text && n)) return FRISK_E_INVALID;
+    *out = nullptr;
+    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
+    frisk_b200_fasta* h = nullptr;
+    const int rc = open_handle(text, n, bgzf, (cudaStream_t)stream, nullptr, &h);
+    if (rc) return rc;
+    if (n_records) *n_records = h->n_rec;
+    if (padded_len) *padded_len = h->padded_len;
+    if (stats) { stats[0] = h->stats[0]; stats[1] = h->stats[1]; stats[2] = h->stats[2]; }
+    *out = h;
+    return FRISK_OK;
+}
+}  // namespace
+
+bool frisk_internal::fasta_open_was_streamed(const frisk_b200_fasta* h) { return h && h->streamed; }
+
+int frisk_internal::fasta_open_planes(const char* text, uint64_t n, bool bgzf, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out) {
+    if (!out || !sink || (!text && n)) return FRISK_E_INVALID;
+    return open_handle(text, n, bgzf, st, sink, out);
+}
+
+int frisk_internal::fasta_device_table(const frisk_b200_fasta* h, const unsigned long long** d_len, const unsigned long long** d_scaf_off,
+                                       const unsigned long long** d_counters, uint64_t* rec_cap, const uint32_t** d_codes,
+                                       const uint32_t** d_inv, const uint32_t** d_low) {
+    if (!h || !h->d_counters || !h->d_len || !h->d_codes) return FRISK_E_INVALID;
+    *d_len = h->d_len; *d_scaf_off = h->d_scaf_off; *d_counters = h->d_counters; *rec_cap = h->rec_cap;
+    *d_codes = h->d_codes; *d_inv = h->d_inv; *d_low = h->d_low;
     return FRISK_OK;
 }
 
@@ -965,27 +1147,18 @@ int frisk_b200_fasta_info(const frisk_b200_fasta* h, uint64_t* n_records, uint64
 
 int frisk_b200_fasta_open(const char* text, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
                           uint64_t* padded_len, uint64_t stats[3]) {
-    if (!out || (!text && n)) return FRISK_E_INVALID;
-    *out = nullptr;
-    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
-    frisk_b200_fasta* h = new (std::nothrow) frisk_b200_fasta();
-    if (!h) return FRISK_E_INVALID;
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc;
-    try {
-        rc = open_any(h, text, n, st, nullptr);
-    } catch (...) {                                   // std::bad_alloc of the record table: nothing crosses the ABI
-        rc = FRISK_E_CAPACITY;
-    }
-    if (rc) {
-        free_all(h, st);
-        delete h;
-        return rc;
-    }
-    if (n_records) *n_records = h->n_rec;
-    if (padded_len) *padded_len = h->padded_len;
-    if (stats) { stats[0] = h->stats[0]; stats[1] = h->stats[1]; stats[2] = h->stats[2]; }
-    *out = h;
+    return open_public(text, n, false, stream, out, n_records, padded_len, stats);
+}
+
+int frisk_b200_fasta_open_bgzf(const char* gz, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
+                               uint64_t* padded_len, uint64_t stats[3]) {
+    return open_public(gz, n, true, stream, out, n_records, padded_len, stats);
+}
+
+int frisk_b200_fasta_name_text(const frisk_b200_fasta* h, const char** text, uint64_t* n) {
+    if (!h || !text || !n) return FRISK_E_INVALID;
+    *text = h->bgzf ? h->name_text.data() : nullptr;
+    *n = h->bgzf ? h->name_text.size() : 0;
     return FRISK_OK;
 }
 

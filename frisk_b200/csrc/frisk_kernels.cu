@@ -2529,7 +2529,8 @@ int stage_get(int dev, int slot, size_t bytes, void** out) {
     return FRISK_OK;
 }
 
-int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, int w, int step, int scaffolds_all,
+// bgzf: h_text / q_text are BGZF buffers, inflated on the device by the ingest (frisk_b200_run_fasta_bgzf)
+int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step, int scaffolds_all,
                    int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
                    uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out, frisk_b200_fasta** host_out,
                    frisk_b200_fasta** query_out, cudaStream_t st, int dev) {
@@ -2652,7 +2653,7 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
             return same ? queue_score(s2) : FRISK_OK;
         };
     g_trace.stamp("call");
-    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, st, &sink, host_out))) return rc;
+    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, bgzf, st, &sink, host_out))) return rc;
     g_trace.stamp("open_returned");
     tm->have[kTmUploaded] = h_n > 0;                                // (recorded behind the last text chunk)
     const bool counted = sink.counted;
@@ -2673,7 +2674,7 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
                 return FRISK_OK;
             };
         qsink.counted = false;
-        if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, st, &qsink, query_out))) return rc;
+        if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, bgzf, st, &qsink, query_out))) return rc;
         qh = *query_out;
         // (qsink has no on_range, so `counted` says nothing: a query that was re-opened exactly has a handle without the
         // speculative table the hook used -- detect it by the hook not having run or the open statistics)
@@ -2734,12 +2735,12 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
                     (int64_t)h_stats[0] - (int64_t)h_stats[1], rows_out, status_out, tables_out, valid_kmax_out, dfwd, st, cc->copy,
                     cc->ev[kMaxChunks + 1], cc->ev[kMaxChunks + 2], tm, &late);
 }
-}  // namespace
 
-int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, int w, int step, int scaffolds_all,
-                         int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
-                         uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
-                         frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
+// frisk_b200_run_fasta and frisk_b200_run_fasta_bgzf
+int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step, int scaffolds_all,
+                  int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
+                  uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
+                  frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
     if (!host_out || !query_out || (!h_text && h_n) || (!q_text && q_n) || (rows_cap && (!rows_out || !status_out)))
         return FRISK_E_INVALID;
     *host_out = *query_out = nullptr;
@@ -2754,7 +2755,7 @@ int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, u
     cudaStream_t st = (cudaStream_t)stream;
     bool threw = false;
     try {
-        rc = run_fasta_body(h_text, h_n, q_text, q_n, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
+        rc = run_fasta_body(h_text, h_n, q_text, q_n, bgzf, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
                             status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, st, dev);
     } catch (...) {
         rc = FRISK_E_CAPACITY;
@@ -2771,6 +2772,24 @@ int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, u
         }
     }
     return rc;
+}
+
+}  // namespace
+
+int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, int w, int step, int scaffolds_all,
+                         int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
+                         uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
+                         frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
+    return run_fasta_any(h_text, h_n, q_text, q_n, false, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
+                         status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
+}
+
+int frisk_b200_run_fasta_bgzf(const char* h_gz, uint64_t h_n, const char* q_gz, uint64_t q_n, int w, int step, int scaffolds_all,
+                              int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
+                              uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
+                              frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
+    return run_fasta_any(h_gz, h_n, q_gz, q_n, true, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
+                         status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
 // Stage times (ms) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call on the current device,

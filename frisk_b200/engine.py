@@ -114,6 +114,51 @@ def read_fasta_file(path: str) -> np.ndarray:
     return np.fromfile(path, dtype=np.uint8)
 
 
+def is_bgzf(buf) -> bool:
+    """Whether ``buf`` begins with a BGZF block (bgzip / samtools): a gzip member with CM 8, FLG = FEXTRA only and a
+    ``BC`` extra subfield of length 2.  Such files are inflated on the device; a plain gzip member is not BGZF."""
+    a = _as_u8(buf)
+    if a.shape[0] < 18 or bytes(a[:4]) != b"\x1f\x8b\x08\x04":
+        return False
+    xlen = int(a[10]) | int(a[11]) << 8
+    extra = bytes(a[12:12 + xlen])
+    q = 0
+    while q + 4 <= len(extra):
+        slen = extra[q + 2] | extra[q + 3] << 8
+        if extra[q:q + 2] == b"BC" and slen == 2:
+            return True
+        q += 4 + slen
+    return False
+
+
+def read_genome_file(path: str) -> Tuple[np.ndarray, bool]:
+    """(bytes, bgzf): a BGZF file as it is on disk (the device inflates it), any other file as ``read_fasta_file``
+    gives it (a single-member ``.gz`` inflated on the host, text as it is)."""
+    raw = np.fromfile(path, dtype=np.uint8)
+    if is_bgzf(raw):
+        return raw, True
+    return (read_fasta_file(path) if path.endswith(".gz") else raw), False
+
+
+def bgzf_text_len(gz) -> int:
+    """Inflated size of a BGZF buffer, from its block headers and trailers alone (FriskError: not BGZF)."""
+    buf = _as_u8(gz)
+    nb, tl = C.c_uint64(0), C.c_uint64(0)
+    _lib.check(_lib.lib().frisk_b200_bgzf_blocks(_ptr(buf), buf.shape[0], 0, None, None, None, None, C.byref(nb), C.byref(tl)),
+               "frisk_b200_bgzf_blocks")
+    return int(tl.value)
+
+
+def _name_source(L, h, buf: np.ndarray, bgzf: bool) -> np.ndarray:
+    """What a handle's name offsets index: the caller's text, or -- a BGZF open, whose text never leaves the device -- the
+    handle's buffer of header lines (copied: it goes with the handle)."""
+    if not bgzf:
+        return buf
+    p, n = C.c_void_p(), C.c_uint64(0)
+    _lib.check(L.frisk_b200_fasta_name_text(h, C.byref(p), C.byref(n)), "frisk_b200_fasta_name_text")
+    return np.frombuffer(C.string_at(p.value, n.value), dtype=np.uint8) if n.value else np.zeros(0, np.uint8)
+
+
 def _decode_names(buf: np.ndarray, name_off: np.ndarray, name_len: np.ndarray) -> List[str]:
     """Header tokens -> str.  All name bytes are gathered with one fancy-index (a 1 M-scaffold
     assembly must not pay a numpy slice of a multi-GB buffer per record), then cut up."""
@@ -340,6 +385,15 @@ class DeviceGenome:
     def from_fasta_bytes_native(cls, text: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
         """``from_fasta_bytes`` without PyTorch: the planes are DevBuf allocations (cudaMalloc through the C
         ABI), work goes to the default stream.  Used by the CLI."""
+        return cls._open_native(text, device, False)
+
+    @classmethod
+    def from_bgzf_bytes_native(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes_native`` for a BGZF buffer: the compressed bytes go to the GPU and are inflated there."""
+        return cls._open_native(gz, device, True)
+
+    @classmethod
+    def _open_native(cls, text, device, bgzf: bool) -> "DeviceGenome":
         _lib.require_device()
         L = _lib.lib()
         buf = _as_u8(text)
@@ -347,9 +401,10 @@ class DeviceGenome:
         h = C.c_void_p()
         nrec, padded = C.c_uint64(0), C.c_uint64(0)
         stats = np.zeros(3, np.uint64)
-        _lib.check(L.frisk_b200_fasta_open(_ptr(buf), buf.shape[0], None, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)),
-                   "frisk_b200_fasta_open")
+        opener, what = (L.frisk_b200_fasta_open_bgzf, "frisk_b200_fasta_open_bgzf") if bgzf else (L.frisk_b200_fasta_open, "frisk_b200_fasta_open")
+        _lib.check(opener(_ptr(buf), buf.shape[0], None, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
         try:
+            names_buf = _name_source(L, h, buf, bgzf)
             R, P = int(nrec.value), int(padded.value)
             name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
             seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
@@ -360,7 +415,7 @@ class DeviceGenome:
             _lib.check(L.frisk_b200_fasta_pack(h, _ptr(codes), _ptr(inv), _ptr(low), None), "frisk_b200_fasta_pack")
         finally:
             L.frisk_b200_fasta_close(h, None)
-        names = _decode_names(buf, name_off, name_len)
+        names = _decode_names(names_buf, name_off, name_len)
         g = PackedGenome(names, seq_len, scaf_off, P, None, None, None, int(stats[0]), int(stats[1]), int(stats[2]), False)
         return cls(g, str(device), planes=(codes, inv, low))
 
@@ -369,19 +424,30 @@ class DeviceGenome:
         """Device-side ingest (frisk_ingest.cu): the raw FASTA text goes to the GPU once and is
         tokenised and 2-bit packed there; only the record table comes back.  ``self.host`` is a
         PackedGenome without host planes (names, lengths, layout, countN statistics)."""
+        return cls._open(text, device, False)
+
+    @classmethod
+    def from_bgzf_bytes(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes`` for a BGZF buffer (bgzip, samtools): the compressed bytes go to the GPU and are inflated
+        there (frisk_bgzf.cu), straight into the ingest's text buffer; the text never exists on the host."""
+        return cls._open(gz, device, True)
+
+    @classmethod
+    def _open(cls, text, device, bgzf: bool) -> "DeviceGenome":
         import torch
         _lib.require_device()
         L = _lib.lib()
         buf = _as_u8(text)
         dev = torch.device(device)
+        opener, what = (L.frisk_b200_fasta_open_bgzf, "frisk_b200_fasta_open_bgzf") if bgzf else (L.frisk_b200_fasta_open, "frisk_b200_fasta_open")
         with torch.cuda.device(dev):
             st = _stream_ptr(dev)
             h = C.c_void_p()
             nrec, padded = C.c_uint64(0), C.c_uint64(0)
             stats = np.zeros(3, np.uint64)
-            _lib.check(L.frisk_b200_fasta_open(_ptr(buf), buf.shape[0], st, C.byref(h), C.byref(nrec), C.byref(padded),
-                                               _ptr(stats)), "frisk_b200_fasta_open")
+            _lib.check(opener(_ptr(buf), buf.shape[0], st, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
             try:
+                names_buf = _name_source(L, h, buf, bgzf)
                 R, P = int(nrec.value), int(padded.value)
                 name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
                 seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
@@ -393,13 +459,15 @@ class DeviceGenome:
                 _lib.check(L.frisk_b200_fasta_pack(h, _ptr(codes), _ptr(inv), _ptr(low), st), "frisk_b200_fasta_pack")
             finally:
                 L.frisk_b200_fasta_close(h, st)
-        names = LazyNames(buf, name_off, name_len)
+        names = LazyNames(names_buf, name_off, name_len)
         g = PackedGenome(names, seq_len, scaf_off, P, None, None, None, int(stats[0]), int(stats[1]), int(stats[2]), False)
         return cls(g, dev, planes=(codes, inv, low))
 
     @classmethod
     def from_fasta(cls, path: str, device="cuda:0") -> "DeviceGenome":
-        return cls.from_fasta_bytes(read_fasta_file(path), device)
+        """A FASTA file: BGZF is inflated on the device, any other ``.gz`` on the host (``read_fasta_file``)."""
+        buf, bgzf = read_genome_file(path)
+        return cls.from_bgzf_bytes(buf, device) if bgzf else cls.from_fasta_bytes(buf, device)
 
     def to_host(self) -> PackedGenome:
         """Copy the planes back (tests; the host packer must agree bit for bit)."""
@@ -989,7 +1057,7 @@ class _HandlePlane:
         return self._p
 
 
-def _genome_from_handle(L, h, buf) -> PackedGenome:
+def _genome_from_handle(L, h, buf, bgzf: bool = False) -> PackedGenome:
     nrec, padded = C.c_uint64(0), C.c_uint64(0)
     stats = np.zeros(3, np.uint64)
     _lib.check(L.frisk_b200_fasta_info(h, C.byref(nrec), C.byref(padded), _ptr(stats)), "frisk_b200_fasta_info")
@@ -998,7 +1066,7 @@ def _genome_from_handle(L, h, buf) -> PackedGenome:
     seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
     _lib.check(L.frisk_b200_fasta_records(h, _ptr(name_off), _ptr(name_len), _ptr(seq_len), _ptr(scaf_off)),
                "frisk_b200_fasta_records")
-    return PackedGenome(LazyNames(buf, name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
+    return PackedGenome(LazyNames(_name_source(L, h, buf, bgzf), name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
                         int(stats[0]), int(stats[1]), int(stats[2]), False)
 
 
@@ -1010,6 +1078,21 @@ def run_fasta(query_text, host_text=None, device="cuda:0", out=None, assemble_re
     derived on the host while the last chunk is still being counted; then tables, IVOM, window kernel, rows.  This is the
     whole of the reference's stages 2+3 (F:1442, F:1478-1494) including its three passes over the file (F:170, F:203,
     F:297).  ``out``: reusable HostOutputs (its row capacity is used; ``out.n_win`` is set)."""
+    return _run_fasta_any(query_text, host_text, False, device, out, assemble_result, kmin, kmax, w, step, mask_host,
+                          scaffolds_all, rip)
+
+
+def run_fasta_bgzf(query_gz, host_gz=None, device="cuda:0", out=None, assemble_result: bool = True, kmin: int = 1,
+                   kmax: int = 8, w: int = 5000, step: int = 2500, mask_host: bool = False, scaffolds_all: bool = False,
+                   rip: bool = True):
+    """``run_fasta`` for BGZF buffers (bgzip, samtools; ideally page-locked): ONE C call (frisk_b200_run_fasta_bgzf) that
+    uploads the compressed bytes, inflates every BGZF block on the device straight into the ingest's text buffer and goes
+    on exactly as ``run_fasta``.  Same results as ``run_fasta`` on the inflated text."""
+    return _run_fasta_any(query_gz, host_gz, True, device, out, assemble_result, kmin, kmax, w, step, mask_host,
+                          scaffolds_all, rip)
+
+
+def _run_fasta_any(query_text, host_text, bgzf, device, out, assemble_result, kmin, kmax, w, step, mask_host, scaffolds_all, rip):
     import torch
     _lib.require_device()
     L = _lib.lib()
@@ -1020,22 +1103,24 @@ def run_fasta(query_text, host_text=None, device="cuda:0", out=None, assemble_re
         # rows: a guess (one window per step of text, one more per 4 KiB for short scaffolds); a text with more windows comes
         # back with FRISK_E_CAPACITY and is scored in a second stage below -- page-locking a far larger buffer "to be safe"
         # would cost more than the run (~0.3 ms per MB)
-        out = HostOutputs(qbuf.shape[0] // step + qbuf.shape[0] // 4096 + 64, kmax)
+        n_text = bgzf_text_len(qbuf) if bgzf else qbuf.shape[0]
+        out = HostOutputs(n_text // step + n_text // 4096 + 64, kmax)
     hh, qh = C.c_void_p(), C.c_void_p()
     n_win = C.c_uint64(0)
+    fn, what = (L.frisk_b200_run_fasta_bgzf, "frisk_b200_run_fasta_bgzf") if bgzf else (L.frisk_b200_run_fasta, "frisk_b200_run_fasta")
     with _device_ctx(dev):
         st = _stream_ptr(dev)
-        rc = L.frisk_b200_run_fasta(_ptr(hbuf), hbuf.shape[0], _ptr(qbuf) if host_text is not None else None,
+        rc = fn(_ptr(hbuf), hbuf.shape[0], _ptr(qbuf) if host_text is not None else None,
                                     qbuf.shape[0] if host_text is not None else 0, w, step, int(scaffolds_all), kmin, kmax,
                                     int(mask_host), int(rip), out.rows.shape[0], _ptr(out.rows), _ptr(out.status),
                                     _ptr(out.tables), _ptr(out.valid), C.byref(n_win), C.byref(hh), C.byref(qh), st)
         try:
             if rc not in (_lib.OK, _lib.E_CAPACITY):
-                _lib.check(rc, "frisk_b200_run_fasta")
+                _lib.check(rc, what)
             n = int(n_win.value)
             need_genomes = assemble_result or rc == _lib.E_CAPACITY
-            host = _genome_from_handle(L, hh, hbuf) if need_genomes else None
-            query = (_genome_from_handle(L, qh, qbuf) if qh else host) if need_genomes else None
+            host = _genome_from_handle(L, hh, hbuf, bgzf) if need_genomes else None
+            query = (_genome_from_handle(L, qh, qbuf, bgzf) if qh else host) if need_genomes else None
             if rc == _lib.E_CAPACITY:
                 # more windows than the guessed row capacity: the planes are on the device, score them into enough rows
                 def planes(h):

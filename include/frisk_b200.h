@@ -371,6 +371,49 @@ int frisk_b200_fasta_info(const frisk_b200_fasta *h, uint64_t *n_records, uint64
 int frisk_b200_fasta_planes(const frisk_b200_fasta *h, const uint32_t **d_codes, const uint32_t **d_inv,
                             const uint32_t **d_low);
 
+/* ------------------------------------------------------------------ BGZF-compressed FASTA (frisk_bgzf.cu)
+ *
+ * BGZF (bgzip, `samtools faidx`) is a series of gzip members of <= 64 KiB each; every member's header gives its
+ * compressed size and its trailer the CRC32 and inflated size, so every member is inflated on the device by a decoder of
+ * its own, straight into the ingest's text buffer.  A single-member .gz (gzip, pigz) is not BGZF: it is FRISK_E_FORMAT
+ * here and is inflated on the host by the Python layer, as before.
+ *
+ * frisk_b200_bgzf_blocks: the block table of a BGZF buffer, from the headers and trailers alone.  comp_off / comp_len: the
+ * raw deflate payload of every member; crc: the CRC32 of its trailer; text_off: the exclusive prefix sum of the inflated
+ * sizes; *text_len their sum.  Every member must be a BGZF block (1f 8b, CM 8, FLG 4, a "BC" subfield of SLEN 2 among the
+ * extra subfields, BSIZE inside the buffer, ISIZE <= 65,536); empty members (the EOF marker) may appear anywhere.
+ * Anything else, trailing bytes included: FRISK_E_FORMAT.  Arrays may be NULL to count only (as frisk_b200_fasta_scan);
+ * *n_blocks always receives the count; FRISK_E_CAPACITY if cap is too small.
+ *
+ * frisk_b200_bgzf_inflate: inflates every member of the table into d_text[text_off[b] ..] (exactly text_len bytes are
+ * written; nothing beyond), one warp per member, and checks each member's size and CRC32 (the CRCs come from the block
+ * table).  Full RFC 1951 (stored, fixed and dynamic Huffman blocks).  Malformed input never faults: d_block_status[b] != 0
+ * marks a member that is not valid deflate, does not fit its ISIZE or fails its CRC; the caller reads the status words
+ * behind the stream's work and treats any non-zero one as FRISK_E_FORMAT.  Only enqueues work on `stream`.
+ * frisk_b200_bgzf_inflate_host: the same decoder run on the CPU over host arrays (test infrastructure: no user path calls it);
+ * returns FRISK_E_FORMAT itself when a status word is non-zero.  `stream` is unused.
+ *
+ * frisk_b200_fasta_open_bgzf / frisk_b200_run_fasta_bgzf: frisk_b200_fasta_open / frisk_b200_run_fasta with BGZF buffers in
+ * place of the texts, same arguments and results: the compressed bytes go up, are inflated into the ingest's text buffer
+ * and are tokenised and packed there.  The inflated text never reaches the host, so the names of a BGZF handle index into
+ * a buffer the handle owns: frisk_b200_fasta_name_text gives it (NULL / 0 for a handle opened from text, whose names index
+ * the caller's text).  ms[0] of frisk_b200_last_run_timing is "compressed bytes uploaded and inflated". */
+int frisk_b200_bgzf_blocks(const uint8_t *gz, uint64_t n, uint64_t cap, uint64_t *comp_off, uint32_t *comp_len,
+                           uint32_t *crc, uint64_t *text_off, uint64_t *n_blocks, uint64_t *text_len);
+int frisk_b200_bgzf_inflate(const uint8_t *d_gz, const uint64_t *d_comp_off, const uint32_t *d_comp_len,
+                            const uint32_t *d_crc, const uint64_t *d_text_off, uint64_t n_blocks, uint64_t text_len,
+                            uint8_t *d_text, uint32_t *d_block_status, void *stream);
+int frisk_b200_bgzf_inflate_host(const uint8_t *gz, const uint64_t *comp_off, const uint32_t *comp_len, const uint32_t *crc,
+                                 const uint64_t *text_off, uint64_t n_blocks, uint64_t text_len, uint8_t *text,
+                                 uint32_t *block_status, void *stream);
+int frisk_b200_fasta_open_bgzf(const char *gz, uint64_t n, void *stream, frisk_b200_fasta **out, uint64_t *n_records,
+                               uint64_t *padded_len, uint64_t stats[3]);
+int frisk_b200_run_fasta_bgzf(const char *h_gz, uint64_t h_n, const char *q_gz, uint64_t q_n, int w, int step,
+                              int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap,
+                              double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
+                              uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
+int frisk_b200_fasta_name_text(const frisk_b200_fasta *h, const char **text, uint64_t *n);
+
 /* Stage times (ms since the start of the call) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call
  * on the current device, from CUDA events recorded on the call's own streams: ms[0] planes uploaded, ms[1] background
  * counted, ms[2] tables + genome IVOM finalised (multi-GPU: includes the wait for the peers' counters), ms[3] window
