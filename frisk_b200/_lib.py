@@ -8,7 +8,6 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get("FRISK_B200_LIB") or os.path.join(HERE, "libfrisk_b200.so")   # override: kernel A/B builds (tools/)
@@ -94,17 +93,6 @@ class FriskError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ""):
         self.code = code
         super().__init__("%s failed: %s%s" % (where, _strerror(code), (" -- " + detail) if detail else ""))
-
-
-def build(force: bool = False) -> str:
-    """Compile the shared library in-tree (nvcc, sm_100a).  Cross-compiles without a GPU."""
-    src_dir = os.path.join(HERE, "csrc")
-    srcs = [os.path.join(src_dir, f) for f in ("frisk_kernels.cu", "frisk_direct.cu", "frisk_device.cuh", "frisk_general.cu", "frisk_ingest.cu", "frisk_bgzf.cu", "frisk_features.cu", "frisk_host.cpp", "frisk_internal.h", "Makefile")]
-    srcs.append(os.path.join(os.path.dirname(HERE), "include", "frisk_b200.h"))
-    stale = not os.path.exists(SO_PATH) or any(os.path.getmtime(s) > os.path.getmtime(SO_PATH) for s in srcs)
-    if force or stale:
-        subprocess.check_call(["make", "-C", src_dir] + (["-B"] if force else []))
-    return SO_PATH
 
 
 def lib():

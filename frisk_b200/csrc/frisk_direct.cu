@@ -31,7 +31,6 @@
 
 namespace {
 using frisk_internal::kRowRedo;
-#define CK(call) FRISK_CK(call)
 
 constexpr uint32_t kSideCap = 64;
 
@@ -367,88 +366,33 @@ score_windows_direct_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
     }
 }
 
-template <int K, int NT, int ROUNDS, bool DUMP, bool ALLK>
-int launch_direct4(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                   const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
-                   double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only) {
-    using L = DirectLayout<K, NT>;
-    auto kern = score_windows_direct_kernel<K, NT, ROUNDS, DUMP, ALLK>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::TOTAL));
-    // three CTAs of 75 KB need the whole 228 KB carve-out (the driver's per-launch heuristic may pick less)
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, NT, L::TOTAL));
-    if (occ_only) { *occ_only = per_sm; return FRISK_OK; }
-    if (per_sm < 1) per_sm = 1;
-    const int sms = frisk_internal::sm_count_cached();
-    if (sms <= 0) return FRISK_E_NO_DEVICE;
-    uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-    if (grid > n_win) grid = n_win;
-    kern<<<(unsigned)grid, NT, L::TOTAL, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len,
-                                               (uint32_t)n_win, reinterpret_cast<const double2*>(ig), kmin, want_rip, rows,
-                                               status, dump, redo_dst);
-    CK(cudaGetLastError());
-    return FRISK_OK;
-}
-
-template <int K, int NT, int ROUNDS>
-int launch_direct3(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                   const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
-                   double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only) {
-    if (dump) return launch_direct4<K, NT, ROUNDS, true, false>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only);
-    if (kmin != 1) return launch_direct4<K, NT, ROUNDS, false, false>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only);
-    return launch_direct4<K, NT, ROUNDS, false, true>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only);
-}
-
-// positions per thread = 4 * ROUNDS (K-mer codes held in registers between the two passes)
 template <int K>
-int launch_direct(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only, int* threads) {
-#define FRISK_DIRECT(NT, R)                                                                                              \
-    do {                                                                                                                 \
-        if (threads) *threads = NT;                                                                                      \
-        return launch_direct3<K, NT, R>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, \
-                                        st, occ_only);                                                                   \
-    } while (0)
-    if (max_len <= 256u * 4u * 2u - 6u) FRISK_DIRECT(256, 2);
-    if (max_len <= 256u * 4u * 5u - 6u) FRISK_DIRECT(256, 5);
-    FRISK_DIRECT(256, 8);
-#undef FRISK_DIRECT
+const void* direct_fn(const frisk_internal::WinPlan& p) {
+    if (p.variant == 2) return FRISK_WIN_INSTANCE(p, score_windows_direct_kernel, K, 256, 2);
+    if (p.variant == 5) return FRISK_WIN_INSTANCE(p, score_windows_direct_kernel, K, 256, 5);
+    return FRISK_WIN_INSTANCE(p, score_windows_direct_kernel, K, 256, 8);
 }
 
 }  // namespace
 
-int frisk_internal::score_direct(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
-                                 int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
-    if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
-    // where the hand-over marks go: `status` itself when it is device memory, device scratch when it is pinned host
-    // memory (the second launch would otherwise read its marks across PCIe, one round trip per window)
-    uint32_t* redo = status;
-    uint32_t* scratch = nullptr;
-    cudaPointerAttributes pa{};
-    if (cudaPointerGetAttributes(&pa, status) != cudaSuccess || pa.type != cudaMemoryTypeDevice) {
-        cudaGetLastError();
-        int rc = pool_ready();
-        if (rc) return rc;
-        CK(cudaMallocAsync((void**)&scratch, n_win * sizeof(uint32_t), st));
-        redo = scratch;
-    }
-    int rc;
-    if (K == 8) rc = launch_direct<8>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo, st, nullptr, nullptr);
-    else rc = launch_direct<7>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo, st, nullptr, nullptr);
-    // windows the byte table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
-    if (!rc) rc = score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump, redo, st);
-    if (scratch) {                                         // freed on every path (stream-ordered: behind the launches above)
-        const cudaError_t e = cudaFreeAsync(scratch, st);
-        if (!rc && e != cudaSuccess) return frisk_internal::cuda_fail(e, "cudaFreeAsync(scratch)");
-    }
-    return rc;
+// 256 threads; at K = 8 three CTAs of 75 KB need the whole 228 KB carve-out
+frisk_internal::LaunchShape frisk_internal::direct_shape(const WinPlan& p, int K) {
+    if (K == 8) return {direct_fn<8>(p), 256, DirectLayout<8, 256>::TOTAL, true};
+    return {direct_fn<7>(p), 256, DirectLayout<7, 256>::TOTAL, true};
 }
 
-int frisk_internal::score_direct_occupancy(int K, uint32_t max_len, int* ctas_per_sm, int* threads_per_cta) {
-    if (K == 8) return launch_direct<8>(nullptr, nullptr, nullptr, nullptr, nullptr, 1, max_len, nullptr, 1, 0, nullptr, nullptr, nullptr, nullptr, 0, ctas_per_sm, threads_per_cta);
-    if (K == 7) return launch_direct<7>(nullptr, nullptr, nullptr, nullptr, nullptr, 1, max_len, nullptr, 1, 0, nullptr, nullptr, nullptr, nullptr, 0, ctas_per_sm, threads_per_cta);
-    return FRISK_E_UNSUPPORTED;
+int frisk_internal::score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
+                                 const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
+                                 int kmin, int K, int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
+    if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
+    return with_redo_marks(status, n_win, false, st, [&](uint32_t* redo) {
+        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
+        const double2* g = reinterpret_cast<const double2*>(ig);
+        uint32_t n = (uint32_t)n_win;
+        void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo};
+        int rc = launch_persistent(direct_shape(p, K), n_win, args, st);
+        // windows the byte table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
+        return rc ? rc : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump,
+                                           redo, st);
+    });
 }

@@ -10,6 +10,12 @@
 
 struct frisk_b200_fasta;
 
+#define FRISK_CK(call)                                                        \
+    do {                                                                      \
+        cudaError_t e_ = (call);                                              \
+        if (e_ != cudaSuccess) return frisk_internal::cuda_fail(e_, #call);   \
+    } while (0)
+
 namespace frisk_internal {
 
 // records the CUDA error text for frisk_b200_last_cuda_error() and returns FRISK_E_CUDA
@@ -74,36 +80,99 @@ int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* lo
                   double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr,
                   int grid_cap = 0);
 
-// kmax 9..12, windows <= 8,186 bases (frisk_nibble_ext.cu): orders 1..8 as in the kmax-8 nibble kernel, orders 9..K from the
-// observation that an 8-mer seen once has only unique extensions (the few repeated ones go through a shared-memory hash
-// table).  What it cannot hold is marked kRowRedo and re-done by general_score behind it.
-int score_nibble_ext(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+// Longest window the shared-memory window kernels hold: an 8,192-base buffer less 6 bases of look-ahead.
+constexpr uint32_t kSmemMaxWindow = 8186u;
+
+// The window kernels of frisk_b200_score and how one of them is instantiated for a call.  plan_score (frisk_kernels.cu)
+// is the one place that chooses them, from (kmin, kmax, longest window, dump) and the kernel forced through
+// frisk_b200_set_option.  variant: ROUNDS of the bucketed and direct kernels or PP of the nibble and extension kernels,
+// positions per thread from the longest window (window_variant).  dump / allk pick the <DUMP, ALLK> instantiation.
+enum class WinKernel { Small, Nibble, Direct, Bucket, Dense, NibbleExt, General };
+struct WinPlan {
+    WinKernel kind;
+    int variant;
+    bool dump, allk;
+};
+int plan_score(int kmin, int kmax, uint32_t max_win_len, bool dump, WinPlan* out);
+int window_variant(WinKernel kind, uint32_t max_win_len);
+// the instantiation of a window kernel template <..., DUMP, ALLK> a plan runs: the table dump and kmin > 1 share the generic
+// <..., DUMP, false> one, the production default (no dump, kmin 1) has its own
+#define FRISK_WIN_INSTANCE(p, kern, ...)                                                                      \
+    ((p).dump ? (const void*)kern<__VA_ARGS__, true, false>                                                   \
+              : ((p).allk ? (const void*)kern<__VA_ARGS__, false, true> : (const void*)kern<__VA_ARGS__, false, false>))
+
+// How a persistent window kernel is launched: each CTA walks windows until none are left, grid = min(SMs x resident CTAs
+// per SM, windows).  max_carveout: ask for the whole shared-memory carve-out instead of leaving the L1 / shared split to
+// the driver's per-launch heuristic (a smaller split silently costs a CTA per SM).
+struct LaunchShape {
+    const void* fn;
+    int threads;
+    size_t smem;
+    bool max_carveout;
+};
+// resident CTAs per SM of `s` on the current device; sets its attributes first (once per device, kernel and smem, cached)
+int ctas_per_sm(const LaunchShape& s, int* out);
+// one persistent launch of `s`; args as for cudaLaunchKernel
+int launch_persistent(const LaunchShape& s, uint64_t n_win, void** args, cudaStream_t st);
+int sm_count_cached();     // multiprocessors of the current device (0: none)
+
+// The hand-over of the nibble, direct and extension kernels: the windows they cannot finish exactly are marked kRowRedo
+// and re-done by a second launch behind them on the same stream.  body(redo) queues both launches.  The marks go into
+// `status` when that is device memory, otherwise into stream-ordered scratch: when `status` is a pinned host buffer
+// written over PCIe the second launch must not read its marks back across the bus one window at a time, and the k sweep
+// (status == nullptr) has eight status arrays.  zero: the window count lives in device memory, so n_win is only the
+// capacity and the second launch walks all of it -- scratch is used and cleared, marks beyond the real count read
+// "nothing to redo".  The scratch is freed behind body's launches on every path.
+constexpr uint32_t kRowRedo = 0x80000000u;
+template <typename F>
+int with_redo_marks(uint32_t* status, uint64_t n_win, bool zero, cudaStream_t st, F body) {
+    uint32_t* scratch = nullptr;
+    cudaPointerAttributes pa{};
+    if (zero || !status || cudaPointerGetAttributes(&pa, status) != cudaSuccess || pa.type != cudaMemoryTypeDevice) {
+        cudaGetLastError();                                  // a host pointer makes the query itself report an error
+        int rc = pool_ready();
+        if (rc) return rc;
+        FRISK_CK(cudaMallocAsync((void**)&scratch, n_win * sizeof(uint32_t), st));
+    }
+    int rc = FRISK_OK;
+    if (zero) {
+        const cudaError_t e = cudaMemsetAsync(scratch, 0, n_win * sizeof(uint32_t), st);
+        if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemsetAsync(redo scratch)");
+    }
+    if (!rc) rc = body(scratch ? scratch : status);
+    if (scratch) {                                           // stream-ordered: behind body's launches
+        const cudaError_t e = cudaFreeAsync(scratch, st);
+        if (!rc && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync(redo scratch)");
+    }
+    return rc;
+}
+
+// kmax 9..12, windows <= kSmemMaxWindow bases (frisk_nibble_ext.cu): orders 1..8 as in the kmax-8 nibble kernel, orders
+// 9..K from the observation that an 8-mer seen once has only unique extensions (the few repeated ones go through a
+// shared-memory hash table).  What it cannot hold is re-done by general_score behind it.
+LaunchShape ext_shape(const WinPlan& p);
+int score_nibble_ext(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                      const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                      double* rows, uint32_t* status, cudaStream_t st);
 
-
-// direct score kernel (frisk_direct.cu): kmax 7, 8 and windows <= 8,186 bases.  Windows it cannot finish exactly
-// (a K-mer seen 256+ times, more than 64 N-boundary words) are marked kRowRedo and re-done by the bucketed kernel
-// (frisk_kernels.cu), launched behind it on the same stream.  The marks live in `status` when that is device memory,
-// in stream-ordered device scratch when `status` is a pinned host buffer written over PCIe (frisk_b200_run_host):
-// the second launch must not read its marks back across the bus one window at a time.
-constexpr uint32_t kRowRedo = 0x80000000u;
-int score_direct(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+// direct score kernel (frisk_direct.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases.  Windows it cannot finish exactly
+// (a K-mer seen 256+ times, more than 64 N-boundary words) are re-done by the bucketed kernel (frisk_kernels.cu).
+LaunchShape direct_shape(const WinPlan& p, int K);
+int score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st);
-int score_direct_occupancy(int K, uint32_t max_len, int* ctas_per_sm, int* threads_per_cta);
 int score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                       const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                       double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src, cudaStream_t st);
-int sm_count_cached();
 
-// nibble score kernel (frisk_nibble.cu): kmax 7, 8 and windows <= 8,186 bases; one 4-bit counter per K-mer, one atomic per
-// position, the first occurrence of a K-mer scores it.  Windows with a K-mer seen 16+ times (or more than 64 N-boundary
-// words) are marked kRowRedo and re-done by the bucketed kernel, exactly like the direct kernel's hand-over.
-int score_nibble(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+// nibble score kernel (frisk_nibble.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases; one 4-bit counter per K-mer, one
+// atomic per position, the first occurrence of a K-mer scores it.  Windows with a K-mer seen 16+ times (or more than 64
+// N-boundary words) are re-done by the bucketed kernel, exactly like the direct kernel's hand-over.  n_win_dev: the window
+// count in device memory, n_win its capacity.
+LaunchShape nibble_shape(const WinPlan& p, int K);
+int score_nibble(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const unsigned long long* n_win_dev = nullptr);
-int score_nibble_occupancy(int K, uint32_t max_len, int* ctas_per_sm, int* threads_per_cta);
 // the k sweep (BASELINE config C3): rows of kmax' = 1..8, kmin 1, from one pass over every window; ig / rows / status are
 // HOST arrays of 8 device pointers
 int score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,
@@ -111,11 +180,5 @@ int score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
                 uint32_t* const* status, cudaStream_t st);
 
 }  // namespace frisk_internal
-
-#define FRISK_CK(call)                                                        \
-    do {                                                                      \
-        cudaError_t e_ = (call);                                              \
-        if (e_ != cudaSuccess) return frisk_internal::cuda_fail(e_, #call);   \
-    } while (0)
 
 #endif

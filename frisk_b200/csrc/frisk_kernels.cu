@@ -22,7 +22,9 @@
 #include <atomic>
 #include <chrono>
 #include <functional>
+#include <map>
 #include <mutex>
+#include <tuple>
 #include <vector>
 
 #include "../../include/frisk_b200.h"
@@ -756,7 +758,6 @@ score_windows_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restr
 // ============================================================================================
 constexpr int kT3 = 256;
 constexpr int kW3 = kT3 / 32;
-constexpr uint32_t kBuf3 = 8192;      // longest window handled by this kernel
 
 struct Score3Smem {
     double q[8];
@@ -1467,11 +1468,7 @@ __global__ void __launch_bounds__(kThreads, 1) smem_atomic_bench_kernel(int iter
 }
 
 thread_local char g_cuda_err[512] = "";
-int g_force_dense = 0;      // tests: force the dense-table kernel (frisk_b200_set_option)
-int g_force_general = 0;    // tests: force the general (global-memory) score kernel
-int g_force_direct = 0;     // tests / A-B: kmax 7, 8 on the direct kernel wherever it can run
-int g_force_bucket = 0;     // tests: keep kmax 4..8 on the bucketed kernel instead of the small-K / direct kernel
-int g_force_nibble = 0;     // tests / A-B: kmax 7, 8 on the nibble kernel wherever it can run
+int g_forced = -1;          // the WinKernel forced through frisk_b200_set_option (tests, A/B measurements), -1: none
 }  // namespace
 
 int frisk_internal::cuda_fail(cudaError_t e, const char* what) {
@@ -1488,14 +1485,12 @@ int frisk_internal::cuda_fail(cudaError_t e, const char* what) {
 
 namespace {
 using frisk_internal::ws_get;
+using frisk_internal::sm_count_cached;
+using frisk_internal::LaunchShape;
+using frisk_internal::WinKernel;
+using frisk_internal::WinPlan;
+using frisk_internal::kSmemMaxWindow;
 #define CK(call) FRISK_CK(call)
-
-int sm_count() {
-    int dev = 0, n = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-    return n;
-}
 
 template <int K>
 int launch_background(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, uint64_t w_lo, uint64_t w_hi,
@@ -1506,7 +1501,7 @@ int launch_background(const uint32_t* codes, const uint32_t* inv, const uint32_t
     const size_t smem = (size_t)NW * 4;
     CK(cudaFuncSetAttribute(bg_count_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const uint64_t n_words = w_hi - w_lo;
-    int grid = sm_count();
+    int grid = sm_count_cached();
     if (grid <= 0) return FRISK_E_NO_DEVICE;
     // at least ~2 rounds of 1024 words per CTA, otherwise fewer CTAs
     const uint64_t want = (n_words + 2047) / 2048;
@@ -1553,7 +1548,7 @@ int launch_finalize_ivom(Fwd f, int kmin, int64_t space, uint64_t* tables, uint6
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0));
         if (per_sm > 0) cached[dev & 63].store(per_sm, std::memory_order_release);
     }
-    const int sms = sm_count();
+    const int sms = sm_count_cached();
     if (sms <= 0) return FRISK_E_NO_DEVICE;
     if (per_sm < 1) return FRISK_E_UNSUPPORTED;
     int grid = sms * (per_sm > 2 ? 2 : per_sm);                          // every CTA resident (grid-wide barriers); 2 per SM measured best
@@ -1589,7 +1584,7 @@ int launch_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* low
     while ((NB / (uint32_t)nseg < max_len ? NB / (uint32_t)nseg : max_len) > kListCap) nseg *= 2;
     if (nseg > kMaxSeg || (uint32_t)nseg > (L::BM_WORDS >= 2u ? L::BM_WORDS / 2u : 1u)) return FRISK_E_UNSUPPORTED;
     CK(cudaFuncSetAttribute(score_windows_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::TOTAL));
-    int grid = sm_count();
+    int grid = sm_count_cached();
     if (grid <= 0) return FRISK_E_NO_DEVICE;
     if ((uint64_t)grid > n_win) grid = (int)n_win;
     score_windows_kernel<K><<<grid, kThreads, L::TOTAL, st>>>(
@@ -1599,106 +1594,67 @@ int launch_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* low
     return FRISK_OK;
 }
 
-template <int K, int ROUNDS, bool DUMP, bool ALLK>
-int launch_score_bucket3(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                         const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                         double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, uint32_t len_min = 0,
-                         uint32_t len_max = 0xffffffffu, const uint32_t* redo_src = nullptr) {
-    using L = Score3Layout<K>;
-    const uint32_t cap = (max_len + 15u) & ~15u;
-    const size_t smem = L::total(cap);
-    auto kern = score_windows_bucket_kernel<K, ROUNDS, DUMP, ALLK>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // four CTAs of 57 KB need the whole 228 KB carve-out: ask for it instead of leaving the L1/shared
-    // split to the driver's per-launch heuristic (a smaller split silently costs a CTA per SM: 0.73 -> 0.83 ms)
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kT3, smem));
-    if (per_sm < 1) per_sm = 1;
-    int sms = sm_count();
-    if (sms <= 0) return FRISK_E_NO_DEVICE;
-    uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-    if (grid > n_win) grid = n_win;
-    kern<<<(unsigned)grid, kT3, smem, st>>>(
-        codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len, (uint32_t)n_win,
-        reinterpret_cast<const double2*>(ig), kmin, want_rip, cap, len_min, len_max, rows, status, dump, redo_src);
-    CK(cudaGetLastError());
-    return FRISK_OK;
-}
-
-template <int K, bool DUMP, bool ALLK>
-int launch_score_bucket2(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                         const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                         double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
-    // positions per thread = 4 * ROUNDS, held in registers: 5 rounds cover the default 5,000-base windows,
-    // 2 rounds short ones (-w 1000 / -w 2000) without dragging three idle rounds through every phase
-    if (max_len <= kT3 * 4u * 2u - 6u)
-        return launch_score_bucket3<K, 2, DUMP, ALLK>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
-    if (max_len <= kT3 * 4u * 5u - 6u)
-        return launch_score_bucket3<K, 5, DUMP, ALLK>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
-    // Longer windows need a bigger buffer, which costs a CTA per SM.  With --scaffoldsAll nearly all windows are
-    // still the standard length and only whole short scaffolds (up to 1.25 w) are longer: two launches, each
-    // taking the windows of its length class, keep the standard ones at four CTAs per SM.
-    constexpr uint32_t kStd = 5104u;                   // largest buffer that still fits four CTAs
-    if (n_win >= 4096) {
-        int rc = launch_score_bucket3<K, 5, DUMP, ALLK>(codes, inv, low, win_off, win_len, n_win, kStd, ig, kmin, want_rip, rows, status,
-                                                       dump, st, 0u, kStd);
-        if (rc) return rc;
-        return launch_score_bucket3<K, 8, DUMP, ALLK>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status,
-                                                      dump, st, kStd + 1u, 0xffffffffu);
+// The small-K kernel (K <= 6: the whole order-K table in shared memory; its L1 / shared split is left to the driver) or the
+// bucketed kernel (K >= 4: buffer sized by the longest window; four CTAs of 57 KB need the whole 228 KB carve-out, which
+// the driver's per-launch heuristic does not always give: 0.73 vs 0.83 ms).
+template <int K>
+int table_shape(const WinPlan& p, uint32_t max_len, LaunchShape* s) {
+    if constexpr (K <= 6) {
+        if (p.kind == WinKernel::Small) {
+            *s = {p.dump ? (const void*)score_windows_small_kernel<K, true> : (const void*)score_windows_small_kernel<K, false>, kT3,
+                  SmallLayout<K>::TOTAL, false};
+            return FRISK_OK;
+        }
     }
-    return launch_score_bucket3<K, 8, DUMP, ALLK>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
+    if constexpr (K >= 4) {
+        if (p.kind == WinKernel::Bucket) {
+            *s = {p.variant == 2   ? FRISK_WIN_INSTANCE(p, score_windows_bucket_kernel, K, 2)
+                  : p.variant == 5 ? FRISK_WIN_INSTANCE(p, score_windows_bucket_kernel, K, 5)
+                                   : FRISK_WIN_INSTANCE(p, score_windows_bucket_kernel, K, 8),
+                  kT3, Score3Layout<K>::total((max_len + 15u) & ~15u), true};
+            return FRISK_OK;
+        }
+    }
+    return FRISK_E_UNSUPPORTED;
 }
 
+// one launch of the small-K or the bucketed kernel; the bucketed one takes the windows of [len_min, len_max] only, and with
+// redo_src only those marked kRowRedo there
 template <int K>
-int launch_score_bucket(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                        const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                        double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
-    // the test-only table dump and kmin > 1 share the generic instantiation; the production default
-    // (no dump, --minWordSize 1) gets the specialised one
-    if (dump || kmin != 1)
-        return dump ? launch_score_bucket2<K, true, false>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st)
-                    : launch_score_bucket2<K, false, false>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
-    return launch_score_bucket2<K, false, true>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
+int launch_table(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip, double* rows,
+                 uint32_t* status, uint16_t* dump, cudaStream_t st, uint32_t len_min = 0, uint32_t len_max = 0xffffffffu,
+                 const uint32_t* redo_src = nullptr) {
+    LaunchShape s;
+    int rc = table_shape<K>(p, max_len, &s);
+    if (rc) return rc;
+    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
+    const double2* g = reinterpret_cast<const double2*>(ig);
+    uint32_t n = (uint32_t)n_win, cap = (max_len + 15u) & ~15u;
+    if (p.kind == WinKernel::Small) {
+        void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo_src};
+        return frisk_internal::launch_persistent(s, n_win, args, st);
+    }
+    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &cap, &len_min, &len_max, &rows, &status, &dump, &redo_src};
+    return frisk_internal::launch_persistent(s, n_win, args, st);
 }
 
-// the windows the direct kernel marked kRowRedo (generic instantiation: any kmin, optional dump)
+// frisk_b200_score on the small-K or the bucketed kernel.  Bucketed windows longer than 5 rounds need a bigger buffer, which
+// costs a CTA per SM.  With --scaffoldsAll nearly all windows are still the standard length and only whole short scaffolds
+// (up to 1.25 w) are longer: two launches, each taking the windows of its length class, keep the standard ones at four
+// CTAs per SM.
 template <int K>
-int launch_score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                             const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                             double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src, cudaStream_t st) {
-#define FRISK_REDO(R)                                                                                                          \
-    (dump ? launch_score_bucket3<K, R, true, false>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, \
-                                                    status, dump, st, 0u, 0xffffffffu, redo_src)                               \
-          : launch_score_bucket3<K, R, false, false>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, \
-                                                     status, dump, st, 0u, 0xffffffffu, redo_src))
-    if (max_len <= kT3 * 4u * 2u - 6u) return FRISK_REDO(2);
-    if (max_len <= kT3 * 4u * 5u - 6u) return FRISK_REDO(5);
-    return FRISK_REDO(8);
-#undef FRISK_REDO
-}
-
-template <int K>
-int launch_score_small(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                       const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
-                       double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr) {
-    using L = SmallLayout<K>;
-    auto launch = [&](auto kern) -> int {
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::TOTAL));
-        int per_sm = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kT3, L::TOTAL));
-        if (per_sm < 1) per_sm = 1;
-        const int sms = sm_count();
-        if (sms <= 0) return FRISK_E_NO_DEVICE;
-        uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-        if (grid > n_win) grid = n_win;
-        kern<<<(unsigned)grid, kT3, L::TOTAL, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len,
-                                                    (uint32_t)n_win, reinterpret_cast<const double2*>(ig), kmin, want_rip, rows,
-                                                    status, dump, redo_src);
-        CK(cudaGetLastError());
-        return FRISK_OK;
-    };
-    return dump ? launch(score_windows_small_kernel<K, true>) : launch(score_windows_small_kernel<K, false>);
+int score_table(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+                const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip, double* rows,
+                uint32_t* status, uint16_t* dump, cudaStream_t st) {
+    constexpr uint32_t kStd = 5104u;                   // largest buffer that still fits four CTAs
+    if (p.kind == WinKernel::Bucket && p.variant == 8 && n_win >= 4096) {
+        const WinPlan std5{p.kind, 5, p.dump, p.allk};
+        int rc = launch_table<K>(std5, codes, inv, low, win_off, win_len, n_win, kStd, ig, kmin, want_rip, rows, status, dump, st, 0u, kStd);
+        if (rc) return rc;
+        return launch_table<K>(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st, kStd + 1u);
+    }
+    return launch_table<K>(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st);
 }
 
 #define DISPATCH_K(kmax, expr)                      \
@@ -1714,24 +1670,28 @@ int launch_score_small(const uint32_t* codes, const uint32_t* inv, const uint32_
         default: return FRISK_E_UNSUPPORTED;        \
     }
 
-// Which window kernel serves kmax 7 and 8 (windows <= 8,186 bases)?  Measured on C2 (tools/direct_vs_bucket.py):
-// the direct kernel wins where the buckets of the bucketed kernel run full (kmax 7: 1,024 buckets) and windows
-// are long; the bucketed kernel keeps kmax 8 and short windows.
-bool use_nibble_kernel(int kmax, uint32_t max_win_len) {
-    if (kmax < 7 || kmax > 8 || max_win_len > kBuf3 - 6u || g_force_dense || g_force_bucket || g_force_direct) return false;
-    if (g_force_nibble) return true;
-    return FRISK_NIBBLE_DEFAULT(kmax, max_win_len);
-}
-
-bool use_direct_kernel(int kmax, uint32_t max_win_len) {
-    if (kmax < 7 || kmax > 8 || max_win_len > kBuf3 - 6u || g_force_dense || g_force_bucket || g_force_nibble) return false;
-    if (g_force_direct) return true;
-    return FRISK_DIRECT_DEFAULT(kmax, max_win_len);
-}
-
 int check_k(int kmin, int kmax) {
     if (kmin < 1 || kmin > kmax) return FRISK_E_INVALID;
     if (kmax > FRISK_B200_MAX_K) return FRISK_E_UNSUPPORTED;
+    return FRISK_OK;
+}
+
+int table_shape_k(const WinPlan& p, int K, uint32_t max_len, LaunchShape* s) { DISPATCH_K(K, table_shape<K>(p, max_len, s)); }
+
+bool forced(WinKernel k) { return g_forced == (int)k; }
+
+// the peers' forward tables and ready flags of a sharded finalize
+int peer_fwd(const uint64_t* const* d_fwd_peers, uint64_t* const* d_flag_peers, int rank, int world, uint64_t epoch, PeerFwd* f) {
+    if (world > kMaxPeers) return FRISK_E_UNSUPPORTED;
+    f->n = world;
+    f->rank = rank;
+    f->epoch = d_flag_peers ? epoch : 0;
+    for (int q = 0; q < kMaxPeers; ++q) { f->p[q] = nullptr; f->flags[q] = nullptr; }
+    for (int q = 0; q < world; ++q) {
+        if (!d_fwd_peers[q] || (d_flag_peers && !d_flag_peers[q])) return FRISK_E_INVALID;
+        f->p[q] = reinterpret_cast<const unsigned long long*>(d_fwd_peers[q]);
+        if (d_flag_peers) f->flags[q] = reinterpret_cast<unsigned long long*>(d_flag_peers[q]);
+    }
     return FRISK_OK;
 }
 
@@ -1746,23 +1706,102 @@ std::mutex g_run_mu[64];     // frisk_b200_run_host / _run_resident share the wo
 
 }  // namespace
 
-int frisk_internal::sm_count_cached() { return sm_count(); }
+// Which window kernel frisk_b200_score runs.  kmax 9..12: the extension kernel on windows the shared-memory kernels hold,
+// the general one otherwise (and for the test-only table dump).  kmax <= 8: the small-K kernel up to kmax 6 (no sorting,
+// 6 CTAs/SM, any window up to 65,535 bases); for kmax 7 and 8 the nibble kernel (4-bit counters, one atomic per position)
+// or the direct kernel (byte table) as measured on C2 (FRISK_NIBBLE_DEFAULT / FRISK_DIRECT_DEFAULT), then the bucketed
+// one over whatever they hand back; the dense-table kernel for windows longer than the shared-memory buffer.  A forced
+// kernel wins wherever it can run.
+int frisk_internal::plan_score(int kmin, int kmax, uint32_t len, bool dump, WinPlan* out) {
+    int rc = check_k(kmin, kmax);
+    if (rc) return rc;
+    const bool smem = len <= kSmemMaxWindow;
+    WinKernel k;
+    if (forced(WinKernel::General) || len > 65535u) k = WinKernel::General;
+    else if (kmax > FRISK_B200_FAST_K) k = kmax <= 12 && smem && !dump ? WinKernel::NibbleExt : WinKernel::General;
+    else if (forced(WinKernel::Dense)) k = WinKernel::Dense;
+    else if (kmax <= 6 && !forced(WinKernel::Bucket)) k = WinKernel::Small;
+    else if (kmax < 4 || !smem) k = WinKernel::Dense;
+    else if (kmax >= 7 && (forced(WinKernel::Nibble) ||
+                           (!forced(WinKernel::Bucket) && !forced(WinKernel::Direct) && FRISK_NIBBLE_DEFAULT(kmax, len))))
+        k = WinKernel::Nibble;
+    else if (kmax >= 7 && (forced(WinKernel::Direct) || (!forced(WinKernel::Bucket) && FRISK_DIRECT_DEFAULT(kmax, len))))
+        k = WinKernel::Direct;
+    else k = WinKernel::Bucket;
+    *out = {k, window_variant(k, len), dump, kmin == 1 && !dump};
+    return FRISK_OK;
+}
+
+// Positions per thread, from the longest window (the K-mer codes stay in registers between the counting and the scoring
+// pass; shorter windows of the same launch use fewer).  All four kernels run 256 threads; a bucketed or direct round is
+// 4 positions and keeps 6 bases of look-ahead.
+int frisk_internal::window_variant(WinKernel kind, uint32_t len) {
+    if (kind == WinKernel::Bucket || kind == WinKernel::Direct)
+        return len <= kT3 * 4u * 2u - 6u ? 2 : (len <= kT3 * 4u * 5u - 6u ? 5 : 8);
+    if (kind == WinKernel::Nibble || kind == WinKernel::NibbleExt) return len <= kT3 * 8u ? 8 : (len <= kT3 * 20u ? 20 : 32);
+    return 0;
+}
+
+int frisk_internal::sm_count_cached() {
+    static std::atomic<int> cached[64];
+    int dev = 0, n = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
+    if ((n = cached[dev & 63].load(std::memory_order_acquire)) > 0) return n;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
+    cached[dev & 63].store(n, std::memory_order_release);
+    return n;
+}
+
+namespace {
+// CTAs per SM by (device, kernel, dynamic shared memory), and the largest dynamic shared memory a kernel has been allowed
+// on a device: the attribute is only ever raised, so that a launch with a smaller cached size stays valid
+std::mutex g_occ_mu;
+std::map<std::tuple<int, const void*, size_t>, int> g_occ;
+std::map<std::pair<int, const void*>, size_t> g_smem_attr;
+}  // namespace
+
+int frisk_internal::ctas_per_sm(const LaunchShape& s, int* out) {
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    std::lock_guard<std::mutex> lock(g_occ_mu);
+    auto it = g_occ.find({dev, s.fn, s.smem});
+    if (it == g_occ.end()) {
+        size_t& attr = g_smem_attr[{dev, s.fn}];
+        if (s.smem > attr) {
+            CK(cudaFuncSetAttribute(s.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem));
+            attr = s.smem;
+        }
+        if (s.max_carveout)
+            CK(cudaFuncSetAttribute(s.fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        int n = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, s.fn, s.threads, s.smem));
+        it = g_occ.emplace(std::make_tuple(dev, s.fn, s.smem), n).first;
+    }
+    *out = it->second;
+    return FRISK_OK;
+}
+
+int frisk_internal::launch_persistent(const LaunchShape& s, uint64_t n_win, void** args, cudaStream_t st) {
+    int per_sm = 0;
+    int rc = ctas_per_sm(s, &per_sm);
+    if (rc) return rc;
+    const int sms = sm_count_cached();
+    if (sms <= 0) return FRISK_E_NO_DEVICE;
+    const uint64_t grid = std::min<uint64_t>((uint64_t)sms * (uint64_t)std::max(per_sm, 1), n_win);
+    CK(cudaLaunchKernel(s.fn, dim3((unsigned)grid), dim3((unsigned)s.threads), args, s.smem, st));
+    return FRISK_OK;
+}
 
 int frisk_internal::score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                                       const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
                                       int want_rip, double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src,
                                       cudaStream_t st) {
-    if (max_len > kBuf3 - 6u || !redo_src) return FRISK_E_UNSUPPORTED;
-    if (K == 8) return launch_score_bucket_redo<8>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo_src, st);
-    if (K == 7) return launch_score_bucket_redo<7>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo_src, st);
-    // the k sweep hands a window over for EVERY kmax': 4..6 on the bucketed kernel too, 1..3 on the small-K kernel
-    if (K == 6) return launch_score_bucket_redo<6>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo_src, st);
-    if (K == 5) return launch_score_bucket_redo<5>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo_src, st);
-    if (K == 4) return launch_score_bucket_redo<4>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo_src, st);
-    if (K == 3) return launch_score_small<3>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, st, redo_src);
-    if (K == 2) return launch_score_small<2>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, st, redo_src);
-    if (K == 1) return launch_score_small<1>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, st, redo_src);
-    return FRISK_E_UNSUPPORTED;
+    if (max_len > kSmemMaxWindow || !redo_src) return FRISK_E_UNSUPPORTED;
+    // the generic instantiation (any kmin, optional dump); the k sweep hands a window over for EVERY kmax': 4..6 on the
+    // bucketed kernel too, 1..3 on the small-K kernel
+    const WinPlan p{K <= 3 ? WinKernel::Small : WinKernel::Bucket, window_variant(WinKernel::Bucket, max_len), dump != nullptr, false};
+    DISPATCH_K(K, launch_table<K>(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st, 0u,
+                                  0xffffffffu, redo_src));
 }
 
 int frisk_internal::pool_ready() {
@@ -1866,17 +1905,9 @@ int frisk_b200_finalize_tables_peers(const uint64_t* const* d_fwd_peers, uint64_
     if (d_flag_peers && epoch == 0) return FRISK_E_INVALID;
     int rc = check_k(1, kmax);
     if (rc) return rc;
-    if (world > kMaxPeers || kmax > FRISK_B200_FAST_K) return FRISK_E_UNSUPPORTED;
+    if (kmax > FRISK_B200_FAST_K) return FRISK_E_UNSUPPORTED;
     PeerFwd f;
-    f.n = world;
-    f.rank = rank;
-    f.epoch = d_flag_peers ? epoch : 0;
-    for (int q = 0; q < kMaxPeers; ++q) { f.p[q] = nullptr; f.flags[q] = nullptr; }
-    for (int q = 0; q < world; ++q) {
-        if (!d_fwd_peers[q] || (d_flag_peers && !d_flag_peers[q])) return FRISK_E_INVALID;
-        f.p[q] = reinterpret_cast<const unsigned long long*>(d_fwd_peers[q]);
-        if (d_flag_peers) f.flags[q] = reinterpret_cast<unsigned long long*>(d_flag_peers[q]);
-    }
+    if ((rc = peer_fwd(d_fwd_peers, d_flag_peers, rank, world, epoch, &f))) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     DISPATCH_K(kmax, (launch_finalize<K, PeerFwd>(f, symmetric, d_tables, d_valid_kmax, st)));
 }
@@ -1899,15 +1930,8 @@ int frisk_b200_finalize_ivom(const uint64_t* d_fwd, const uint64_t* const* d_fwd
         const LocalFwd f{reinterpret_cast<const unsigned long long*>(d_fwd)};
         DISPATCH_K(kmax, (launch_finalize_ivom<K, LocalFwd>(f, kmin, genome_space, d_tables, d_valid_kmax, d_ig, st)));
     }
-    if (world > kMaxPeers) return FRISK_E_UNSUPPORTED;
     PeerFwd f;
-    f.n = world; f.rank = rank; f.epoch = d_flag_peers ? epoch : 0;
-    for (int q = 0; q < kMaxPeers; ++q) { f.p[q] = nullptr; f.flags[q] = nullptr; }
-    for (int q = 0; q < world; ++q) {
-        if (!d_fwd_peers[q] || (d_flag_peers && !d_flag_peers[q])) return FRISK_E_INVALID;
-        f.p[q] = reinterpret_cast<const unsigned long long*>(d_fwd_peers[q]);
-        if (d_flag_peers) f.flags[q] = reinterpret_cast<unsigned long long*>(d_flag_peers[q]);
-    }
+    if ((rc = peer_fwd(d_fwd_peers, d_flag_peers, rank, world, epoch, &f))) return rc;
     DISPATCH_K(kmax, (launch_finalize_ivom<K, PeerFwd>(f, kmin, genome_space, d_tables, d_valid_kmax, d_ig, st)));
 }
 
@@ -1925,52 +1949,34 @@ int frisk_b200_score(const uint32_t* d_codes, const uint32_t* d_inv, const uint3
                      int kmax, int want_rip, double* d_rows, uint32_t* d_status, uint16_t* d_dump, void* stream) {
     if (n_win == 0) return FRISK_OK;
     if (!d_codes || !d_inv || !d_win_off || !d_win_len || !d_ig || !d_rows || !d_status) return FRISK_E_INVALID;
-    int rc = check_k(kmin, kmax);
+    WinPlan p;
+    int rc = frisk_internal::plan_score(kmin, kmax, max_win_len, d_dump != nullptr, &p);
     if (rc) return rc;
     if (max_win_len > FRISK_B200_MAX_WINDOW || n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     const int rip = want_rip && kmin <= 2 && kmax >= 2;
-    // kmax 9..12 on windows the shared-memory kernels hold: the extension kernel (orders 1..8 as at kmax 8, 9..K from the few
-    // repeated 8-mers); the test-only table dump stays on the general kernel
-    if (kmax > FRISK_B200_FAST_K && kmax <= 12 && max_win_len <= kBuf3 - 6u && !d_dump && !g_force_general)
-        return frisk_internal::score_nibble_ext(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax,
-                                                rip, d_rows, d_status, st);
-    if (kmax > FRISK_B200_FAST_K || max_win_len > 65535u || g_force_general)
-        return frisk_internal::general_score(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax,
-                                             rip, d_rows, d_status, d_dump, st);
-    // word sizes up to 6: the whole order-K table is small -- no sorting, 6 CTAs/SM, any window up to 65,535 bases
-    if (kmax <= 6 && !g_force_dense && !g_force_bucket) {
-        switch (kmax) {
-            case 1: return launch_score_small<1>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 2: return launch_score_small<2>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 3: return launch_score_small<3>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 4: return launch_score_small<4>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 5: return launch_score_small<5>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 6: return launch_score_small<6>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            default: break;
-        }
+    switch (p.kind) {
+        case WinKernel::NibbleExt:
+            return frisk_internal::score_nibble_ext(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax,
+                                                    rip, d_rows, d_status, st);
+        case WinKernel::General:
+            return frisk_internal::general_score(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
+                                                 d_rows, d_status, d_dump, st);
+        case WinKernel::Nibble:
+            return frisk_internal::score_nibble(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
+                                                d_rows, d_status, d_dump, st);
+        case WinKernel::Direct:
+            return frisk_internal::score_direct(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
+                                                d_rows, d_status, d_dump, st);
+        case WinKernel::Small:
+        case WinKernel::Bucket:
+            DISPATCH_K(kmax, score_table<K>(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows,
+                                            d_status, d_dump, st));
+        case WinKernel::Dense:
+            DISPATCH_K(kmax, launch_score<K>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows,
+                                             d_status, d_dump, st));
     }
-    // kmax 7 and 8: the nibble kernel (4-bit counters, one atomic per position) or the direct kernel (byte table), then the
-    // bucketed one over whatever they handed back
-    if (use_nibble_kernel(kmax, max_win_len))
-        return frisk_internal::score_nibble(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                            d_rows, d_status, d_dump, st);
-    if (use_direct_kernel(kmax, max_win_len))
-        return frisk_internal::score_direct(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                            d_rows, d_status, d_dump, st);
-    // kmax 4..8 when forced: bucketed kernel (4 CTAs/SM); the dense-table kernel covers long windows
-    if (kmax >= 4 && max_win_len <= kBuf3 - 6u && !g_force_dense) {
-        switch (kmax) {
-            case 4: return launch_score_bucket<4>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 5: return launch_score_bucket<5>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 6: return launch_score_bucket<6>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 7: return launch_score_bucket<7>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            case 8: return launch_score_bucket<8>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip, d_rows, d_status, d_dump, st);
-            default: break;
-        }
-    }
-    DISPATCH_K(kmax, launch_score<K>(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, rip,
-                                     d_rows, d_status, d_dump, st));
+    return FRISK_E_UNSUPPORTED;
 }
 
 int frisk_b200_score_sweep(const uint32_t* d_codes, const uint32_t* d_inv, const uint32_t* d_low, const uint64_t* d_win_off,
@@ -1978,89 +1984,61 @@ int frisk_b200_score_sweep(const uint32_t* d_codes, const uint32_t* d_inv, const
                            int want_rip, double* const* d_rows, uint32_t* const* d_status, void* stream) {
     if (n_win == 0) return FRISK_OK;
     if (!d_codes || !d_inv || !d_win_off || !d_win_len || !d_ig || !d_rows || !d_status) return FRISK_E_INVALID;
-    if (kmax != 8 || max_win_len > kBuf3 - 6u || n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
+    if (kmax != 8 || max_win_len > kSmemMaxWindow || n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
     return frisk_internal::score_sweep(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, want_rip, d_rows, d_status,
                                        (cudaStream_t)stream);
 }
 
 int frisk_b200_score_occupancy(int kmax, uint32_t max_win_len, int* ctas_per_sm, int* threads_per_cta) {
     if (!ctas_per_sm || !threads_per_cta) return FRISK_E_INVALID;
-    int rc = check_k(1, kmax);
+    WinPlan p;
+    int rc = frisk_internal::plan_score(1, kmax, max_win_len, false, &p);
     if (rc) return rc;
-    *ctas_per_sm = 1;
-    *threads_per_cta = kThreads;
-    if (kmax > FRISK_B200_FAST_K || max_win_len > 65535u) { *threads_per_cta = 1024; return FRISK_OK; }   // general kernel
-    if (kmax <= 6 && !g_force_dense && !g_force_bucket) {                                                       // small-K kernel
-        *threads_per_cta = kT3;
-        switch (kmax) {
-#define FRISK_OCC_S(KK)                                                                                                         \
-    case KK:                                                                                                                    \
-        CK(cudaFuncSetAttribute(score_windows_small_kernel<KK, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,              \
-                                (int)SmallLayout<KK>::TOTAL));                                                                  \
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, score_windows_small_kernel<KK, false>, kT3,               \
-                                                         SmallLayout<KK>::TOTAL));                                              \
-        return FRISK_OK;
-            FRISK_OCC_S(1) FRISK_OCC_S(2) FRISK_OCC_S(3) FRISK_OCC_S(4) FRISK_OCC_S(5) FRISK_OCC_S(6)
-#undef FRISK_OCC_S
-            default: break;
-        }
+    LaunchShape s;
+    switch (p.kind) {
+        case WinKernel::Dense:                              // one CTA of 1,024 threads per SM, like the general kernel
+        case WinKernel::General: *ctas_per_sm = 1; *threads_per_cta = kThreads; return FRISK_OK;
+        case WinKernel::Nibble: s = frisk_internal::nibble_shape(p, kmax); break;
+        case WinKernel::Direct: s = frisk_internal::direct_shape(p, kmax); break;
+        case WinKernel::NibbleExt: s = frisk_internal::ext_shape(p); break;
+        default: if ((rc = table_shape_k(p, kmax, max_win_len, &s))) return rc;
     }
-    if (kmax < 4 || max_win_len > kBuf3 - 6u || g_force_dense) return FRISK_OK;                                // dense kernel
-    if (use_nibble_kernel(kmax, max_win_len)) return frisk_internal::score_nibble_occupancy(kmax, max_win_len, ctas_per_sm, threads_per_cta);
-    if (use_direct_kernel(kmax, max_win_len)) return frisk_internal::score_direct_occupancy(kmax, max_win_len, ctas_per_sm, threads_per_cta);
-    const uint32_t cap = (max_win_len + 15u) & ~15u;
-    *threads_per_cta = kT3;
-#define FRISK_OCC(KK)                                                                                                   \
-    case KK: {                                                                                                          \
-        auto kern = max_win_len <= kT3 * 4u * 2u - 6u ? score_windows_bucket_kernel<KK, 2, false, true>                 \
-                    : (max_win_len <= kT3 * 4u * 5u - 6u ? score_windows_bucket_kernel<KK, 5, false, true>              \
-                                                          : score_windows_bucket_kernel<KK, 8, false, true>);           \
-        const size_t smem = Score3Layout<KK>::total(cap);                                                               \
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                         \
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kern, kT3, smem));                                \
-        return FRISK_OK;                                                                                                \
-    }
-    switch (kmax) {
-        FRISK_OCC(4) FRISK_OCC(5) FRISK_OCC(6) FRISK_OCC(7) FRISK_OCC(8)
-        default: break;
-    }
-#undef FRISK_OCC
-    return FRISK_OK;
+    *threads_per_cta = s.threads;
+    return frisk_internal::ctas_per_sm(s, ctas_per_sm);
 }
 
-// Which window kernel frisk_b200_score launches for these parameters, spelled the way ncu prints it (without the
-// "<unnamed>::" prefix and the argument list): the same decisions as frisk_b200_score above, so a profile or a bench
-// line can be labelled from the launcher's own selection instead of a string constant.
+// Which window kernel frisk_b200_score launches for these parameters (the plan), spelled the way ncu prints it (without
+// the "<unnamed>::" prefix and the argument list), so that a profile or a bench line is labelled from the launcher's own
+// selection instead of a string constant.
 int frisk_b200_score_kernel_name(int kmin, int kmax, uint32_t max_win_len, char* buf, uint64_t cap) {
     if (!buf || cap < 8) return FRISK_E_INVALID;
-    int rc = check_k(kmin, kmax);
+    WinPlan p;
+    int rc = frisk_internal::plan_score(kmin, kmax, max_win_len, false, &p);
     if (rc) return rc;
-    const int allk = kmin == 1 ? 1 : 0;
-    auto chunk = [&](uint32_t a, uint32_t b, uint32_t c) { return max_win_len <= kT3 * a ? a : (max_win_len <= kT3 * b ? b : c); };
-    if (kmax > FRISK_B200_FAST_K && kmax <= 12 && max_win_len <= kBuf3 - 6u && !g_force_general)
-        snprintf(buf, cap, "score_windows_nibble_ext_kernel<%u, %d>", chunk(8u, 20u, 32u), allk);
-    else if (kmax > FRISK_B200_FAST_K || max_win_len > 65535u || g_force_general) snprintf(buf, cap, "gen_score_kernel");
-    else if (kmax <= 6 && !g_force_dense && !g_force_bucket) snprintf(buf, cap, "score_windows_small_kernel<%d, 0>", kmax);
-    else if (use_nibble_kernel(kmax, max_win_len))
-        snprintf(buf, cap, "score_windows_nibble_kernel<%d, %u, 0, %d, 0>", kmax, chunk(8u, 20u, 32u), allk);
-    else if (use_direct_kernel(kmax, max_win_len)) {
-        const uint32_t r = max_win_len <= 256u * 4u * 2u - 6u ? 2u : (max_win_len <= 256u * 4u * 5u - 6u ? 5u : 8u);
-        snprintf(buf, cap, "score_windows_direct_kernel<%d, 256, %u, 0, %d>", kmax, r, allk);
-    } else if (kmax >= 4 && max_win_len <= kBuf3 - 6u && !g_force_dense) {
-        const uint32_t r = max_win_len <= kT3 * 4u * 2u - 6u ? 2u : (max_win_len <= kT3 * 4u * 5u - 6u ? 5u : 8u);
-        snprintf(buf, cap, "score_windows_bucket_kernel<%d, %u, 0, %d>", kmax, r, allk);
-    } else snprintf(buf, cap, "score_windows_kernel<%d>", kmax);
+    const int v = p.variant, allk = p.allk;
+    switch (p.kind) {
+        case WinKernel::Small: snprintf(buf, cap, "score_windows_small_kernel<%d, 0>", kmax); break;
+        case WinKernel::Nibble: snprintf(buf, cap, "score_windows_nibble_kernel<%d, %d, 0, %d, 0>", kmax, v, allk); break;
+        case WinKernel::Direct: snprintf(buf, cap, "score_windows_direct_kernel<%d, 256, %d, 0, %d>", kmax, v, allk); break;
+        case WinKernel::Bucket: snprintf(buf, cap, "score_windows_bucket_kernel<%d, %d, 0, %d>", kmax, v, allk); break;
+        case WinKernel::Dense: snprintf(buf, cap, "score_windows_kernel<%d>", kmax); break;
+        case WinKernel::NibbleExt: snprintf(buf, cap, "score_windows_nibble_ext_kernel<%d, %d>", v, allk); break;
+        case WinKernel::General: snprintf(buf, cap, "gen_score_kernel"); break;
+    }
     return FRISK_OK;
 }
 
 int frisk_b200_set_option(const char* name, int value) {
     if (!name) return FRISK_E_INVALID;
-    if (strcmp(name, "force_dense_kernel") == 0) { g_force_dense = value; return FRISK_OK; }
-    if (strcmp(name, "force_general_kernel") == 0) { g_force_general = value; return FRISK_OK; }
-    if (strcmp(name, "force_bucket_kernel") == 0) { g_force_bucket = value; return FRISK_OK; }
-    if (strcmp(name, "force_direct_kernel") == 0) { g_force_direct = value; return FRISK_OK; }
-    if (strcmp(name, "force_nibble_kernel") == 0) { g_force_nibble = value; return FRISK_OK; }
+    static const struct { const char* name; WinKernel kind; } kForce[] = {
+        {"force_dense_kernel", WinKernel::Dense},   {"force_general_kernel", WinKernel::General}, {"force_bucket_kernel", WinKernel::Bucket},
+        {"force_direct_kernel", WinKernel::Direct}, {"force_nibble_kernel", WinKernel::Nibble}};
+    for (const auto& f : kForce)
+        if (strcmp(name, f.name) == 0) {                    // the last switch set wins; clearing another one changes nothing
+            if (value) g_forced = (int)f.kind;
+            else if (g_forced == (int)f.kind) g_forced = -1;
+            return FRISK_OK;
+        }
     if (strcmp(name, "ingest_exact_open") == 0) { frisk_internal::g_ingest_exact = value; return FRISK_OK; }
     if (strcmp(name, "ingest_chunk_tiles") == 0) { frisk_internal::g_ingest_chunk_tiles = value; return FRISK_OK; }
     return FRISK_E_INVALID;
@@ -2074,6 +2052,19 @@ int frisk_b200_kld(const double* d_genome_ivom, const double* d_window_ivom, uin
 }
 
 namespace {
+// Result buffers the window kernel writes itself: rows and status both page-locked host memory with a device view (40 + 4
+// bytes per window, posted PCIe writes while it runs, no download behind it).  Then *k_rows / *k_stat become those views
+// and the result is true; pageable buffers leave them as they are and get a copy.
+bool pinned_views(double* rows, uint32_t* status, double** k_rows, uint32_t** k_stat) {
+    cudaPointerAttributes pa_rows{}, pa_stat{};
+    const bool direct = cudaPointerGetAttributes(&pa_rows, rows) == cudaSuccess && pa_rows.type == cudaMemoryTypeHost &&
+                        cudaPointerGetAttributes(&pa_stat, status) == cudaSuccess && pa_stat.type == cudaMemoryTypeHost &&
+                        pa_rows.devicePointer && pa_stat.devicePointer;
+    cudaGetLastError();                                 // a pageable pointer makes the query itself report an error
+    if (direct) { *k_rows = (double*)pa_rows.devicePointer; *k_stat = (uint32_t*)pa_stat.devicePointer; }
+    return direct;
+}
+
 // Stage marks of the last frisk_b200_run_host* / _run_resident call on a device (frisk_b200_last_run_timing): timing-enabled
 // events recorded on the call's streams; reading them back costs nothing on the data path.
 enum { kTmStart = 0, kTmUploaded, kTmCounted, kTmFinalised, kTmScored, kTmEnd, kTmScoreStart, kTmCount };
@@ -2206,15 +2197,9 @@ static int run_tail(const PeerArgs& peers, const uint32_t* dhc, const uint32_t* 
     }
     if (copy) CK(cudaStreamWaitEvent(st, copy_done, 0));
     if (n_win) {
-        // Pinned result buffers are written by the score kernel itself (40 + 4 bytes per window, posted
-        // PCIe writes while it runs): no download after the kernel.  Pageable ones get a copy.
-        cudaPointerAttributes pa_rows{}, pa_stat{};
-        const bool direct = cudaPointerGetAttributes(&pa_rows, rows_out) == cudaSuccess && pa_rows.type == cudaMemoryTypeHost &&
-                            cudaPointerGetAttributes(&pa_stat, status_out) == cudaSuccess && pa_stat.type == cudaMemoryTypeHost &&
-                            pa_rows.devicePointer && pa_stat.devicePointer;
-        cudaGetLastError();                             // a pageable pointer makes the query itself report an error
-        double* k_rows = direct ? (double*)pa_rows.devicePointer : (double*)drows;
-        uint32_t* k_stat = direct ? (uint32_t*)pa_stat.devicePointer : (uint32_t*)dstat;
+        double* k_rows = (double*)drows;
+        uint32_t* k_stat = (uint32_t*)dstat;
+        const bool direct = pinned_views(rows_out, status_out, &k_rows, &k_stat);
         if ((rc = mark(tm, kTmScoreStart, st))) return rc;
         rc = frisk_b200_score(dqc, dqi, dql, (const uint64_t*)dwo, (const uint32_t*)dwl, n_win, max_win_len,
                               (const double*)dig, kmin, kmax, want_rip, k_rows, k_stat, nullptr, st);
@@ -2565,8 +2550,10 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
     // the caller's row buffers (inside their capacity) and is simply done again by the host-driven tail below.
     const double min_size = (double)w + (((double)w * 0.75) - (double)step);
     const uint32_t len_bound = (uint32_t)std::min<double>(4.0e9, std::max<double>((double)w, scaffolds_all ? min_size : 0.0));
-    const bool dev_tail = kmax <= FRISK_B200_FAST_K && rows_cap > 0 && rows_cap <= 0xffffffffull && (uint64_t)w <= FRISK_B200_MAX_WINDOW &&
-                          len_bound <= 8186u && use_nibble_kernel(kmax, len_bound) && !getenv("FRISK_RUN_FASTA_HOST_TAIL");
+    WinPlan tail_plan;
+    const bool dev_tail = rows_cap > 0 && rows_cap <= 0xffffffffull && (uint64_t)w <= FRISK_B200_MAX_WINDOW &&
+                          frisk_internal::plan_score(kmin, kmax, len_bound, false, &tail_plan) == FRISK_OK &&
+                          tail_plan.kind == WinKernel::Nibble && !getenv("FRISK_RUN_FASTA_HOST_TAIL");
     void *dtab = nullptr, *dig = nullptr, *dwin = nullptr, *dfirst = nullptr, *dscal = nullptr;
     bool tail_queued = false;
     double* k_rows = rows_out;
@@ -2577,14 +2564,8 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
         if ((rc = ws_get(8, (size_t)pow4(kmax) * 16, &dig))) return rc;
         if ((rc = ws_get(9, rows_cap * 12, &dwin))) return rc;
         if ((rc = ws_get(20, 64, &dscal))) return rc;              // [0] number of windows, [1] genome space
-        cudaPointerAttributes pa_rows{}, pa_stat{};
-        const bool direct = cudaPointerGetAttributes(&pa_rows, rows_out) == cudaSuccess && pa_rows.type == cudaMemoryTypeHost &&
-                            cudaPointerGetAttributes(&pa_stat, status_out) == cudaSuccess && pa_stat.type == cudaMemoryTypeHost &&
-                            pa_rows.devicePointer && pa_stat.devicePointer;
-        cudaGetLastError();
-        rows_direct = direct;
-        if (direct) { k_rows = (double*)pa_rows.devicePointer; k_stat = (uint32_t*)pa_stat.devicePointer; }
-        else {
+        rows_direct = pinned_views(rows_out, status_out, &k_rows, &k_stat);
+        if (!rows_direct) {
             void *drows, *dstat;
             if ((rc = ws_get(11, rows_cap * 40, &drows))) return rc;
             if ((rc = ws_get(12, rows_cap * 4, &dstat))) return rc;
@@ -2611,18 +2592,7 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
     auto queue_finalize = [&](cudaStream_t s2) -> int {
         const LocalFwd f{reinterpret_cast<const unsigned long long*>(dfwd), (const long long*)((unsigned long long*)dscal + 1)};
         uint64_t* dvalid = (uint64_t*)dtab + tsz;
-        int rc2 = FRISK_E_UNSUPPORTED;
-        switch (kmax) {
-            case 1: rc2 = launch_finalize_ivom<1, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 2: rc2 = launch_finalize_ivom<2, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 3: rc2 = launch_finalize_ivom<3, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 4: rc2 = launch_finalize_ivom<4, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 5: rc2 = launch_finalize_ivom<5, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 6: rc2 = launch_finalize_ivom<6, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 7: rc2 = launch_finalize_ivom<7, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            case 8: rc2 = launch_finalize_ivom<8, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2); break;
-            default: break;
-        }
+        int rc2 = [&]() -> int { DISPATCH_K(kmax, (launch_finalize_ivom<K, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2))); }();
         if (rc2) return rc2;
         if ((rc2 = mark(tm, kTmFinalised, s2))) return rc2;
         // the genome tables (0.7 MB) go back on the copy stream while the window kernel runs
@@ -2635,7 +2605,7 @@ int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_
     auto queue_score = [&](cudaStream_t s2) -> int {
         int rc2;
         if ((rc2 = mark(tm, kTmScoreStart, s2))) return rc2;
-        rc2 = frisk_internal::score_nibble(win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
+        rc2 = frisk_internal::score_nibble(tail_plan, win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
                                            (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound, (const double*)dig,
                                            kmin, kmax, want_rip && kmin <= 2 && kmax >= 2 /* as frisk_b200_score: RIP needs orders 1 and 2 */,
                                            k_rows, k_stat, nullptr, s2, (const unsigned long long*)dscal);

@@ -28,15 +28,12 @@
 #include <math_constants.h>
 #include <stdint.h>
 
-#include <atomic>
-
 #include "../../include/frisk_b200.h"
 #include "frisk_internal.h"
 #include "frisk_device.cuh"
 
 namespace {
 using frisk_internal::kRowRedo;
-#define CK(call) FRISK_CK(call)
 
 constexpr uint32_t kSideCap = 64;
 constexpr int kNT = 256;
@@ -770,126 +767,45 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
     }
 }
 
-template <int K, int PP, bool DUMP, bool ALLK>
-int launch_nibble4(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                   const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
-                   double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only,
-                   const unsigned long long* n_win_dev = nullptr) {
-    using L = NibLayout<K>;
-    auto kern = score_windows_nibble_kernel<K, PP, DUMP, ALLK>;
-    // attributes and occupancy once per device and instantiation: three runtime calls less in front of every launch
-    static std::atomic<int> cached[64];
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    int per_sm = cached[dev & 63].load(std::memory_order_acquire);
-    if (per_sm == 0) {
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::TOTAL));
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kNT, L::TOTAL));
-        if (per_sm > 0) cached[dev & 63].store(per_sm, std::memory_order_release);
-    }
-    if (occ_only) { *occ_only = per_sm; return FRISK_OK; }
-    if (per_sm < 1) per_sm = 1;
-    const int sms = frisk_internal::sm_count_cached();
-    if (sms <= 0) return FRISK_E_NO_DEVICE;
-    uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-    if (grid > n_win) grid = n_win;
-    NibSweep sw{};
-    sw.n_win_dev = n_win_dev;
-    kern<<<(unsigned)grid, kNT, L::TOTAL, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len,
-                                                (uint32_t)n_win, reinterpret_cast<const double2*>(ig), kmin, want_rip, rows,
-                                                status, dump, redo_dst, sw);
-    CK(cudaGetLastError());
-    return FRISK_OK;
-}
-
-template <int PP>
-int launch_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,
-                 uint64_t n_win, const NibSweep& sw, int want_rip, uint32_t* redo_dst, cudaStream_t st) {
-    using L = NibLayout<8>;
-    if constexpr (!NIB_PRE5) return FRISK_E_UNSUPPORTED;               // (an A/B build without the order-5 fold has no sweep kernel)
-    auto kern = score_windows_nibble_kernel<8, PP, false, true, NIB_PRE5>;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::TOTAL));
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    int per_sm = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kNT, L::TOTAL));
-    if (per_sm < 1) per_sm = 1;
-    const int sms = frisk_internal::sm_count_cached();
-    if (sms <= 0) return FRISK_E_NO_DEVICE;
-    uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-    if (grid > n_win) grid = n_win;
-    kern<<<(unsigned)grid, kNT, L::TOTAL, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len,
-                                                (uint32_t)n_win, nullptr, 1, want_rip, nullptr, nullptr, nullptr, redo_dst, sw);
-    CK(cudaGetLastError());
-    return FRISK_OK;
-}
-
-template <int K, int PP>
-int launch_nibble3(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                   const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
-                   double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only,
-                   const unsigned long long* n_win_dev = nullptr) {
-    if (dump) return launch_nibble4<K, PP, true, false>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-    if (kmin != 1) return launch_nibble4<K, PP, false, false>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-    return launch_nibble4<K, PP, false, true>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-}
-
-// positions per thread: the longest window of the launch spread over the CTA (K-mer codes stay in registers between
-// the counting and the scoring pass); shorter windows of the same launch use shorter chunks
 template <int K>
-int launch_nibble(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, cudaStream_t st, int* occ_only,
-                  const unsigned long long* n_win_dev = nullptr) {
-    if (max_len <= kNT * 8u)
-        return launch_nibble3<K, 8>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-    if (max_len <= kNT * 20u)
-        return launch_nibble3<K, 20>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-    if (max_len <= kNT * 32u)
-        return launch_nibble3<K, 32>(codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump, redo_dst, st, occ_only, n_win_dev);
-    return FRISK_E_UNSUPPORTED;
+const void* nibble_fn(const frisk_internal::WinPlan& p) {
+    if (p.variant == 8) return FRISK_WIN_INSTANCE(p, score_windows_nibble_kernel, K, 8);
+    if (p.variant == 20) return FRISK_WIN_INSTANCE(p, score_windows_nibble_kernel, K, 20);
+    return FRISK_WIN_INSTANCE(p, score_windows_nibble_kernel, K, 32);
+}
+
+// one launch of a nibble-kernel instantiation, the sweep's included (they share the signature)
+int launch_nibble(const frisk_internal::LaunchShape& s, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
+                  const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
+                  double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, NibSweep sw, cudaStream_t st) {
+    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
+    const double2* g = reinterpret_cast<const double2*>(ig);
+    uint32_t n = (uint32_t)n_win;
+    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo_dst, &sw};
+    return frisk_internal::launch_persistent(s, n_win, args, st);
 }
 
 }  // namespace
 
-int frisk_internal::score_nibble(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
-                                 int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st,
-                                 const unsigned long long* n_win_dev) {
-    if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
-    if (max_len > 8186u) return FRISK_E_UNSUPPORTED;
-    // where the hand-over marks go: `status` itself when it is device memory, device scratch when it is pinned host
-    // memory (the second launch would otherwise read its marks across PCIe, one round trip per window)
-    uint32_t* redo = status;
-    uint32_t* scratch = nullptr;
-    cudaPointerAttributes pa{};
-    if (n_win_dev || cudaPointerGetAttributes(&pa, status) != cudaSuccess || pa.type != cudaMemoryTypeDevice) {
-        cudaGetLastError();
-        int rc = pool_ready();
-        if (rc) return rc;
-        CK(cudaMallocAsync((void**)&scratch, n_win * sizeof(uint32_t), st));
-        // window count in device memory: n_win is only the capacity, and the hand-over launch below walks all of it --
-        // marks beyond the real count must read "nothing to redo"
-        if (n_win_dev) CK(cudaMemsetAsync(scratch, 0, n_win * sizeof(uint32_t), st));
-        redo = scratch;
-    }
-    int rc;
-    if (K == 8) rc = launch_nibble<8>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo, st, nullptr, n_win_dev);
-    else rc = launch_nibble<7>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, redo, st, nullptr, n_win_dev);
-    // windows the nibble table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
-    if (!rc) rc = score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump, redo, st);
-    if (scratch) {                                         // freed on every path (stream-ordered: behind the launches above)
-        const cudaError_t e = cudaFreeAsync(scratch, st);
-        if (!rc && e != cudaSuccess) return frisk_internal::cuda_fail(e, "cudaFreeAsync(scratch)");
-    }
-    return rc;
+frisk_internal::LaunchShape frisk_internal::nibble_shape(const WinPlan& p, int K) {
+    if (K == 8) return {nibble_fn<8>(p), kNT, NibLayout<8>::TOTAL, true};
+    return {nibble_fn<7>(p), kNT, NibLayout<7>::TOTAL, true};
 }
 
-int frisk_internal::score_nibble_occupancy(int K, uint32_t max_len, int* ctas_per_sm, int* threads_per_cta) {
-    if (threads_per_cta) *threads_per_cta = kNT;
-    if (K == 8) return launch_nibble<8>(nullptr, nullptr, nullptr, nullptr, nullptr, 1, max_len, nullptr, 1, 0, nullptr, nullptr, nullptr, nullptr, 0, ctas_per_sm);
-    if (K == 7) return launch_nibble<7>(nullptr, nullptr, nullptr, nullptr, nullptr, 1, max_len, nullptr, 1, 0, nullptr, nullptr, nullptr, nullptr, 0, ctas_per_sm);
-    return FRISK_E_UNSUPPORTED;
+int frisk_internal::score_nibble(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
+                                 const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
+                                 int kmin, int K, int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st,
+                                 const unsigned long long* n_win_dev) {
+    if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
+    NibSweep sw{};
+    sw.n_win_dev = n_win_dev;
+    return with_redo_marks(status, n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
+        int rc = launch_nibble(nibble_shape(p, K), codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump,
+                               redo, sw, st);
+        // windows the nibble table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
+        return rc ? rc : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump,
+                                           redo, st);
+    });
 }
 
 // The k sweep: rows of kmax' = 1..8 (kmin 1) for every window from one pass (see NibSweep).  A window the 4-bit counters
@@ -897,23 +813,23 @@ int frisk_internal::score_nibble_occupancy(int K, uint32_t max_len, int* ctas_pe
 int frisk_internal::score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* const* ig, int want_rip,
                                 double* const* rows, uint32_t* const* status, cudaStream_t st) {
-    if (max_len > kNT * 32u || max_len > 8186u) return FRISK_E_UNSUPPORTED;
+    if (max_len > kSmemMaxWindow) return FRISK_E_UNSUPPORTED;
+    if (!NIB_PRE5) return FRISK_E_UNSUPPORTED;                         // (an A/B build without the order-5 fold has no sweep kernel)
     NibSweep sw{};
     for (int k = 0; k < 8; ++k) {
         if (!ig[k] || !rows[k] || !status[k]) return FRISK_E_INVALID;
         sw.ig[k] = reinterpret_cast<const double2*>(ig[k]); sw.rows[k] = rows[k]; sw.status[k] = status[k];
     }
-    int rc = pool_ready();
-    if (rc) return rc;
-    uint32_t* redo = nullptr;
-    CK(cudaMallocAsync((void**)&redo, n_win * sizeof(uint32_t), st));
-    if (max_len <= kNT * 8u) rc = launch_sweep<8>(codes, inv, low, win_off, win_len, n_win, sw, want_rip, redo, st);
-    else if (max_len <= kNT * 20u) rc = launch_sweep<20>(codes, inv, low, win_off, win_len, n_win, sw, want_rip, redo, st);
-    else rc = launch_sweep<32>(codes, inv, low, win_off, win_len, n_win, sw, want_rip, redo, st);
-    for (int k = 1; k <= 8 && !rc; ++k)
-        rc = score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig[k - 1], 1, k, want_rip && k >= 2, rows[k - 1],
-                               status[k - 1], nullptr, redo, st);
-    const cudaError_t e = cudaFreeAsync(redo, st);
-    if (!rc && e != cudaSuccess) return frisk_internal::cuda_fail(e, "cudaFreeAsync(redo)");
-    return rc;
+    const int pp = window_variant(WinKernel::Nibble, max_len);
+    const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, NIB_PRE5>
+                     : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, NIB_PRE5>
+                                : (const void*)score_windows_nibble_kernel<8, 32, false, true, NIB_PRE5>;
+    return with_redo_marks(nullptr, n_win, false, st, [&](uint32_t* redo) {
+        int rc = launch_nibble({fn, kNT, NibLayout<8>::TOTAL, true}, codes, inv, low, win_off, win_len, n_win, nullptr, 1, want_rip,
+                               nullptr, nullptr, nullptr, redo, sw, st);
+        for (int k = 1; k <= 8 && !rc; ++k)
+            rc = score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig[k - 1], 1, k, want_rip && k >= 2, rows[k - 1],
+                                   status[k - 1], nullptr, redo, st);
+        return rc;
+    });
 }

@@ -27,7 +27,6 @@
 
 namespace {
 using frisk_internal::kRowRedo;
-#define CK(call) FRISK_CK(call)
 
 constexpr uint32_t kSideCap = 64;
 constexpr int kNT = 256;
@@ -484,56 +483,28 @@ score_windows_nibble_ext_kernel(const uint32_t* __restrict__ codes, const uint32
     }
 }
 
-template <int PP>
-int launch_ext(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,
-               uint64_t n_win, const double* ig, int kmin, int K, int want_rip, double* rows, uint32_t* status, uint32_t* redo,
-               cudaStream_t st) {
-    auto launch = [&](auto kern) -> int {
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ExtLayout::TOTAL));
-        CK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        int per_sm = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kNT, ExtLayout::TOTAL));
-        if (per_sm < 1) per_sm = 1;
-        const int sms = frisk_internal::sm_count_cached();
-        if (sms <= 0) return FRISK_E_NO_DEVICE;
-        uint64_t grid = (uint64_t)sms * (uint64_t)per_sm;
-        if (grid > n_win) grid = n_win;
-        kern<<<(unsigned)grid, kNT, ExtLayout::TOTAL, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len,
-                                                            (uint32_t)n_win, reinterpret_cast<const double2*>(ig), kmin, K, want_rip, rows,
-                                                            status, redo);
-        CK(cudaGetLastError());
-        return FRISK_OK;
-    };
-    return kmin == 1 ? launch(score_windows_nibble_ext_kernel<PP, true>) : launch(score_windows_nibble_ext_kernel<PP, false>);
-}
-
 }  // namespace
 
-int frisk_internal::score_nibble_ext(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                                     const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
-                                     int want_rip, double* rows, uint32_t* status, cudaStream_t st) {
-    if (K < 9 || K > 12 || max_len > 8186u) return FRISK_E_UNSUPPORTED;
-    uint32_t* redo = status;
-    uint32_t* scratch = nullptr;
-    cudaPointerAttributes pa{};
-    if (cudaPointerGetAttributes(&pa, status) != cudaSuccess || pa.type != cudaMemoryTypeDevice) {
-        cudaGetLastError();
-        int rc = pool_ready();
-        if (rc) return rc;
-        CK(cudaMallocAsync((void**)&scratch, n_win * sizeof(uint32_t), st));
-        redo = scratch;
-    }
-    int rc;
-    if (max_len <= kNT * 8u) rc = launch_ext<8>(codes, inv, low, win_off, win_len, n_win, ig, kmin, K, want_rip, rows, status, redo, st);
-    else if (max_len <= kNT * 20u) rc = launch_ext<20>(codes, inv, low, win_off, win_len, n_win, ig, kmin, K, want_rip, rows, status, redo, st);
-    else rc = launch_ext<32>(codes, inv, low, win_off, win_len, n_win, ig, kmin, K, want_rip, rows, status, redo, st);
-    // the windows this kernel could not hold: exact re-run on the general kernel (a few CTAs: its per-CTA slab is large)
-    // (few CTAs: the slab is 156 MB per CTA at kmax 12, and a hand-over launch usually has nothing to do)
-    if (!rc) rc = general_score(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, nullptr, st, redo,
-                                K <= 10 ? 8 : 2);
-    if (scratch) {
-        const cudaError_t e = cudaFreeAsync(scratch, st);
-        if (!rc && e != cudaSuccess) return frisk_internal::cuda_fail(e, "cudaFreeAsync(scratch)");
-    }
-    return rc;
+frisk_internal::LaunchShape frisk_internal::ext_shape(const WinPlan& p) {
+#define FRISK_EXT(PP) (p.allk ? (const void*)score_windows_nibble_ext_kernel<PP, true> : (const void*)score_windows_nibble_ext_kernel<PP, false>)
+    const void* fn = p.variant == 8 ? FRISK_EXT(8) : (p.variant == 20 ? FRISK_EXT(20) : FRISK_EXT(32));
+#undef FRISK_EXT
+    return {fn, kNT, ExtLayout::TOTAL, true};
+}
+
+int frisk_internal::score_nibble_ext(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
+                                     const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
+                                     int kmin, int K, int want_rip, double* rows, uint32_t* status, cudaStream_t st) {
+    if (K < 9 || K > 12) return FRISK_E_UNSUPPORTED;
+    return with_redo_marks(status, n_win, false, st, [&](uint32_t* redo) {
+        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
+        const double2* g = reinterpret_cast<const double2*>(ig);
+        uint32_t n = (uint32_t)n_win;
+        void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &K, &want_rip, &rows, &status, &redo};
+        int rc = launch_persistent(ext_shape(p), n_win, args, st);
+        // the windows this kernel could not hold: exact re-run on the general kernel (few CTAs: the slab is 156 MB per CTA
+        // at kmax 12, and a hand-over launch usually has nothing to do)
+        return rc ? rc : general_score(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, nullptr, st,
+                                       redo, K <= 10 ? 8 : 2);
+    });
 }

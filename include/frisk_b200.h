@@ -206,7 +206,8 @@ int frisk_b200_genome_ivom(const uint64_t *d_tables, int kmin, int kmax, int64_t
  * kmin <= 2 <= kmax).  d_status: n_win FRISK_ROW_* words.  d_dump (nullable, tests only):
  * n_win x frisk_b200_table_size(1,kmax) uint16 window tables, orders 1..kmax.
  * max_win_len: the largest win_len (<= FRISK_B200_MAX_WINDOW).  kmax <= 8 and windows <= 65,535 bases
- * run in the shared-memory kernels; anything else in the general kernel (frisk_general.cu), same results.
+ * run in the shared-memory kernels, kmax 9..12 on windows <= 8,186 bases (without d_dump) in the extension kernel,
+ * anything else in the general kernel (frisk_general.cu); same results.  frisk_b200_score_kernel_name names the kernel.
  */
 int frisk_b200_score(const uint32_t *d_codes, const uint32_t *d_inv, const uint32_t *d_low,
                      const uint64_t *d_win_off, const uint32_t *d_win_len, uint64_t n_win, uint32_t max_win_len,
@@ -230,14 +231,17 @@ int frisk_b200_region_features(const uint32_t *d_codes, const uint32_t *d_inv, c
                                uint64_t n_features, double *d_out, void *stream);
 
 /* How frisk_b200_score would run the default (kmin = 1, no dump) configuration on the current device:
- * resident CTAs per SM and threads per CTA of the window kernel it selects (diagnostic; bench.py reports it). */
+ * resident CTAs per SM and threads per CTA of the window kernel it selects, a forced one included (diagnostic;
+ * bench.py reports it). */
 int frisk_b200_score_occupancy(int kmax, uint32_t max_win_len, int *ctas_per_sm, int *threads_per_cta);
 
-/* Tuning/test switches (0 = default behaviour).  "force_dense_kernel" = 1 makes frisk_b200_score use the
- * dense-table kernel (the path for windows of 8,187..65,535 bases) for every input; "force_bucket_kernel" = 1 keeps
- * kmax 4..8 on the bucketed kernel (default for kmax 8); "force_direct_kernel" = 1 runs kmax 7 and 8 on the direct
- * kernel (default for kmax 7) wherever windows are <= 8,186 bases; "force_general_kernel" = 1 selects the general
- * (global-memory, run-time K) path.  All of them produce the same rows (tests/test_gpu_parity.py).
+/* Tuning/test switches (0 = default behaviour).  "force_dense_kernel", "force_bucket_kernel", "force_direct_kernel",
+ * "force_nibble_kernel" and "force_general_kernel" = 1 make frisk_b200_score run that window kernel wherever it can:
+ * dense-table (the kernel for windows of 8,187..65,535 bases) for kmax <= 8; bucketed for kmax 4..8 and direct or nibble
+ * for kmax 7 and 8, on windows <= 8,186 bases; general (global-memory, run-time K) for everything.  Elsewhere the default
+ * choice stands (kmax 9..12 keep the extension kernel unless the general one is forced).  One kernel is forced at a time:
+ * the last switch set to 1 wins, and setting a switch to 0 clears it only if it is the one in force.  Every entry point
+ * that scores windows honours it, and all of them produce the same rows (tests/test_gpu_parity.py).
  * "ingest_exact_open" = 1 makes frisk_b200_fasta_open copy the text in one piece and count the records before it
  * allocates the record table (the fallback of the default chunked open); "ingest_chunk_tiles" = t lets texts of
  * 2t or more 4096-byte tiles be uploaded in chunks (default 512: 2 MiB per chunk, at most 8 chunks).  Same genome
