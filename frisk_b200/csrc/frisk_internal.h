@@ -21,10 +21,7 @@ namespace frisk_internal {
 // records the CUDA error text for frisk_b200_last_cuda_error() and returns FRISK_E_CUDA
 int cuda_fail(cudaError_t e, const char* what);
 
-// cached per-device workspace (grown on demand, freed by frisk_b200_release_workspace)
-int ws_get(int slot, size_t bytes, void** out);
-
-// once per device: let the default memory pool keep up to 1 GiB of freed cudaMallocAsync scratch
+// once per device: let the default memory pool keep up to 32 GiB of freed cudaMallocAsync scratch (frisk_kernels.cu says why)
 int pool_ready();
 extern int g_ingest_exact, g_ingest_chunk_tiles;   // frisk_ingest.cu; set through frisk_b200_set_option
 
@@ -79,6 +76,17 @@ int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* lo
                   const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                   double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr,
                   int grid_cap = 0);
+
+// FRISK_E_INVALID unless 1 <= kmin <= kmax; FRISK_E_UNSUPPORTED for kmax > FRISK_B200_MAX_K
+int check_k(int kmin, int kmax);
+
+// most ranks a sharded finalize sums over (frisk_b200_finalize_ivom, frisk_b200_run_host_peers)
+constexpr int kMaxPeers = 16;
+// frisk_b200_finalize_ivom without its argument checks (the run paths of frisk_run.cu have made them).  space_dev
+// (nullable, single GPU, kmax <= FRISK_B200_FAST_K): the genome space in device memory, read in place of `space`.
+int finalize_ivom(const uint64_t* d_fwd, const uint64_t* const* d_fwd_peers, uint64_t* const* d_flag_peers, int rank, int world,
+                  uint64_t epoch, int kmin, int kmax, int64_t space, const long long* space_dev, uint64_t* tables, uint64_t* valid,
+                  double* ig, cudaStream_t st);
 
 // Longest window the shared-memory window kernels hold: an 8,192-base buffer less 6 bases of look-ahead.
 constexpr uint32_t kSmemMaxWindow = 8186u;

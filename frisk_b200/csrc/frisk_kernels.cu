@@ -20,12 +20,9 @@
 
 #include <algorithm>
 #include <atomic>
-#include <chrono>
-#include <functional>
 #include <map>
 #include <mutex>
 #include <tuple>
-#include <vector>
 
 #include "../../include/frisk_b200.h"
 #include "frisk_internal.h"
@@ -207,7 +204,7 @@ struct LocalFwd {
     __device__ __forceinline__ void arrive_and_wait() const {}
     __device__ __forceinline__ long long space(long long by_value) const { return space_dev ? *space_dev : by_value; }
 };
-constexpr int kMaxPeers = 16;
+using frisk_internal::kMaxPeers;
 struct PeerFwd {
     const unsigned long long* p[kMaxPeers];
     unsigned long long* flags[kMaxPeers];     // flags[q][r]: "rank r's counters of epoch >= value are complete", in rank q's memory
@@ -1484,12 +1481,12 @@ int frisk_internal::cuda_fail(cudaError_t e, const char* what) {
 #endif
 
 namespace {
-using frisk_internal::ws_get;
 using frisk_internal::sm_count_cached;
 using frisk_internal::LaunchShape;
 using frisk_internal::WinKernel;
 using frisk_internal::WinPlan;
 using frisk_internal::kSmemMaxWindow;
+using frisk_internal::check_k;
 #define CK(call) FRISK_CK(call)
 
 template <int K>
@@ -1670,12 +1667,6 @@ int score_table(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, co
         default: return FRISK_E_UNSUPPORTED;        \
     }
 
-int check_k(int kmin, int kmax) {
-    if (kmin < 1 || kmin > kmax) return FRISK_E_INVALID;
-    if (kmax > FRISK_B200_MAX_K) return FRISK_E_UNSUPPORTED;
-    return FRISK_OK;
-}
-
 int table_shape_k(const WinPlan& p, int K, uint32_t max_len, LaunchShape* s) { DISPATCH_K(K, table_shape<K>(p, max_len, s)); }
 
 bool forced(WinKernel k) { return g_forced == (int)k; }
@@ -1694,15 +1685,6 @@ int peer_fwd(const uint64_t* const* d_fwd_peers, uint64_t* const* d_flag_peers, 
     }
     return FRISK_OK;
 }
-
-// cached device workspace of frisk_b200_run_host (one per device, grown on demand)
-struct Workspace {
-    int device = -1;
-    void* buf[32] = {};
-    size_t cap[32] = {};
-};
-Workspace g_ws[64];
-std::mutex g_run_mu[64];     // frisk_b200_run_host / _run_resident share the workspace: one call at a time per device
 
 }  // namespace
 
@@ -1735,6 +1717,12 @@ int frisk_internal::plan_score(int kmin, int kmax, uint32_t len, bool dump, WinP
 // Positions per thread, from the longest window (the K-mer codes stay in registers between the counting and the scoring
 // pass; shorter windows of the same launch use fewer).  All four kernels run 256 threads; a bucketed or direct round is
 // 4 positions and keeps 6 bases of look-ahead.
+int frisk_internal::check_k(int kmin, int kmax) {
+    if (kmin < 1 || kmin > kmax) return FRISK_E_INVALID;
+    if (kmax > FRISK_B200_MAX_K) return FRISK_E_UNSUPPORTED;
+    return FRISK_OK;
+}
+
 int frisk_internal::window_variant(WinKernel kind, uint32_t len) {
     if (kind == WinKernel::Bucket || kind == WinKernel::Direct)
         return len <= kT3 * 4u * 2u - 6u ? 2 : (len <= kT3 * 4u * 5u - 6u ? 5 : 8);
@@ -1804,6 +1792,25 @@ int frisk_internal::score_bucket_redo(const uint32_t* codes, const uint32_t* inv
                                   0xffffffffu, redo_src));
 }
 
+int frisk_internal::finalize_ivom(const uint64_t* d_fwd, const uint64_t* const* d_fwd_peers, uint64_t* const* d_flag_peers, int rank,
+                                  int world, uint64_t epoch, int kmin, int kmax, int64_t space, const long long* space_dev,
+                                  uint64_t* tables, uint64_t* valid, double* ig, cudaStream_t st) {
+    int rc;
+    if (kmax > FRISK_B200_FAST_K) {                                   // general path: separate launches
+        if (world > 0 || space_dev) return FRISK_E_UNSUPPORTED;
+        if ((rc = frisk_internal::general_finalize(d_fwd, kmax, 1, tables, valid, st))) return rc;
+        return frisk_internal::general_genome_ivom(tables, kmin, kmax, space, ig, st);
+    }
+    if (world == 0) {
+        const LocalFwd f{reinterpret_cast<const unsigned long long*>(d_fwd), space_dev};
+        DISPATCH_K(kmax, (launch_finalize_ivom<K, LocalFwd>(f, kmin, space, tables, valid, ig, st)));
+    }
+    if (space_dev) return FRISK_E_UNSUPPORTED;
+    PeerFwd f;
+    if ((rc = peer_fwd(d_fwd_peers, d_flag_peers, rank, world, epoch, &f))) return rc;
+    DISPATCH_K(kmax, (launch_finalize_ivom<K, PeerFwd>(f, kmin, space, tables, valid, ig, st)));
+}
+
 int frisk_internal::pool_ready() {
     static bool done[64] = {};
     int dev = 0;
@@ -1818,21 +1825,6 @@ int frisk_internal::pool_ready() {
         CK(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep));
         done[dev & 63] = true;
     }
-    return FRISK_OK;
-}
-
-int frisk_internal::ws_get(int slot, size_t bytes, void** out) {
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    Workspace& w = g_ws[dev & 63];
-    if (w.cap[slot] < bytes) {
-        if (w.buf[slot]) CK(cudaFree(w.buf[slot]));
-        w.buf[slot] = nullptr; w.cap[slot] = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        CK(cudaMalloc(&w.buf[slot], want));
-        w.cap[slot] = want;
-    }
-    *out = w.buf[slot];
     return FRISK_OK;
 }
 
@@ -1920,19 +1912,8 @@ int frisk_b200_finalize_ivom(const uint64_t* d_fwd, const uint64_t* const* d_fwd
     if (world > 0 && d_flag_peers && epoch == 0) return FRISK_E_INVALID;
     int rc = check_k(kmin, kmax);
     if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (kmax > FRISK_B200_FAST_K) {                                   // general path: separate launches
-        if (world > 0) return FRISK_E_UNSUPPORTED;
-        if ((rc = frisk_internal::general_finalize(d_fwd, kmax, 1, d_tables, d_valid_kmax, st))) return rc;
-        return frisk_internal::general_genome_ivom(d_tables, kmin, kmax, genome_space, d_ig, st);
-    }
-    if (world == 0) {
-        const LocalFwd f{reinterpret_cast<const unsigned long long*>(d_fwd)};
-        DISPATCH_K(kmax, (launch_finalize_ivom<K, LocalFwd>(f, kmin, genome_space, d_tables, d_valid_kmax, d_ig, st)));
-    }
-    PeerFwd f;
-    if ((rc = peer_fwd(d_fwd_peers, d_flag_peers, rank, world, epoch, &f))) return rc;
-    DISPATCH_K(kmax, (launch_finalize_ivom<K, PeerFwd>(f, kmin, genome_space, d_tables, d_valid_kmax, d_ig, st)));
+    return frisk_internal::finalize_ivom(d_fwd, d_fwd_peers, d_flag_peers, rank, world, epoch, kmin, kmax, genome_space, nullptr,
+                                         d_tables, d_valid_kmax, d_ig, (cudaStream_t)stream);
 }
 
 int frisk_b200_genome_ivom(const uint64_t* d_tables, int kmin, int kmax, int64_t genome_space, double* d_ig, void* stream) {
@@ -2048,753 +2029,6 @@ int frisk_b200_kld(const double* d_genome_ivom, const double* d_window_ivom, uin
     if (!d_out || (n && (!d_genome_ivom || !d_window_ivom)) || n > 0xffffffffull) return FRISK_E_INVALID;
     kld_kernel<<<1, kThreads, 0, (cudaStream_t)stream>>>(d_genome_ivom, d_window_ivom, (uint32_t)n, d_out);
     CK(cudaGetLastError());
-    return FRISK_OK;
-}
-
-namespace {
-// Result buffers the window kernel writes itself: rows and status both page-locked host memory with a device view (40 + 4
-// bytes per window, posted PCIe writes while it runs, no download behind it).  Then *k_rows / *k_stat become those views
-// and the result is true; pageable buffers leave them as they are and get a copy.
-bool pinned_views(double* rows, uint32_t* status, double** k_rows, uint32_t** k_stat) {
-    cudaPointerAttributes pa_rows{}, pa_stat{};
-    const bool direct = cudaPointerGetAttributes(&pa_rows, rows) == cudaSuccess && pa_rows.type == cudaMemoryTypeHost &&
-                        cudaPointerGetAttributes(&pa_stat, status) == cudaSuccess && pa_stat.type == cudaMemoryTypeHost &&
-                        pa_rows.devicePointer && pa_stat.devicePointer;
-    cudaGetLastError();                                 // a pageable pointer makes the query itself report an error
-    if (direct) { *k_rows = (double*)pa_rows.devicePointer; *k_stat = (uint32_t*)pa_stat.devicePointer; }
-    return direct;
-}
-
-// Stage marks of the last frisk_b200_run_host* / _run_resident call on a device (frisk_b200_last_run_timing): timing-enabled
-// events recorded on the call's streams; reading them back costs nothing on the data path.
-enum { kTmStart = 0, kTmUploaded, kTmCounted, kTmFinalised, kTmScored, kTmEnd, kTmScoreStart, kTmCount };
-struct RunMarks {
-    cudaEvent_t ev[kTmCount] = {};
-    bool have[kTmCount] = {};
-    bool ready = false;
-};
-RunMarks g_marks[64];
-int run_marks(RunMarks** out) {
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    RunMarks& m = g_marks[dev & 63];
-    if (!m.ready) {
-        for (auto& e : m.ev) CK(cudaEventCreate(&e));
-        m.ready = true;
-    }
-    for (auto& h : m.have) h = false;
-    *out = &m;
-    return FRISK_OK;
-}
-int mark(RunMarks* m, int which, cudaStream_t st) {
-    if (!m) return FRISK_OK;
-    CK(cudaEventRecord(m->ev[which], st));
-    m->have[which] = true;
-    return FRISK_OK;
-}
-}  // namespace
-
-// Everything after the planes are on the device: [background], finalize, genome IVOM, window
-// upload, score, download.  `copy` (nullable) already carries the uploads this run must wait for.
-// multi-GPU: where the other ranks' counters are (frisk_b200_finalize_tables_peers); world == 0: single GPU
-struct PeerArgs {
-    uint64_t* d_fwd_local = nullptr;
-    const uint64_t* const* d_fwd_peers = nullptr;
-    uint64_t* const* d_flag_peers = nullptr;
-    int rank = 0, world = 0;
-    uint64_t epoch = 0;
-};
-
-// A window list that points outside the planes would become an illegal-address fault (and a sticky context error) in the
-// score kernel; the arrays are host memory here, so check them: O(n), ~1 ns per window.
-static int check_windows(const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_win_len, uint64_t padded_len) {
-    for (uint64_t i = 0; i < n_win; ++i) {
-        const uint64_t l = win_len[i];
-        if (l == 0 || l > max_win_len || win_off[i] > padded_len || l > padded_len - win_off[i]) return FRISK_E_INVALID;
-    }
-    return FRISK_OK;
-}
-
-typedef std::function<int(const uint64_t** win_off, const uint32_t** win_len, uint64_t* n_win, uint32_t* max_win_len)> LateWindows;
-
-// FRISK_RUN_TRACE=1: host-side timeline of a one-call run on stderr (microseconds since the first stamp)
-struct HostTrace {
-    bool on = getenv("FRISK_RUN_TRACE") != nullptr;
-    std::chrono::steady_clock::time_point t0;
-    char buf[512]; int len = 0; bool started = false;
-    void stamp(const char* what) {
-        if (!on) return;
-        const auto now = std::chrono::steady_clock::now();
-        if (!started) { t0 = now; started = true; }
-        len += snprintf(buf + len, sizeof(buf) - (size_t)len, " %s=%.1f", what, std::chrono::duration<double, std::micro>(now - t0).count());
-    }
-    void flush() { if (on && len) fprintf(stderr, "host trace (us):%s\n", buf); len = 0; started = false; }
-};
-static thread_local HostTrace g_trace;
-
-static int run_tail(const PeerArgs& peers, const uint32_t* dhc, const uint32_t* dhi, const uint32_t* dhl, uint64_t h_padded_len, bool bg_enqueued,
-                    const uint32_t* dqc, const uint32_t* dqi, const uint32_t* dql, const uint64_t* win_off,
-                    const uint32_t* win_len, uint64_t n_win, uint32_t max_win_len, int kmin, int kmax, int mask_host,
-                    int want_rip, int64_t genome_space, double* rows_out, uint32_t* status_out, uint64_t* tables_out,
-                    uint64_t* valid_kmax_out, void* dfwd, cudaStream_t st, cudaStream_t copy, cudaEvent_t copy_done,
-                    cudaEvent_t tables_ready, RunMarks* tm, const LateWindows* late = nullptr) {
-    // late: the window list is produced by the caller AFTER the tables' finalisation has been queued (frisk_b200_run_fasta:
-    // the host derives the windows while the device is still counting)
-    const size_t tsz = (size_t)frisk_b200_table_size(1, kmax);
-    void *dtab, *dig, *dwo = nullptr, *dwl = nullptr, *drows = nullptr, *dstat = nullptr;
-    int rc;
-    if ((rc = ws_get(7, (tsz + 1) * 8, &dtab))) return rc;
-    if ((rc = ws_get(8, (size_t)pow4(kmax) * 16, &dig))) return rc;
-    auto upload_windows = [&]() -> int {
-        if (n_win) {
-            int rc2;
-            // (offsets and lengths in one host block -- frisk_b200_run_fasta's staging -- travel as one copy)
-            const bool one_block = (const void*)win_len == (const void*)(win_off + n_win);
-            if ((rc2 = ws_get(9, one_block ? n_win * 12 : n_win * 8, &dwo))) return rc2;
-            if (one_block) dwl = (char*)dwo + n_win * 8;
-            else if ((rc2 = ws_get(10, n_win * 4, &dwl))) return rc2;
-            if ((rc2 = ws_get(11, n_win * 40, &drows))) return rc2;
-            if ((rc2 = ws_get(12, n_win * 4, &dstat))) return rc2;
-            // the window list rides behind the planes -- but a late one goes on the compute stream: the copy stream is busy
-            // bringing the tables back by then, and the window kernel would wait 0.03 ms for its 190 KB behind them
-            cudaStream_t up = (copy && !late) ? copy : st;
-            if (one_block) CK(cudaMemcpyAsync(dwo, win_off, n_win * 12, cudaMemcpyHostToDevice, up));
-            else {
-                CK(cudaMemcpyAsync(dwo, win_off, n_win * 8, cudaMemcpyHostToDevice, up));
-                CK(cudaMemcpyAsync(dwl, win_len, n_win * 4, cudaMemcpyHostToDevice, up));
-            }
-        }
-        if (copy) CK(cudaEventRecord(copy_done, copy));
-        return FRISK_OK;
-    };
-    if (!late && (rc = upload_windows())) return rc;
-    if (!bg_enqueued) {
-        CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, st));
-        // the last 32-base word is padding by construction and is only ever read as look-ahead
-        rc = frisk_b200_background(dhc, dhi, dhl, 0, h_padded_len - 32, kmax, mask_host, (uint64_t*)dfwd, st);
-        if (rc) return rc;
-        if ((rc = mark(tm, kTmCounted, st))) return rc;
-    }
-    uint64_t* dvalid = (uint64_t*)dtab + tsz;
-    rc = frisk_b200_finalize_ivom((const uint64_t*)dfwd, peers.d_fwd_peers, peers.d_flag_peers, peers.rank, peers.world, peers.epoch,
-                                  kmin, kmax, genome_space, (uint64_t*)dtab, dvalid, (double*)dig, st);
-    if (rc) return rc;
-    if ((rc = mark(tm, kTmFinalised, st))) return rc;
-    // the genome tables (0.7 MB) go back on the copy stream while the window kernel runs, not behind it
-    const bool tables_aside = copy && tables_ready && (tables_out || valid_kmax_out);
-    if (tables_aside) {
-        CK(cudaEventRecord(tables_ready, st));
-        CK(cudaStreamWaitEvent(copy, tables_ready, 0));
-        if (tables_out) CK(cudaMemcpyAsync(tables_out, dtab, tsz * 8, cudaMemcpyDeviceToHost, copy));
-        if (valid_kmax_out) CK(cudaMemcpyAsync(valid_kmax_out, dvalid, 8, cudaMemcpyDeviceToHost, copy));
-    }
-    g_trace.stamp("finalize_queued");
-    if (late) {
-        if ((rc = (*late)(&win_off, &win_len, &n_win, &max_win_len))) return rc;
-        g_trace.stamp("windows");
-        if ((rc = upload_windows())) return rc;
-        g_trace.stamp("windows_queued");
-    }
-    if (copy) CK(cudaStreamWaitEvent(st, copy_done, 0));
-    if (n_win) {
-        double* k_rows = (double*)drows;
-        uint32_t* k_stat = (uint32_t*)dstat;
-        const bool direct = pinned_views(rows_out, status_out, &k_rows, &k_stat);
-        if ((rc = mark(tm, kTmScoreStart, st))) return rc;
-        rc = frisk_b200_score(dqc, dqi, dql, (const uint64_t*)dwo, (const uint32_t*)dwl, n_win, max_win_len,
-                              (const double*)dig, kmin, kmax, want_rip, k_rows, k_stat, nullptr, st);
-        if (rc) return rc;
-        g_trace.stamp("score_queued");
-        if ((rc = mark(tm, kTmScored, st))) return rc;
-        if (!direct) {
-            CK(cudaMemcpyAsync(rows_out, drows, n_win * 40, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(status_out, dstat, n_win * 4, cudaMemcpyDeviceToHost, st));
-        }
-    }
-    if (!tables_aside) {
-        if (tables_out) CK(cudaMemcpyAsync(tables_out, dtab, tsz * 8, cudaMemcpyDeviceToHost, st));
-        if (valid_kmax_out) CK(cudaMemcpyAsync(valid_kmax_out, dvalid, 8, cudaMemcpyDeviceToHost, st));
-    }
-    if ((rc = mark(tm, kTmEnd, st))) return rc;
-    CK(cudaStreamSynchronize(st));
-    g_trace.stamp("done");
-    g_trace.flush();
-    if (tables_aside) CK(cudaStreamSynchronize(copy));
-    return FRISK_OK;
-}
-
-// per-device copy stream + events of frisk_b200_run_host (uploads overlap the background count)
-namespace {
-constexpr int kMaxChunks = 16;
-struct CopyCtx {
-    cudaStream_t copy = nullptr;
-    cudaEvent_t ev[kMaxChunks + 3] = {};
-};
-CopyCtx g_copy[64];
-
-int copy_ctx(CopyCtx** out) {
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    CopyCtx& c = g_copy[dev & 63];
-    if (!c.copy) {
-        CK(cudaStreamCreateWithFlags(&c.copy, cudaStreamNonBlocking));
-        for (auto& e : c.ev) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    }
-    *out = &c;
-    return FRISK_OK;
-}
-}  // namespace
-
-// One genome's planes in host memory; the invalid plane either dense or as its non-zero words.
-struct HostPlanes {
-    const uint32_t* codes;
-    const uint32_t* inv;            // dense (padded_len / 32 words) or nullptr
-    const uint32_t* inv_idx;        // sparse: word indices ...
-    const uint32_t* inv_val;        // ... and the words
-    uint64_t inv_n;
-    const uint32_t* low;            // nullable
-    uint64_t padded_len;
-};
-
-__global__ void __launch_bounds__(256)
-plane_scatter_kernel(const uint32_t* __restrict__ idx, const uint32_t* __restrict__ val, uint64_t n, uint32_t* __restrict__ plane) {
-    const uint64_t i = (uint64_t)blockIdx.x * 256u + threadIdx.x;
-    if (i < n) plane[idx[i]] = val[i];
-}
-
-// invalid plane of `hp` -> d_inv on the copy stream (sparse: zero fill + pairs + scatter)
-static int upload_inv(const HostPlanes& hp, void* d_inv, int slot_idx, int slot_val, cudaStream_t copy) {
-    if (hp.inv) return FRISK_OK;                      // dense: goes up with the code chunks
-    CK(cudaMemsetAsync(d_inv, 0, hp.padded_len / 8, copy));
-    if (hp.inv_n) {
-        void *di, *dv;
-        int rc;
-        if ((rc = ws_get(slot_idx, hp.inv_n * 4, &di))) return rc;
-        if ((rc = ws_get(slot_val, hp.inv_n * 4, &dv))) return rc;
-        CK(cudaMemcpyAsync(di, hp.inv_idx, hp.inv_n * 4, cudaMemcpyHostToDevice, copy));
-        CK(cudaMemcpyAsync(dv, hp.inv_val, hp.inv_n * 4, cudaMemcpyHostToDevice, copy));
-        plane_scatter_kernel<<<(unsigned)((hp.inv_n + 255) / 256), 256, 0, copy>>>((const uint32_t*)di, (const uint32_t*)dv,
-                                                                                  hp.inv_n, (uint32_t*)d_inv);
-        CK(cudaGetLastError());
-    }
-    return FRISK_OK;
-}
-
-static int run_host_body(const PeerArgs& peers, const HostPlanes& h, const HostPlanes& q, bool same, const uint64_t* win_off, const uint32_t* win_len,
-                         uint64_t n_win, uint32_t max_win_len, int kmin, int kmax, int mask_host, int want_rip,
-                         int64_t genome_space, double* rows_out, uint32_t* status_out, uint64_t* tables_out,
-                         uint64_t* valid_kmax_out, void* stream);
-
-// On an error the copies and kernels already queued still target the caller's (pinned) buffers: drain both streams
-// before handing control -- and with it the right to free those buffers -- back.
-static int run_host_impl(const PeerArgs& peers, const HostPlanes& h, const HostPlanes& q, bool same, const uint64_t* win_off, const uint32_t* win_len,
-                         uint64_t n_win, uint32_t max_win_len, int kmin, int kmax, int mask_host, int want_rip,
-                         int64_t genome_space, double* rows_out, uint32_t* status_out, uint64_t* tables_out,
-                         uint64_t* valid_kmax_out, void* stream) {
-    const int rc = run_host_body(peers, h, q, same, win_off, win_len, n_win, max_win_len, kmin, kmax, mask_host, want_rip, genome_space,
-                                 rows_out, status_out, tables_out, valid_kmax_out, stream);
-    if (rc != FRISK_OK && rc != FRISK_E_INVALID && rc != FRISK_E_NO_DEVICE && rc != FRISK_E_UNSUPPORTED) {
-        int dev = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess) {
-            cudaStreamSynchronize((cudaStream_t)stream);
-            if (g_copy[dev & 63].copy) cudaStreamSynchronize(g_copy[dev & 63].copy);
-        }
-        cudaGetLastError();
-    }
-    return rc;
-}
-
-static int run_host_body(const PeerArgs& peers, const HostPlanes& h, const HostPlanes& q, bool same, const uint64_t* win_off, const uint32_t* win_len,
-                         uint64_t n_win, uint32_t max_win_len, int kmin, int kmax, int mask_host, int want_rip,
-                         int64_t genome_space, double* rows_out, uint32_t* status_out, uint64_t* tables_out,
-                         uint64_t* valid_kmax_out, void* stream) {
-    const uint64_t h_padded_len = h.padded_len, q_padded_len = q.padded_len;
-    if (!h.codes || !q.codes || (!h.inv && !h.inv_idx && h.inv_n) || (!q.inv && !q.inv_idx && q.inv_n) ||
-        (h_padded_len & 127) || (q_padded_len & 127) || h_padded_len < 128 || q_padded_len < 128)
-        return FRISK_E_INVALID;
-    if (n_win && (!win_off || !win_len || !rows_out || !status_out)) return FRISK_E_INVALID;
-    int rc = check_k(kmin, kmax);
-    if (rc) return rc;
-    if ((rc = check_windows(win_off, win_len, n_win, max_win_len, q_padded_len))) return rc;
-    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
-    int dev_ = 0;
-    CK(cudaGetDevice(&dev_));
-    std::lock_guard<std::mutex> lock(g_run_mu[dev_ & 63]);
-    cudaStream_t st = (cudaStream_t)stream;
-    CopyCtx* cc = nullptr;
-    if ((rc = copy_ctx(&cc))) return rc;
-    RunMarks* tm = nullptr;
-    if ((rc = run_marks(&tm))) return rc;
-    if ((rc = mark(tm, kTmStart, st))) return rc;
-    const size_t tsz = (size_t)frisk_b200_table_size(1, kmax);
-    void *dhc, *dhi, *dhl = nullptr, *dqc, *dqi, *dql = nullptr, *dfwd;
-    if ((rc = ws_get(0, h_padded_len / 4, &dhc))) return rc;
-    if ((rc = ws_get(1, h_padded_len / 8, &dhi))) return rc;
-    if (h.low && (rc = ws_get(2, h_padded_len / 8, &dhl))) return rc;
-    if (peers.world) {
-        if (!peers.d_fwd_local || !peers.d_fwd_peers) return FRISK_E_INVALID;
-        dfwd = peers.d_fwd_local;                     // this rank's counters live where the peers can read them
-        CK(cudaMemsetAsync(dfwd, 0, tsz * 8, st));
-    } else {
-        if ((rc = ws_get(6, (tsz + 1) * 8, &dfwd))) return rc;
-        CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, st));
-    }
-    // The planes go up in chunks on the copy stream; the background count of a chunk starts as soon
-    // as the chunk has landed (it stops 128 bases short of the chunk's end: the kernel looks ahead),
-    // so only the last chunk's count is not hidden behind PCIe.
-    CK(cudaEventRecord(cc->ev[kMaxChunks], st));
-    CK(cudaStreamWaitEvent(cc->copy, cc->ev[kMaxChunks], 0));          // order behind earlier work on `stream`
-    // sparse invalid plane: zero fill + pairs + scatter on the COMPUTE stream, behind the first code chunk's transfer
-    // (on the copy stream they would delay that chunk by four small operations); the counts on `st` follow in order
-    if ((rc = upload_inv(h, dhi, 15, 16, st))) return rc;
-    // Chunk plan: equal chunks of <= 64 M bases.  Measured on C2 (40 Mbp, profiles/r02_upload_plans.txt): one chunk -- upload,
-    // then one count of 0.07 ms -- beats every split (2 chunks +0.02 ms, 3 chunks +0.04..0.1 ms): a count that runs beside
-    // the copy takes about twice as long, every extra copy and count launch has a fixed cost, and the whole count is short
-    // next to the upload.  Genomes of hundreds of Mbp and more keep the split: there the last chunk's count is what shows.
-    // FRISK_UPLOAD_PLAN="f0,f1,..." (relative chunk sizes) overrides the plan (tools/upload_plans.sh).
-    uint64_t bounds[kMaxChunks + 1];
-    uint64_t n_chunks = 0;
-    bounds[0] = 0;
-    {
-        int parts[kMaxChunks];
-        int n_parts = (int)((h_padded_len + (64ull << 20) - 1) / (64ull << 20));
-        if (n_parts > kMaxChunks - 1) n_parts = kMaxChunks - 1;
-        if (n_parts < 1) n_parts = 1;
-        // (also when eight ranks share the host's H2D bandwidth and the upload takes twice as long, profiles/
-        // r02_pcie_contention_8gpu.json: two chunks measured 0.50 ms to the end of the count against 0.48 for one)
-        for (int i = 0; i < n_parts; ++i) parts[i] = 1;
-        if (const char* e = getenv("FRISK_UPLOAD_PLAN")) {
-            n_parts = 0;
-            for (const char* p = e; *p && n_parts < kMaxChunks - 1;) {
-                parts[n_parts++] = atoi(p);
-                while (*p && *p != ',') ++p;
-                if (*p == ',') ++p;
-            }
-        }
-        int total = 0, acc = 0;
-        for (int i = 0; i < n_parts; ++i) total += parts[i] > 0 ? parts[i] : 0;
-        for (int i = 0; i < n_parts && total > 0; ++i) {
-            if (parts[i] <= 0) continue;
-            acc += parts[i];
-            uint64_t b = i == n_parts - 1 ? h_padded_len : ((h_padded_len / (uint64_t)total) * (uint64_t)acc + 127) & ~127ull;
-            if (b > h_padded_len) b = h_padded_len;
-            if (b > bounds[n_chunks]) bounds[++n_chunks] = b;
-        }
-        if (n_chunks == 0 || bounds[n_chunks] != h_padded_len) bounds[++n_chunks] = h_padded_len;
-    }
-    uint64_t counted = 0;
-    for (uint64_t c = 0; c < n_chunks; ++c) {
-        const uint64_t b0 = bounds[c], b1 = bounds[c + 1];
-        if (b0 >= b1) continue;
-        CK(cudaMemcpyAsync((char*)dhc + b0 / 4, (const char*)h.codes + b0 / 4, (b1 - b0) / 4, cudaMemcpyHostToDevice, cc->copy));
-        if (h.inv) CK(cudaMemcpyAsync((char*)dhi + b0 / 8, (const char*)h.inv + b0 / 8, (b1 - b0) / 8, cudaMemcpyHostToDevice, cc->copy));
-        if (h.low) CK(cudaMemcpyAsync((char*)dhl + b0 / 8, (const char*)h.low + b0 / 8, (b1 - b0) / 8, cudaMemcpyHostToDevice, cc->copy));
-        CK(cudaEventRecord(cc->ev[c], cc->copy));
-        CK(cudaStreamWaitEvent(st, cc->ev[c], 0));
-        const uint64_t upto = (b1 == h_padded_len) ? h_padded_len - 32 : b1 - 128;
-        if (upto > counted) {
-            rc = frisk_b200_background((const uint32_t*)dhc, (const uint32_t*)dhi, (const uint32_t*)dhl, counted, upto, kmax,
-                                       mask_host, (uint64_t*)dfwd, st);
-            if (rc) return rc;
-            counted = upto;
-        }
-    }
-    if ((rc = mark(tm, kTmUploaded, cc->copy))) return rc;
-    if ((rc = mark(tm, kTmCounted, st))) return rc;
-    if (same) { dqc = dhc; dqi = dhi; dql = dhl; }
-    else {
-        if ((rc = ws_get(3, q_padded_len / 4, &dqc))) return rc;
-        if ((rc = ws_get(4, q_padded_len / 8, &dqi))) return rc;
-        if (q.low && (rc = ws_get(5, q_padded_len / 8, &dql))) return rc;
-        CK(cudaMemcpyAsync(dqc, q.codes, q_padded_len / 4, cudaMemcpyHostToDevice, cc->copy));
-        if (q.inv) CK(cudaMemcpyAsync(dqi, q.inv, q_padded_len / 8, cudaMemcpyHostToDevice, cc->copy));
-        else if ((rc = upload_inv(q, dqi, 17, 18, cc->copy))) return rc;
-        if (q.low) CK(cudaMemcpyAsync(dql, q.low, q_padded_len / 8, cudaMemcpyHostToDevice, cc->copy));
-    }
-    return run_tail(peers, (const uint32_t*)dhc, (const uint32_t*)dhi, (const uint32_t*)dhl, h_padded_len, true,
-                    (const uint32_t*)dqc, (const uint32_t*)dqi, (const uint32_t*)dql, win_off, win_len, n_win, max_win_len,
-                    kmin, kmax, mask_host, want_rip, genome_space, rows_out, status_out, tables_out, valid_kmax_out, dfwd, st,
-                    cc->copy, cc->ev[kMaxChunks + 1], cc->ev[kMaxChunks + 2], tm);
-}
-
-int frisk_b200_run_host(const uint32_t* h_codes, const uint32_t* h_inv, const uint32_t* h_low, uint64_t h_padded_len,
-                        const uint32_t* q_codes, const uint32_t* q_inv, const uint32_t* q_low, uint64_t q_padded_len,
-                        const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_win_len,
-                        int kmin, int kmax, int mask_host, int want_rip, int64_t genome_space, double* rows_out,
-                        uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, void* stream) {
-    if (!h_inv || !q_inv) return FRISK_E_INVALID;
-    const HostPlanes h{h_codes, h_inv, nullptr, nullptr, 0, h_low, h_padded_len};
-    const HostPlanes q{q_codes, q_inv, nullptr, nullptr, 0, q_low, q_padded_len};
-    const bool same = (h_codes == q_codes) && (h_inv == q_inv) && (h_padded_len == q_padded_len);
-    return run_host_impl(PeerArgs(), h, q, same, win_off, win_len, n_win, max_win_len, kmin, kmax, mask_host, want_rip, genome_space,
-                         rows_out, status_out, tables_out, valid_kmax_out, stream);
-}
-
-int frisk_b200_run_host_sparse(const uint32_t* h_codes, const uint32_t* h_inv_idx, const uint32_t* h_inv_val, uint64_t h_inv_n,
-                               const uint32_t* h_low, uint64_t h_padded_len, const uint32_t* q_codes,
-                               const uint32_t* q_inv_idx, const uint32_t* q_inv_val, uint64_t q_inv_n, const uint32_t* q_low,
-                               uint64_t q_padded_len, const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win,
-                               uint32_t max_win_len, int kmin, int kmax, int mask_host, int want_rip, int64_t genome_space,
-                               double* rows_out, uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out,
-                               void* stream) {
-    if ((h_inv_n && (!h_inv_idx || !h_inv_val)) || (q_inv_n && (!q_inv_idx || !q_inv_val))) return FRISK_E_INVALID;
-    if (h_padded_len / 32 > 0xffffffffull || q_padded_len / 32 > 0xffffffffull) return FRISK_E_UNSUPPORTED;   // 32-bit word indices
-    const HostPlanes h{h_codes, nullptr, h_inv_idx, h_inv_val, h_inv_n, h_low, h_padded_len};
-    const HostPlanes q{q_codes, nullptr, q_inv_idx, q_inv_val, q_inv_n, q_low, q_padded_len};
-    const bool same = (h_codes == q_codes) && (h_inv_idx == q_inv_idx) && (h_inv_n == q_inv_n) && (h_padded_len == q_padded_len);
-    return run_host_impl(PeerArgs(), h, q, same, win_off, win_len, n_win, max_win_len, kmin, kmax, mask_host, want_rip, genome_space,
-                         rows_out, status_out, tables_out, valid_kmax_out, stream);
-}
-
-int frisk_b200_run_host_peers(const uint32_t* h_codes, const uint32_t* h_inv_idx, const uint32_t* h_inv_val, uint64_t h_inv_n,
-                              const uint32_t* h_low, uint64_t h_padded_len, const uint64_t* win_off, const uint32_t* win_len,
-                              uint64_t n_win, uint32_t max_win_len, int kmin, int kmax, int mask_host, int want_rip,
-                              int64_t genome_space, uint64_t* d_fwd_local, const uint64_t* const* d_fwd_peers,
-                              uint64_t* const* d_flag_peers, int rank, int world, uint64_t epoch, double* rows_out,
-                              uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, void* stream) {
-    if ((h_inv_n && (!h_inv_idx || !h_inv_val)) || world < 1 || rank < 0 || rank >= world || !d_fwd_local || !d_fwd_peers ||
-        !d_flag_peers || epoch == 0)
-        return FRISK_E_INVALID;
-    if (h_padded_len / 32 > 0xffffffffull || kmax > FRISK_B200_FAST_K || world > kMaxPeers) return FRISK_E_UNSUPPORTED;
-    const HostPlanes h{h_codes, nullptr, h_inv_idx, h_inv_val, h_inv_n, h_low, h_padded_len};
-    PeerArgs peers;
-    peers.d_fwd_local = d_fwd_local; peers.d_fwd_peers = d_fwd_peers; peers.d_flag_peers = d_flag_peers;
-    peers.rank = rank; peers.world = world; peers.epoch = epoch;
-    return run_host_impl(peers, h, h, true, win_off, win_len, n_win, max_win_len, kmin, kmax, mask_host, want_rip, genome_space,
-                         rows_out, status_out, tables_out, valid_kmax_out, stream);
-}
-
-int frisk_b200_run_resident(const uint32_t* d_h_codes, const uint32_t* d_h_inv, const uint32_t* d_h_low,
-                            uint64_t h_padded_len, const uint32_t* d_q_codes, const uint32_t* d_q_inv,
-                            const uint32_t* d_q_low, uint64_t q_padded_len, const uint64_t* win_off,
-                            const uint32_t* win_len, uint64_t n_win, uint32_t max_win_len, int kmin, int kmax,
-                            int mask_host, int want_rip, int64_t genome_space, double* rows_out, uint32_t* status_out,
-                            uint64_t* tables_out, uint64_t* valid_kmax_out, void* stream) {
-    if (!d_h_codes || !d_h_inv || !d_q_codes || !d_q_inv || (h_padded_len & 127) || (q_padded_len & 127) ||
-        h_padded_len < 128 || q_padded_len < 128)
-        return FRISK_E_INVALID;
-    if (n_win && (!win_off || !win_len || !rows_out || !status_out)) return FRISK_E_INVALID;
-    int rc = check_k(kmin, kmax);
-    if (rc) return rc;
-    if ((rc = check_windows(win_off, win_len, n_win, max_win_len, q_padded_len))) return rc;
-    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
-    int dev_ = 0;
-    CK(cudaGetDevice(&dev_));
-    std::lock_guard<std::mutex> lock(g_run_mu[dev_ & 63]);
-    void* dfwd;
-    if ((rc = ws_get(6, ((size_t)frisk_b200_table_size(1, kmax) + 1) * 8, &dfwd))) return rc;
-    RunMarks* tm = nullptr;
-    if ((rc = run_marks(&tm))) return rc;
-    if ((rc = mark(tm, kTmStart, (cudaStream_t)stream))) return rc;
-    rc = run_tail(PeerArgs(), d_h_codes, d_h_inv, d_h_low, h_padded_len, false, d_q_codes, d_q_inv, d_q_low, win_off, win_len, n_win,
-                  max_win_len, kmin, kmax, mask_host, want_rip, genome_space, rows_out, status_out, tables_out,
-                  valid_kmax_out, dfwd, (cudaStream_t)stream, nullptr, nullptr, nullptr, tm);
-    if (rc) { cudaStreamSynchronize((cudaStream_t)stream); cudaGetLastError(); }   // queued copies still target the caller's buffers
-    return rc;
-}
-
-// ---- FASTA text in, rows out, one call -------------------------------------------------------------------------------
-// The text goes up in chunks; each chunk is tokenised, laid out, packed and (kmax <= 8) counted on the device while the
-// next one is on the bus (frisk_ingest.cu).  The host sees the record table as soon as the last chunk is tokenised, derives
-// names and windows while that chunk is still being packed and counted, and queues tables -> IVOM -> window kernel behind it.
-namespace {
-struct HostStage { void* p = nullptr; size_t cap = 0; };
-HostStage g_stage[64][2];        // pinned staging of the window list (off, len), grown on demand
-
-int stage_get(int dev, int slot, size_t bytes, void** out) {
-    HostStage& s = g_stage[dev & 63][slot];
-    if (s.cap < bytes) {
-        if (s.p) CK(cudaFreeHost(s.p));
-        s.p = nullptr; s.cap = 0;
-        const size_t want = bytes + bytes / 2 + 4096;
-        CK(cudaHostAlloc(&s.p, want, cudaHostAllocDefault));
-        s.cap = want;
-    }
-    *out = s.p;
-    return FRISK_OK;
-}
-
-// bgzf: h_text / q_text are BGZF buffers, inflated on the device by the ingest (frisk_b200_run_fasta_bgzf)
-int run_fasta_body(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step, int scaffolds_all,
-                   int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
-                   uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out, frisk_b200_fasta** host_out,
-                   frisk_b200_fasta** query_out, cudaStream_t st, int dev) {
-    int rc;
-    CopyCtx* cc = nullptr;
-    if ((rc = copy_ctx(&cc))) return rc;
-    RunMarks* tm = nullptr;
-    if ((rc = run_marks(&tm))) return rc;
-    if ((rc = mark(tm, kTmStart, st))) return rc;
-    const size_t tsz = (size_t)frisk_b200_table_size(1, kmax);
-    void* dfwd;
-    if ((rc = ws_get(6, (tsz + 1) * 8, &dfwd))) return rc;
-    CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, st));
-
-    frisk_internal::IngestSink sink;
-    if (kmax <= FRISK_B200_FAST_K)
-        sink.on_range = [&](const uint32_t* c, const uint32_t* i, const uint32_t* l, const unsigned long long* d_range,
-                            uint64_t hint, cudaStream_t s2) {
-            return frisk_internal::background_device_range(c, i, l, d_range, hint, kmax, mask_host, (uint64_t*)dfwd, s2);
-        };
-    sink.abandon = [&](cudaStream_t s2) {
-        CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, s2));
-        return (int)FRISK_OK;
-    };
-    sink.uploaded_mark = tm->ev[kTmUploaded];
-    const bool same = !q_text || (q_text == h_text && q_n == h_n);
-
-    // ---- the device-only tail: with the nibble kernel (kmax 7, 8; windows <= 8,186 bases) everything behind the ingest is queued
-    // from inside the open, before the host has seen the record table -- genome space and window list by frisk_windows.cu,
-    // the window count read by the window kernel from device memory -- so that no launch waits for the host.  If the
-    // streamed open has to be redone (sink.counted comes back false), what was queued here ran on provisional data into
-    // the caller's row buffers (inside their capacity) and is simply done again by the host-driven tail below.
-    const double min_size = (double)w + (((double)w * 0.75) - (double)step);
-    const uint32_t len_bound = (uint32_t)std::min<double>(4.0e9, std::max<double>((double)w, scaffolds_all ? min_size : 0.0));
-    WinPlan tail_plan;
-    const bool dev_tail = rows_cap > 0 && rows_cap <= 0xffffffffull && (uint64_t)w <= FRISK_B200_MAX_WINDOW &&
-                          frisk_internal::plan_score(kmin, kmax, len_bound, false, &tail_plan) == FRISK_OK &&
-                          tail_plan.kind == WinKernel::Nibble && !getenv("FRISK_RUN_FASTA_HOST_TAIL");
-    void *dtab = nullptr, *dig = nullptr, *dwin = nullptr, *dfirst = nullptr, *dscal = nullptr;
-    bool tail_queued = false;
-    double* k_rows = rows_out;
-    uint32_t* k_stat = status_out;
-    bool rows_direct = false;
-    if (dev_tail) {
-        if ((rc = ws_get(7, (tsz + 1) * 8, &dtab))) return rc;
-        if ((rc = ws_get(8, (size_t)pow4(kmax) * 16, &dig))) return rc;
-        if ((rc = ws_get(9, rows_cap * 12, &dwin))) return rc;
-        if ((rc = ws_get(20, 64, &dscal))) return rc;              // [0] number of windows, [1] genome space
-        rows_direct = pinned_views(rows_out, status_out, &k_rows, &k_stat);
-        if (!rows_direct) {
-            void *drows, *dstat;
-            if ((rc = ws_get(11, rows_cap * 40, &drows))) return rc;
-            if ((rc = ws_get(12, rows_cap * 4, &dstat))) return rc;
-            k_rows = (double*)drows; k_stat = (uint32_t*)dstat;
-        }
-    }
-    const uint32_t* win_codes[3] = {nullptr, nullptr, nullptr};      // planes of the genome whose windows are scored
-    auto queue_windows_and_score = [&](frisk_b200_fasta* h, bool with_space, cudaStream_t s2) -> int {
-        const unsigned long long *d_len, *d_off, *d_ctr;
-        uint64_t rec_cap = 0;
-        int rc2;
-        if ((rc2 = frisk_internal::fasta_device_table(h, &d_len, &d_off, &d_ctr, &rec_cap, &win_codes[0], &win_codes[1], &win_codes[2])))
-            return rc2;
-        if ((rc2 = ws_get(19, (rec_cap + 2) * 8, &dfirst))) return rc2;
-        unsigned long long* const scal = (unsigned long long*)dscal;
-        if ((rc2 = frisk_internal::windows_device(d_len, d_off, d_ctr + frisk_internal::kIngestRecords, d_ctr + frisk_internal::kIngestOverflow,
-                                                  d_ctr + frisk_internal::kIngestNonUpper, rec_cap, w, step, scaffolds_all, rows_cap,
-                                                  (unsigned long long*)dfirst, (unsigned long long*)dwin,
-                                                  (uint32_t*)((unsigned long long*)dwin + rows_cap), scal,
-                                                  with_space ? (long long*)(scal + 1) : nullptr, s2)))
-            return rc2;
-        return FRISK_OK;
-    };
-    auto queue_finalize = [&](cudaStream_t s2) -> int {
-        const LocalFwd f{reinterpret_cast<const unsigned long long*>(dfwd), (const long long*)((unsigned long long*)dscal + 1)};
-        uint64_t* dvalid = (uint64_t*)dtab + tsz;
-        int rc2 = [&]() -> int { DISPATCH_K(kmax, (launch_finalize_ivom<K, LocalFwd>(f, kmin, 0, (uint64_t*)dtab, dvalid, (double*)dig, s2))); }();
-        if (rc2) return rc2;
-        if ((rc2 = mark(tm, kTmFinalised, s2))) return rc2;
-        // the genome tables (0.7 MB) go back on the copy stream while the window kernel runs
-        CK(cudaEventRecord(cc->ev[kMaxChunks + 2], s2));
-        CK(cudaStreamWaitEvent(cc->copy, cc->ev[kMaxChunks + 2], 0));
-        if (tables_out) CK(cudaMemcpyAsync(tables_out, dtab, tsz * 8, cudaMemcpyDeviceToHost, cc->copy));
-        if (valid_kmax_out) CK(cudaMemcpyAsync(valid_kmax_out, dvalid, 8, cudaMemcpyDeviceToHost, cc->copy));
-        return FRISK_OK;
-    };
-    auto queue_score = [&](cudaStream_t s2) -> int {
-        int rc2;
-        if ((rc2 = mark(tm, kTmScoreStart, s2))) return rc2;
-        rc2 = frisk_internal::score_nibble(tail_plan, win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
-                                           (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound, (const double*)dig,
-                                           kmin, kmax, want_rip && kmin <= 2 && kmax >= 2 /* as frisk_b200_score: RIP needs orders 1 and 2 */,
-                                           k_rows, k_stat, nullptr, s2, (const unsigned long long*)dscal);
-        if (rc2) return rc2;
-        tail_queued = true;
-        return mark(tm, kTmScored, s2);
-    };
-    if (dev_tail)
-        sink.on_complete = [&](frisk_b200_fasta* h, cudaStream_t s2) -> int {
-            int rc2;
-            if ((rc2 = mark(tm, kTmCounted, s2))) return rc2;
-            // genome space of the host genome (and, when it is the scored genome too, its window list), tables, IVOM, score
-            if ((rc2 = queue_windows_and_score(h, true, s2))) return rc2;
-            if ((rc2 = queue_finalize(s2))) return rc2;
-            return same ? queue_score(s2) : FRISK_OK;
-        };
-    g_trace.stamp("call");
-    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, bgzf, st, &sink, host_out))) return rc;
-    g_trace.stamp("open_returned");
-    tm->have[kTmUploaded] = h_n > 0;                                // (recorded behind the last text chunk)
-    const bool counted = sink.counted;
-    bool tail_ok = dev_tail && counted && (tail_queued || !same);   // (an exact re-open leaves counted == false)
-    if (!tail_ok) tm->have[kTmFinalised] = tm->have[kTmScoreStart] = tm->have[kTmScored] = false;
-    if (counted && !dev_tail && (rc = mark(tm, kTmCounted, st))) return rc;
-    frisk_b200_fasta* hh = *host_out;
-    frisk_b200_fasta* qh = hh;
-    if (!same) {
-        frisk_internal::IngestSink qsink;                            // planes only: nothing of the query is counted
-        bool q_queued = false;
-        if (tail_ok)
-            qsink.on_complete = [&](frisk_b200_fasta* h, cudaStream_t s2) -> int {
-                int rc2;
-                if ((rc2 = queue_windows_and_score(h, false, s2))) return rc2;
-                if ((rc2 = queue_score(s2))) return rc2;
-                q_queued = true;
-                return FRISK_OK;
-            };
-        qsink.counted = false;
-        if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, bgzf, st, &qsink, query_out))) return rc;
-        qh = *query_out;
-        // (qsink has no on_range, so `counted` says nothing: a query that was re-opened exactly has a handle without the
-        // speculative table the hook used -- detect it by the hook not having run or the open statistics)
-        tail_ok = tail_ok && q_queued && frisk_internal::fasta_open_was_streamed(qh);
-    }
-    uint64_t h_rec = 0, h_padded = 0, h_stats[3], q_rec = 0, q_padded = 0, q_stats[3];
-    if ((rc = frisk_b200_fasta_info(hh, &h_rec, &h_padded, h_stats))) return rc;
-    if ((rc = frisk_b200_fasta_info(qh, &q_rec, &q_padded, q_stats))) return rc;
-    const uint32_t *dhc, *dhi, *dhl, *dqc, *dqi, *dql;
-    if ((rc = frisk_b200_fasta_planes(hh, &dhc, &dhi, &dhl))) return rc;
-    if ((rc = frisk_b200_fasta_planes(qh, &dqc, &dqi, &dql))) return rc;
-
-    // windows of the query (F:194-251), into pinned staging -- produced once the tables' finalisation is queued
-    const LateWindows late = [&](const uint64_t** win_off, const uint32_t** win_len, uint64_t* n_win, uint32_t* max_len) -> int {
-        int rc2;
-        std::vector<uint64_t> seq_len((size_t)q_rec), scaf_off((size_t)q_rec);
-        if ((rc2 = frisk_b200_fasta_records(qh, nullptr, nullptr, seq_len.data(), scaf_off.data()))) return rc2;
-        void *wo = nullptr, *wl = nullptr;
-        if ((rc2 = stage_get(dev, 0, (rows_cap + 1) * 12, &wo))) return rc2;
-        if ((rc2 = stage_get(dev, 1, (rows_cap + 1) * 4, &wl))) return rc2;
-        uint64_t nw = 0;
-        rc2 = frisk_b200_windows(seq_len.data(), scaf_off.data(), q_rec, w, step, scaffolds_all, rows_cap, (uint64_t*)wo, (uint32_t*)wl,
-                                 nullptr, nullptr, nullptr, &nw);
-        if (n_win_out) *n_win_out = nw;
-        if (rc2) return rc2;                                         // (FRISK_E_CAPACITY: more windows than rows_cap)
-        uint32_t mx = 0;
-        uint32_t* const packed = (uint32_t*)((uint64_t*)wo + nw);    // the lengths move right behind the offsets: one H2D copy
-        for (uint64_t i = 0; i < nw; ++i) {
-            const uint32_t l = ((const uint32_t*)wl)[i];
-            packed[i] = l;
-            mx = l > mx ? l : mx;
-        }
-        *win_off = (const uint64_t*)wo; *win_len = packed; *n_win = nw; *max_len = mx;
-        return FRISK_OK;
-    };
-    if (tail_ok) {
-        // everything is queued: bring the tables and the window count back, wait, check the capacity
-        void* h_scal = nullptr;
-        if ((rc = stage_get(dev, 1, 64, &h_scal))) return rc;
-        if (!rows_direct) {                                          // pageable result buffers: the rows come back by copy
-            CK(cudaMemcpyAsync(rows_out, k_rows, rows_cap * 40, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(status_out, k_stat, rows_cap * 4, cudaMemcpyDeviceToHost, st));
-        }
-        CK(cudaMemcpyAsync(h_scal, dscal, 16, cudaMemcpyDeviceToHost, st));
-        if ((rc = mark(tm, kTmEnd, st))) return rc;
-        CK(cudaStreamSynchronize(st));
-        CK(cudaStreamSynchronize(cc->copy));                         // the tables came back beside the window kernel
-        g_trace.stamp("done");
-        g_trace.flush();
-        const uint64_t n_win = ((const uint64_t*)h_scal)[0];
-        if (n_win_out) *n_win_out = n_win;
-        if ((int64_t)((const uint64_t*)h_scal)[1] != (int64_t)h_stats[0] - (int64_t)h_stats[1]) return FRISK_E_CUDA;   // (cannot happen)
-        return n_win > rows_cap ? FRISK_E_CAPACITY : FRISK_OK;
-    }
-    CK(cudaEventRecord(cc->ev[kMaxChunks], st));                    // the copy stream joins behind the ingest
-    CK(cudaStreamWaitEvent(cc->copy, cc->ev[kMaxChunks], 0));
-    return run_tail(PeerArgs(), dhc, dhi, dhl, h_padded, counted, dqc, dqi, dql, nullptr, nullptr, 0, 0, kmin, kmax, mask_host, want_rip,
-                    (int64_t)h_stats[0] - (int64_t)h_stats[1], rows_out, status_out, tables_out, valid_kmax_out, dfwd, st, cc->copy,
-                    cc->ev[kMaxChunks + 1], cc->ev[kMaxChunks + 2], tm, &late);
-}
-
-// frisk_b200_run_fasta and frisk_b200_run_fasta_bgzf
-int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step, int scaffolds_all,
-                  int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
-                  uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
-                  frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    if (!host_out || !query_out || (!h_text && h_n) || (!q_text && q_n) || (rows_cap && (!rows_out || !status_out)))
-        return FRISK_E_INVALID;
-    *host_out = *query_out = nullptr;
-    if (n_win_out) *n_win_out = 0;
-    int rc = check_k(kmin, kmax);
-    if (rc) return rc;
-    if (w < 1 || step < 1) return FRISK_E_INVALID;
-    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    std::lock_guard<std::mutex> lock(g_run_mu[dev & 63]);
-    cudaStream_t st = (cudaStream_t)stream;
-    bool threw = false;
-    try {
-        rc = run_fasta_body(h_text, h_n, q_text, q_n, bgzf, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
-                            status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, st, dev);
-    } catch (...) {
-        rc = FRISK_E_CAPACITY;
-        threw = true;
-    }
-    if (rc != FRISK_OK) {                                           // queued work still targets the caller's buffers
-        cudaStreamSynchronize(st);
-        if (g_copy[dev & 63].copy) cudaStreamSynchronize(g_copy[dev & 63].copy);
-        cudaGetLastError();
-        if (rc != FRISK_E_CAPACITY || threw) {                      // (too few rows: the handles stay, with their planes)
-            if (*query_out) frisk_b200_fasta_close(*query_out, st);
-            if (*host_out) frisk_b200_fasta_close(*host_out, st);
-            *host_out = *query_out = nullptr;
-        }
-    }
-    return rc;
-}
-
-}  // namespace
-
-int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, int w, int step, int scaffolds_all,
-                         int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
-                         uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
-                         frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_text, h_n, q_text, q_n, false, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
-                         status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
-}
-
-int frisk_b200_run_fasta_bgzf(const char* h_gz, uint64_t h_n, const char* q_gz, uint64_t q_n, int w, int step, int scaffolds_all,
-                              int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
-                              uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
-                              frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_gz, h_n, q_gz, q_n, true, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
-                         status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
-}
-
-// Stage times (ms) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call on the current device,
-// from events recorded on its streams: [0] upload of the planes finished, [1] background count finished, [2] tables
-// finalised + genome IVOM table (multi-GPU: includes the wait for the peers' counters), [3] window kernel(s) finished,
-// [4] results on the host -- each since the start of the call -- and [5] the moment the window kernel could start
-// (everything it waits for is done and its launch has reached the device).  A mark the call did not set
-// (run_resident has no upload) reads -1.
-int frisk_b200_last_run_timing(float* ms, int cap, int* n) {
-    if (!ms || cap < 1) return FRISK_E_INVALID;
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    RunMarks& m = g_marks[dev & 63];
-    if (!m.ready || !m.have[kTmStart] || !m.have[kTmEnd]) return FRISK_E_INVALID;
-    CK(cudaEventSynchronize(m.ev[kTmEnd]));
-    const int order[6] = {kTmUploaded, kTmCounted, kTmFinalised, kTmScored, kTmEnd, kTmScoreStart};
-    int k = 0;
-    for (; k < 6 && k < cap; ++k) {
-        ms[k] = -1.0f;
-        if (!m.have[order[k]]) continue;
-        if (order[k] == kTmUploaded) CK(cudaEventSynchronize(m.ev[kTmUploaded]));
-        CK(cudaEventElapsedTime(&ms[k], m.ev[kTmStart], m.ev[order[k]]));
-    }
-    if (n) *n = k;
-    return FRISK_OK;
-}
-
-int frisk_b200_release_workspace(void) {
-    int dev = 0;
-    CK(cudaGetDevice(&dev));
-    Workspace& w = g_ws[dev & 63];
-    for (int i = 0; i < 32; ++i) {
-        if (w.buf[i]) CK(cudaFree(w.buf[i]));
-        w.buf[i] = nullptr; w.cap[i] = 0;
-    }
     return FRISK_OK;
 }
 
