@@ -352,10 +352,10 @@ def score_genome(args, device="cuda:0") -> engine.HotPathResult:
     # (the reference reads each file three times in Python: F:170, F:203, F:297)
     # ... and everything goes through the C ABI alone (DevBuf planes, one frisk_b200_run_resident call): PyTorch is
     # never imported on this path -- its import takes several seconds, the run itself milliseconds
-    # A BGZF file (bgzip, samtools) goes up compressed and is inflated on the device; any other .gz is inflated on the host.
+    # A BGZF file (bgzip, samtools) or a single gzip member (gzip, pigz) goes up compressed and is inflated on the device;
+    # a multi-member .gz is inflated on the host.
     def ingest(path):
-        buf, bgzf = engine.read_genome_file(path)
-        return (engine.DeviceGenome.from_bgzf_bytes_native if bgzf else engine.DeviceGenome.from_fasta_bytes_native)(buf, device)
+        return engine.open_genome_file(path, lambda buf, kind: engine.DeviceGenome._open_native(buf, device, kind))
     host = ingest(args.hostSeq)
     query = host if not args.querySeq or args.querySeq == args.hostSeq else ingest(args.querySeq)
     res = engine.run_resident(query, host if query is not host else None, kmin=args.minWordSize, kmax=args.maxWordSize,

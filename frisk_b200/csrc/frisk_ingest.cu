@@ -23,6 +23,8 @@
 // with exact sizes (open_any).  The planes belong to the handle.
 // A BGZF source (frisk_b200_fasta_open_bgzf, frisk_b200_run_fasta_bgzf) shares all of it: the compressed bytes go up on the
 // upload lane, frisk_bgzf.cu inflates them into the text buffer, and the passes wait on that instead of on the text's copy.
+// A gzip source (frisk_b200_fasta_open_gzip, frisk_b200_run_fasta_gzip) is inflated first (frisk_gzip.cu synchronises: its
+// text length is only known at the end) and the open takes over the text buffer it filled, as the BGZF exact re-open does.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -677,11 +679,11 @@ struct frisk_b200_fasta {
     void *d_scan_slab = nullptr, *d_out_slab = nullptr;                  // what the pointers above (but d_text) are carved from
     uint64_t rec_cap = 0;                                                // entries of the device record table
     bool streamed = false;                                               // opened on the chunked, speculatively sized path
-    bool bgzf = false;                                                   // opened from BGZF: names index name_text
+    bool device_text = false;                                            // opened from BGZF or gzip: names index name_text
     void* d_gz_slab = nullptr;                                           // BGZF: compressed bytes, block table, status words
     std::vector<uint64_t> name_off, seq_len, scaf_off, hdr_pos;
     std::vector<uint32_t> name_len;
-    std::vector<char> name_text;                                         // BGZF: the header lines, one after the other
+    std::vector<char> name_text;                                         // BGZF / gzip: the header lines, one after the other
 };
 
 namespace {
@@ -736,19 +738,48 @@ int upload_lane(UploadLane** out) {
     return FRISK_OK;
 }
 
-// What an open reads: a host text, or a BGZF buffer with its block table (the text is inflated on the device).
+// What an open reads: a host text, a BGZF buffer with its block table, or a gzip member (the text is inflated on the device).
 struct Source {
-    const char* text = nullptr;           // host text (nullptr for BGZF)
-    uint64_t n = 0;                       // text bytes (BGZF: inflated)
-    bool bgzf = false;
+    const char* text = nullptr;           // host text (nullptr for BGZF and gzip)
+    uint64_t n = 0;                       // text bytes (BGZF, gzip: inflated)
+    bool bgzf = false, gzip = false;
     const uint8_t* gz = nullptr;
     uint64_t gz_n = 0, n_blocks = 0;
     std::vector<uint64_t> table;          // per block: comp_off, text_off (8 bytes each), comp_len, crc (4 bytes each)
-    uint8_t* d_ready = nullptr;           // the exact re-open: the text the first attempt inflated (the handle takes it)
+    uint8_t* d_ready = nullptr;           // gzip, the exact re-open: the text inflated already (the handle takes it)
+    bool device() const { return bgzf || gzip; }   // the text exists on the device only
 };
 
-int make_source(const char* text, uint64_t n, bool bgzf, Source* src) {
-    if (!bgzf) { src->text = text; src->n = n; return FRISK_OK; }
+// the text buffer of an open: kTile-padded, '\n' behind the text
+int alloc_text(uint64_t n, cudaStream_t st, uint8_t** out) {
+    const uint64_t padded_text = (n + kTile - 1) / kTile * kTile + 16;
+    FRISK_CK(cudaMallocAsync((void**)out, padded_text, st));
+    FRISK_CK(cudaMemsetAsync(*out + n, '\n', padded_text - n, st));
+    return FRISK_OK;
+}
+
+// gzip: the member goes up and is inflated into a text buffer of its own (src->d_ready)
+int gzip_source(const char* gz, uint64_t n, cudaStream_t st, Source* src) {
+    src->gzip = true;
+    uint8_t* d_gz = nullptr;
+    FRISK_CK(cudaMallocAsync((void**)&d_gz, n ? n : 1, st));
+    auto alloc = [&](uint64_t len, uint8_t** out) -> int {
+        *out = nullptr;
+        if (!len) return FRISK_OK;                        // no text: the open's empty path
+        const int rc = alloc_text(len, st, out);
+        src->d_ready = *out;
+        return rc;
+    };
+    const cudaError_t e = cudaMemcpyAsync(d_gz, gz, n, cudaMemcpyHostToDevice, st);
+    int rc = e == cudaSuccess ? frisk_internal::gzip_inflate(d_gz, reinterpret_cast<const uint8_t*>(gz), n, alloc, &src->n, nullptr, st)
+                              : frisk_internal::cuda_fail(e, "cudaMemcpyAsync(d_gz)");
+    cudaFreeAsync(d_gz, st);                              // (every exit; a failed text buffer is freed by open_handle)
+    return rc;
+}
+
+int make_source(const char* text, uint64_t n, frisk_internal::TextFormat fmt, cudaStream_t st, Source* src) {
+    if (fmt == frisk_internal::kFmtGzip) return gzip_source(text, n, st, src);
+    if (fmt != frisk_internal::kFmtBgzf) { src->text = text; src->n = n; return FRISK_OK; }
     src->bgzf = true;
     src->gz = reinterpret_cast<const uint8_t*>(text);
     src->gz_n = n;
@@ -836,7 +867,7 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
     const char* const text = src.text;
     const uint64_t n = src.n;
     h->n = n;
-    h->bgzf = src.bgzf;
+    h->device_text = src.device();
     unsigned int* d_any_bad = nullptr;                                  // BGZF: some member failed to inflate
     h->n_tiles = n ? (n + kTile - 1) / kTile : 0;
     if (h->n_tiles > 0x7fffffffull) return FRISK_E_UNSUPPORTED;         // 8 TB of text per call
@@ -882,15 +913,12 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
             FRISK_CK(cudaMemcpyAsync(&bad, d_any_bad, 4, cudaMemcpyDeviceToHost, st));
             FRISK_CK(cudaStreamSynchronize(st));
             if (bad) return FRISK_E_FORMAT;
+        } else if (src.gzip && sink && sink->uploaded_mark) {          // (inflated before the open)
+            FRISK_CK(cudaEventRecord(sink->uploaded_mark, st));
         }
     } else {
-        const uint64_t padded_text = T * kTile + 16;
-        if (src.d_ready) {
-            h->d_text = src.d_ready;                                    // (its padding is in place)
-        } else {
-            FRISK_CK(cudaMallocAsync((void**)&h->d_text, padded_text, st));
-            FRISK_CK(cudaMemsetAsync(h->d_text + n, '\n', padded_text - n, st));
-        }
+        if (src.d_ready) h->d_text = src.d_ready;                      // (its padding is in place)
+        else if ((rc = alloc_text(n, st, &h->d_text))) return rc;
         // Chunk plan (tile bounds, multiples of kSP): equal chunks of >= 1400 tiles (5.6 MiB; ingest_chunk_tiles overrides), at most
         // kMaxChunks.  Measured on C2 (40.8 MB, 52 GB/s over PCIe): beside a running H2D copy the three passes + count of a
         // chunk take about as long as the chunk's copy, and every launch of a short chunk costs ~10 us whatever its size, so
@@ -904,7 +932,7 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
         if (!exact) {
             auto round_sp = [](uint64_t v) { return (v + kSP - 1) / kSP * kSP; };
             const uint64_t min_tiles = frisk_internal::g_ingest_chunk_tiles > 0 ? (uint64_t)frisk_internal::g_ingest_chunk_tiles : kMinChunkTiles;
-            const uint64_t want = src.bgzf && frisk_internal::g_ingest_chunk_tiles <= 0
+            const uint64_t want = src.device() && frisk_internal::g_ingest_chunk_tiles <= 0
                                       ? 1 : std::max<uint64_t>(1, std::min<uint64_t>(kMaxChunks, T / min_tiles));
             const uint64_t per = round_sp((T + want - 1) / want);
             n_chunks = 0;
@@ -926,7 +954,7 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
         };
         tmark(st);
         auto issue_copy = [&](int c) -> int {
-            if (src.bgzf) return FRISK_OK;                              // (uploaded and inflated below, all chunks at once)
+            if (src.device()) return FRISK_OK;                          // (inflated already or below, all chunks at once)
             const uint64_t b0 = bound[c] * kTile, b1 = std::min<uint64_t>(bound[c + 1] * kTile, n);
             FRISK_CK(cudaMemcpyAsync(h->d_text + b0, text + b0, b1 - b0, cudaMemcpyHostToDevice, lane->copy));
             FRISK_CK(cudaEventRecord(lane->done[c], lane->copy));
@@ -936,9 +964,9 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
         // page-locked text: every copy is queued before anything else is set up (the first byte leaves ~20 us earlier);
         // pageable text: a copy returns when its chunk is staged, so each one is issued just before its chunk's passes
         cudaPointerAttributes pa{};
-        const bool pinned = !src.bgzf && cudaPointerGetAttributes(&pa, text) == cudaSuccess && pa.type == cudaMemoryTypeHost;
+        const bool pinned = !src.device() && cudaPointerGetAttributes(&pa, text) == cudaSuccess && pa.type == cudaMemoryTypeHost;
         cudaGetLastError();
-        if (src.bgzf) {
+        if (src.device()) {
             if (!src.d_ready && (rc = bgzf_upload_inflate(h, src, st, lane->copy, &d_any_bad))) return rc;
             for (int c = 0; c <= last_chunk; ++c) FRISK_CK(cudaEventRecord(lane->done[c], lane->copy));
             if (sink && sink->uploaded_mark) FRISK_CK(cudaEventRecord(sink->uploaded_mark, lane->copy));
@@ -957,7 +985,7 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
         for (int c = 0; c <= last_chunk; ++c) {
             const uint64_t t0 = bound[c], t1 = bound[c + 1];
             const uint64_t b1 = std::min<uint64_t>(t1 * kTile, n);
-            const uint64_t avail = src.bgzf ? n : b1;                   // bytes on the device when the chunk's passes run
+            const uint64_t avail = src.device() ? n : b1;               // bytes on the device when the chunk's passes run
             const bool final = c == last_chunk;
             if (!pinned || trace) {
                 if ((rc = issue_copy(c))) return rc;
@@ -1037,7 +1065,7 @@ int open_impl(frisk_b200_fasta* h, const Source& src, cudaStream_t st, bool exac
     // names (F:156) and the 128-base aligned layout
     const uint64_t R = h->n_rec;
     h->name_off.resize(R); h->name_len.resize(R); h->scaf_off.resize(R);
-    if (src.bgzf) {
+    if (src.device()) {
         if (h->d_gz_slab) FRISK_CK(cudaFreeAsync(h->d_gz_slab, st));    // (the inflate is behind the synchronisation above)
         h->d_gz_slab = nullptr;
         // beside the tail run_fasta may have queued on `st`: on the upload lane, which follows the last chunk's pack
@@ -1069,30 +1097,32 @@ int open_any(frisk_b200_fasta* h, Source& src, cudaStream_t st, frisk_internal::
         g_open_stats[1].fetch_add(1);
         FRISK_CK(cudaStreamSynchronize(st));                            // (the abandoned attempt's work targets what is freed next)
         if (sink && sink->abandon && (rc = sink->abandon(st))) return rc;
-        if (src.bgzf) { src.d_ready = h->d_text; h->d_text = nullptr; }  // inflated once: the re-open keeps the text
+        if (src.device()) { src.d_ready = h->d_text; h->d_text = nullptr; }   // inflated once: the re-open keeps the text
         if ((rc = free_all(h, st))) return rc;
         *h = frisk_b200_fasta();
         rc = open_impl(h, src, st, true, nullptr);
-        if (src.bgzf && !h->d_text && src.d_ready) FRISK_CK(cudaFreeAsync(src.d_ready, st));   // (not taken over)
+        if (!h->d_text && src.d_ready) FRISK_CK(cudaFreeAsync(src.d_ready, st));   // (not taken over)
         src.d_ready = nullptr;
         if (sink) sink->counted = false;
     }
     return rc;
 }
 
-// the public opens and the one-call path: block table (BGZF), open with retry; no handle on failure
-int open_handle(const char* text, uint64_t n, bool bgzf, cudaStream_t st, frisk_internal::IngestSink* sink, frisk_b200_fasta** out) {
+// the public opens and the one-call path: block table (BGZF) or inflate (gzip), open with retry; no handle on failure
+int open_handle(const char* text, uint64_t n, frisk_internal::TextFormat fmt, cudaStream_t st, frisk_internal::IngestSink* sink,
+                frisk_b200_fasta** out) {
     *out = nullptr;
     frisk_b200_fasta* h = new (std::nothrow) frisk_b200_fasta();
     if (!h) return FRISK_E_INVALID;
     int rc;
+    Source src;
     try {                                                 // std::bad_alloc of the record table: nothing crosses the ABI
-        Source src;
-        rc = make_source(text, n, bgzf, &src);
+        rc = make_source(text, n, fmt, st, &src);
         if (!rc) rc = open_any(h, src, st, sink);
     } catch (...) {
         rc = FRISK_E_CAPACITY;
     }
+    if (src.d_ready && h->d_text != src.d_ready) cudaFreeAsync(src.d_ready, st);   // gzip: a text the handle did not take
     if (rc) {
         free_all(h, st);
         delete h;
@@ -1102,14 +1132,14 @@ int open_handle(const char* text, uint64_t n, bool bgzf, cudaStream_t st, frisk_
     return FRISK_OK;
 }
 
-// frisk_b200_fasta_open and frisk_b200_fasta_open_bgzf
-int open_public(const char* text, uint64_t n, bool bgzf, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
+// frisk_b200_fasta_open, _open_bgzf and _open_gzip
+int open_public(const char* text, uint64_t n, frisk_internal::TextFormat fmt, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
                 uint64_t* padded_len, uint64_t stats[3]) {
     if (!out || (!text && n)) return FRISK_E_INVALID;
     *out = nullptr;
     if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
     frisk_b200_fasta* h = nullptr;
-    const int rc = open_handle(text, n, bgzf, (cudaStream_t)stream, nullptr, &h);
+    const int rc = open_handle(text, n, fmt, (cudaStream_t)stream, nullptr, &h);
     if (rc) return rc;
     if (n_records) *n_records = h->n_rec;
     if (padded_len) *padded_len = h->padded_len;
@@ -1121,9 +1151,10 @@ int open_public(const char* text, uint64_t n, bool bgzf, void* stream, frisk_b20
 
 bool frisk_internal::fasta_open_was_streamed(const frisk_b200_fasta* h) { return h && h->streamed; }
 
-int frisk_internal::fasta_open_planes(const char* text, uint64_t n, bool bgzf, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out) {
+int frisk_internal::fasta_open_planes(const char* text, uint64_t n, TextFormat fmt, cudaStream_t st, IngestSink* sink,
+                                      frisk_b200_fasta** out) {
     if (!out || !sink || (!text && n)) return FRISK_E_INVALID;
-    return open_handle(text, n, bgzf, st, sink, out);
+    return open_handle(text, n, fmt, st, sink, out);
 }
 
 int frisk_internal::fasta_device_table(const frisk_b200_fasta* h, const unsigned long long** d_len, const unsigned long long** d_scaf_off,
@@ -1147,18 +1178,23 @@ int frisk_b200_fasta_info(const frisk_b200_fasta* h, uint64_t* n_records, uint64
 
 int frisk_b200_fasta_open(const char* text, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
                           uint64_t* padded_len, uint64_t stats[3]) {
-    return open_public(text, n, false, stream, out, n_records, padded_len, stats);
+    return open_public(text, n, frisk_internal::kFmtText, stream, out, n_records, padded_len, stats);
 }
 
 int frisk_b200_fasta_open_bgzf(const char* gz, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
                                uint64_t* padded_len, uint64_t stats[3]) {
-    return open_public(gz, n, true, stream, out, n_records, padded_len, stats);
+    return open_public(gz, n, frisk_internal::kFmtBgzf, stream, out, n_records, padded_len, stats);
+}
+
+int frisk_b200_fasta_open_gzip(const char* gz, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
+                               uint64_t* padded_len, uint64_t stats[3]) {
+    return open_public(gz, n, frisk_internal::kFmtGzip, stream, out, n_records, padded_len, stats);
 }
 
 int frisk_b200_fasta_name_text(const frisk_b200_fasta* h, const char** text, uint64_t* n) {
     if (!h || !text || !n) return FRISK_E_INVALID;
-    *text = h->bgzf ? h->name_text.data() : nullptr;
-    *n = h->bgzf ? h->name_text.size() : 0;
+    *text = h->device_text ? h->name_text.data() : nullptr;
+    *n = h->device_text ? h->name_text.size() : 0;
     return FRISK_OK;
 }
 

@@ -46,12 +46,19 @@ bool fasta_open_was_streamed(const frisk_b200_fasta* h);     // false: the handl
 int fasta_device_table(const frisk_b200_fasta* h, const unsigned long long** d_len, const unsigned long long** d_scaf_off,
                        const unsigned long long** d_counters, uint64_t* rec_cap, const uint32_t** d_codes, const uint32_t** d_inv,
                        const uint32_t** d_low);
-// bgzf = true: `text` / `n` are a BGZF buffer (frisk_b200_fasta_open_bgzf), inflated on the device into the text buffer
-int fasta_open_planes(const char* text, uint64_t n, bool bgzf, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out);
+// what the bytes handed to an open are: the text, a BGZF buffer (frisk_b200_fasta_open_bgzf) or one gzip member
+// (frisk_b200_fasta_open_gzip); compressed input is inflated on the device into the text buffer
+enum TextFormat : int { kFmtText = 0, kFmtBgzf = 1, kFmtGzip = 2 };
+int fasta_open_planes(const char* text, uint64_t n, TextFormat fmt, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out);
 // frisk_b200_bgzf_inflate's kernel (frisk_bgzf.cu); d_any_bad (nullable) receives a non-zero word when a member fails
 int bgzf_inflate(const uint8_t* d_gz, const uint64_t* d_comp_off, const uint32_t* d_comp_len, const uint32_t* d_crc,
                  const uint64_t* d_text_off, uint64_t n_blocks, uint64_t text_len, uint8_t* d_text, uint32_t* d_block_status,
                  unsigned int* d_any_bad, cudaStream_t st);
+// frisk_b200_gzip_inflate (frisk_gzip.cu) with the text buffer from alloc_text(text_len, &d_text), called once the length
+// is known; h_gz (nullable) is a host copy of the member, read instead of d_gz for the header and trailer.  Synchronises st.
+extern int g_gzip_chunk_bytes;                     // compressed bytes per nominal chunk (0 = default); frisk_b200_set_option
+int gzip_inflate(const uint8_t* d_gz, const uint8_t* h_gz, uint64_t n, const std::function<int(uint64_t, uint8_t**)>& alloc_text,
+                 uint64_t* text_len, uint64_t stats[4], cudaStream_t st);
 // background count of a word range that lives in device memory (frisk_kernels.cu); kmax <= FRISK_B200_FAST_K
 int background_device_range(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const unsigned long long* d_word_range,
                             uint64_t words_hint, int kmax, int mask_host, uint64_t* fwd, cudaStream_t st);

@@ -2022,6 +2022,7 @@ int frisk_b200_set_option(const char* name, int value) {
         }
     if (strcmp(name, "ingest_exact_open") == 0) { frisk_internal::g_ingest_exact = value; return FRISK_OK; }
     if (strcmp(name, "ingest_chunk_tiles") == 0) { frisk_internal::g_ingest_chunk_tiles = value; return FRISK_OK; }
+    if (strcmp(name, "gzip_chunk_bytes") == 0) { frisk_internal::g_gzip_chunk_bytes = value; return FRISK_OK; }
     return FRISK_E_INVALID;
 }
 

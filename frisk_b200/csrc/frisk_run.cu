@@ -1,5 +1,5 @@
 // frisk_b200 one-call run paths: host planes, resident planes or FASTA text in, rows out, in one C call
-// (frisk_b200_run_host / _sparse / _peers, frisk_b200_run_resident, frisk_b200_run_fasta / _bgzf).  Every path enters and
+// (frisk_b200_run_host / _sparse / _peers, frisk_b200_run_resident, frisk_b200_run_fasta / _bgzf / _gzip).  Every path enters and
 // leaves through RunCall (device lock, stage marks, error drain), finalises through queue_tables and ends in results.  The
 // per-device state they share lives here too: the workspace, the copy stream, the stage marks and the window staging.
 #include <cuda_runtime.h>
@@ -493,10 +493,10 @@ int stage_get(int dev, int slot, size_t bytes, void** out) {
     return FRISK_OK;
 }
 
-// bgzf: h_text / q_text are BGZF buffers, inflated on the device by the ingest (frisk_b200_run_fasta_bgzf)
-int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step,
-                   int scaffolds_all, const Job& j, uint64_t rows_cap, uint64_t* n_win_out, frisk_b200_fasta** host_out,
-                   frisk_b200_fasta** query_out) {
+// fmt: h_text / q_text are texts, BGZF buffers or gzip members (the last two inflated on the device by the ingest)
+int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt,
+                   int w, int step, int scaffolds_all, const Job& j, uint64_t rows_cap, uint64_t* n_win_out,
+                   frisk_b200_fasta** host_out, frisk_b200_fasta** query_out) {
     const int kmin = j.kmin, kmax = j.kmax;
     const size_t tsz = table_words(kmax);
     void* dfwd;
@@ -574,7 +574,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
             return same ? queue_score(s2) : FRISK_OK;
         };
     g_trace.stamp("call");
-    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, bgzf, c.st, &sink, host_out))) return rc;
+    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, fmt, c.st, &sink, host_out))) return rc;
     g_trace.stamp("open_returned");
     c.tm->have[kTmUploaded] = h_n > 0;                              // (recorded behind the last text chunk)
     const bool counted = sink.counted;
@@ -595,7 +595,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
                 return FRISK_OK;
             };
         qsink.counted = false;
-        if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, bgzf, c.st, &qsink, query_out))) return rc;
+        if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, fmt, c.st, &qsink, query_out))) return rc;
         qh = *query_out;
         // (qsink has no on_range, so `counted` says nothing: a query that was re-opened exactly has a handle without the
         // speculative table the hook used -- detect it by the hook not having run or the open statistics)
@@ -648,9 +648,9 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
                     &late);
 }
 
-// frisk_b200_run_fasta and frisk_b200_run_fasta_bgzf
-int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, bool bgzf, int w, int step, int scaffolds_all,
-                  int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
+// frisk_b200_run_fasta, _run_fasta_bgzf and _run_fasta_gzip
+int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
+                  int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                   uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                   frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
     if (!host_out || !query_out || (!h_text && h_n) || (!q_text && q_n) || (rows_cap && (!rows_out || !status_out)))
@@ -665,7 +665,7 @@ int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t
     bool threw = false;
     if (!(rc = c.enter(stream, true))) {
         try {
-            rc = run_fasta_body(c, h_text, h_n, q_text, q_n, bgzf, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
+            rc = run_fasta_body(c, h_text, h_n, q_text, q_n, fmt, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
         } catch (...) {
             rc = FRISK_E_CAPACITY;
             threw = true;
@@ -747,7 +747,7 @@ int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, u
                          int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                          uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                          frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_text, h_n, q_text, q_n, false, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
+    return run_fasta_any(h_text, h_n, q_text, q_n, frisk_internal::kFmtText, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
                          status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
@@ -755,8 +755,16 @@ int frisk_b200_run_fasta_bgzf(const char* h_gz, uint64_t h_n, const char* q_gz, 
                               int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                               uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                               frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_gz, h_n, q_gz, q_n, true, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
-                         status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
+    return run_fasta_any(h_gz, h_n, q_gz, q_n, frisk_internal::kFmtBgzf, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+                         rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
+}
+
+int frisk_b200_run_fasta_gzip(const char* h_gz, uint64_t h_n, const char* q_gz, uint64_t q_n, int w, int step, int scaffolds_all,
+                              int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
+                              uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
+                              frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
+    return run_fasta_any(h_gz, h_n, q_gz, q_n, frisk_internal::kFmtGzip, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+                         rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
 // Stage times (ms) of the last frisk_b200_run_* call on the current device,

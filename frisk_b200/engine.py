@@ -131,6 +131,13 @@ def is_bgzf(buf) -> bool:
     return False
 
 
+def is_gzip(buf) -> bool:
+    """Whether ``buf`` begins with a gzip member (1f 8b, CM 8) that is not BGZF: gzip, pigz, NCBI / Ensembl / UCSC
+    ``.fa.gz``.  Such files are inflated on the device too (frisk_gzip.cu)."""
+    a = _as_u8(buf)
+    return a.shape[0] >= 18 and bytes(a[:3]) == b"\x1f\x8b\x08" and not is_bgzf(a)
+
+
 def read_genome_file(path: str) -> Tuple[np.ndarray, bool]:
     """(bytes, bgzf): a BGZF file as it is on disk (the device inflates it), any other file as ``read_fasta_file``
     gives it (a single-member ``.gz`` inflated on the host, text as it is)."""
@@ -138,6 +145,31 @@ def read_genome_file(path: str) -> Tuple[np.ndarray, bool]:
     if is_bgzf(raw):
         return raw, True
     return (read_fasta_file(path) if path.endswith(".gz") else raw), False
+
+
+def read_genome_raw(path: str) -> Tuple[np.ndarray, str]:
+    """(bytes, kind) as the file is on disk: kind "bgzf" (BGZF), "gzip" (a ``.gz`` with a plain gzip member) or "text".
+    Compressed files are left to the device to inflate; a ``.gz`` that is neither is read by ``read_fasta_file``."""
+    raw = np.fromfile(path, dtype=np.uint8)
+    if is_bgzf(raw):
+        return raw, "bgzf"
+    if path.endswith(".gz"):
+        return (raw, "gzip") if is_gzip(raw) else (read_fasta_file(path), "text")
+    return raw, "text"
+
+
+def open_genome_file(path: str, opener) -> "DeviceGenome":
+    """``opener(bytes, kind)`` on the file as it is on disk; a gzip file the device refuses as unsupported (more than one
+    member) is inflated on the host by ``read_fasta_file`` and opened as text."""
+    buf, kind = read_genome_raw(path)
+    if kind != "gzip":
+        return opener(buf, kind)
+    try:
+        return opener(buf, kind)
+    except _lib.FriskError as e:
+        if e.code != _lib.E_UNSUPPORTED:
+            raise
+    return opener(read_fasta_file(path), "text")
 
 
 def bgzf_text_len(gz) -> int:
@@ -149,10 +181,10 @@ def bgzf_text_len(gz) -> int:
     return int(tl.value)
 
 
-def _name_source(L, h, buf: np.ndarray, bgzf: bool) -> np.ndarray:
-    """What a handle's name offsets index: the caller's text, or -- a BGZF open, whose text never leaves the device -- the
-    handle's buffer of header lines (copied: it goes with the handle)."""
-    if not bgzf:
+def _name_source(L, h, buf: np.ndarray, device_text: bool) -> np.ndarray:
+    """What a handle's name offsets index: the caller's text, or -- a BGZF or gzip open, whose text never leaves the
+    device -- the handle's buffer of header lines (copied: it goes with the handle)."""
+    if not device_text:
         return buf
     p, n = C.c_void_p(), C.c_uint64(0)
     _lib.check(L.frisk_b200_fasta_name_text(h, C.byref(p), C.byref(n)), "frisk_b200_fasta_name_text")
@@ -385,15 +417,21 @@ class DeviceGenome:
     def from_fasta_bytes_native(cls, text: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
         """``from_fasta_bytes`` without PyTorch: the planes are DevBuf allocations (cudaMalloc through the C
         ABI), work goes to the default stream.  Used by the CLI."""
-        return cls._open_native(text, device, False)
+        return cls._open_native(text, device, "text")
 
     @classmethod
     def from_bgzf_bytes_native(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
         """``from_fasta_bytes_native`` for a BGZF buffer: the compressed bytes go to the GPU and are inflated there."""
-        return cls._open_native(gz, device, True)
+        return cls._open_native(gz, device, "bgzf")
 
     @classmethod
-    def _open_native(cls, text, device, bgzf: bool) -> "DeviceGenome":
+    def from_gzip_bytes_native(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes_native`` for one gzip member: the compressed bytes go to the GPU and are inflated there
+        (FriskError E_UNSUPPORTED for a multi-member file)."""
+        return cls._open_native(gz, device, "gzip")
+
+    @classmethod
+    def _open_native(cls, text, device, kind: str) -> "DeviceGenome":
         _lib.require_device()
         L = _lib.lib()
         buf = _as_u8(text)
@@ -401,10 +439,10 @@ class DeviceGenome:
         h = C.c_void_p()
         nrec, padded = C.c_uint64(0), C.c_uint64(0)
         stats = np.zeros(3, np.uint64)
-        opener, what = (L.frisk_b200_fasta_open_bgzf, "frisk_b200_fasta_open_bgzf") if bgzf else (L.frisk_b200_fasta_open, "frisk_b200_fasta_open")
-        _lib.check(opener(_ptr(buf), buf.shape[0], None, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
+        what = _OPENERS[kind]
+        _lib.check(getattr(L, what)(_ptr(buf), buf.shape[0], None, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
         try:
-            names_buf = _name_source(L, h, buf, bgzf)
+            names_buf = _name_source(L, h, buf, kind != "text")
             R, P = int(nrec.value), int(padded.value)
             name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
             seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
@@ -424,22 +462,29 @@ class DeviceGenome:
         """Device-side ingest (frisk_ingest.cu): the raw FASTA text goes to the GPU once and is
         tokenised and 2-bit packed there; only the record table comes back.  ``self.host`` is a
         PackedGenome without host planes (names, lengths, layout, countN statistics)."""
-        return cls._open(text, device, False)
+        return cls._open(text, device, "text")
 
     @classmethod
     def from_bgzf_bytes(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
         """``from_fasta_bytes`` for a BGZF buffer (bgzip, samtools): the compressed bytes go to the GPU and are inflated
         there (frisk_bgzf.cu), straight into the ingest's text buffer; the text never exists on the host."""
-        return cls._open(gz, device, True)
+        return cls._open(gz, device, "bgzf")
 
     @classmethod
-    def _open(cls, text, device, bgzf: bool) -> "DeviceGenome":
+    def from_gzip_bytes(cls, gz: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes`` for one gzip member (gzip, pigz): the compressed bytes go to the GPU and are inflated there
+        (frisk_gzip.cu), straight into the ingest's text buffer.  FriskError E_UNSUPPORTED for a multi-member file."""
+        return cls._open(gz, device, "gzip")
+
+    @classmethod
+    def _open(cls, text, device, kind: str) -> "DeviceGenome":
         import torch
         _lib.require_device()
         L = _lib.lib()
         buf = _as_u8(text)
         dev = torch.device(device)
-        opener, what = (L.frisk_b200_fasta_open_bgzf, "frisk_b200_fasta_open_bgzf") if bgzf else (L.frisk_b200_fasta_open, "frisk_b200_fasta_open")
+        what = _OPENERS[kind]
+        opener = getattr(L, what)
         with torch.cuda.device(dev):
             st = _stream_ptr(dev)
             h = C.c_void_p()
@@ -447,7 +492,7 @@ class DeviceGenome:
             stats = np.zeros(3, np.uint64)
             _lib.check(opener(_ptr(buf), buf.shape[0], st, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
             try:
-                names_buf = _name_source(L, h, buf, bgzf)
+                names_buf = _name_source(L, h, buf, kind != "text")
                 R, P = int(nrec.value), int(padded.value)
                 name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
                 seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
@@ -465,9 +510,9 @@ class DeviceGenome:
 
     @classmethod
     def from_fasta(cls, path: str, device="cuda:0") -> "DeviceGenome":
-        """A FASTA file: BGZF is inflated on the device, any other ``.gz`` on the host (``read_fasta_file``)."""
-        buf, bgzf = read_genome_file(path)
-        return cls.from_bgzf_bytes(buf, device) if bgzf else cls.from_fasta_bytes(buf, device)
+        """A FASTA file: BGZF and single-member gzip are inflated on the device, a multi-member ``.gz`` on the host
+        (``read_fasta_file``)."""
+        return open_genome_file(path, lambda buf, kind: cls._open(buf, device, kind))
 
     def to_host(self) -> PackedGenome:
         """Copy the planes back (tests; the host packer must agree bit for bit)."""
@@ -1057,7 +1102,7 @@ class _HandlePlane:
         return self._p
 
 
-def _genome_from_handle(L, h, buf, bgzf: bool = False) -> PackedGenome:
+def _genome_from_handle(L, h, buf, device_text: bool = False) -> PackedGenome:
     nrec, padded = C.c_uint64(0), C.c_uint64(0)
     stats = np.zeros(3, np.uint64)
     _lib.check(L.frisk_b200_fasta_info(h, C.byref(nrec), C.byref(padded), _ptr(stats)), "frisk_b200_fasta_info")
@@ -1066,7 +1111,7 @@ def _genome_from_handle(L, h, buf, bgzf: bool = False) -> PackedGenome:
     seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
     _lib.check(L.frisk_b200_fasta_records(h, _ptr(name_off), _ptr(name_len), _ptr(seq_len), _ptr(scaf_off)),
                "frisk_b200_fasta_records")
-    return PackedGenome(LazyNames(_name_source(L, h, buf, bgzf), name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
+    return PackedGenome(LazyNames(_name_source(L, h, buf, device_text), name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
                         int(stats[0]), int(stats[1]), int(stats[2]), False)
 
 
@@ -1078,7 +1123,7 @@ def run_fasta(query_text, host_text=None, device="cuda:0", out=None, assemble_re
     derived on the host while the last chunk is still being counted; then tables, IVOM, window kernel, rows.  This is the
     whole of the reference's stages 2+3 (F:1442, F:1478-1494) including its three passes over the file (F:170, F:203,
     F:297).  ``out``: reusable HostOutputs (its row capacity is used; ``out.n_win`` is set)."""
-    return _run_fasta_any(query_text, host_text, False, device, out, assemble_result, kmin, kmax, w, step, mask_host,
+    return _run_fasta_any(query_text, host_text, "text", device, out, assemble_result, kmin, kmax, w, step, mask_host,
                           scaffolds_all, rip)
 
 
@@ -1088,11 +1133,34 @@ def run_fasta_bgzf(query_gz, host_gz=None, device="cuda:0", out=None, assemble_r
     """``run_fasta`` for BGZF buffers (bgzip, samtools; ideally page-locked): ONE C call (frisk_b200_run_fasta_bgzf) that
     uploads the compressed bytes, inflates every BGZF block on the device straight into the ingest's text buffer and goes
     on exactly as ``run_fasta``.  Same results as ``run_fasta`` on the inflated text."""
-    return _run_fasta_any(query_gz, host_gz, True, device, out, assemble_result, kmin, kmax, w, step, mask_host,
+    return _run_fasta_any(query_gz, host_gz, "bgzf", device, out, assemble_result, kmin, kmax, w, step, mask_host,
                           scaffolds_all, rip)
 
 
-def _run_fasta_any(query_text, host_text, bgzf, device, out, assemble_result, kmin, kmax, w, step, mask_host, scaffolds_all, rip):
+def run_fasta_gzip(query_gz, host_gz=None, device="cuda:0", out=None, assemble_result: bool = True, kmin: int = 1,
+                   kmax: int = 8, w: int = 5000, step: int = 2500, mask_host: bool = False, scaffolds_all: bool = False,
+                   rip: bool = True):
+    """``run_fasta`` for single gzip members (gzip, pigz): ONE C call (frisk_b200_run_fasta_gzip) that uploads the
+    compressed bytes, inflates them on the device straight into the ingest's text buffer and goes on exactly as
+    ``run_fasta``.  Same results as ``run_fasta`` on the inflated text; FriskError E_UNSUPPORTED for a multi-member file."""
+    return _run_fasta_any(query_gz, host_gz, "gzip", device, out, assemble_result, kmin, kmax, w, step, mask_host,
+                          scaffolds_all, rip)
+
+
+_OPENERS = {"text": "frisk_b200_fasta_open", "bgzf": "frisk_b200_fasta_open_bgzf", "gzip": "frisk_b200_fasta_open_gzip"}
+_RUNNERS = {"text": "frisk_b200_run_fasta", "bgzf": "frisk_b200_run_fasta_bgzf", "gzip": "frisk_b200_run_fasta_gzip"}
+
+
+def _text_len_hint(buf: np.ndarray, kind: str) -> int:
+    """The text's length: exact for text and BGZF; for gzip, ISIZE (the length mod 2^32 -- a guess for sizing rows)."""
+    if kind == "bgzf":
+        return bgzf_text_len(buf)
+    if kind == "gzip":
+        return int.from_bytes(bytes(buf[-4:]), "little") if buf.shape[0] >= 4 else 0
+    return buf.shape[0]
+
+
+def _run_fasta_any(query_text, host_text, kind, device, out, assemble_result, kmin, kmax, w, step, mask_host, scaffolds_all, rip):
     import torch
     _lib.require_device()
     L = _lib.lib()
@@ -1103,11 +1171,12 @@ def _run_fasta_any(query_text, host_text, bgzf, device, out, assemble_result, km
         # rows: a guess (one window per step of text, one more per 4 KiB for short scaffolds); a text with more windows comes
         # back with FRISK_E_CAPACITY and is scored in a second stage below -- page-locking a far larger buffer "to be safe"
         # would cost more than the run (~0.3 ms per MB)
-        n_text = bgzf_text_len(qbuf) if bgzf else qbuf.shape[0]
+        n_text = _text_len_hint(qbuf, kind)
         out = HostOutputs(n_text // step + n_text // 4096 + 64, kmax)
     hh, qh = C.c_void_p(), C.c_void_p()
     n_win = C.c_uint64(0)
-    fn, what = (L.frisk_b200_run_fasta_bgzf, "frisk_b200_run_fasta_bgzf") if bgzf else (L.frisk_b200_run_fasta, "frisk_b200_run_fasta")
+    what = _RUNNERS[kind]
+    fn = getattr(L, what)
     with _device_ctx(dev):
         st = _stream_ptr(dev)
         rc = fn(_ptr(hbuf), hbuf.shape[0], _ptr(qbuf) if host_text is not None else None,
@@ -1119,8 +1188,8 @@ def _run_fasta_any(query_text, host_text, bgzf, device, out, assemble_result, km
                 _lib.check(rc, what)
             n = int(n_win.value)
             need_genomes = assemble_result or rc == _lib.E_CAPACITY
-            host = _genome_from_handle(L, hh, hbuf, bgzf) if need_genomes else None
-            query = (_genome_from_handle(L, qh, qbuf, bgzf) if qh else host) if need_genomes else None
+            host = _genome_from_handle(L, hh, hbuf, kind != "text") if need_genomes else None
+            query = (_genome_from_handle(L, qh, qbuf, kind != "text") if qh else host) if need_genomes else None
             if rc == _lib.E_CAPACITY:
                 # more windows than the guessed row capacity: the planes are on the device, score them into enough rows
                 def planes(h):

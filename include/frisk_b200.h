@@ -245,7 +245,8 @@ int frisk_b200_score_occupancy(int kmax, uint32_t max_win_len, int *ctas_per_sm,
  * "ingest_exact_open" = 1 makes frisk_b200_fasta_open copy the text in one piece and count the records before it
  * allocates the record table (the fallback of the default chunked open); "ingest_chunk_tiles" = t lets texts of
  * 2t or more 4096-byte tiles be uploaded in chunks (default 512: 2 MiB per chunk, at most 8 chunks).  Same genome
- * either way (tests/test_ingest_gpu.py). */
+ * either way (tests/test_ingest_gpu.py).  "gzip_chunk_bytes" = c places the gzip inflate's nominal chunk starts every c
+ * compressed bytes (0: default); same text either way. */
 int frisk_b200_set_option(const char *name, int value);
 
 /*
@@ -380,7 +381,7 @@ int frisk_b200_fasta_planes(const frisk_b200_fasta *h, const uint32_t **d_codes,
  * BGZF (bgzip, `samtools faidx`) is a series of gzip members of <= 64 KiB each; every member's header gives its
  * compressed size and its trailer the CRC32 and inflated size, so every member is inflated on the device by a decoder of
  * its own, straight into the ingest's text buffer.  A single-member .gz (gzip, pigz) is not BGZF: it is FRISK_E_FORMAT
- * here and is inflated on the host by the Python layer, as before.
+ * here and goes to the gzip entry points below.
  *
  * frisk_b200_bgzf_blocks: the block table of a BGZF buffer, from the headers and trailers alone.  comp_off / comp_len: the
  * raw deflate payload of every member; crc: the CRC32 of its trailer; text_off: the exclusive prefix sum of the inflated
@@ -417,6 +418,47 @@ int frisk_b200_run_fasta_bgzf(const char *h_gz, uint64_t h_n, const char *q_gz, 
                               double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
                               uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
 int frisk_b200_fasta_name_text(const frisk_b200_fasta *h, const char **text, uint64_t *n);
+
+/* ------------------------------------------------------------------ gzip-compressed FASTA (frisk_gzip.cu)
+ *
+ * One plain gzip member (gzip, pigz, NCBI / Ensembl / UCSC .fa.gz) is one deflate stream, inflated on the device in two
+ * passes: decoders start at block boundaries found by a search for valid dynamic block headers, every C compressed bytes,
+ * and write matches that reach before their chunk as placeholders; the host accepts a chunk only where its predecessor
+ * ended exactly at its start and decodes the others again from there; the placeholders are then resolved in chunk order.
+ * A file without dynamic blocks (level 0, Z_FIXED) is one chunk.  "gzip_chunk_bytes" (frisk_b200_set_option) sets C
+ * (0: the default, 16 KiB).  Device memory: besides the member and the text, the first pass takes about 16 bytes of
+ * scratch per compressed byte (16-bit symbols, 8 per compressed byte), about 14 GB for a 900 MB .gz.
+ *
+ * frisk_b200_gzip_member: the header of the member at gz (1f 8b, CM 8; FTEXT, FHCRC (checked), FEXTRA, FNAME, FCOMMENT;
+ * reserved flag bits are FRISK_E_FORMAT): the deflate payload's offset and length up to the last 8 bytes, and the CRC32 and
+ * ISIZE of those last 8 bytes (the trailer of a single-member file).  Any pointer but gz may be NULL.
+ *
+ * frisk_b200_gzip_inflate: inflates the member in d_gz[0, n) (device memory) into d_text.  Synchronises `stream`.
+ * *text_len receives the text's length (exact: no ISIZE guess; ISIZE must equal it mod 2^32); FRISK_E_CAPACITY, with
+ * *text_len set, when text_cap is smaller.  stats (nullable): {chunks, joins accepted on the first pass, chunks decoded
+ * again from their predecessor's end, chain chunks decoded again because their scratch was too small}.  Not valid
+ * deflate, a CRC32 or ISIZE mismatch, truncation or trailing bytes: FRISK_E_FORMAT.  Another gzip member after the
+ * trailer (a multi-member file): FRISK_E_UNSUPPORTED (the Python layer then inflates on the host); so are chunks of 4 GiB
+ * of text or more.  Malformed input never faults and leaves no CUDA error behind.
+ * frisk_b200_gzip_inflate_host: the same plan, joins and repairs run on the CPU over host memory (test infrastructure: no
+ * user path calls it); same text, same stats, same return codes.  `stream` is unused.
+ *
+ * frisk_b200_fasta_open_gzip / frisk_b200_run_fasta_gzip: frisk_b200_fasta_open / frisk_b200_run_fasta with one gzip member
+ * in place of the texts, same arguments and results, as the _bgzf pair: the member goes up and is inflated into the
+ * ingest's text buffer; the names come from frisk_b200_fasta_name_text; ms[0] of frisk_b200_last_run_timing is
+ * "compressed bytes uploaded and inflated". */
+int frisk_b200_gzip_member(const uint8_t *gz, uint64_t n, uint64_t *payload_off, uint64_t *payload_len, uint32_t *crc,
+                           uint32_t *isize);
+int frisk_b200_gzip_inflate(const uint8_t *d_gz, uint64_t n, uint8_t *d_text, uint64_t text_cap, uint64_t *text_len,
+                            uint64_t stats[4], void *stream);
+int frisk_b200_gzip_inflate_host(const uint8_t *gz, uint64_t n, uint8_t *text, uint64_t text_cap, uint64_t *text_len,
+                                 uint64_t stats[4], void *stream);
+int frisk_b200_fasta_open_gzip(const char *gz, uint64_t n, void *stream, frisk_b200_fasta **out, uint64_t *n_records,
+                               uint64_t *padded_len, uint64_t stats[3]);
+int frisk_b200_run_fasta_gzip(const char *h_gz, uint64_t h_n, const char *q_gz, uint64_t q_n, int w, int step,
+                              int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap,
+                              double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
+                              uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
 
 /* Stage times (ms since the start of the call) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call
  * on the current device, from CUDA events recorded on the call's own streams: ms[0] planes uploaded, ms[1] background
