@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SO_PATH = os.environ.get("FRISK_B200_LIB") or os.path.join(HERE, "libfrisk_b200.so")   # override: kernel A/B builds (tools/)
+SO_PATH = os.environ.get("FRISK_B200_LIB") or os.path.join(HERE, "libfrisk_b200.so")   # override: load another build (A/B of two commits in one GPU call)
 
 OK, E_INVALID, E_UNSUPPORTED, E_CUDA, E_NO_DEVICE, E_CAPACITY, E_FORMAT = 0, -1, -2, -3, -4, -5, -6
 ROW_KLD_ZERODIV, ROW_GC_ZERODIV, ROW_LOG_DOMAIN, ROW_EXCLUDED = 1, 2, 4, 8

@@ -13,7 +13,7 @@
 //   * every POSITION scores its own K-mer with weight 1/c_K (c_K = its count in the window), so the sum over
 //     positions equals the sum over distinct K-mers (F:448-472 iterate the distinct keys) without ever
 //     enumerating them; a thread's positions are fixed and so is the reduction tree -> bit-reproducible rows.
-// Two atomics and one epilogue per position; 3 CTAs per SM (75 KB each).
+// Two atomics and one epilogue per position; 3 CTAs per SM (73 KB each).
 //
 // What a byte cannot hold is handed to the bucketed kernel (frisk_kernels.cu), exactly: a window in which some
 // K-mer occurs 256+ times (the thread whose increment wraps the byte sees 255 in the word it got back), or
@@ -54,24 +54,15 @@ struct DirectLayout {
     static constexpr uint32_t ZERO_BYTES = TOP_BYTES + LOW_BYTES;
     static constexpr uint32_t OFF_LOW = TOP_BYTES;
     static constexpr uint32_t OFF_PRE = ZERO_BYTES;
-    static constexpr uint32_t OFF_LOG = OFF_PRE + NPRE * 16u;
-    static constexpr uint32_t OFF_SS = OFF_LOG + 128u * 16u;
+    static constexpr uint32_t OFF_SS = OFF_PRE + NPRE * 16u;
     static constexpr uint32_t TOTAL = OFF_SS + (uint32_t)sizeof(DirectSmem<NT>);
 };
 
 __device__ __forceinline__ uint32_t bytes_sum(uint32_t w, uint32_t acc) { return __dp4a(w, 0x01010101u, acc); }
 
-#ifndef FRISK_DIRECT_K7_CTAS
-#define FRISK_DIRECT_K7_CTAS 4
-#endif
-#define FRISK_DIRECT_MIN_CTAS(K) ((K) == 7 ? FRISK_DIRECT_K7_CTAS : 3)   // K = 8: 75 KB of shared memory each; K = 7: registers decide
-#ifndef FRISK_DIRECT_TABLOG
-#define FRISK_DIRECT_TABLOG 0
-#endif
-constexpr bool TABLOG = FRISK_DIRECT_TABLOG;      // log2 by series: no shared-memory table read in the epilogue
-
+// CTAs per SM: K = 8: 73 KB of shared memory each; K = 7: registers decide
 template <int K, int NT, int ROUNDS, bool DUMP, bool ALLK>
-__global__ void __launch_bounds__(NT, FRISK_DIRECT_MIN_CTAS(K))
+__global__ void __launch_bounds__(NT, K == 7 ? 4 : 3)
 score_windows_direct_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ inv, const uint32_t* __restrict__ low,
                             const unsigned long long* __restrict__ win_off, const uint32_t* __restrict__ win_len, uint32_t n_win,
                             const double2* __restrict__ ig, int kmin_arg, int want_rip,
@@ -85,17 +76,11 @@ score_windows_direct_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
     uint16_t* tab16 = reinterpret_cast<uint16_t*>(smem + L::OFF_LOW);    // orders 1..A at lvl_off(x)
     uint32_t* tab32 = reinterpret_cast<uint32_t*>(smem + L::OFF_LOW);
     double2* pre = reinterpret_cast<double2*>(smem + L::OFF_PRE);       // .x = num, .y = {flag, den} as two u32
-    double2* logtab = reinterpret_cast<double2*>(smem + L::OFF_LOG);
     DirectSmem<NT>& ss = *reinterpret_cast<DirectSmem<NT>*>(smem + L::OFF_SS);
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (uint32_t i = tid; i < L::ZERO_BYTES / 16u; i += NT) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
     if (tid < 8) ss.cnt[tid >> 2][tid & 3] = 0;
-    if (tid < 128) {
-        const double c = 1.0 + ((double)tid + 0.5) / 128.0;
-        const double ic = 1.0 / c;
-        logtab[tid] = make_double2(ic, -log2(ic));
-    }
     __syncthreads();
 
     int par = 1;
@@ -309,7 +294,7 @@ score_windows_direct_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             const double om = dden * r;
             s_w += a;
             s_g = fma(g.x, om, s_g);                       // a NaN entry (reference: ZeroDivisionError) poisons the sum
-            s_t = fma(a, (TABLOG ? log2_pos(iw, logtab) : log2_series(iw)) - g.y, s_t);
+            s_t = fma(a, log2_series(iw) - g.y, s_t);
         };
 #pragma unroll 1
         for (int r = 0; r < ROUNDS; ++r) {
@@ -375,7 +360,7 @@ const void* direct_fn(const frisk_internal::WinPlan& p) {
 
 }  // namespace
 
-// 256 threads; at K = 8 three CTAs of 75 KB need the whole 228 KB carve-out
+// 256 threads; at K = 8 three CTAs of 73 KB need the whole 228 KB carve-out
 frisk_internal::LaunchShape frisk_internal::direct_shape(const WinPlan& p, int K) {
     if (K == 8) return {direct_fn<8>(p), 256, DirectLayout<8, 256>::TOTAL, true};
     return {direct_fn<7>(p), 256, DirectLayout<7, 256>::TOTAL, true};

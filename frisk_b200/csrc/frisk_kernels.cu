@@ -28,13 +28,6 @@
 #include "frisk_internal.h"
 #include "frisk_device.cuh"
 
-// log2 in the window-kernel epilogues: table-driven (log2_pos) or table-free series (log2_series)
-#ifdef FRISK_SERIES_LOG2
-#define FRISK_LOG2(x, tab) log2_series(x)
-#else
-#define FRISK_LOG2(x, tab) log2_pos(x, tab)
-#endif
-
 namespace {
 
 constexpr int kThreads = 1024;          // one CTA per SM: the 4^8 u16 window table takes 128 KiB of smem
@@ -680,7 +673,7 @@ score_windows_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restr
                 const double2 g = __ldg(ig + kappa);
                 s_w += iw;
                 s_g += g.x;
-                s_t = fma(iw, FRISK_LOG2(iw, logtab) - g.y, s_t);
+                s_t = fma(iw, log2_pos(iw, logtab) - g.y, s_t);
                 bad |= (g.x != g.x);
             }
             __syncthreads();                               // list is reused by the next segment
@@ -1134,7 +1127,7 @@ score_windows_bucket_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             const double2 g = __ldg(ig + kappa);
             s_w += iw;
             s_g += g.x;                                    // a NaN entry (reference: ZeroDivisionError) poisons the sum
-            s_t = fma(iw, FRISK_LOG2(iw, logtab) - g.y, s_t);
+            s_t = fma(iw, log2_pos(iw, logtab) - g.y, s_t);
         };
         for (uint32_t e = tid; e < n_clean; e += kT3) {
             const uint32_t kappa = list[e];
@@ -1365,7 +1358,7 @@ score_windows_small_kernel(const uint32_t* __restrict__ codes, const uint32_t* _
                 const double2 g = __ldg(ig + kappa);
                 s_w += iw;
                 s_g += g.x;
-                s_t = fma(iw, FRISK_LOG2(iw, logtab) - g.y, s_t);
+                s_t = fma(iw, log2_pos(iw, logtab) - g.y, s_t);
                 any = 1;
             }
         }
@@ -1472,13 +1465,6 @@ int frisk_internal::cuda_fail(cudaError_t e, const char* what) {
     snprintf(g_cuda_err, sizeof(g_cuda_err), "%s: %s (%s)", what, cudaGetErrorName(e), cudaGetErrorString(e));
     return FRISK_E_CUDA;
 }
-
-#ifndef FRISK_DIRECT_DEFAULT
-#define FRISK_DIRECT_DEFAULT(kmax, len) ((kmax) == 7)   // (reached for short windows only: w = 1000 / 500: 1.00 / 1.59 ms vs 1.05 / 1.76 nibble, 1.14 / 1.85 bucketed)
-#endif
-#ifndef FRISK_NIBBLE_DEFAULT
-#define FRISK_NIBBLE_DEFAULT(kmax, len) ((kmax) == 8 || ((kmax) == 7 && (len) > 1500u))   // measured: tools/k8_ab.py
-#endif
 
 namespace {
 using frisk_internal::sm_count_cached;
@@ -1686,12 +1672,15 @@ int peer_fwd(const uint64_t* const* d_fwd_peers, uint64_t* const* d_flag_peers, 
     return FRISK_OK;
 }
 
+constexpr bool nibble_default(int kmax, uint32_t len) { return kmax == 8 || (kmax == 7 && len > 1500u); }   // measured: tools/k8_ab.py
+constexpr bool direct_default(int kmax) { return kmax == 7; }   // (reached for short windows only: w = 1000 / 500: 1.00 / 1.59 ms vs 1.05 / 1.76 nibble, 1.14 / 1.85 bucketed)
+
 }  // namespace
 
 // Which window kernel frisk_b200_score runs.  kmax 9..12: the extension kernel on windows the shared-memory kernels hold,
 // the general one otherwise (and for the test-only table dump).  kmax <= 8: the small-K kernel up to kmax 6 (no sorting,
 // 6 CTAs/SM, any window up to 65,535 bases); for kmax 7 and 8 the nibble kernel (4-bit counters, one atomic per position)
-// or the direct kernel (byte table) as measured on C2 (FRISK_NIBBLE_DEFAULT / FRISK_DIRECT_DEFAULT), then the bucketed
+// or the direct kernel (byte table) as measured on C2 (nibble_default / direct_default), then the bucketed
 // one over whatever they hand back; the dense-table kernel for windows longer than the shared-memory buffer.  A forced
 // kernel wins wherever it can run.
 int frisk_internal::plan_score(int kmin, int kmax, uint32_t len, bool dump, WinPlan* out) {
@@ -1705,9 +1694,9 @@ int frisk_internal::plan_score(int kmin, int kmax, uint32_t len, bool dump, WinP
     else if (kmax <= 6 && !forced(WinKernel::Bucket)) k = WinKernel::Small;
     else if (kmax < 4 || !smem) k = WinKernel::Dense;
     else if (kmax >= 7 && (forced(WinKernel::Nibble) ||
-                           (!forced(WinKernel::Bucket) && !forced(WinKernel::Direct) && FRISK_NIBBLE_DEFAULT(kmax, len))))
+                           (!forced(WinKernel::Bucket) && !forced(WinKernel::Direct) && nibble_default(kmax, len))))
         k = WinKernel::Nibble;
-    else if (kmax >= 7 && (forced(WinKernel::Direct) || (!forced(WinKernel::Bucket) && FRISK_DIRECT_DEFAULT(kmax, len))))
+    else if (kmax >= 7 && (forced(WinKernel::Direct) || (!forced(WinKernel::Bucket) && direct_default(kmax))))
         k = WinKernel::Direct;
     else k = WinKernel::Bucket;
     *out = {k, window_variant(k, len), dump, kmin == 1 && !dump};

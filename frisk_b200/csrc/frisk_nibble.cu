@@ -47,24 +47,6 @@ struct NibSmem {
     uint32_t side[kSideCap];          // v << 16 | code of a word valid for v = K-1 or K-2 bases only
 };
 
-#ifndef FRISK_NIBBLE_TABLOG
-#define FRISK_NIBBLE_TABLOG 0
-#endif
-constexpr bool NIB_TABLOG = FRISK_NIBBLE_TABLOG;   // 0: log2 by series, no shared-memory table read in the epilogue
-#ifndef FRISK_NIBBLE_PRE5
-#define FRISK_NIBBLE_PRE5 1
-#endif
-constexpr bool NIB_PRE5 = FRISK_NIBBLE_PRE5;       // K = 8: order 5 folded into `pre` too (one 16-byte read instead of 16 + 2)
-#ifndef FRISK_NIBBLE_PREFETCH
-#define FRISK_NIBBLE_PREFETCH 0
-#endif
-#ifndef FRISK_NIBBLE_WINPF
-#define FRISK_NIBBLE_WINPF 0
-#endif
-constexpr bool NIB_WINPF = FRISK_NIBBLE_WINPF;         // L2 prefetch of the CTA's next window while this one is processed
-                                                       // (measured: 0.655 vs 0.658 ms on C2 -- within noise, off)
-constexpr bool NIB_PREFETCH = FRISK_NIBBLE_PREFETCH;   // request the next K-mer's genome IVOM entry before scoring this one
-
 template <int K>
 struct NibLayout {
     static_assert(K == 7 || K == 8, "nibble kernel: K = 7 or 8");
@@ -78,11 +60,11 @@ struct NibLayout {
     static constexpr uint32_t ZERO_BYTES = NIB_BYTES + LOW_BYTES;
     static constexpr uint32_t OFF_LOW = NIB_BYTES;
     static constexpr uint32_t OFF_PRE = ZERO_BYTES;
-    static constexpr bool FOLD_A = NIB_PRE5 && A > LP;                   // `pre` extended to order A (its own array, after the order-4 one)
+    // K = 8: `pre` extended to order A (its own array, after the order-4 one): one 16-byte read instead of 16 + 2
+    static constexpr bool FOLD_A = A > LP;
     static constexpr uint32_t NPREA = FOLD_A ? pow4(A) : 0u;
     static constexpr uint32_t OFF_PREA = OFF_PRE + NPRE * 16u;
-    static constexpr uint32_t OFF_LOG = OFF_PREA + NPREA * 16u;
-    static constexpr uint32_t OFF_SS = OFF_LOG + (NIB_TABLOG ? 128u * 16u : 0u);
+    static constexpr uint32_t OFF_SS = OFF_PREA + NPREA * 16u;
     static constexpr uint32_t TOTAL = OFF_SS + (uint32_t)sizeof(NibSmem);
 };
 
@@ -112,24 +94,6 @@ template <typename MT> __device__ __forceinline__ MT top_bits(int n) {       // 
     return n >= MB ? ~MT(0) : ~(~MT(0) >> n);
 }
 
-#ifndef FRISK_NIBBLE_WALK
-#define FRISK_NIBBLE_WALK 0
-#endif
-constexpr bool NIB_WALK = FRISK_NIBBLE_WALK;       // scoring pass re-reads the thread's code words and walks them with a 2-bit
-                                                   // shift register instead of keeping PP K-mer codes in registers
-#ifndef FRISK_NIBBLE_GATHER_CG
-#define FRISK_NIBBLE_GATHER_CG 1
-#endif
-#if FRISK_NIBBLE_GATHER_CG
-#define NIB_GATHER(p) __ldcg(p)                    // L2 only: the 1 MiB table never survives in a ~30 KB L1 anyway, and
-                                                   // not allocating there measured 4.7 % faster (0.703 -> 0.671 ms on C2)
-#else
-#define NIB_GATHER(p) __ldg(p)
-#endif
-#ifndef FRISK_NIBBLE_CTAS
-#define FRISK_NIBBLE_CTAS 4
-#endif
-
 // The k sweep of BASELINE config C3 (scores for kmax' = 1..K with kmin = 1, i.e. K reference runs `-m 1 -k k'`, F:1197-1206)
 // from ONE pass over the window: the counts of every order are there after the marginalisation, so the SWEEP
 // instantiation evaluates all K scores -- kmax' <= K-2 by walking that order's bins (coalesced genome-IVOM reads),
@@ -146,13 +110,13 @@ struct NibSweep {
 // (cs = the window length spread over the CTA, a multiple of 4), reads the three or four code words and two or three
 // mask words that cover it once, and issues the atomics of its full K-words back to back from registers.
 template <int K, int PP, bool DUMP, bool ALLK, bool SWEEP = false>
-__global__ void __launch_bounds__(kNT, FRISK_NIBBLE_CTAS)
+__global__ void __launch_bounds__(kNT, 4)
 score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ inv, const uint32_t* __restrict__ low,
                             const unsigned long long* __restrict__ win_off, const uint32_t* __restrict__ win_len, uint32_t n_win,
                             const double2* __restrict__ ig, int kmin_arg, int want_rip,
                             double* __restrict__ rows, uint32_t* __restrict__ status, uint16_t* __restrict__ dump,
                             uint32_t* redo_dst, const NibSweep sw) {
-    static_assert(!SWEEP || (K == 8 && ALLK && !DUMP && NIB_PRE5), "the sweep instantiation: K = 8, kmin = 1");
+    static_assert(!SWEEP || (K == 8 && ALLK && !DUMP), "the sweep instantiation: K = 8, kmin = 1");
     using L = NibLayout<K>;
     static_assert(PP % 4 == 0 && PP >= 4 && PP + K - 1 <= 64, "chunk size");
     constexpr int A = L::A, LP = L::LP, NT = kNT, NW = NT / 32;
@@ -169,18 +133,11 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
     uint32_t* tab32 = reinterpret_cast<uint32_t*>(smem + L::OFF_LOW);
     double2* pre = reinterpret_cast<double2*>(smem + L::OFF_PRE);       // .x = num, .y = {flag, den} as two u32
     double2* preA = reinterpret_cast<double2*>(smem + L::OFF_PREA);     // FOLD_A: the same pair through order A, per order-A prefix
-    double2* logtab = reinterpret_cast<double2*>(smem + L::OFF_LOG);
     NibSmem& ss = *reinterpret_cast<NibSmem*>(smem + L::OFF_SS);
-    (void)logtab; (void)preA;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (uint32_t i = tid; i < L::ZERO_BYTES / 16u; i += NT) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
     if (tid < 12) ss.cnt[tid / 6][tid % 6] = 0;
-    if (NIB_TABLOG && tid < 128) {
-        const double c = 1.0 + ((double)tid + 0.5) / 128.0;
-        const double ic = 1.0 / c;
-        logtab[tid] = make_double2(ic, -log2(ic));
-    }
     __syncthreads();
 
     if (sw.n_win_dev) n_win = (uint32_t)min((unsigned long long)n_win, *sw.n_win_dev);
@@ -196,18 +153,6 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         const uint32_t* __restrict__ lw = low ? low + (o >> 5) : nullptr;
         const uint32_t cs = max(4u, ((len + NT - 1) / NT + 3u) & ~3u);    // positions per thread (<= PP: checked by the launcher)
         const uint32_t p0 = (uint32_t)tid * cs;                          // this thread's first position
-        if (NIB_WINPF && warp == 0 && win + gridDim.x < n_win) {
-            // the planes of this CTA's NEXT window into L2 (every step starts with a cold L2: P1 would wait for HBM):
-            // lanes 0..15 the code lines, 16..23 the invalid-mask lines, 24..31 the lower-case lines
-            const uint64_t on = win_off[win + gridDim.x];
-            const uint32_t ln = win_len[win + gridDim.x] + (uint32_t)K;
-            const char* pc = reinterpret_cast<const char*>(codes + (on >> 5) * 2);
-            const char* pm = reinterpret_cast<const char*>(inv + (on >> 5));
-            if (lane < 16) { if ((uint32_t)lane * 128u < ln / 4u + 8u) asm volatile("prefetch.global.L2 [%0];" ::"l"(pc + lane * 128)); }
-            else if (lane < 24) { if ((uint32_t)(lane - 16) * 128u < ln / 8u + 8u) asm volatile("prefetch.global.L2 [%0];" ::"l"(pm + (lane - 16) * 128)); }
-            else if (low && (uint32_t)(lane - 24) * 128u < ln / 8u + 8u)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(low + (on >> 5)) + (lane - 24) * 128));
-        }
 
         // ---- P1: composition + ONE atomic per full K-word, all from registers ----------------------------
         uint32_t kk[PP / 2];                                             // two K-mer codes per register
@@ -265,7 +210,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                         const uint32_t k0 = kmer_at(i), k1 = kmer_at(i + 1);
                         atomicAdd(&nib32[k0 >> 3], 1u << ((k0 & 7u) * 4u));
                         atomicAdd(&nib32[k1 >> 3], 1u << ((k1 & 7u) * 4u));
-                        if (!NIB_WALK || SWEEP) kk[i >> 1] = k0 | (k1 << 16);
+                        kk[i >> 1] = k0 | (k1 << 16);
                     }
                 } else {
 #pragma unroll
@@ -273,7 +218,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                         if (vm & (MT(1) << (MB - 1 - i))) {
                             const uint32_t kap = kmer_at(i);
                             atomicAdd(&nib32[kap >> 3], 1u << ((kap & 7u) * 4u));
-                            if (!NIB_WALK || SWEEP) kk[i >> 1] |= kap << (16 * (i & 1));
+                            kk[i >> 1] |= kap << (16 * (i & 1));
                         }
                     }
                 }
@@ -535,7 +480,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             };
             auto eval7 = [&](uint32_t code7, const uint2 v, const double2 pp, uint32_t c6, uint32_t c7) {
                 weighted(fma(q7, u32_to_double(c7 * c7), fma(q6, u32_to_double(c6 * c6), pp.x)),
-                         (uint32_t)__double2loint(pp.y) + (c6 << 12) + (c7 << 14), c7, NIB_GATHER(sw.ig[6] + code7), w7, g7, t7);
+                         (uint32_t)__double2loint(pp.y) + (c6 << 12) + (c7 << 14), c7, __ldcg(sw.ig[6] + code7), w7, g7, t7);
                 (void)v;
             };
             {
@@ -546,7 +491,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                     for (int j = 0; j < 4; ++j) {
                         if (vm & (MT(1) << (MB - 1 - j))) {
                             const uint32_t kap = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-                            const double2 gg8 = NIB_GATHER(sw.ig[7] + kap);
+                            const double2 gg8 = __ldcg(sw.ig[7] + kap);           // L2 only, as in P3
                             const uint2 v = nib64[kap >> 4];
                             const uint32_t ws = (kap & 8u) ? v.y : v.x, wo = (kap & 8u) ? v.x : v.y;
                             const uint32_t c8 = (ws >> ((kap & 7u) * 4u)) & 15u;
@@ -620,7 +565,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
 
         // ---- P3: every position scores its own K-mer with weight 1 / (its count) --------------------
         double s_w = 0.0, s_g = 0.0, s_t = 0.0;
-        const double qA = ss.q[A - 1], qK2 = ss.q[K - 3], qK1 = ss.q[K - 2], qK = ss.q[K - 1];
+        const double qK2 = ss.q[K - 3], qK1 = ss.q[K - 2], qK = ss.q[K - 1];
         auto score_one = [&](uint32_t kap, const double2 g) {
             const uint2 v = nib64[kap >> 4];
             const uint32_t ws = (kap & 8u) ? v.y : v.x, wo = (kap & 8u) ? v.x : v.y;
@@ -632,22 +577,12 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             const double2 pp = L::FOLD_A ? preA[kap >> (2 * (K - A))] : pre[kap >> (2 * (K - LP))];
             double num = pp.x;
             uint32_t den = (uint32_t)__double2loint(pp.y);
-            uint32_t cA = 0, flag;
-            if constexpr (A > LP && !L::FOLD_A) {
-                const uint32_t raw = tab16[lvl_off(A) + (kap >> (2 * (K - A)))];
-                cA = raw & 0x7fffu; flag = raw >> 15;
-            } else {
-                flag = (uint32_t)__double2hiint(pp.y);
-            }
-            if (flag) {                                    // rare: a short word of K-1 / K-2 bases lies below this bin
+            if (__double2hiint(pp.y)) {                    // rare: a short word of K-1 / K-2 bases lies below this bin
                 for (uint32_t i = 0; i < n_side; ++i) {
                     const uint32_t e = ss.side[i], sv = e >> 16, code = e & 0xffffu;
                     if (sv == (uint32_t)(K - 1)) { cK1 += (code == (kap >> 2)); cK2 += ((code >> 2) == (kap >> 4)); }
                     else cK2 += (code == (kap >> 4));
                 }
-            }
-            if constexpr (A > LP && !L::FOLD_A) {
-                if (A >= kmin) { den += cA << (2 * A); num = fma(qA, u32_to_double(cA * cA), num); }
             }
             if (K - 2 >= kmin) { den += cK2 << (2 * (K - 2)); num = fma(qK2, u32_to_double(cK2 * cK2), num); }
             if (K - 1 >= kmin) { den += cK1 << (2 * (K - 1)); num = fma(qK1, u32_to_double(cK1 * cK1), num); }
@@ -666,52 +601,24 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             const double om = dden * r;
             s_w += a;
             s_g = fma(g.x, om, s_g);                       // a NaN entry (reference: ZeroDivisionError) poisons the sum
-            s_t = fma(a, (NIB_TABLOG ? log2_pos(iw, logtab) : log2_series(iw)) - g.y, s_t);
+            s_t = fma(a, log2_series(iw) - g.y, s_t);
         };
-        if constexpr (NIB_WALK && !SWEEP) {
-            if (p0 < len) {
-                constexpr int NWK = (PP + K - 1 + 15 + 15) / 16;               // aligned words: the chunk, K-1 bases of look-ahead, 16 for the walk
-                const uint32_t r0 = o_lo + p0;
-                uint32_t rw[NWK + 1];
-#pragma unroll
-                for (int j = 0; j <= NWK; ++j) rw[j] = __ldg(cw + (r0 >> 4) + j);
-                const uint32_t sc = (r0 & 15u) * 2u;
-                uint32_t Wa = __funnelshift_l(rw[1], rw[0], sc), Wb = __funnelshift_l(rw[2], rw[1], sc);
-                uint32_t Wc = NWK > 2 ? __funnelshift_l(rw[NWK > 2 ? 3 : 0], rw[2], sc) : 0u;
-                uint32_t Wd = NWK > 3 ? __funnelshift_l(rw[NWK > 3 ? 4 : 0], rw[NWK > 3 ? 3 : 0], sc) : 0u;
-                const int n_pos = (int)(len - p0) < (int)cs ? (int)(len - p0) : (int)cs;
+        const int rounds = (int)(cs >> 2);
 #pragma unroll 1
-                for (int i = 0; i < n_pos; ++i) {
-                    if (vm & (MT(1) << (MB - 1))) score_one(Wa >> (32 - 2 * K), NIB_GATHER(ig + (Wa >> (32 - 2 * K))));
-                    vm <<= 1;
-                    Wa = __funnelshift_l(Wb, Wa, 2); Wb = __funnelshift_l(Wc, Wb, 2); Wc = __funnelshift_l(Wd, Wc, 2); Wd <<= 2;
-                }
-            }
-        } else {
-            const int rounds = (int)(cs >> 2);
-            double2 gnext = NIB_PREFETCH ? NIB_GATHER(ig + (kk[0] & 0xffffu)) : make_double2(0.0, 0.0);
-#pragma unroll 1
-            for (int r = 0; r < rounds; ++r) {
-                uint32_t kp[5];
+        for (int r = 0; r < rounds; ++r) {
+            uint32_t kp[4];
 #pragma unroll
-                for (int j = 0; j < 4; ++j) kp[j] = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-                kp[4] = PP / 2 > 2 ? (kk[2 < PP / 2 ? 2 : 0] & 0xffffu) : 0u;   // first K-mer of the next round (0 past the end: a valid entry)
+            for (int j = 0; j < 4; ++j) kp[j] = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
+            // the gather is L2 only (__ldcg): the 1 MiB table never survives in a ~30 KB L1 anyway, and not allocating
+            // there measured 4.7 % faster (0.703 -> 0.671 ms on C2)
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    if constexpr (NIB_PREFETCH) {
-                        const double2 g = gnext;
-                        gnext = NIB_GATHER(ig + kp[j + 1]);                      // unconditional: an unused position holds code 0
-                        if (vm & (MT(1) << (MB - 1 - j))) score_one(kp[j], g);
-                    } else {
-                        if (vm & (MT(1) << (MB - 1 - j))) score_one(kp[j], NIB_GATHER(ig + kp[j]));
-                    }
-                }
-                vm <<= 4;
+            for (int j = 0; j < 4; ++j)
+                if (vm & (MT(1) << (MB - 1 - j))) score_one(kp[j], __ldcg(ig + kp[j]));
+            vm <<= 4;
 #pragma unroll
-                for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];     // rotate: the loop body stays one round long
+            for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];         // rotate: the loop body stays one round long
 #pragma unroll
-                for (int i = (PP / 2 > 2 ? PP / 2 - 2 : 0); i < PP / 2; ++i) kk[i] = 0;
-            }
+            for (int i = (PP / 2 > 2 ? PP / 2 - 2 : 0); i < PP / 2; ++i) kk[i] = 0;
         }
 #pragma unroll
         for (int ofs = 16; ofs; ofs >>= 1) {
@@ -814,16 +721,15 @@ int frisk_internal::score_sweep(const uint32_t* codes, const uint32_t* inv, cons
                                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* const* ig, int want_rip,
                                 double* const* rows, uint32_t* const* status, cudaStream_t st) {
     if (max_len > kSmemMaxWindow) return FRISK_E_UNSUPPORTED;
-    if (!NIB_PRE5) return FRISK_E_UNSUPPORTED;                         // (an A/B build without the order-5 fold has no sweep kernel)
     NibSweep sw{};
     for (int k = 0; k < 8; ++k) {
         if (!ig[k] || !rows[k] || !status[k]) return FRISK_E_INVALID;
         sw.ig[k] = reinterpret_cast<const double2*>(ig[k]); sw.rows[k] = rows[k]; sw.status[k] = status[k];
     }
     const int pp = window_variant(WinKernel::Nibble, max_len);
-    const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, NIB_PRE5>
-                     : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, NIB_PRE5>
-                                : (const void*)score_windows_nibble_kernel<8, 32, false, true, NIB_PRE5>;
+    const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, true>
+                     : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, true>
+                                : (const void*)score_windows_nibble_kernel<8, 32, false, true, true>;
     return with_redo_marks(nullptr, n_win, false, st, [&](uint32_t* redo) {
         int rc = launch_nibble({fn, kNT, NibLayout<8>::TOTAL, true}, codes, inv, low, win_off, win_len, n_win, nullptr, 1, want_rip,
                                nullptr, nullptr, nullptr, redo, sw, st);

@@ -399,36 +399,18 @@ int run_host_body(RunCall& c, const PeerArgs& peers, const HostPlanes& h, const 
     // then one count of 0.07 ms -- beats every split (2 chunks +0.02 ms, 3 chunks +0.04..0.1 ms): a count that runs beside
     // the copy takes about twice as long, every extra copy and count launch has a fixed cost, and the whole count is short
     // next to the upload.  Genomes of hundreds of Mbp and more keep the split: there the last chunk's count is what shows.
-    // FRISK_UPLOAD_PLAN="f0,f1,..." (relative chunk sizes) overrides the plan (tools/upload_plans.sh).
+    // (One chunk wins also when eight ranks share the host's H2D bandwidth and the upload takes twice as long, profiles/
+    // r02_pcie_contention_8gpu.json: two chunks measured 0.50 ms to the end of the count against 0.48 for one.)
+    int n_parts = (int)((h_padded_len + (64ull << 20) - 1) / (64ull << 20));
+    if (n_parts > kMaxChunks - 1) n_parts = kMaxChunks - 1;
+    if (n_parts < 1) n_parts = 1;
     uint64_t bounds[kMaxChunks + 1];
     uint64_t n_chunks = 0;
     bounds[0] = 0;
-    {
-        int parts[kMaxChunks];
-        int n_parts = (int)((h_padded_len + (64ull << 20) - 1) / (64ull << 20));
-        if (n_parts > kMaxChunks - 1) n_parts = kMaxChunks - 1;
-        if (n_parts < 1) n_parts = 1;
-        // (also when eight ranks share the host's H2D bandwidth and the upload takes twice as long, profiles/
-        // r02_pcie_contention_8gpu.json: two chunks measured 0.50 ms to the end of the count against 0.48 for one)
-        for (int i = 0; i < n_parts; ++i) parts[i] = 1;
-        if (const char* e = getenv("FRISK_UPLOAD_PLAN")) {
-            n_parts = 0;
-            for (const char* p = e; *p && n_parts < kMaxChunks - 1;) {
-                parts[n_parts++] = atoi(p);
-                while (*p && *p != ',') ++p;
-                if (*p == ',') ++p;
-            }
-        }
-        int total = 0, acc = 0;
-        for (int i = 0; i < n_parts; ++i) total += parts[i] > 0 ? parts[i] : 0;
-        for (int i = 0; i < n_parts && total > 0; ++i) {
-            if (parts[i] <= 0) continue;
-            acc += parts[i];
-            uint64_t b = i == n_parts - 1 ? h_padded_len : ((h_padded_len / (uint64_t)total) * (uint64_t)acc + 127) & ~127ull;
-            if (b > h_padded_len) b = h_padded_len;
-            if (b > bounds[n_chunks]) bounds[++n_chunks] = b;
-        }
-        if (n_chunks == 0 || bounds[n_chunks] != h_padded_len) bounds[++n_chunks] = h_padded_len;
+    for (int i = 1; i <= n_parts; ++i) {
+        uint64_t b = i == n_parts ? h_padded_len : ((h_padded_len / (uint64_t)n_parts) * (uint64_t)i + 127) & ~127ull;
+        if (b > h_padded_len) b = h_padded_len;
+        if (b > bounds[n_chunks]) bounds[++n_chunks] = b;
     }
     uint64_t counted = 0;
     for (uint64_t k = 0; k < n_chunks; ++k) {
@@ -527,7 +509,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
     WinPlan tail_plan;
     const bool dev_tail = rows_cap > 0 && rows_cap <= 0xffffffffull && (uint64_t)w <= FRISK_B200_MAX_WINDOW &&
                           frisk_internal::plan_score(kmin, kmax, len_bound, false, &tail_plan) == FRISK_OK &&
-                          tail_plan.kind == WinKernel::Nibble && !getenv("FRISK_RUN_FASTA_HOST_TAIL");
+                          tail_plan.kind == WinKernel::Nibble;
     void *dtab = nullptr, *dig = nullptr, *dwin = nullptr, *dfirst = nullptr, *dscal = nullptr;
     Rows r{};
     bool tail_queued = false;
