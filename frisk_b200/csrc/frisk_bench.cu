@@ -4,7 +4,8 @@
 //                                {I_g, log2 I_g} pair per distinct K-mer out of a 1 MiB table)
 //   frisk_b200_bench_smem_loads  random 4/8/16-byte loads from a 32 KiB shared-memory table (bank-conflicted reads:
 //                                what a position-ordered epilogue does to its count tables)
-// (the shared-memory ATOMIC rate is frisk_b200_bench_smem_atomics in frisk_kernels.cu)
+//   frisk_b200_bench_smem_atomics  u32 shared-memory atomics on a 64 KiB table: one lane per bank, random bins or one
+//                                address (the counting step of the window and table kernels)
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -201,6 +202,28 @@ smem_load_kernel(int iters, T* sink) {
     if (acc == 0xdeadbeefu) *reinterpret_cast<uint32_t*>(sink) = acc;
 }
 
+// Shared-memory atomic micro-benchmark (roofline denominator for the counting step): one CTA of 1,024 threads per SM
+constexpr int kThreads = 1024;
+
+__global__ void __launch_bounds__(kThreads, 1) smem_atomic_bench_kernel(int iters, int mode, uint32_t* sink) {
+    extern __shared__ __align__(16) uint32_t tab[];
+    constexpr uint32_t N = 16384;   // 64 KiB of u32 bins
+    for (uint32_t i = threadIdx.x; i < N; i += kThreads) tab[i] = 0;
+    __syncthreads();
+    uint32_t x = threadIdx.x * 2654435761u + blockIdx.x * 40503u + 12345u;
+    for (int it = 0; it < iters; ++it) {
+        uint32_t idx;
+        if (mode == 0) idx = (threadIdx.x + 32u * (uint32_t)it) & (N - 1);        // one lane per bank
+        else if (mode == 1) { x = x * 1664525u + 1013904223u; idx = (x >> 10) & (N - 1); }   // random bins
+        else idx = 0;                                                              // one address
+        atomicAdd(&tab[idx], 1u);
+    }
+    __syncthreads();
+    uint32_t s = 0;
+    for (uint32_t i = threadIdx.x; i < N; i += kThreads) s += tab[i];
+    if (s == 0xdeadbeefu) sink[0] = s;
+}
+
 template <typename F>
 int time_twice(F launch, cudaStream_t st, float* ms) {
     cudaEvent_t a, b;
@@ -296,6 +319,28 @@ int frisk_b200_bench_smem_loads(int blocks, int iters, int elem_bytes, float* ms
     else rc = FRISK_E_INVALID;
     cudaFree(sink);
     return rc;
+}
+
+int frisk_b200_bench_smem_atomics(int blocks, int iters, int mode, float* ms, void* stream) {
+    if (blocks <= 0 || iters <= 0 || !ms) return FRISK_E_INVALID;
+    cudaStream_t st = (cudaStream_t)stream;
+    CK(cudaFuncSetAttribute(smem_atomic_bench_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 65536));
+    uint32_t* sink = nullptr;
+    CK(cudaMalloc(&sink, 4));
+    cudaEvent_t a, b;
+    CK(cudaEventCreate(&a));
+    CK(cudaEventCreate(&b));
+    smem_atomic_bench_kernel<<<blocks, kThreads, 65536, st>>>(iters, mode, sink);   // warm-up
+    CK(cudaEventRecord(a, st));
+    smem_atomic_bench_kernel<<<blocks, kThreads, 65536, st>>>(iters, mode, sink);
+    CK(cudaEventRecord(b, st));
+    CK(cudaEventSynchronize(b));
+    CK(cudaEventElapsedTime(ms, a, b));
+    CK(cudaEventDestroy(a));
+    CK(cudaEventDestroy(b));
+    CK(cudaFree(sink));
+    CK(cudaGetLastError());
+    return FRISK_OK;
 }
 
 }  // extern "C"

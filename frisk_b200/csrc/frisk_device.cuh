@@ -1,4 +1,4 @@
-// Device helpers shared by the translation units that hold score kernels (frisk_kernels.cu, frisk_direct.cu).
+// Device helpers shared by the translation units that hold the table and window kernels.
 #ifndef FRISK_DEVICE_CUH
 #define FRISK_DEVICE_CUH
 
@@ -12,6 +12,19 @@ constexpr uint32_t kFull = 0xffffffffu;
 __host__ __device__ constexpr uint32_t pow4(int k) { return 1u << (2 * k); }
 // offset (in entries) of order x inside a concatenation of orders 1..: sum_{y<x} 4^y
 __host__ __device__ constexpr uint32_t lvl_off(int x) { return (pow4(x) - 4u) / 3u; }
+
+// gather bit1 of each of the 16 2-bit codes of a word into 16 contiguous bits (order kept)
+__device__ __forceinline__ uint32_t high_bits16(uint32_t w) {
+    uint32_t x = (w >> 1) & 0x55555555u;
+    x = (x | (x >> 1)) & 0x33333333u;
+    x = (x | (x >> 2)) & 0x0f0f0f0fu;
+    x = (x | (x >> 4)) & 0x00ff00ffu;
+    x = (x | (x >> 8)) & 0x0000ffffu;
+    return x;
+}
+
+// bytes of the result = sums of the two nibbles of each byte of w (<= 30)
+__device__ __forceinline__ uint32_t nib_pairs(uint32_t w) { return (w & 0x0f0f0f0fu) + ((w >> 4) & 0x0f0f0f0fu); }
 
 __device__ __forceinline__ double u32_to_double(uint32_t v) {
     // exact: 2^52 + v has v in the low mantissa bits

@@ -15,7 +15,7 @@
 //     enumerating them; a thread's positions are fixed and so is the reduction tree -> bit-reproducible rows.
 // Two atomics and one epilogue per position; 3 CTAs per SM (73 KB each).
 //
-// What a byte cannot hold is handed to the bucketed kernel (frisk_kernels.cu), exactly: a window in which some
+// What a byte cannot hold is handed to the bucketed kernel (frisk_bucket.cu), exactly: a window in which some
 // K-mer occurs 256+ times (the thread whose increment wraps the byte sees 255 in the word it got back), or
 // with more than kSideCap words cut short by an N / the window end at K-1 or K-2 bases, is marked kRowRedo in
 // `status` and re-done by the launch that follows on the same stream.  Short words of K-1 / K-2 bases (every

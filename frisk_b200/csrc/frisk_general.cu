@@ -1,7 +1,7 @@
 // frisk_b200 general path: runtime K (1..12) and windows of any length.
 //
 // The reference accepts any --minWordSize/--maxWordSize/--windowlen (F:1197-1216); its defaults are
-// 1..8 and 5,000.  The tuned kernels in frisk_kernels.cu keep a window's tables in shared memory,
+// 1..8 and 5,000.  The tuned window kernels keep a window's tables in shared memory,
 // which caps them at K <= 8 and 65,535 bases.  Everything beyond that comes here: same arithmetic,
 // same table/row conventions, but the tables of orders >= 7 live in a per-CTA slab of global memory
 // (L2-resident for the sizes that matter) and K is a run-time value.
@@ -96,7 +96,7 @@ gen_sym_kernel(unsigned long long* __restrict__ tables, int K) {
     }
 }
 
-// ---- genome IVOM (closed form, see genome_ivom_kernel in frisk_kernels.cu) -----------------------
+// ---- genome IVOM (closed form, see genome_ivom_kernel in frisk_tables.cu) ------------------------
 __global__ void __launch_bounds__(256)
 gen_ivom_kernel(const unsigned long long* __restrict__ tables, int kmin, int K, long long space, double2* __restrict__ ig) {
     const uint64_t kappa = (uint64_t)blockIdx.x * 256u + threadIdx.x;

@@ -21,7 +21,7 @@ namespace frisk_internal {
 // records the CUDA error text for frisk_b200_last_cuda_error() and returns FRISK_E_CUDA
 int cuda_fail(cudaError_t e, const char* what);
 
-// once per device: let the default memory pool keep up to 32 GiB of freed cudaMallocAsync scratch (frisk_kernels.cu says why)
+// once per device: let the default memory pool keep up to 32 GiB of freed cudaMallocAsync scratch (frisk_common.cu says why)
 int pool_ready();
 extern int g_ingest_exact, g_ingest_chunk_tiles;   // frisk_ingest.cu; set through frisk_b200_set_option
 
@@ -59,7 +59,7 @@ int bgzf_inflate(const uint8_t* d_gz, const uint64_t* d_comp_off, const uint32_t
 extern int g_gzip_chunk_bytes;                     // compressed bytes per nominal chunk (0 = default); frisk_b200_set_option
 int gzip_inflate(const uint8_t* d_gz, const uint8_t* h_gz, uint64_t n, const std::function<int(uint64_t, uint8_t**)>& alloc_text,
                  uint64_t* text_len, uint64_t stats[4], cudaStream_t st);
-// background count of a word range that lives in device memory (frisk_kernels.cu); kmax <= FRISK_B200_FAST_K
+// background count of a word range that lives in device memory (frisk_tables.cu); kmax <= FRISK_B200_FAST_K
 int background_device_range(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const unsigned long long* d_word_range,
                             uint64_t words_hint, int kmax, int mask_host, uint64_t* fwd, cudaStream_t st);
 
@@ -87,6 +87,20 @@ int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* lo
 // FRISK_E_INVALID unless 1 <= kmin <= kmax; FRISK_E_UNSUPPORTED for kmax > FRISK_B200_MAX_K
 int check_k(int kmin, int kmax);
 
+// `return expr;` with the run-time kmax as the compile-time constant K (1..8); FRISK_E_UNSUPPORTED for any other kmax
+#define DISPATCH_K(kmax, expr)                      \
+    switch (kmax) {                                 \
+        case 1: { constexpr int K = 1; return expr; } \
+        case 2: { constexpr int K = 2; return expr; } \
+        case 3: { constexpr int K = 3; return expr; } \
+        case 4: { constexpr int K = 4; return expr; } \
+        case 5: { constexpr int K = 5; return expr; } \
+        case 6: { constexpr int K = 6; return expr; } \
+        case 7: { constexpr int K = 7; return expr; } \
+        case 8: { constexpr int K = 8; return expr; } \
+        default: return FRISK_E_UNSUPPORTED;        \
+    }
+
 // most ranks a sharded finalize sums over (frisk_b200_finalize_ivom, frisk_b200_run_host_peers)
 constexpr int kMaxPeers = 16;
 // frisk_b200_finalize_ivom without its argument checks (the run paths of frisk_run.cu have made them).  space_dev
@@ -98,7 +112,7 @@ int finalize_ivom(const uint64_t* d_fwd, const uint64_t* const* d_fwd_peers, uin
 // Longest window the shared-memory window kernels hold: an 8,192-base buffer less 6 bases of look-ahead.
 constexpr uint32_t kSmemMaxWindow = 8186u;
 
-// The window kernels of frisk_b200_score and how one of them is instantiated for a call.  plan_score (frisk_kernels.cu)
+// The window kernels of frisk_b200_score and how one of them is instantiated for a call.  plan_score (frisk_score.cu)
 // is the one place that chooses them, from (kmin, kmax, longest window, dump) and the kernel forced through
 // frisk_b200_set_option.  variant: ROUNDS of the bucketed and direct kernels or PP of the nibble and extension kernels,
 // positions per thread from the longest window (window_variant).  dump / allk pick the <DUMP, ALLK> instantiation.
@@ -162,6 +176,30 @@ int with_redo_marks(uint32_t* status, uint64_t n_win, bool zero, cudaStream_t st
     return rc;
 }
 
+// A *_shape function expects a K its kernel serves (a plan only picks a kernel for those); a score_* entry refuses any
+// other K with FRISK_E_UNSUPPORTED.
+//
+// small-K kernel (frisk_small.cu): kmax 1..6, windows <= 65,535 bases.  redo_src: only the windows marked kRowRedo there.
+LaunchShape small_shape(const WinPlan& p, int K);
+int score_small(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+                const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int K, int want_rip, double* rows,
+                uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr);
+// bucketed kernel (frisk_bucket.cu): kmax 4..8, windows <= kSmemMaxWindow bases; its buffer is sized by max_len
+LaunchShape bucket_shape(const WinPlan& p, int K, uint32_t max_len);
+int score_bucket(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
+                 double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr);
+// The hand-over target of the direct and nibble kernels and of the k sweep (frisk_score.cu): the windows marked kRowRedo
+// in redo_src, re-done on the small-K kernel for K <= 3 and on the bucketed kernel for K >= 4.
+int score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
+                      const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
+                      double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src, cudaStream_t st);
+// dense-table kernel (frisk_dense.cu): kmax 1..8, windows <= 65,535 bases; one CTA of dense_shape(K).threads per SM
+LaunchShape dense_shape(int K);
+int score_dense(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,
+                uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip, double* rows, uint32_t* status,
+                uint16_t* dump, cudaStream_t st);
+
 // kmax 9..12, windows <= kSmemMaxWindow bases (frisk_nibble_ext.cu): orders 1..8 as in the kmax-8 nibble kernel, orders
 // 9..K from the observation that an 8-mer seen once has only unique extensions (the few repeated ones go through a
 // shared-memory hash table).  What it cannot hold is re-done by general_score behind it.
@@ -171,14 +209,11 @@ int score_nibble_ext(const WinPlan& p, const uint32_t* codes, const uint32_t* in
                      double* rows, uint32_t* status, cudaStream_t st);
 
 // direct score kernel (frisk_direct.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases.  Windows it cannot finish exactly
-// (a K-mer seen 256+ times, more than 64 N-boundary words) are re-done by the bucketed kernel (frisk_kernels.cu).
+// (a K-mer seen 256+ times, more than 64 N-boundary words) are re-done by score_bucket_redo.
 LaunchShape direct_shape(const WinPlan& p, int K);
 int score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st);
-int score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                      const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                      double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src, cudaStream_t st);
 
 // nibble score kernel (frisk_nibble.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases; one 4-bit counter per K-mer, one
 // atomic per position, the first occurrence of a K-mer scores it.  Windows with a K-mer seen 16+ times (or more than 64

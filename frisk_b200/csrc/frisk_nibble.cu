@@ -18,7 +18,7 @@
 //   * a thread's positions are fixed and so is the reduction tree -> bit-reproducible rows.
 // 40-56 KB of shared memory per CTA (K = 8).
 //
-// What a nibble cannot hold is handed to the bucketed kernel (frisk_kernels.cu), exactly: a window in which some
+// What a nibble cannot hold is handed to the bucketed kernel (frisk_bucket.cu), exactly: a window in which some
 // K-mer occurs 16+ times (the thread whose increment wraps the nibble sees 15 in the word it got back), or with
 // more than kSideCap words cut short by an N / the window end at K-1 or K-2 bases, is marked kRowRedo and re-done
 // by the launch that follows on the same stream.  Short words of K-1 / K-2 bases (every window has two at its
@@ -67,19 +67,6 @@ struct NibLayout {
     static constexpr uint32_t OFF_SS = OFF_PREA + NPREA * 16u;
     static constexpr uint32_t TOTAL = OFF_SS + (uint32_t)sizeof(NibSmem);
 };
-
-// bytes of the result = sums of the two nibbles of each byte of w (<= 30)
-__device__ __forceinline__ uint32_t nib_pairs(uint32_t w) { return (w & 0x0f0f0f0fu) + ((w >> 4) & 0x0f0f0f0fu); }
-
-// gather bit1 of each of the 16 2-bit codes of a word into 16 contiguous bits (order kept)
-__device__ __forceinline__ uint32_t nib_high_bits16(uint32_t w) {
-    uint32_t x = (w >> 1) & 0x55555555u;
-    x = (x | (x >> 1)) & 0x33333333u;
-    x = (x | (x >> 2)) & 0x0f0f0f0fu;
-    x = (x | (x >> 4)) & 0x00ff00ffu;
-    x = (x | (x >> 8)) & 0x0000ffffu;
-    return x;
-}
 
 // Per-thread position masks: position i of the thread's chunk is bit (MB - 1 - i).  32 bits when the chunk and the
 // K - 1 bases of look-ahead fit (PP + K - 1 <= 32), 64 bits otherwise.
@@ -193,7 +180,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                 MT G = 0;                                                // bit 1 of the code: G = 2, C = 3 (invalid bases carry code 0)
 #pragma unroll
                 for (int j = 0; j < NA; ++j)
-                    if (MB - 16 - 16 * j >= 0) G |= (MT)nib_high_bits16(W[j]) << (MB - 16 - 16 * j);
+                    if (MB - 16 - 16 * j >= 0) G |= (MT)high_bits16(W[j]) << (MB - 16 - 16 * j);
                 non = popc_m(unres);
                 gc = popc_m(G & in_p & ~unres);
                 nfull = popc_m(vm);

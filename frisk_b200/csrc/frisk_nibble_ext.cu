@@ -58,17 +58,6 @@ struct ExtLayout {
     static constexpr uint32_t TOTAL = OFF_SS + (uint32_t)sizeof(ExtSmem);
 };
 
-__device__ __forceinline__ uint32_t nib_pairs(uint32_t w) { return (w & 0x0f0f0f0fu) + ((w >> 4) & 0x0f0f0f0fu); }
-
-__device__ __forceinline__ uint32_t ext_high_bits16(uint32_t w) {
-    uint32_t x = (w >> 1) & 0x55555555u;
-    x = (x | (x >> 1)) & 0x33333333u;
-    x = (x | (x >> 2)) & 0x0f0f0f0fu;
-    x = (x | (x >> 4)) & 0x00ff00ffu;
-    x = (x | (x >> 8)) & 0x0000ffffu;
-    return x;
-}
-
 __device__ __forceinline__ unsigned long long top_bits64(int n) { return n >= 64 ? ~0ull : ~(~0ull >> n); }
 
 // tag of the order-x prefix `code` (2x bits, x = 9..12): never 0
@@ -154,7 +143,7 @@ score_windows_nibble_ext_kernel(const uint32_t* __restrict__ codes, const uint32
                 const MT vm8 = ~sm & in_p;                               // 8+ valid bases from here
                 MT G = 0;
 #pragma unroll
-                for (int j = 0; j < NAW && j < 4; ++j) G |= (MT)ext_high_bits16(W[j]) << (MB - 16 - 16 * j);
+                for (int j = 0; j < NAW && j < 4; ++j) G |= (MT)high_bits16(W[j]) << (MB - 16 - 16 * j);
                 non = __popcll(unres);
                 gc = __popcll(G & in_p & ~unres);
                 nfull = __popcll(vm8);
