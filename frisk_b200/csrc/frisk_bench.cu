@@ -1,7 +1,8 @@
 // frisk_b200: micro-benchmarks that measure the roofline denominators of the window kernels on the GPU at hand
 // (bench.py calls them live; SURVEY.md section 8d asks for measured, not assumed, rates):
 //   frisk_b200_bench_l2_gather   random 16-byte gathers from an L2-resident table (the genome-IVOM lookup: one
-//                                {I_g, log2 I_g} pair per distinct K-mer out of a 1 MiB table)
+//                                {I_g, log2 I_g} pair per distinct K-mer out of a 1 MiB table); mode 7: 32-byte entries
+//                                with one 256-bit load each (the nibble kernel's (K+1)-mer pair table)
 //   frisk_b200_bench_smem_loads  random 4/8/16-byte loads from a 32 KiB shared-memory table (bank-conflicted reads:
 //                                what a position-ordered epilogue does to its count tables)
 //   frisk_b200_bench_smem_atomics  u32 shared-memory atomics on a 64 KiB table: one lane per bank, random bins or one
@@ -12,6 +13,7 @@
 
 #include "../../include/frisk_b200.h"
 #include "frisk_internal.h"
+#include "frisk_device.cuh"
 
 namespace {
 #define CK(call) FRISK_CK(call)
@@ -164,6 +166,23 @@ l2_gather4_kernel(const __grid_constant__ CUtensorMap map, uint32_t n_mask, int 
     if (a0 == 1.2345e-300) sink[0] = a0;
 }
 
+// mode 7: the random gather of mode 0 with 32-byte entries, each read by one 256-bit load (ldcg_pair): the nibble kernel's
+// (K+1)-mer pair table, 8 MiB at K = 8 and 2 MiB at K = 7
+__global__ void __launch_bounds__(256, 4)
+l2_gather32_kernel(const double2* __restrict__ tab, uint32_t n_mask, int iters, double* sink) {
+    uint32_t x = (blockIdx.x * 256u + threadIdx.x) * 2654435761u + 12345u;
+    double a0 = 0, a1 = 0, a2 = 0, a3 = 0;
+    for (int it = 0; it < iters; it += 4) {
+        const uint32_t i0 = lcg(x), i1 = lcg(x), i2 = lcg(x), i3 = lcg(x);
+        double2 u0, v0, u1, v1, u2, v2, u3, v3;
+        ldcg_pair(tab + 2u * (i0 & n_mask), u0, v0); ldcg_pair(tab + 2u * (i1 & n_mask), u1, v1);
+        ldcg_pair(tab + 2u * (i2 & n_mask), u2, v2); ldcg_pair(tab + 2u * (i3 & n_mask), u3, v3);
+        a0 += u0.x + v0.y; a1 += u1.x + v1.y; a2 += u2.x + v2.y; a3 += u3.x + v3.y;
+    }
+    const double s = a0 + a1 + a2 + a3;
+    if (s == 1.2345e-300) sink[0] = s;
+}
+
 __global__ void fill_pattern_kernel(double2* tab, uint32_t n) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) tab[i] = make_double2((double)i, -(double)i);
@@ -245,7 +264,7 @@ int time_twice(F launch, cudaStream_t st, float* ms) {
 extern "C" {
 
 int frisk_b200_bench_l2_gather(int blocks, int iters, uint64_t table_bytes, int mode, float* ms, void* stream) {
-    if (blocks <= 0 || iters <= 0 || (iters & 3) || !ms || table_bytes < 4096 || (table_bytes & (table_bytes - 1)) || mode < 0 || mode > 6)
+    if (blocks <= 0 || iters <= 0 || (iters & 3) || !ms || table_bytes < 4096 || (table_bytes & (table_bytes - 1)) || mode < 0 || mode > 7)
         return FRISK_E_INVALID;
     if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -299,6 +318,7 @@ int frisk_b200_bench_l2_gather(int blocks, int iters, uint64_t table_bytes, int 
         if (!rc && h_bad) rc = h_bad >= 1000000u ? FRISK_E_UNSUPPORTED : FRISK_E_FORMAT;   // never completed / wrong data
     } else if (mode == 2) rc = time_twice([&] { l2_gather_async_kernel<<<blocks, 256, 0, st>>>(tab, n_mask, iters, sink); }, st, ms);
     else if (mode == 4) rc = time_twice([&] { l2_gather_bulk_kernel<<<blocks, 256, 0, st>>>(tab, n_mask, iters, sink); }, st, ms);
+    else if (mode == 7) rc = time_twice([&] { l2_gather32_kernel<<<blocks, 256, 0, st>>>(tab, (n_mask - 1u) / 2u, iters, sink); }, st, ms);
     else if (mode == 3) rc = time_twice([&] { l2_gather8_kernel<<<blocks, 256, 0, st>>>((const double*)tab, 2u * n_mask + 1u, iters, sink); }, st, ms);
     else rc = time_twice([&] { l2_gather_kernel<<<blocks, 256, 0, st>>>(tab, n_mask, iters, mode, gap, sink); }, st, ms);
     cudaFree(tab);

@@ -91,6 +91,13 @@ __device__ __forceinline__ double div_pos(double n, double d) {
     return fma(fma(-d, q, n), r, q);
 }
 
+// The 32-byte entry at p (32-byte aligned) as two double2, with ONE 256-bit load cached in L2 only (as __ldcg): on sm_100
+// this is a single LDG.E.ENL2.256, so a fully divergent gather of 32-byte entries costs a warp no more wavefronts than one
+// of 16-byte entries.
+__device__ __forceinline__ void ldcg_pair(const double2* p, double2& a, double2& b) {
+    asm volatile("ld.global.cg.v4.f64 {%0, %1, %2, %3}, [%4];" : "=d"(a.x), "=d"(a.y), "=d"(b.x), "=d"(b.y) : "l"(p));
+}
+
 // One round of the position walk: the four absolute-aligned bases of group `gi` (see below), with
 // the words they need loaded once.  f(j, p, c32, m, low_bit) for the positions inside the window:
 // j = 0..3, p = position in the window, c32 = the 16 bases from p (2 bits each, first base on top),

@@ -218,7 +218,8 @@ int score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, c
 // nibble score kernel (frisk_nibble.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases; one 4-bit counter per K-mer, one
 // atomic per position, the first occurrence of a K-mer scores it.  Windows with a K-mer seen 16+ times (or more than 64
 // N-boundary words) are re-done by the bucketed kernel, exactly like the direct kernel's hand-over.  n_win_dev: the window
-// count in device memory, n_win its capacity.
+// count in device memory, n_win its capacity.  It reads ig through a (K+1)-mer pair table it builds in stream-ordered scratch
+// before its launch (frisk_nibble.cu); the hand-over reads ig itself.
 LaunchShape nibble_shape(const WinPlan& p, int K);
 int score_nibble(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,

@@ -100,7 +100,7 @@ template <int K, int PP, bool DUMP, bool ALLK, bool SWEEP = false>
 __global__ void __launch_bounds__(kNT, 4)
 score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ inv, const uint32_t* __restrict__ low,
                             const unsigned long long* __restrict__ win_off, const uint32_t* __restrict__ win_len, uint32_t n_win,
-                            const double2* __restrict__ ig, int kmin_arg, int want_rip,
+                            const double2* __restrict__ pair, int kmin_arg, int want_rip,
                             double* __restrict__ rows, uint32_t* __restrict__ status, uint16_t* __restrict__ dump,
                             uint32_t* redo_dst, const NibSweep sw) {
     static_assert(!SWEEP || (K == 8 && ALLK && !DUMP), "the sweep instantiation: K = 8, kmin = 1");
@@ -596,11 +596,21 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             uint32_t kp[4];
 #pragma unroll
             for (int j = 0; j < 4; ++j) kp[j] = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-            // the gather is L2 only (__ldcg): the 1 MiB table never survives in a ~30 KB L1 anyway, and not allocating
-            // there measured 4.7 % faster (0.703 -> 0.671 ms on C2)
+            // positions j and j + 1 fetch both genome-IVOM entries with ONE 32-byte load from the pair table, at the
+            // (K+1)-mer of bases j .. j+K.  Only j + 1 valid: its K-mer with a leading A (the second half is still its
+            // entry).  Only j valid: the first half is used, kp[j + 1] & 3 only keeps mu in range.  L2 only (.cg): the
+            // table never survives in a ~30 KB L1 anyway, and not allocating there measured faster (0.703 -> 0.671 ms on C2)
 #pragma unroll
-            for (int j = 0; j < 4; ++j)
-                if (vm & (MT(1) << (MB - 1 - j))) score_one(kp[j], __ldcg(ig + kp[j]));
+            for (int j = 0; j < 4; j += 2) {
+                const bool v0 = vm & (MT(1) << (MB - 1 - j)), v1 = vm & (MT(1) << (MB - 2 - j));
+                if (v0 || v1) {
+                    const uint32_t mu = v0 ? ((kp[j] << 2) | (kp[j + 1] & 3u)) : kp[j + 1];
+                    double2 g0, g1;
+                    ldcg_pair(pair + 2u * mu, g0, g1);
+                    if (v0) score_one(kp[j], g0);
+                    if (v1) score_one(kp[j + 1], g1);
+                }
+            }
             vm <<= 4;
 #pragma unroll
             for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];         // rotate: the loop body stays one round long
@@ -661,6 +671,16 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
     }
 }
 
+// The pair table of P3: P[mu] = {ig[mu >> 2], ig[mu & (4^K - 1)]} for every (K+1)-mer mu, i.e. the genome-IVOM entries of
+// the K-mers at two adjacent positions p, p + 1 (bases p .. p+K) in one 32-byte entry, 4^(K+1) x 32 B (8 MiB at K = 8, 2 MiB
+// at K = 7).  Bits are copied: a NaN entry (query k-mer absent from the host, the reference's ZeroDivisionError) stays NaN.
+template <int K>
+__global__ void __launch_bounds__(256) ivom_pair_kernel(const uint4* __restrict__ ig, uint4* __restrict__ pair) {
+    const uint32_t mu = blockIdx.x * 256u + threadIdx.x;                 // the grid covers 4^(K+1) exactly
+    pair[2u * mu] = __ldg(ig + (mu >> 2));
+    pair[2u * mu + 1u] = __ldg(ig + (mu & (pow4(K) - 1u)));
+}
+
 template <int K>
 const void* nibble_fn(const frisk_internal::WinPlan& p) {
     if (p.variant == 8) return FRISK_WIN_INSTANCE(p, score_windows_nibble_kernel, K, 8);
@@ -670,12 +690,11 @@ const void* nibble_fn(const frisk_internal::WinPlan& p) {
 
 // one launch of a nibble-kernel instantiation, the sweep's included (they share the signature)
 int launch_nibble(const frisk_internal::LaunchShape& s, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                  const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int want_rip,
+                  const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, const double2* pair, int kmin, int want_rip,
                   double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, NibSweep sw, cudaStream_t st) {
     const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-    const double2* g = reinterpret_cast<const double2*>(ig);
     uint32_t n = (uint32_t)n_win;
-    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo_dst, &sw};
+    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &pair, &kmin, &want_rip, &rows, &status, &dump, &redo_dst, &sw};
     return frisk_internal::launch_persistent(s, n_win, args, st);
 }
 
@@ -693,13 +712,26 @@ int frisk_internal::score_nibble(const WinPlan& p, const uint32_t* codes, const 
     if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
     NibSweep sw{};
     sw.n_win_dev = n_win_dev;
-    return with_redo_marks(status, n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
-        int rc = launch_nibble(nibble_shape(p, K), codes, inv, low, win_off, win_len, n_win, ig, kmin, want_rip, rows, status, dump,
-                               redo, sw, st);
-        // windows the nibble table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
-        return rc ? rc : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump,
-                                           redo, st);
-    });
+    // the pair table: stream-ordered scratch, built from ig right before the window kernel, freed behind the hand-over
+    int rc = pool_ready();
+    if (rc) return rc;
+    const uint32_t n_pair = pow4(K + 1);
+    uint4* pair = nullptr;
+    FRISK_CK(cudaMallocAsync((void**)&pair, (size_t)n_pair * 32u, st));
+    (K == 8 ? ivom_pair_kernel<8> : ivom_pair_kernel<7>)<<<n_pair / 256u, 256, 0, st>>>(reinterpret_cast<const uint4*>(ig), pair);
+    const cudaError_t le = cudaGetLastError();
+    if (le != cudaSuccess) rc = cuda_fail(le, "ivom_pair_kernel");
+    if (!rc)
+        rc = with_redo_marks(status, n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
+            int rc2 = launch_nibble(nibble_shape(p, K), codes, inv, low, win_off, win_len, n_win, reinterpret_cast<const double2*>(pair),
+                                    kmin, want_rip, rows, status, dump, redo, sw, st);
+            // windows the nibble table could not hold (marked kRowRedo): exact re-run on the bucketed kernel, which reads ig
+            return rc2 ? rc2 : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status,
+                                                 dump, redo, st);
+        });
+    const cudaError_t e = cudaFreeAsync(pair, st);                     // stream-ordered: behind the launches above
+    if (!rc && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync(pair table)");
+    return rc;
 }
 
 // The k sweep: rows of kmax' = 1..8 (kmin 1) for every window from one pass (see NibSweep).  A window the 4-bit counters

@@ -505,8 +505,8 @@ int frisk_b200_bench_smem_atomics(int blocks, int iters, int mode, float *ms, vo
  *   entry; mode 1: a warp's lanes read increasing entries with random gaps (the sorted epilogue's pattern); mode 2: mode 0
  *   as 16-byte cp.async into shared memory; mode 3: mode 0 with 8-byte entries; mode 4: mode 0 as 16-byte cp.async.bulk
  *   copies (the TMA engine) completing on an mbarrier; mode 5: as TMA tile::gather4 loads (4 rows per instruction; the
- *   gathered data is verified: FRISK_E_UNSUPPORTED = never completed, FRISK_E_FORMAT = wrong data).
- *   gathers = blocks*256*iters.
+ *   gathered data is verified: FRISK_E_UNSUPPORTED = never completed, FRISK_E_FORMAT = wrong data); mode 7: mode 0 with
+ *   32-byte entries, each read by one 256-bit load.  gathers = blocks*256*iters.
  * _smem_loads: `blocks` x 256 threads each issue `iters` random loads of `elem_bytes` (4, 8 or 16) from a 32 KiB
  *   shared-memory table (bank-conflicted reads).  loads = blocks*256*iters. */
 int frisk_b200_bench_l2_gather(int blocks, int iters, uint64_t table_bytes, int mode, float *ms, void *stream);

@@ -48,6 +48,24 @@ if len(sys.argv) > 1 and sys.argv[1] == "tex":
                                               "ldg_random_64KiB": best(lambda: gathers(0, 1 << 16)),
                                               "tex1Dfetch_random_64KiB": best(lambda: gathers(6, 1 << 16))}}))
     sys.exit(0)
+if len(sys.argv) > 1 and sys.argv[1] == "pairs":
+    # the nibble kernel's pair gather: one 256-bit load of a 32-byte entry out of the (K+1)-mer pair table (8 MiB at K = 8,
+    # 2 MiB at K = 7) against today's 16-byte gather from the 1 MiB genome-IVOM table; the three alternate, 7 rounds
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    legs = {"mode0_16B_1MiB": (0, 1 << 20), "mode7_32B_8MiB": (7, 1 << 23), "mode7_32B_2MiB": (7, 1 << 21)}
+    runs = {k: [] for k in legs}
+    for _ in range(7):
+        for k, (mode, nbytes) in legs.items():
+            runs[k].append(gathers(mode, nbytes))
+    med = {k: sorted(v)[len(v) // 2] for k, v in runs.items()}
+    print(json.dumps({"gpu": q.stdout.strip() if q.returncode == 0 else "not available",
+                      "gathers_per_s_median": med, "gathers_per_s_runs": runs,
+                      "ratio_to_mode0": {k: med[k] / med["mode0_16B_1MiB"] for k in med},
+                      "note": "requests (one entry per lane) per second, 148 x 4 CTAs of 256 threads, 2,048 loads per thread, "
+                              "uniformly random entries; mode 0 is __ldg of 16 B, mode 7 ld.global.cg.v4.f64 of 32 B"}))
+    sys.exit(0)
 if len(sys.argv) > 1 and sys.argv[1] == "gather4":
     # (probed and removed: a tensor-map box of 4 rows is rejected, and destinations that are only 64- or 80-byte aligned
     # fault with cudaErrorMisalignedAddress: every gather4 needs a 128-byte aligned 64-byte landing slot)
