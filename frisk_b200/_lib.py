@@ -77,6 +77,11 @@ PROTOTYPES = {
     "frisk_b200_fasta_open_gzip": (_i, [_p, _u64, _p, C.POINTER(C.c_void_p), C.POINTER(_u64), C.POINTER(_u64), _p]),
     "frisk_b200_run_fasta_gzip": (_i, [_p, _u64, _p, _u64, _i, _i, _i, _i, _i, _i, _i, _u64, _p, _p, _p, _p, C.POINTER(_u64),
                                        C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _p]),
+    "frisk_b200_2bit_records": (_i, [_p, _u64, _u64, _p, _p, _p, C.POINTER(_u64), C.POINTER(_u64)]),
+    "frisk_b200_2bit_unpack_host": (_i, [_p, _u64, _u64, _p, _p, _p, _p]),
+    "frisk_b200_fasta_open_2bit": (_i, [_p, _u64, _p, C.POINTER(C.c_void_p), C.POINTER(_u64), C.POINTER(_u64), _p]),
+    "frisk_b200_run_2bit": (_i, [_p, _u64, _p, _u64, _i, _i, _i, _i, _i, _i, _i, _u64, _p, _p, _p, _p, C.POINTER(_u64),
+                                 C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _p]),
     "frisk_b200_fasta_planes": (_i, [_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     "frisk_b200_last_run_timing": (_i, [C.POINTER(C.c_float), _i, C.POINTER(_i)]),
     "frisk_b200_score_sweep": (_i, [_p, _p, _p, _p, _p, _u64, C.c_uint32, _p, _i, _i, _p, _p, _p]),

@@ -25,6 +25,8 @@
 // upload lane, frisk_bgzf.cu inflates them into the text buffer, and the passes wait on that instead of on the text's copy.
 // A gzip source (frisk_b200_fasta_open_gzip, frisk_b200_run_fasta_gzip) is inflated first (frisk_gzip.cu synchronises: its
 // text length is only known at the end) and the open takes over the text buffer it filled, as the BGZF exact re-open does.
+// A .2bit file (frisk_b200_fasta_open_2bit, frisk_b200_run_2bit) is not text: frisk_twobit.cu decodes it into planes and a
+// record table of its own, and fasta_adopt makes the handle and does what the passes above do behind the last chunk.
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -61,7 +63,8 @@ enum { kCtrRecords = 0, kCtrNonUpper = 1, kCtrLower = 2, kCtrWhitespace = 3, kCt
        kRangeSlots = 2 };      // per chunk, behind the counters: {word_lo, word_hi}
 
 static_assert((int)kCtrRecords == (int)frisk_internal::kIngestRecords && (int)kCtrNonUpper == (int)frisk_internal::kIngestNonUpper &&
-              (int)kCtrOverflow == (int)frisk_internal::kIngestOverflow, "frisk_internal.h names these counters");
+              (int)kCtrLower == (int)frisk_internal::kIngestLower && (int)kCtrOverflow == (int)frisk_internal::kIngestOverflow &&
+              (int)kCtrCount == (int)frisk_internal::kIngestRange, "frisk_internal.h names these counters");
 
 // class of a byte: 0..3 = A,T,G,C (F:70 order); 4..7 = a,t,g,c; 8 = anything else; 9 = whitespace
 // removed by the reference's line.strip() (F:149)
@@ -1115,6 +1118,14 @@ int open_handle(const char* text, uint64_t n, frisk_internal::TextFormat fmt, cu
     frisk_b200_fasta* h = new (std::nothrow) frisk_b200_fasta();
     if (!h) return FRISK_E_INVALID;
     int rc;
+    if (fmt == frisk_internal::kFmt2bit) {                // planes decoded by frisk_twobit.cu, handle made by fasta_adopt
+        delete h;
+        try {
+            return frisk_internal::twobit_open(text, n, st, sink, out);
+        } catch (...) {
+            return FRISK_E_CAPACITY;
+        }
+    }
     Source src;
     try {                                                 // std::bad_alloc of the record table: nothing crosses the ABI
         rc = make_source(text, n, fmt, st, &src);
@@ -1147,7 +1158,58 @@ int open_public(const char* text, uint64_t n, frisk_internal::TextFormat fmt, vo
     *out = h;
     return FRISK_OK;
 }
+
+// fasta_adopt behind the take-over: on_range over every word, the counters back on the upload lane beside on_complete's work
+int adopt_finish(frisk_b200_fasta* h, cudaStream_t st, frisk_internal::IngestSink* sink) {
+    UploadLane* lane = nullptr;
+    int rc = upload_lane(&lane);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> one_open(lane->mu);
+    FRISK_CK(cudaEventRecord(lane->ready, st));                         // the planes and counters are final here
+    FRISK_CK(cudaStreamWaitEvent(lane->copy, lane->ready, 0));
+    FRISK_CK(cudaMemcpyAsync(lane->stage, h->d_counters, frisk_internal::kIngestCounters * 8, cudaMemcpyDeviceToHost, lane->copy));
+    if (sink && sink->on_range &&
+        (rc = sink->on_range(h->d_codes, h->d_inv, h->d_low, h->d_counters + frisk_internal::kIngestRange, h->padded_len / 32, st)))
+        return rc;
+    if (sink && sink->on_complete && (rc = sink->on_complete(h, st))) return rc;
+    FRISK_CK(cudaStreamSynchronize(lane->copy));
+    h->stats[1] = lane->stage[kCtrNonUpper];
+    h->stats[2] = lane->stage[kCtrLower];
+    if (sink) sink->counted = (bool)sink->on_range;
+    return FRISK_OK;
+}
 }  // namespace
+
+int frisk_internal::fasta_adopt(AdoptedGenome& g, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out) {
+    *out = nullptr;
+    if (sink) sink->counted = false;
+    frisk_b200_fasta* h = new (std::nothrow) frisk_b200_fasta();
+    if (!h) {
+        cudaFreeAsync(g.d_slab, st);
+        return FRISK_E_CAPACITY;
+    }
+    h->d_out_slab = g.d_slab;
+    g.d_slab = nullptr;
+    h->d_codes = g.d_codes; h->d_inv = g.d_inv; h->d_low = g.d_low;
+    h->d_len = g.d_len; h->d_scaf_off = g.d_scaf_off; h->d_counters = g.d_counters;
+    h->rec_cap = g.rec_cap;
+    h->n_rec = g.seq_len.size();
+    h->padded_len = g.padded_len;
+    h->stats[0] = g.total;
+    h->name_off = std::move(g.name_off); h->name_len = std::move(g.name_len);
+    h->seq_len = std::move(g.seq_len); h->scaf_off = std::move(g.scaf_off);
+    h->name_text = std::move(g.name_text);
+    h->device_text = true;                                             // the names index the handle's buffer
+    h->streamed = true;                                                // what on_complete queued ran on the final table
+    const int rc = adopt_finish(h, st, sink);
+    if (rc) {
+        free_all(h, st);
+        delete h;
+        return rc;
+    }
+    *out = h;
+    return FRISK_OK;
+}
 
 bool frisk_internal::fasta_open_was_streamed(const frisk_b200_fasta* h) { return h && h->streamed; }
 
@@ -1189,6 +1251,11 @@ int frisk_b200_fasta_open_bgzf(const char* gz, uint64_t n, void* stream, frisk_b
 int frisk_b200_fasta_open_gzip(const char* gz, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
                                uint64_t* padded_len, uint64_t stats[3]) {
     return open_public(gz, n, frisk_internal::kFmtGzip, stream, out, n_records, padded_len, stats);
+}
+
+int frisk_b200_fasta_open_2bit(const char* buf, uint64_t n, void* stream, frisk_b200_fasta** out, uint64_t* n_records,
+                               uint64_t* padded_len, uint64_t stats[3]) {
+    return open_public(buf, n, frisk_internal::kFmt2bit, stream, out, n_records, padded_len, stats);
 }
 
 int frisk_b200_fasta_name_text(const frisk_b200_fasta* h, const char** text, uint64_t* n) {

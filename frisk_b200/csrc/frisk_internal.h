@@ -7,6 +7,7 @@
 #include <stdint.h>
 
 #include <functional>
+#include <vector>
 
 struct frisk_b200_fasta;
 
@@ -40,16 +41,36 @@ struct IngestSink {
     bool counted = false;                    // out: on_range saw every word of [0, padded_len / 32 - 1)
 };
 // the device side of a handle's record table, for on_complete: lengths, offsets, capacity, and the ingest's counters
-// (records at [kIngestRecords], non-upper-case bases at [kIngestNonUpper], "capacities exceeded" at [kIngestOverflow])
-enum { kIngestRecords = 0, kIngestNonUpper = 1, kIngestOverflow = 5 };
+// (records at [kIngestRecords], non-upper-case bases at [kIngestNonUpper], lower-case acgt at [kIngestLower], "capacities
+// exceeded" at [kIngestOverflow]; an adopted handle's {first, last} word of on_range at [kIngestRange]; kIngestCounters words)
+enum { kIngestRecords = 0, kIngestNonUpper = 1, kIngestLower = 2, kIngestOverflow = 5, kIngestRange = 12, kIngestCounters = 14 };
 bool fasta_open_was_streamed(const frisk_b200_fasta* h);     // false: the handle comes from the exact re-open
 int fasta_device_table(const frisk_b200_fasta* h, const unsigned long long** d_len, const unsigned long long** d_scaf_off,
                        const unsigned long long** d_counters, uint64_t* rec_cap, const uint32_t** d_codes, const uint32_t** d_inv,
                        const uint32_t** d_low);
-// what the bytes handed to an open are: the text, a BGZF buffer (frisk_b200_fasta_open_bgzf) or one gzip member
-// (frisk_b200_fasta_open_gzip); compressed input is inflated on the device into the text buffer
-enum TextFormat : int { kFmtText = 0, kFmtBgzf = 1, kFmtGzip = 2 };
+// what the bytes handed to an open are: the text, a BGZF buffer (frisk_b200_fasta_open_bgzf), one gzip member
+// (frisk_b200_fasta_open_gzip) -- compressed input is inflated on the device into the text buffer -- or a UCSC .2bit file
+// (frisk_b200_fasta_open_2bit), decoded on the device straight into the planes
+enum TextFormat : int { kFmtText = 0, kFmtBgzf = 1, kFmtGzip = 2, kFmt2bit = 3 };
 int fasta_open_planes(const char* text, uint64_t n, TextFormat fmt, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out);
+// A genome whose record table and planes were built in device memory by an open other than the text ingest (frisk_twobit.cu).
+// d_slab is one stream-ordered allocation holding every d_ pointer; d_counters has kIngestCounters words, with the records,
+// overflow (0) and on_range's word range set, and nnTotal / lower-case counts that are final once the work queued on the
+// open's stream is done.  Names index name_text.
+struct AdoptedGenome {
+    void* d_slab = nullptr;
+    uint32_t *d_codes = nullptr, *d_inv = nullptr, *d_low = nullptr;
+    unsigned long long *d_len = nullptr, *d_scaf_off = nullptr, *d_counters = nullptr;
+    uint64_t rec_cap = 0, padded_len = 0, total = 0;
+    std::vector<uint64_t> name_off, seq_len, scaf_off;
+    std::vector<uint32_t> name_len;
+    std::vector<char> name_text;
+};
+// frisk_ingest.cu: a handle takes g over (its slab is freed with the handle, or here on failure) and does what the text open
+// does behind its last chunk: the planes go to sink->on_range (every word), the counters come back, sink->on_complete runs.
+int fasta_adopt(AdoptedGenome& g, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out);
+// frisk_twobit.cu: the open of a .2bit file (kFmt2bit)
+int twobit_open(const char* buf, uint64_t n, cudaStream_t st, IngestSink* sink, frisk_b200_fasta** out);
 // frisk_b200_bgzf_inflate's kernel (frisk_bgzf.cu); d_any_bad (nullable) receives a non-zero word when a member fails
 int bgzf_inflate(const uint8_t* d_gz, const uint64_t* d_comp_off, const uint32_t* d_comp_len, const uint32_t* d_crc,
                  const uint64_t* d_text_off, uint64_t n_blocks, uint64_t text_len, uint8_t* d_text, uint32_t* d_block_status,

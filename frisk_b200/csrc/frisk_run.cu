@@ -1,5 +1,5 @@
-// frisk_b200 one-call run paths: host planes, resident planes or FASTA text in, rows out, in one C call
-// (frisk_b200_run_host / _sparse / _peers, frisk_b200_run_resident, frisk_b200_run_fasta / _bgzf / _gzip).  Every path enters and
+// frisk_b200 one-call run paths: host planes, resident planes, FASTA text or a .2bit file in, rows out, in one C call
+// (frisk_b200_run_host / _sparse / _peers, frisk_b200_run_resident, frisk_b200_run_fasta / _bgzf / _gzip, frisk_b200_run_2bit).  Every path enters and
 // leaves through RunCall (device lock, stage marks, error drain), finalises through queue_tables and ends in results.  The
 // per-device state they share lives here too: the workspace, the copy stream, the stage marks and the window staging.
 #include <cuda_runtime.h>
@@ -475,7 +475,8 @@ int stage_get(int dev, int slot, size_t bytes, void** out) {
     return FRISK_OK;
 }
 
-// fmt: h_text / q_text are texts, BGZF buffers or gzip members (the last two inflated on the device by the ingest)
+// fmt: h_text / q_text are texts, BGZF buffers or gzip members (the last two inflated on the device by the ingest), or .2bit
+// files (decoded on the device into the planes by frisk_twobit.cu)
 int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt,
                    int w, int step, int scaffolds_all, const Job& j, uint64_t rows_cap, uint64_t* n_win_out,
                    frisk_b200_fasta** host_out, frisk_b200_fasta** query_out) {
@@ -630,7 +631,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
                     &late);
 }
 
-// frisk_b200_run_fasta, _run_fasta_bgzf and _run_fasta_gzip
+// frisk_b200_run_fasta, _run_fasta_bgzf, _run_fasta_gzip and _run_2bit
 int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
                   int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                   uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
@@ -746,6 +747,14 @@ int frisk_b200_run_fasta_gzip(const char* h_gz, uint64_t h_n, const char* q_gz, 
                               uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                               frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
     return run_fasta_any(h_gz, h_n, q_gz, q_n, frisk_internal::kFmtGzip, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+                         rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
+}
+
+int frisk_b200_run_2bit(const char* h_2bit, uint64_t h_n, const char* q_2bit, uint64_t q_n, int w, int step, int scaffolds_all,
+                        int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
+                        uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out, frisk_b200_fasta** host_out,
+                        frisk_b200_fasta** query_out, void* stream) {
+    return run_fasta_any(h_2bit, h_n, q_2bit, q_n, frisk_internal::kFmt2bit, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
                          rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 

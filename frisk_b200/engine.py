@@ -138,6 +138,16 @@ def is_gzip(buf) -> bool:
     return a.shape[0] >= 18 and bytes(a[:3]) == b"\x1f\x8b\x08" and not is_bgzf(a)
 
 
+TWOBIT_SIGNATURE = 0x1A412743
+
+
+def is_2bit(buf) -> bool:
+    """Whether ``buf`` begins with the signature of a UCSC .2bit file, in either byte order (a big-endian file stores
+    every integer byte-swapped).  Such files are decoded on the device straight into the planes (frisk_twobit.cu)."""
+    a = _as_u8(buf)
+    return a.shape[0] >= 16 and int.from_bytes(bytes(a[:4]), "little") in (TWOBIT_SIGNATURE, 0x4327411A)
+
+
 def read_genome_file(path: str) -> Tuple[np.ndarray, bool]:
     """(bytes, bgzf): a BGZF file as it is on disk (the device inflates it), any other file as ``read_fasta_file``
     gives it (a single-member ``.gz`` inflated on the host, text as it is)."""
@@ -148,9 +158,12 @@ def read_genome_file(path: str) -> Tuple[np.ndarray, bool]:
 
 
 def read_genome_raw(path: str) -> Tuple[np.ndarray, str]:
-    """(bytes, kind) as the file is on disk: kind "bgzf" (BGZF), "gzip" (a ``.gz`` with a plain gzip member) or "text".
-    Compressed files are left to the device to inflate; a ``.gz`` that is neither is read by ``read_fasta_file``."""
+    """(bytes, kind) as the file is on disk: kind "2bit" (a UCSC .2bit file, by its signature, whatever the extension),
+    "bgzf" (BGZF), "gzip" (a ``.gz`` with a plain gzip member) or "text".  Compressed files are left to the device to
+    inflate; a ``.gz`` that is neither is read by ``read_fasta_file``."""
     raw = np.fromfile(path, dtype=np.uint8)
+    if is_2bit(raw):
+        return raw, "2bit"
     if is_bgzf(raw):
         return raw, "bgzf"
     if path.endswith(".gz"):
@@ -181,9 +194,24 @@ def bgzf_text_len(gz) -> int:
     return int(tl.value)
 
 
+def twobit_records(buf) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """(name_off, name_len, seq_len) of a .2bit buffer, parsed and checked on the host (frisk_b200_2bit_records;
+    FriskError E_FORMAT for a malformed file).  Name offsets index ``buf``."""
+    L = _lib.lib()
+    a = _as_u8(buf)
+    n, bases = C.c_uint64(0), C.c_uint64(0)
+    _lib.check(L.frisk_b200_2bit_records(_ptr(a), a.shape[0], 0, None, None, None, C.byref(n), C.byref(bases)),
+               "frisk_b200_2bit_records")
+    R = int(n.value)
+    name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32); seq_len = np.zeros(R, np.uint64)
+    _lib.check(L.frisk_b200_2bit_records(_ptr(a), a.shape[0], R, _ptr(name_off), _ptr(name_len), _ptr(seq_len), C.byref(n),
+                                         C.byref(bases)), "frisk_b200_2bit_records")
+    return name_off, name_len, seq_len
+
+
 def _name_source(L, h, buf: np.ndarray, device_text: bool) -> np.ndarray:
-    """What a handle's name offsets index: the caller's text, or -- a BGZF or gzip open, whose text never leaves the
-    device -- the handle's buffer of header lines (copied: it goes with the handle)."""
+    """What a handle's name offsets index: the caller's text, or -- a BGZF, gzip or .2bit open, whose text never leaves
+    the device or does not exist -- the handle's buffer of names (copied: it goes with the handle)."""
     if not device_text:
         return buf
     p, n = C.c_void_p(), C.c_uint64(0)
@@ -309,8 +337,34 @@ class PackedGenome:
                          threads)
 
     @classmethod
+    def from_2bit_bytes(cls, buf: Union[bytes, np.ndarray], pinned: bool = False) -> "PackedGenome":
+        """A UCSC .2bit buffer decoded on the host (frisk_b200_2bit_unpack_host): the same planes, records and countN
+        statistics as the genome's FASTA through ``from_fasta_bytes``."""
+        L = _lib.lib()
+        a = _as_u8(buf)
+        name_off, name_len, lens = twobit_records(a)
+        n = len(lens)
+        scaf_off = np.zeros(n, np.uint64)
+        padded = C.c_uint64(0)
+        _lib.check(L.frisk_b200_pack_layout(_ptr(lens), n, _ptr(scaf_off), C.byref(padded)), "frisk_b200_pack_layout")
+        P = int(padded.value)
+        codes = _alloc_u32(P // 16, pinned)
+        inv = _alloc_u32(P // 32, pinned)
+        low = _alloc_u32(P // 32, pinned)
+        stats = np.zeros(3, np.uint64)
+        _lib.check(L.frisk_b200_2bit_unpack_host(_ptr(a), a.shape[0], P, _ptr(codes), _ptr(inv), _ptr(low), _ptr(stats)),
+                   "frisk_b200_2bit_unpack_host")
+        n_lower = int(stats[2])
+        return cls(_decode_names(a, name_off, name_len), lens, scaf_off, P, codes, inv, low if n_lower else None, int(stats[0]),
+                   int(stats[1]), n_lower, bool(pinned))
+
+    @classmethod
     def from_fasta(cls, path: str, pinned: bool = False, threads: int = 0) -> "PackedGenome":
-        return cls.from_fasta_bytes(read_fasta_file(path), pinned, threads)
+        """A FASTA file (``.gz`` inflated on the host), or a .2bit file, recognised by its signature."""
+        raw = np.fromfile(path, dtype=np.uint8)
+        if is_2bit(raw):
+            return cls.from_2bit_bytes(raw, pinned)
+        return cls.from_fasta_bytes(read_fasta_file(path) if path.endswith(".gz") else raw, pinned, threads)
 
     @classmethod
     def _pack(cls, names, src, src_off, src_end, lens, pinned, threads) -> "PackedGenome":
@@ -431,6 +485,11 @@ class DeviceGenome:
         return cls._open_native(gz, device, "gzip")
 
     @classmethod
+    def from_2bit_bytes_native(cls, buf: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes_native`` for a UCSC .2bit buffer: the file goes to the GPU and is decoded there."""
+        return cls._open_native(buf, device, "2bit")
+
+    @classmethod
     def _open_native(cls, text, device, kind: str) -> "DeviceGenome":
         _lib.require_device()
         L = _lib.lib()
@@ -477,6 +536,12 @@ class DeviceGenome:
         return cls._open(gz, device, "gzip")
 
     @classmethod
+    def from_2bit_bytes(cls, buf: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
+        """``from_fasta_bytes`` for a UCSC .2bit buffer (frisk_twobit.cu): the file goes to the GPU in one copy and its
+        packed bases, N blocks and mask blocks are decoded there straight into the planes."""
+        return cls._open(buf, device, "2bit")
+
+    @classmethod
     def _open(cls, text, device, kind: str) -> "DeviceGenome":
         import torch
         _lib.require_device()
@@ -511,7 +576,7 @@ class DeviceGenome:
     @classmethod
     def from_fasta(cls, path: str, device="cuda:0") -> "DeviceGenome":
         """A FASTA file: BGZF and single-member gzip are inflated on the device, a multi-member ``.gz`` on the host
-        (``read_fasta_file``)."""
+        (``read_fasta_file``); a .2bit file is decoded on the device."""
         return open_genome_file(path, lambda buf, kind: cls._open(buf, device, kind))
 
     def to_host(self) -> PackedGenome:
@@ -1147,12 +1212,27 @@ def run_fasta_gzip(query_gz, host_gz=None, device="cuda:0", out=None, assemble_r
                           scaffolds_all, rip)
 
 
-_OPENERS = {"text": "frisk_b200_fasta_open", "bgzf": "frisk_b200_fasta_open_bgzf", "gzip": "frisk_b200_fasta_open_gzip"}
-_RUNNERS = {"text": "frisk_b200_run_fasta", "bgzf": "frisk_b200_run_fasta_bgzf", "gzip": "frisk_b200_run_fasta_gzip"}
+def run_2bit(query_2bit, host_2bit=None, device="cuda:0", out=None, assemble_result: bool = True, kmin: int = 1,
+             kmax: int = 8, w: int = 5000, step: int = 2500, mask_host: bool = False, scaffolds_all: bool = False,
+             rip: bool = True):
+    """``run_fasta`` for UCSC .2bit files (ideally page-locked): ONE C call (frisk_b200_run_2bit) that uploads the file,
+    decodes it on the device straight into the planes and goes on exactly as ``run_fasta``.  Same results as
+    ``run_fasta`` on the genome's FASTA."""
+    return _run_fasta_any(query_2bit, host_2bit, "2bit", device, out, assemble_result, kmin, kmax, w, step, mask_host,
+                          scaffolds_all, rip)
+
+
+_OPENERS = {"text": "frisk_b200_fasta_open", "bgzf": "frisk_b200_fasta_open_bgzf", "gzip": "frisk_b200_fasta_open_gzip",
+            "2bit": "frisk_b200_fasta_open_2bit"}
+_RUNNERS = {"text": "frisk_b200_run_fasta", "bgzf": "frisk_b200_run_fasta_bgzf", "gzip": "frisk_b200_run_fasta_gzip",
+            "2bit": "frisk_b200_run_2bit"}
 
 
 def _text_len_hint(buf: np.ndarray, kind: str) -> int:
-    """The text's length: exact for text and BGZF; for gzip, ISIZE (the length mod 2^32 -- a guess for sizing rows)."""
+    """The text's length: exact for text and BGZF; for gzip, ISIZE (the length mod 2^32 -- a guess for sizing rows); for
+    .2bit, the number of bases."""
+    if kind == "2bit":
+        return int(twobit_records(buf)[2].sum())
     if kind == "bgzf":
         return bgzf_text_len(buf)
     if kind == "gzip":

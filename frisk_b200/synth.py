@@ -262,6 +262,50 @@ def fasta_bytes(scaffolds: List[Scaffold], width: int = 60) -> bytes:
     return b"".join(parts)
 
 
+_TWOBIT_CODE = np.zeros(256, np.uint8)                   # T=0, C=1, A=2, G=3; anything else (an N) is stored as T
+for _c, _v in zip(b"TCAGtcag", (0, 1, 2, 3, 0, 1, 2, 3)):
+    _TWOBIT_CODE[_c] = _v
+
+
+def _runs(flag: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+    """(starts, sizes) of the runs of True in a boolean array."""
+    d = np.diff(np.concatenate([[0], flag.astype(np.int8), [0]]))
+    starts = np.nonzero(d == 1)[0]
+    return starts.astype(np.uint32), (np.nonzero(d == -1)[0] - starts).astype(np.uint32)
+
+
+def twobit_bytes(scaffolds: List[Scaffold], big_endian: bool = False, version: int = 0) -> bytes:
+    """The scaffolds as a UCSC .2bit file (faToTwoBit's format): N blocks = the runs of characters that are not one of
+    ACGTacgt, mask blocks = the runs of lower-case characters, 4 bases per byte with the first in the top two bits.
+    ``version`` 1 writes 64-bit index offsets; ``big_endian`` writes every integer byte-swapped."""
+    e = ">" if big_endian else "<"
+    u32 = np.dtype(e + "u4")
+    idx_entry = 4 if version == 0 else 8
+    index_len = sum(1 + len(name.encode()) + idx_entry for name, _ in scaffolds)
+    records = []
+    for _, seq in scaffolds:
+        s = np.ascontiguousarray(seq, dtype=np.uint8)
+        n = len(s)
+        up = s & 0xDF
+        n_starts, n_sizes = _runs(~np.isin(up, np.frombuffer(b"ACGT", np.uint8)))
+        m_starts, m_sizes = _runs((s >= ord("a")) & (s <= ord("z")))
+        codes = np.zeros((n + 3) // 4 * 4, np.uint8)
+        codes[:n] = _TWOBIT_CODE[s]
+        q = codes.reshape(-1, 4)
+        packed = (q[:, 0] << 6) | (q[:, 1] << 4) | (q[:, 2] << 2) | q[:, 3]
+        head = np.array([n, len(n_starts)], u32).tobytes() + n_starts.astype(u32).tobytes() + n_sizes.astype(u32).tobytes()
+        head += np.array([len(m_starts)], u32).tobytes() + m_starts.astype(u32).tobytes() + m_sizes.astype(u32).tobytes()
+        records.append(head + np.array([0], u32).tobytes() + packed.astype(np.uint8).tobytes())
+    off = 16 + index_len
+    index = []
+    for (name, _), rec in zip(scaffolds, records):
+        nb = name.encode()
+        index.append(bytes([len(nb)]) + nb + np.array([off], np.dtype(e + ("u4" if version == 0 else "u8"))).tobytes())
+        off += len(rec)
+    header = np.array([0x1A412743, version, len(scaffolds), 0], u32).tobytes()
+    return header + b"".join(index) + b"".join(records)
+
+
 def write_fasta(scaffolds: List[Scaffold], path: str, width: int = 60) -> None:
     with open(path, "wb") as fh:
         fh.write(fasta_bytes(scaffolds, width))

@@ -460,6 +460,42 @@ int frisk_b200_run_fasta_gzip(const char *h_gz, uint64_t h_n, const char *q_gz, 
                               double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
                               uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
 
+/* ------------------------------------------------------------------ UCSC .2bit genomes (frisk_twobit.cu)
+ *
+ * A twoBit file (UCSC hg38.2bit, faToTwoBit; versions 0 and 1, either byte order: a signature that reads 0x4327411A means
+ * every integer of the file is byte-swapped) holds 2-bit bases, N blocks and soft-mask blocks: exactly what the planes hold.
+ * Every non-ACGT character of a FASTA is an N there and every lower-case character lies in a mask block, so a .2bit file and
+ * its FASTA give the same records, planes, tables and rows, bit for bit.  Nothing is tokenised: the bases are remapped and
+ * realigned to the 128-base layout, the blocks expanded into the invalid and lower-case planes (N blocks: invalid, code 0;
+ * mask blocks minus N blocks: lower case).  The name of a record is its index name, verbatim.
+ *
+ * frisk_b200_2bit_records: parses and checks the whole file on the host: header, index and record headers, every block
+ * inside its sequence (zero-size blocks are ignored; blocks may overlap and come in any order), the packed bases inside the
+ * buffer.  A bad signature, a version other than 0 or 1, an empty name, an offset, count or length that reaches beyond the
+ * buffer, or a block beyond its sequence: FRISK_E_FORMAT, before any byte beyond the buffer is read.  name_off / name_len:
+ * the index names in buf; seq_len: dnaSize; *bases (nullable): their sum.  Arrays may be NULL to count only; *n_records
+ * always receives the count; FRISK_E_CAPACITY if cap is too small.
+ *
+ * frisk_b200_2bit_unpack_host: the planes of the file on the CPU, with the device path's plan and per-word code (test
+ * infrastructure, and the producer of host planes).  padded_len must be frisk_b200_pack_layout's for the record lengths
+ * (FRISK_E_INVALID otherwise); codes / inv / low as frisk_b200_pack (low may be NULL when the file has no mask bases,
+ * FRISK_E_FORMAT if it has some); stats[3] as frisk_b200_pack (totalLen, nnTotal, lower-case acgt).
+ *
+ * frisk_b200_fasta_open_2bit / frisk_b200_run_2bit: frisk_b200_fasta_open / frisk_b200_run_fasta with .2bit files in place of
+ * the texts, same arguments and results.  The file goes up in one copy and is decoded into planes the handle owns; the names
+ * come from frisk_b200_fasta_name_text; with kmax 7 or 8 and windows of <= 8,186 bases the one-call path takes the
+ * device-only tail as text does.  ms[0] of frisk_b200_last_run_timing is "file uploaded and decoded". */
+int frisk_b200_2bit_records(const uint8_t *buf, uint64_t n, uint64_t cap, uint64_t *name_off, uint32_t *name_len,
+                            uint64_t *seq_len, uint64_t *n_records, uint64_t *bases);
+int frisk_b200_2bit_unpack_host(const uint8_t *buf, uint64_t n, uint64_t padded_len, uint32_t *codes, uint32_t *inv,
+                                uint32_t *low, uint64_t stats[3]);
+int frisk_b200_fasta_open_2bit(const char *buf, uint64_t n, void *stream, frisk_b200_fasta **out, uint64_t *n_records,
+                               uint64_t *padded_len, uint64_t stats[3]);
+int frisk_b200_run_2bit(const char *h_2bit, uint64_t h_n, const char *q_2bit, uint64_t q_n, int w, int step,
+                        int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap,
+                        double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
+                        uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
+
 /* Stage times (ms since the start of the call) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call
  * on the current device, from CUDA events recorded on the call's own streams: ms[0] planes uploaded, ms[1] background
  * counted, ms[2] tables + genome IVOM finalised (multi-GPU: includes the wait for the peers' counters), ms[3] window
