@@ -16,6 +16,7 @@
 
 namespace {
 using frisk_internal::LaunchShape;
+using frisk_internal::WinJob;
 using frisk_internal::WinPlan;
 
 // ============================================================================================
@@ -490,16 +491,15 @@ LaunchShape bucket_shape_k(const WinPlan& p, uint32_t max_len) {
 }
 
 // one launch; it takes the windows of [len_min, len_max] only, and with redo_src only those marked kRowRedo there
-int launch_bucket(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, uint32_t len_min, uint32_t len_max,
-                  const uint32_t* redo_src) {
-    const LaunchShape s = frisk_internal::bucket_shape(p, K, max_len);
-    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-    const double2* g = reinterpret_cast<const double2*>(ig);
-    uint32_t n = (uint32_t)n_win, cap = (max_len + 15u) & ~15u;
-    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &cap, &len_min, &len_max, &rows, &status, &dump, &redo_src};
-    return frisk_internal::launch_persistent(s, n_win, args, st);
+int launch_bucket(const WinPlan& p, const WinJob& j, uint32_t len_min, uint32_t len_max, const uint32_t* redo_src) {
+    const LaunchShape s = frisk_internal::bucket_shape(p, j.K, j.max_len);
+    WinJob a = j;                                      // the kernel arguments are read from their addresses
+    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(a.win_off);
+    const double2* g = reinterpret_cast<const double2*>(a.ig);
+    uint32_t n = (uint32_t)a.n_win, cap = (a.max_len + 15u) & ~15u;
+    void* args[] = {&a.codes, &a.inv, &a.low, &off, &a.win_len, &n, &g, &a.kmin, &a.rip, &cap, &len_min, &len_max,
+                    &a.rows, &a.status, &a.dump, &redo_src};
+    return frisk_internal::launch_persistent(s, a.n_win, args, a.st);
 }
 
 }  // namespace
@@ -519,20 +519,16 @@ frisk_internal::LaunchShape frisk_internal::bucket_shape(const WinPlan& p, int K
 // Windows longer than 5 rounds need a bigger buffer, which costs a CTA per SM.  With --scaffoldsAll nearly all windows are
 // still the standard length and only whole short scaffolds (up to 1.25 w) are longer: two launches, each taking the
 // windows of its length class, keep the standard ones at four CTAs per SM.  A hand-over launch (redo_src) is one launch.
-int frisk_internal::score_bucket(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                                 const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
-                                 int kmin, int K, int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st,
-                                 const uint32_t* redo_src) {
-    if (K < 4 || K > 8) return FRISK_E_UNSUPPORTED;
+int frisk_internal::score_bucket(const WinPlan& p, const WinJob& j, const uint32_t* redo_src) {
+    if (j.K < 4 || j.K > 8) return FRISK_E_UNSUPPORTED;
     constexpr uint32_t kStd = 5104u;                   // largest buffer that still fits four CTAs
-    if (!redo_src && p.variant == 8 && n_win >= 4096) {
+    if (!redo_src && p.variant == 8 && j.n_win >= 4096) {
         const WinPlan std5{p.kind, 5, p.dump, p.allk};
-        int rc = launch_bucket(std5, codes, inv, low, win_off, win_len, n_win, kStd, ig, kmin, K, want_rip, rows, status, dump, st, 0u,
-                               kStd, nullptr);
+        WinJob std_len = j;
+        std_len.max_len = kStd;
+        int rc = launch_bucket(std5, std_len, 0u, kStd, nullptr);
         if (rc) return rc;
-        return launch_bucket(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump, st,
-                             kStd + 1u, 0xffffffffu, nullptr);
+        return launch_bucket(p, j, kStd + 1u, 0xffffffffu, nullptr);
     }
-    return launch_bucket(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump, st, 0u,
-                         0xffffffffu, redo_src);
+    return launch_bucket(p, j, 0u, 0xffffffffu, redo_src);
 }

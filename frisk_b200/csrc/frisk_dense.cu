@@ -17,6 +17,7 @@
 
 namespace {
 using frisk_internal::LaunchShape;
+using frisk_internal::WinJob;
 using frisk_internal::sm_count_cached;
 #define CK(call) FRISK_CK(call)
 
@@ -349,24 +350,22 @@ LaunchShape dense_shape_k() {
 
 // grid: one CTA per SM (or per window, when there are fewer windows than SMs)
 template <int K>
-int score_dense_k(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
+int score_dense_k(const WinJob& j) {
     using L = ScoreLayout<K>;
     constexpr uint32_t NB = pow4(K);
     const LaunchShape s = dense_shape_k<K>();
     // a segment = a contiguous 1/nseg of the k-mer space (and of the threads owning its bitmap words);
     // its distinct k-mers (<= bins in it, <= window length) must fit the list
     int nseg = 1;
-    while ((NB / (uint32_t)nseg < max_len ? NB / (uint32_t)nseg : max_len) > kListCap) nseg *= 2;
+    while ((NB / (uint32_t)nseg < j.max_len ? NB / (uint32_t)nseg : j.max_len) > kListCap) nseg *= 2;
     if (nseg > kMaxSeg || (uint32_t)nseg > (L::BM_WORDS >= 2u ? L::BM_WORDS / 2u : 1u)) return FRISK_E_UNSUPPORTED;
     CK(cudaFuncSetAttribute(s.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem));
     int grid = sm_count_cached();
     if (grid <= 0) return FRISK_E_NO_DEVICE;
-    if ((uint64_t)grid > n_win) grid = (int)n_win;
-    score_windows_kernel<K><<<grid, s.threads, s.smem, st>>>(
-        codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off), win_len, (uint32_t)n_win,
-        reinterpret_cast<const double2*>(ig), kmin, want_rip, nseg, rows, status, dump);
+    if ((uint64_t)grid > j.n_win) grid = (int)j.n_win;
+    score_windows_kernel<K><<<grid, s.threads, s.smem, j.st>>>(
+        j.codes, j.inv, j.low, reinterpret_cast<const unsigned long long*>(j.win_off), j.win_len, (uint32_t)j.n_win,
+        reinterpret_cast<const double2*>(j.ig), j.kmin, j.rip, nseg, j.rows, j.status, j.dump);
     CK(cudaGetLastError());
     return FRISK_OK;
 }
@@ -386,8 +385,6 @@ frisk_internal::LaunchShape frisk_internal::dense_shape(int K) {
     }
 }
 
-int frisk_internal::score_dense(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                                const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
-                                int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
-    DISPATCH_K(K, score_dense_k<K>(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, want_rip, rows, status, dump, st));
+int frisk_internal::score_dense(const WinPlan&, const WinJob& j) {
+    DISPATCH_K(j.K, score_dense_k<K>(j));
 }

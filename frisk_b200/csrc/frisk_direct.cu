@@ -366,18 +366,16 @@ frisk_internal::LaunchShape frisk_internal::direct_shape(const WinPlan& p, int K
     return {direct_fn<7>(p), 256, DirectLayout<7, 256>::TOTAL, true};
 }
 
-int frisk_internal::score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                                 const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
-                                 int kmin, int K, int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st) {
-    if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
-    return with_redo_marks(status, n_win, false, st, [&](uint32_t* redo) {
-        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-        const double2* g = reinterpret_cast<const double2*>(ig);
-        uint32_t n = (uint32_t)n_win;
-        void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo};
-        int rc = launch_persistent(direct_shape(p, K), n_win, args, st);
+int frisk_internal::score_direct(const WinPlan& p, const WinJob& j) {
+    if (j.K != 7 && j.K != 8) return FRISK_E_UNSUPPORTED;
+    return with_redo_marks(j.status, j.n_win, false, j.st, [&](uint32_t* redo) {
+        WinJob a = j;                                  // the kernel arguments are read from their addresses
+        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(a.win_off);
+        const double2* g = reinterpret_cast<const double2*>(a.ig);
+        uint32_t n = (uint32_t)a.n_win;
+        void* args[] = {&a.codes, &a.inv, &a.low, &off, &a.win_len, &n, &g, &a.kmin, &a.rip, &a.rows, &a.status, &a.dump, &redo};
+        int rc = launch_persistent(direct_shape(p, a.K), a.n_win, args, a.st);
         // windows the byte table could not hold (marked kRowRedo): exact re-run on the bucketed kernel
-        return rc ? rc : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump,
-                                           redo, st);
+        return rc ? rc : score_bucket_redo(j, redo);
     });
 }

@@ -354,10 +354,11 @@ int general_genome_ivom(const uint64_t* tables, int kmin, int K, int64_t space, 
     return FRISK_OK;
 }
 
-int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src, int grid_cap) {
-    if (dump && max_len > 65535u) return FRISK_E_UNSUPPORTED;          // the test dump is 16-bit
+int general_score(const WinPlan&, const WinJob& j, const uint32_t* redo_src, int grid_cap) {
+    const uint64_t n_win = j.n_win;
+    const int K = j.K;
+    const cudaStream_t st = j.st;
+    if (j.dump && j.max_len > 65535u) return FRISK_E_UNSUPPORTED;      // the test dump is 16-bit
     const int n = sms();
     if (n <= 0) return FRISK_E_NO_DEVICE;
     uint64_t grid = (uint64_t)n;
@@ -390,10 +391,10 @@ int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* lo
     const int KS = K < kSmemOrders ? K : kSmemOrders;
     const size_t smem = ((sizeof(GenSmem) + 15) & ~(size_t)15) + (size_t)loff(KS + 1) * 4 + (K <= kSmemOrders ? (size_t)p4(K) * 4 : 0);
     FRISK_CK(cudaFuncSetAttribute(gen_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (dump) gen_zero_dump_kernel<<<1024, 256, 0, st>>>(dump, n_win * loff(K + 1));
-    gen_score_kernel<<<(unsigned)grid, kGT, smem, st>>>(codes, inv, low, reinterpret_cast<const unsigned long long*>(win_off),
-                                                       win_len, (uint32_t)n_win, reinterpret_cast<const double2*>(ig), kmin, K,
-                                                       want_rip, slab, slab_words, rows, status, dump, redo_list, redo_count);
+    if (j.dump) gen_zero_dump_kernel<<<1024, 256, 0, st>>>(j.dump, n_win * loff(K + 1));
+    gen_score_kernel<<<(unsigned)grid, kGT, smem, st>>>(j.codes, j.inv, j.low, reinterpret_cast<const unsigned long long*>(j.win_off),
+                                                       j.win_len, (uint32_t)n_win, reinterpret_cast<const double2*>(j.ig), j.kmin, K,
+                                                       j.rip, slab, slab_words, j.rows, j.status, j.dump, redo_list, redo_count);
     FRISK_CK(cudaGetLastError());
     if (redo_list) FRISK_CK(cudaFreeAsync(redo_list, st));
     if (slab) FRISK_CK(cudaFreeAsync(slab, st));

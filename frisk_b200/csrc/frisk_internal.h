@@ -100,10 +100,6 @@ int general_background(const uint32_t* codes, const uint32_t* inv, const uint32_
                        int mask_host, uint64_t* fwd, cudaStream_t st);
 int general_finalize(const uint64_t* fwd, int K, int symmetric, uint64_t* tables, uint64_t* valid, cudaStream_t st);
 int general_genome_ivom(const uint64_t* tables, int kmin, int K, int64_t space, double* ig, cudaStream_t st);
-int general_score(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                  const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr,
-                  int grid_cap = 0);
 
 // FRISK_E_INVALID unless 1 <= kmin <= kmax; FRISK_E_UNSUPPORTED for kmax > FRISK_B200_MAX_K
 int check_k(int kmin, int kmax);
@@ -145,6 +141,29 @@ struct WinPlan {
 };
 int plan_score(int kmin, int kmax, uint32_t max_win_len, bool dump, WinPlan* out);
 int window_variant(WinKernel kind, uint32_t max_win_len);
+
+// One score call's device inputs and outputs: the query planes (low nullable), the window list, its count and longest
+// window, the genome IVOM table, the orders kmin..K, the RIP flag, the outputs (dump nullable) and the stream.
+struct WinJob {
+    const uint32_t *codes, *inv, *low;
+    const uint64_t* win_off;
+    const uint32_t* win_len;
+    uint64_t n_win;
+    uint32_t max_len;
+    const double* ig;
+    int kmin, K, rip;
+    double* rows;
+    uint32_t* status;
+    uint16_t* dump;
+    cudaStream_t st;
+};
+// the RIP flag a launcher is handed: RIP needs orders 1 and 2
+inline int rip_orders(int want_rip, int kmin, int kmax) { return want_rip && kmin <= 2 && kmax >= 2; }
+// The score call behind frisk_b200_score and the device-only tail of the one-call run (frisk_score.cu): reduces j.rip (the
+// caller's want_rip) by rip_orders, refuses windows longer than FRISK_B200_MAX_WINDOW and more than 2^32-1 windows with
+// FRISK_E_UNSUPPORTED, and runs the launcher of p.kind.  n_win_dev (nibble kernel only): the window count in device
+// memory, j.n_win its capacity.
+int score(const WinPlan& p, WinJob j, const unsigned long long* n_win_dev = nullptr);
 // the instantiation of a window kernel template <..., DUMP, ALLK> a plan runs: the table dump and kmin > 1 share the generic
 // <..., DUMP, false> one, the production default (no dump, kmin 1) has its own
 #define FRISK_WIN_INSTANCE(p, kern, ...)                                                                      \
@@ -197,54 +216,43 @@ int with_redo_marks(uint32_t* status, uint64_t n_win, bool zero, cudaStream_t st
     return rc;
 }
 
-// A *_shape function expects a K its kernel serves (a plan only picks a kernel for those); a score_* entry refuses any
-// other K with FRISK_E_UNSUPPORTED.
+// A *_shape function expects a K its kernel serves (a plan only picks a kernel for those).  A launcher takes the plan and
+// the job, runs the kernel of p.kind for j.K, and refuses any other K with FRISK_E_UNSUPPORTED; j.rip is passed to the
+// kernel as it is.  Only an argument that one launcher alone uses is a parameter of its own.
 //
 // small-K kernel (frisk_small.cu): kmax 1..6, windows <= 65,535 bases.  redo_src: only the windows marked kRowRedo there.
 LaunchShape small_shape(const WinPlan& p, int K);
-int score_small(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int K, int want_rip, double* rows,
-                uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr);
+int score_small(const WinPlan& p, const WinJob& j, const uint32_t* redo_src = nullptr);
 // bucketed kernel (frisk_bucket.cu): kmax 4..8, windows <= kSmemMaxWindow bases; its buffer is sized by max_len
 LaunchShape bucket_shape(const WinPlan& p, int K, uint32_t max_len);
-int score_bucket(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                 double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const uint32_t* redo_src = nullptr);
+int score_bucket(const WinPlan& p, const WinJob& j, const uint32_t* redo_src = nullptr);
 // The hand-over target of the direct and nibble kernels and of the k sweep (frisk_score.cu): the windows marked kRowRedo
-// in redo_src, re-done on the small-K kernel for K <= 3 and on the bucketed kernel for K >= 4.
-int score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                      const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                      double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src, cudaStream_t st);
+// in redo_src, re-done on the small-K kernel for K <= 3 and on the bucketed kernel for K >= 4, with a plan of its own.
+int score_bucket_redo(const WinJob& j, const uint32_t* redo_src);
 // dense-table kernel (frisk_dense.cu): kmax 1..8, windows <= 65,535 bases; one CTA of dense_shape(K).threads per SM
 LaunchShape dense_shape(int K);
-int score_dense(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,
-                uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip, double* rows, uint32_t* status,
-                uint16_t* dump, cudaStream_t st);
+int score_dense(const WinPlan& p, const WinJob& j);
+// general path (frisk_general.cu): K up to FRISK_B200_MAX_K, windows of any length.  grid_cap > 0: at most that many CTAs.
+int general_score(const WinPlan& p, const WinJob& j, const uint32_t* redo_src = nullptr, int grid_cap = 0);
 
 // kmax 9..12, windows <= kSmemMaxWindow bases (frisk_nibble_ext.cu): orders 1..8 as in the kmax-8 nibble kernel, orders
 // 9..K from the observation that an 8-mer seen once has only unique extensions (the few repeated ones go through a
-// shared-memory hash table).  What it cannot hold is re-done by general_score behind it.
+// shared-memory hash table).  What it cannot hold is re-done by general_score behind it.  No table dump (j.dump unused).
 LaunchShape ext_shape(const WinPlan& p);
-int score_nibble_ext(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                     const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                     double* rows, uint32_t* status, cudaStream_t st);
+int score_nibble_ext(const WinPlan& p, const WinJob& j);
 
 // direct score kernel (frisk_direct.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases.  Windows it cannot finish exactly
 // (a K-mer seen 256+ times, more than 64 N-boundary words) are re-done by score_bucket_redo.
 LaunchShape direct_shape(const WinPlan& p, int K);
-int score_direct(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                 double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st);
+int score_direct(const WinPlan& p, const WinJob& j);
 
 // nibble score kernel (frisk_nibble.cu): kmax 7, 8 and windows <= kSmemMaxWindow bases; one 4-bit counter per K-mer, one
 // atomic per position, the first occurrence of a K-mer scores it.  Windows with a K-mer seen 16+ times (or more than 64
 // N-boundary words) are re-done by the bucketed kernel, exactly like the direct kernel's hand-over.  n_win_dev: the window
-// count in device memory, n_win its capacity.  It reads ig through a (K+1)-mer pair table it builds in stream-ordered scratch
-// before its launch (frisk_nibble.cu); the hand-over reads ig itself.
+// count in device memory, j.n_win its capacity.  It reads j.ig through a (K+1)-mer pair table it builds in stream-ordered
+// scratch before its launch (frisk_nibble.cu); the hand-over reads j.ig itself.
 LaunchShape nibble_shape(const WinPlan& p, int K);
-int score_nibble(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                 const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K, int want_rip,
-                 double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st, const unsigned long long* n_win_dev = nullptr);
+int score_nibble(const WinPlan& p, const WinJob& j, const unsigned long long* n_win_dev = nullptr);
 // the k sweep (BASELINE config C3): rows of kmax' = 1..8, kmin 1, from one pass over every window; ig / rows / status are
 // HOST arrays of 8 device pointers
 int score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,

@@ -688,14 +688,15 @@ const void* nibble_fn(const frisk_internal::WinPlan& p) {
     return FRISK_WIN_INSTANCE(p, score_windows_nibble_kernel, K, 32);
 }
 
-// one launch of a nibble-kernel instantiation, the sweep's included (they share the signature)
-int launch_nibble(const frisk_internal::LaunchShape& s, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                  const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, const double2* pair, int kmin, int want_rip,
-                  double* rows, uint32_t* status, uint16_t* dump, uint32_t* redo_dst, NibSweep sw, cudaStream_t st) {
-    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-    uint32_t n = (uint32_t)n_win;
-    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &pair, &kmin, &want_rip, &rows, &status, &dump, &redo_dst, &sw};
-    return frisk_internal::launch_persistent(s, n_win, args, st);
+// one launch of a nibble-kernel instantiation, the sweep's included (they share the signature); the kernel reads pair in
+// place of j.ig
+int launch_nibble(const frisk_internal::LaunchShape& s, const frisk_internal::WinJob& j, const double2* pair, uint32_t* redo_dst,
+                  NibSweep sw) {
+    frisk_internal::WinJob a = j;                      // the kernel arguments are read from their addresses
+    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(a.win_off);
+    uint32_t n = (uint32_t)a.n_win;
+    void* args[] = {&a.codes, &a.inv, &a.low, &off, &a.win_len, &n, &pair, &a.kmin, &a.rip, &a.rows, &a.status, &a.dump, &redo_dst, &sw};
+    return frisk_internal::launch_persistent(s, a.n_win, args, a.st);
 }
 
 }  // namespace
@@ -705,10 +706,9 @@ frisk_internal::LaunchShape frisk_internal::nibble_shape(const WinPlan& p, int K
     return {nibble_fn<7>(p), kNT, NibLayout<7>::TOTAL, true};
 }
 
-int frisk_internal::score_nibble(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                                 const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
-                                 int kmin, int K, int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st,
-                                 const unsigned long long* n_win_dev) {
+int frisk_internal::score_nibble(const WinPlan& p, const WinJob& j, const unsigned long long* n_win_dev) {
+    const int K = j.K;
+    const cudaStream_t st = j.st;
     if (K != 7 && K != 8) return FRISK_E_UNSUPPORTED;
     NibSweep sw{};
     sw.n_win_dev = n_win_dev;
@@ -718,16 +718,14 @@ int frisk_internal::score_nibble(const WinPlan& p, const uint32_t* codes, const 
     const uint32_t n_pair = pow4(K + 1);
     uint4* pair = nullptr;
     FRISK_CK(cudaMallocAsync((void**)&pair, (size_t)n_pair * 32u, st));
-    (K == 8 ? ivom_pair_kernel<8> : ivom_pair_kernel<7>)<<<n_pair / 256u, 256, 0, st>>>(reinterpret_cast<const uint4*>(ig), pair);
+    (K == 8 ? ivom_pair_kernel<8> : ivom_pair_kernel<7>)<<<n_pair / 256u, 256, 0, st>>>(reinterpret_cast<const uint4*>(j.ig), pair);
     const cudaError_t le = cudaGetLastError();
     if (le != cudaSuccess) rc = cuda_fail(le, "ivom_pair_kernel");
     if (!rc)
-        rc = with_redo_marks(status, n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
-            int rc2 = launch_nibble(nibble_shape(p, K), codes, inv, low, win_off, win_len, n_win, reinterpret_cast<const double2*>(pair),
-                                    kmin, want_rip, rows, status, dump, redo, sw, st);
+        rc = with_redo_marks(j.status, j.n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
+            int rc2 = launch_nibble(nibble_shape(p, K), j, reinterpret_cast<const double2*>(pair), redo, sw);
             // windows the nibble table could not hold (marked kRowRedo): exact re-run on the bucketed kernel, which reads ig
-            return rc2 ? rc2 : score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status,
-                                                 dump, redo, st);
+            return rc2 ? rc2 : score_bucket_redo(j, redo);
         });
     const cudaError_t e = cudaFreeAsync(pair, st);                     // stream-ordered: behind the launches above
     if (!rc && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync(pair table)");
@@ -749,12 +747,14 @@ int frisk_internal::score_sweep(const uint32_t* codes, const uint32_t* inv, cons
     const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, true>
                      : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, true>
                                 : (const void*)score_windows_nibble_kernel<8, 32, false, true, true>;
+    const WinJob all{codes, inv, low, win_off, win_len, n_win, max_len, nullptr, 1, 8, want_rip, nullptr, nullptr, nullptr, st};
     return with_redo_marks(nullptr, n_win, false, st, [&](uint32_t* redo) {
-        int rc = launch_nibble({fn, kNT, NibLayout<8>::TOTAL, true}, codes, inv, low, win_off, win_len, n_win, nullptr, 1, want_rip,
-                               nullptr, nullptr, nullptr, redo, sw, st);
-        for (int k = 1; k <= 8 && !rc; ++k)
-            rc = score_bucket_redo(codes, inv, low, win_off, win_len, n_win, max_len, ig[k - 1], 1, k, want_rip && k >= 2, rows[k - 1],
-                                   status[k - 1], nullptr, redo, st);
+        int rc = launch_nibble({fn, kNT, NibLayout<8>::TOTAL, true}, all, nullptr, redo, sw);
+        for (int k = 1; k <= 8 && !rc; ++k) {
+            WinJob one = all;                                          // kmax' = k alone
+            one.ig = ig[k - 1]; one.K = k; one.rip = rip_orders(want_rip, 1, k); one.rows = rows[k - 1]; one.status = status[k - 1];
+            rc = score_bucket_redo(one, redo);
+        }
         return rc;
     });
 }

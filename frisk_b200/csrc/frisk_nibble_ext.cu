@@ -481,19 +481,18 @@ frisk_internal::LaunchShape frisk_internal::ext_shape(const WinPlan& p) {
     return {fn, kNT, ExtLayout::TOTAL, true};
 }
 
-int frisk_internal::score_nibble_ext(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                                     const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig,
-                                     int kmin, int K, int want_rip, double* rows, uint32_t* status, cudaStream_t st) {
-    if (K < 9 || K > 12) return FRISK_E_UNSUPPORTED;
-    return with_redo_marks(status, n_win, false, st, [&](uint32_t* redo) {
-        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-        const double2* g = reinterpret_cast<const double2*>(ig);
-        uint32_t n = (uint32_t)n_win;
-        void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &K, &want_rip, &rows, &status, &redo};
-        int rc = launch_persistent(ext_shape(p), n_win, args, st);
+int frisk_internal::score_nibble_ext(const WinPlan& p, const WinJob& j) {
+    if (j.K < 9 || j.K > 12) return FRISK_E_UNSUPPORTED;
+    return with_redo_marks(j.status, j.n_win, false, j.st, [&](uint32_t* redo) {
+        WinJob a = j;                                  // the kernel arguments are read from their addresses
+        const unsigned long long* off = reinterpret_cast<const unsigned long long*>(a.win_off);
+        const double2* g = reinterpret_cast<const double2*>(a.ig);
+        uint32_t n = (uint32_t)a.n_win;
+        void* args[] = {&a.codes, &a.inv, &a.low, &off, &a.win_len, &n, &g, &a.kmin, &a.K, &a.rip, &a.rows, &a.status, &redo};
+        int rc = launch_persistent(ext_shape(p), a.n_win, args, a.st);
         // the windows this kernel could not hold: exact re-run on the general kernel (few CTAs: the slab is 156 MB per CTA
         // at kmax 12, and a hand-over launch usually has nothing to do)
-        return rc ? rc : general_score(codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, nullptr, st,
-                                       redo, K <= 10 ? 8 : 2);
+        a.dump = nullptr;
+        return rc ? rc : general_score(p, a, redo, a.K <= 10 ? 8 : 2);
     });
 }

@@ -508,7 +508,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
     const double min_size = (double)w + (((double)w * 0.75) - (double)step);
     const uint32_t len_bound = (uint32_t)std::min<double>(4.0e9, std::max<double>((double)w, scaffolds_all ? min_size : 0.0));
     WinPlan tail_plan;
-    const bool dev_tail = rows_cap > 0 && rows_cap <= 0xffffffffull && (uint64_t)w <= FRISK_B200_MAX_WINDOW &&
+    const bool dev_tail = rows_cap > 0 && rows_cap <= 0xffffffffull &&
                           frisk_internal::plan_score(kmin, kmax, len_bound, false, &tail_plan) == FRISK_OK &&
                           tail_plan.kind == WinKernel::Nibble;
     void *dtab = nullptr, *dig = nullptr, *dwin = nullptr, *dfirst = nullptr, *dscal = nullptr;
@@ -539,10 +539,10 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
     auto queue_score = [&](cudaStream_t s2) -> int {
         int rc2;
         if ((rc2 = mark(c.tm, kTmScoreStart, s2))) return rc2;
-        rc2 = frisk_internal::score_nibble(tail_plan, win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
-                                           (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound, (const double*)dig,
-                                           kmin, kmax, j.want_rip && kmin <= 2 && kmax >= 2 /* as frisk_b200_score: RIP needs orders 1 and 2 */,
-                                           r.rows, r.status, nullptr, s2, scal);
+        rc2 = frisk_internal::score(tail_plan, {win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
+                                                (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound,
+                                                (const double*)dig, kmin, kmax, j.want_rip, r.rows, r.status, nullptr, s2},
+                                    scal);
         if (rc2) return rc2;
         tail_queued = true;
         return mark(c.tm, kTmScored, s2);

@@ -1,6 +1,6 @@
 // frisk_b200: the window-kernel layer -- which window kernel frisk_b200_score runs (plan_score), how a persistent window
-// kernel is launched, the hand-over to the small-K and bucketed kernels, the score entry points of the C ABI and the
-// options that force a kernel -- and the KLD of two IVOM vectors.
+// kernel is launched, the hand-over to the small-K and bucketed kernels, the internal score entry that runs a plan, the
+// score entry points of the C ABI and the options that force a kernel -- and the KLD of two IVOM vectors.
 //
 // Replaces the reference's per-window loop (/root/reference/frisk/__init__.py F:1478-1494) by a choice of one kernel
 // for all windows; the kernels are in frisk_small.cu, frisk_bucket.cu, frisk_dense.cu, frisk_direct.cu, frisk_nibble.cu,
@@ -144,17 +144,30 @@ int frisk_internal::launch_persistent(const LaunchShape& s, uint64_t n_win, void
     return FRISK_OK;
 }
 
-int frisk_internal::score_bucket_redo(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
-                                      const uint32_t* win_len, uint64_t n_win, uint32_t max_len, const double* ig, int kmin, int K,
-                                      int want_rip, double* rows, uint32_t* status, uint16_t* dump, const uint32_t* redo_src,
-                                      cudaStream_t st) {
-    if (max_len > kSmemMaxWindow || !redo_src) return FRISK_E_UNSUPPORTED;
+int frisk_internal::score_bucket_redo(const WinJob& j, const uint32_t* redo_src) {
+    if (j.max_len > kSmemMaxWindow || !redo_src) return FRISK_E_UNSUPPORTED;
     // the generic instantiation (any kmin, optional dump); the k sweep hands a window over for EVERY kmax': 4..6 on the
     // bucketed kernel too, 1..3 on the small-K kernel
-    const WinPlan p{K <= 3 ? WinKernel::Small : WinKernel::Bucket, window_variant(WinKernel::Bucket, max_len), dump != nullptr, false};
-    if (K <= 3)
-        return score_small(p, codes, inv, low, win_off, win_len, n_win, ig, kmin, K, want_rip, rows, status, dump, st, redo_src);
-    return score_bucket(p, codes, inv, low, win_off, win_len, n_win, max_len, ig, kmin, K, want_rip, rows, status, dump, st, redo_src);
+    const WinPlan p{j.K <= 3 ? WinKernel::Small : WinKernel::Bucket, window_variant(WinKernel::Bucket, j.max_len), j.dump != nullptr,
+                    false};
+    if (j.K <= 3) return score_small(p, j, redo_src);
+    return score_bucket(p, j, redo_src);
+}
+
+int frisk_internal::score(const WinPlan& p, WinJob j, const unsigned long long* n_win_dev) {
+    if (j.max_len > FRISK_B200_MAX_WINDOW || j.n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
+    if (n_win_dev && p.kind != WinKernel::Nibble) return FRISK_E_UNSUPPORTED;
+    j.rip = rip_orders(j.rip, j.kmin, j.K);
+    switch (p.kind) {
+        case WinKernel::NibbleExt: return score_nibble_ext(p, j);
+        case WinKernel::General: return general_score(p, j);
+        case WinKernel::Nibble: return score_nibble(p, j, n_win_dev);
+        case WinKernel::Direct: return score_direct(p, j);
+        case WinKernel::Small: return score_small(p, j);
+        case WinKernel::Bucket: return score_bucket(p, j);
+        case WinKernel::Dense: return score_dense(p, j);
+    }
+    return FRISK_E_UNSUPPORTED;
 }
 
 extern "C" {
@@ -167,33 +180,8 @@ int frisk_b200_score(const uint32_t* d_codes, const uint32_t* d_inv, const uint3
     WinPlan p;
     int rc = frisk_internal::plan_score(kmin, kmax, max_win_len, d_dump != nullptr, &p);
     if (rc) return rc;
-    if (max_win_len > FRISK_B200_MAX_WINDOW || n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int rip = want_rip && kmin <= 2 && kmax >= 2;
-    switch (p.kind) {
-        case WinKernel::NibbleExt:
-            return frisk_internal::score_nibble_ext(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax,
-                                                    rip, d_rows, d_status, st);
-        case WinKernel::General:
-            return frisk_internal::general_score(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                                 d_rows, d_status, d_dump, st);
-        case WinKernel::Nibble:
-            return frisk_internal::score_nibble(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                                d_rows, d_status, d_dump, st);
-        case WinKernel::Direct:
-            return frisk_internal::score_direct(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                                d_rows, d_status, d_dump, st);
-        case WinKernel::Small:
-            return frisk_internal::score_small(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, d_ig, kmin, kmax, rip, d_rows,
-                                               d_status, d_dump, st);
-        case WinKernel::Bucket:
-            return frisk_internal::score_bucket(p, d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                                d_rows, d_status, d_dump, st);
-        case WinKernel::Dense:
-            return frisk_internal::score_dense(d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, rip,
-                                               d_rows, d_status, d_dump, st);
-    }
-    return FRISK_E_UNSUPPORTED;
+    return frisk_internal::score(p, {d_codes, d_inv, d_low, d_win_off, d_win_len, n_win, max_win_len, d_ig, kmin, kmax, want_rip,
+                                     d_rows, d_status, d_dump, (cudaStream_t)stream});
 }
 
 int frisk_b200_score_sweep(const uint32_t* d_codes, const uint32_t* d_inv, const uint32_t* d_low, const uint64_t* d_win_off,

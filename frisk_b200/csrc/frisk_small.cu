@@ -264,14 +264,12 @@ frisk_internal::LaunchShape frisk_internal::small_shape(const WinPlan& p, int K)
     }
 }
 
-int frisk_internal::score_small(const WinPlan& p, const uint32_t* codes, const uint32_t* inv, const uint32_t* low,
-                                const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win, const double* ig, int kmin, int K,
-                                int want_rip, double* rows, uint32_t* status, uint16_t* dump, cudaStream_t st,
-                                const uint32_t* redo_src) {
-    if (K < 1 || K > 6) return FRISK_E_UNSUPPORTED;
-    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(win_off);
-    const double2* g = reinterpret_cast<const double2*>(ig);
-    uint32_t n = (uint32_t)n_win;
-    void* args[] = {&codes, &inv, &low, &off, &win_len, &n, &g, &kmin, &want_rip, &rows, &status, &dump, &redo_src};
-    return launch_persistent(small_shape(p, K), n_win, args, st);
+int frisk_internal::score_small(const WinPlan& p, const WinJob& j, const uint32_t* redo_src) {
+    if (j.K < 1 || j.K > 6) return FRISK_E_UNSUPPORTED;
+    WinJob a = j;                                      // the kernel arguments are read from their addresses
+    const unsigned long long* off = reinterpret_cast<const unsigned long long*>(a.win_off);
+    const double2* g = reinterpret_cast<const double2*>(a.ig);
+    uint32_t n = (uint32_t)a.n_win;
+    void* args[] = {&a.codes, &a.inv, &a.low, &off, &a.win_len, &n, &g, &a.kmin, &a.rip, &a.rows, &a.status, &a.dump, &redo_src};
+    return launch_persistent(small_shape(p, a.K), a.n_win, args, a.st);
 }
