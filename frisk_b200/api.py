@@ -38,7 +38,7 @@ __all__ = ["LETTERS", "tempPathCheck", "countN", "calcGC", "iterFasta", "crawlGe
            "scrubMirrors", "flattenKmerMap", "pcaFeatures", "pcaFeaturesFromIntervals", "score_genome", "FRISK_VERSION"]
 
 FRISK_VERSION = "b200-0.1"
-LETTERS = ("A", "T", "G", "C")             # F:70 -- alphabet and table order
+LETTERS = engine.LETTERS                   # F:70 -- alphabet and table order
 _UPPER = b"ATGC"
 
 
@@ -118,17 +118,7 @@ def crawlGenome(args, querySeq: str) -> Iterator[Tuple[str, str, int, int]]:
         yield seq, names[s], int(wins.start[i]), int(wins.stop[i])
 
 
-_KEYS: Dict[int, List[str]] = {}
-
-
-def _kmer_keys(k: int) -> List[str]:
-    """All 4^k words in the reference's dict order (F:253-265)."""
-    if k not in _KEYS:
-        words = [""]
-        for _ in range(k):
-            words = [w + c for w in words for c in LETTERS]
-        _KEYS[k] = words
-    return _KEYS[k]
+_kmer_keys = engine.kmer_words              # all 4^k words in the reference's dict order (F:253-265)
 
 
 def prepareMaps(k: int, maxk: int, kmers: Sequence[str]) -> Dict[str, int]:
@@ -367,13 +357,23 @@ def score_genome(args, device="cuda:0") -> engine.HotPathResult:
 
 def genome_kmers_from_result(res: engine.HotPathResult) -> list:
     """The reference's genomeKmers object (F:356-359) from a batch result."""
-    full = np.zeros(_lib.table_size(1, res.kmax), dtype=np.uint64)
-    full[_lib.table_size(1, res.kmin - 1) if res.kmin > 1 else 0:] = res.tables
-    maps = _tables_to_dicts(full, res.kmin, res.kmax)
-    maps.append({"totalLen": res.meta[0]})
-    maps.append({"exMax": res.meta[1]})
-    maps.append({"nnTotal": res.meta[2]})
-    return maps
+    return engine.genome_kmers(res.tables, res.kmin, res.kmax, res.meta)
+
+
+def score_background(args, background, source: str, device="cuda:0") -> engine.HotPathResult:
+    """Every window row of ``args.querySeq or args.hostSeq`` scored against stored background tables instead of tables
+    counted from ``args.hostSeq``, which is only opened when it is also the query.  ``background``: (tables, kmin, kmax,
+    meta) of ``engine.genome_kmers_tables``, from the reference's genomeKmers object loaded from ``source`` (F:1437)."""
+    tables, kmin, kmax, meta = background
+    path = args.querySeq or args.hostSeq
+    query = engine.open_genome_file(path, lambda buf, kind: engine.DeviceGenome._open_native(buf, device, kind))
+    # (the reference's cache key has no --maskHost, SURVEY section 5: the stored tables win, whatever the flag says now)
+    logging.info("Scoring %s against the background tables in %s (orders %d..%d, totalLen %d, nnTotal %d); %s is not "
+                 "counted again" % (path, source, kmin, kmax, meta[0], meta[2], args.hostSeq))
+    with engine.Background(tables, kmin, kmax, meta, device) as bg:
+        res = bg.run_resident(query, w=args.windowlen, step=args.increment, scaffolds_all=args.scaffoldsAll, rip=bool(args.RIP))
+    res.raise_reference_errors()                 # the reference aborts on ZeroDivisionError (F:437, F:136)
+    return res
 
 
 def windows_frame(res: engine.HotPathResult, with_rip: bool):
@@ -469,14 +469,22 @@ def main(argv=None):
     have_genome = os.path.isfile(genomepickle) and args.recalc      # F:1437
     have_windows = os.path.isfile(windowsPickle) and args.recalcWin  # F:1454
     res = None
-    if not have_genome or not have_windows:
-        logging.info("Calculating kmers for host sequence: %s" % args.hostSeq)
-        res = score_genome(args)                                    # one GPU pass produces both products
     if have_genome:
         logging.info("Importing previously calculated genome kmers from %s" % genomepickle)
         with open(genomepickle, "rb") as fh:
             genomeKmers = pickle.load(fh)
-    else:
+    if not have_genome or not have_windows:
+        if have_genome:                                             # the windows against the stored tables (F:1437)
+            try:                                                    # orders -m..-k of 4^k words + meta, before any device work
+                background = engine.genome_kmers_tables(genomeKmers, args.minWordSize, args.maxWordSize)
+            except ValueError as e:
+                logging.error("[ERROR] %s: %s" % (genomepickle, e))
+                sys.exit(1)
+            res = score_background(args, background, genomepickle)
+        else:
+            logging.info("Calculating kmers for host sequence: %s" % args.hostSeq)
+            res = score_genome(args)                                # one GPU pass produces both products
+    if not have_genome:
         genomeKmers = genome_kmers_from_result(res)
         with open(genomepickle, "wb") as fh:
             pickle.dump(genomeKmers, fh, protocol=2)                # F:363 (protocol 2: readable by a py2 frisk)

@@ -11,10 +11,23 @@
 #include <chrono>
 #include <functional>
 #include <mutex>
+#include <new>
 #include <vector>
 
 #include "../../include/frisk_b200.h"
 #include "frisk_internal.h"
+
+// A resident background (frisk_b200_background_open): the genome IVOM table of finalised tables, in device memory of its
+// own -- not the run workspace, which the next ordinary run on the device reuses.
+struct frisk_b200_background {
+    int dev, kmin, kmax;
+    int64_t space;
+    double* ig;
+};
+
+static_assert(FRISK_FORMAT_TEXT == (int)frisk_internal::kFmtText && FRISK_FORMAT_BGZF == (int)frisk_internal::kFmtBgzf &&
+                  FRISK_FORMAT_GZIP == (int)frisk_internal::kFmtGzip && FRISK_FORMAT_2BIT == (int)frisk_internal::kFmt2bit,
+              "FRISK_FORMAT_* are the public names of frisk_internal::TextFormat");
 
 namespace {
 using frisk_internal::WinKernel;
@@ -187,6 +200,13 @@ struct PeerArgs {
 size_t table_words(int kmax) { return (size_t)frisk_b200_table_size(1, kmax); }
 size_t ivom_bytes(int kmax) { return (size_t)16 << (2 * kmax); }
 
+// a background handle serves the device it was opened on
+int bg_current(const struct frisk_b200_background* bg) {
+    int dev = 0;
+    CK(cudaGetDevice(&dev));
+    return dev == bg->dev ? FRISK_OK : FRISK_E_INVALID;
+}
+
 // The checks of a run from planes, before anything touches a device: the planes are there and padded to whole 128-base
 // tiles, kmin / kmax, and every window lies inside the query planes -- the window list is host memory here, and a window
 // outside the planes would be an illegal-address fault (and a sticky context error) in the window kernel: O(n), ~1 ns
@@ -275,15 +295,18 @@ int results(RunCall& c, uint64_t n, const Rows& r, const Job& j, const void* dta
 typedef std::function<int(WindowList* wins)> LateWindows;
 
 // Everything after the planes are on the device (or on their way, on the copy stream): [background count unless
-// `counted`], tables, window list, window kernel, results.
+// `counted`], tables, window list, window kernel, results.  bg_ig (nullable): a resident background's genome IVOM table,
+// which takes the place of the count and the tables step.
 int run_tail(RunCall& c, const PeerArgs& peers, const Planes& h, bool counted, const Planes& q, WindowList wins, const Job& j,
-             int64_t space, void* dfwd, const LateWindows* late = nullptr) {
+             int64_t space, void* dfwd, const LateWindows* late = nullptr, const double* bg_ig = nullptr) {
     const size_t tsz = table_words(j.kmax);
-    void *dtab = nullptr, *dig = nullptr, *dwo = nullptr, *dwl = nullptr;
+    void *dtab = nullptr, *dig = (void*)bg_ig, *dwo = nullptr, *dwl = nullptr;
     Rows r{};
     int rc;
-    if ((rc = ws_get(kWsTables, (tsz + 1) * 8, &dtab))) return rc;
-    if ((rc = ws_get(kWsIvom, ivom_bytes(j.kmax), &dig))) return rc;
+    if (!bg_ig) {
+        if ((rc = ws_get(kWsTables, (tsz + 1) * 8, &dtab))) return rc;
+        if ((rc = ws_get(kWsIvom, ivom_bytes(j.kmax), &dig))) return rc;
+    }
     auto upload_windows = [&]() -> int {
         if (wins.n) {
             int rc2;
@@ -306,15 +329,17 @@ int run_tail(RunCall& c, const PeerArgs& peers, const Planes& h, bool counted, c
         return FRISK_OK;
     };
     if (!late && (rc = upload_windows())) return rc;
-    if (!counted) {
+    if (!counted && !bg_ig) {
         CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, c.st));
         // the last 32-base word is padding by construction and is only ever read as look-ahead
         rc = frisk_b200_background(h.codes, h.inv, h.low, 0, h.padded_len - 32, j.kmax, j.mask_host, (uint64_t*)dfwd, c.st);
         if (rc) return rc;
         if ((rc = mark(c.tm, kTmCounted, c.st))) return rc;
     }
-    if ((rc = queue_tables(c, peers, dfwd, j, space, nullptr, dtab, dig, c.st))) return rc;
-    g_trace.stamp("finalize_queued");
+    if (!bg_ig) {
+        if ((rc = queue_tables(c, peers, dfwd, j, space, nullptr, dtab, dig, c.st))) return rc;
+        g_trace.stamp("finalize_queued");
+    }
     if (late) {
         if ((rc = (*late)(&wins))) return rc;
         g_trace.stamp("windows");
@@ -476,16 +501,20 @@ int stage_get(int dev, int slot, size_t bytes, void** out) {
 }
 
 // fmt: h_text / q_text are texts, BGZF buffers or gzip members (the last two inflated on the device by the ingest), or .2bit
-// files (decoded on the device into the planes by frisk_twobit.cu)
-int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt,
-                   int w, int step, int scaffolds_all, const Job& j, uint64_t rows_cap, uint64_t* n_win_out,
-                   frisk_b200_fasta** host_out, frisk_b200_fasta** query_out) {
+// files (decoded on the device into the planes by frisk_twobit.cu).  bg (nullable): a resident background in place of the
+// host genome -- there is no h_text, q_text is ingested as planes only, and bg's genome IVOM table is what the windows are
+// scored against.  That table's source is the one thing the two kinds of call do differently.
+int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n,
+                   frisk_internal::TextFormat fmt, int w, int step, int scaffolds_all, const Job& j, uint64_t rows_cap,
+                   uint64_t* n_win_out, frisk_b200_fasta** host_out, frisk_b200_fasta** query_out) {
     const int kmin = j.kmin, kmax = j.kmax;
     const size_t tsz = table_words(kmax);
-    void* dfwd;
+    void* dfwd = nullptr;
     int rc;
-    if ((rc = ws_get(kWsFwd, (tsz + 1) * 8, &dfwd))) return rc;
-    CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, c.st));
+    if (!bg) {
+        if ((rc = ws_get(kWsFwd, (tsz + 1) * 8, &dfwd))) return rc;
+        CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, c.st));
+    }
 
     frisk_internal::IngestSink sink;
     if (kmax <= FRISK_B200_FAST_K)
@@ -498,7 +527,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
         return (int)FRISK_OK;
     };
     sink.uploaded_mark = c.tm->ev[kTmUploaded];
-    const bool same = !q_text || (q_text == h_text && q_n == h_n);
+    const bool same = !bg && (!q_text || (q_text == h_text && q_n == h_n));
 
     // ---- the device-only tail: with the nibble kernel (kmax 7, 8; windows <= 8,186 bases) everything behind the ingest is queued
     // from inside the open, before the host has seen the record table -- genome space and window list by frisk_windows.cu,
@@ -515,8 +544,8 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
     Rows r{};
     bool tail_queued = false;
     if (dev_tail) {
-        if ((rc = ws_get(kWsTables, (tsz + 1) * 8, &dtab))) return rc;
-        if ((rc = ws_get(kWsIvom, ivom_bytes(kmax), &dig))) return rc;
+        if (bg) dig = (void*)bg->ig;
+        else if ((rc = ws_get(kWsTables, (tsz + 1) * 8, &dtab)) || (rc = ws_get(kWsIvom, ivom_bytes(kmax), &dig))) return rc;
         if ((rc = ws_get(kWsWinOff, rows_cap * 12, &dwin))) return rc;
         if ((rc = ws_get(kWsScalars, 64, &dscal))) return rc;
         if ((rc = rows_for(rows_cap, j, &r))) return rc;
@@ -557,17 +586,22 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
             return same ? queue_score(s2) : FRISK_OK;
         };
     g_trace.stamp("call");
-    if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, fmt, c.st, &sink, host_out))) return rc;
-    g_trace.stamp("open_returned");
-    c.tm->have[kTmUploaded] = h_n > 0;                              // (recorded behind the last text chunk)
-    const bool counted = sink.counted;
-    bool tail_ok = dev_tail && counted && (tail_queued || !same);   // (an exact re-open leaves counted == false)
-    if (!tail_ok) c.tm->have[kTmFinalised] = c.tm->have[kTmScoreStart] = c.tm->have[kTmScored] = false;
-    if (counted && !dev_tail && (rc = mark(c.tm, kTmCounted, c.st))) return rc;
-    frisk_b200_fasta* hh = *host_out;
+    frisk_b200_fasta* hh = nullptr;
+    bool counted = true, tail_ok = dev_tail;
+    if (!bg) {
+        if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, fmt, c.st, &sink, host_out))) return rc;
+        g_trace.stamp("open_returned");
+        c.tm->have[kTmUploaded] = h_n > 0;                          // (recorded behind the last text chunk)
+        counted = sink.counted;
+        tail_ok = dev_tail && counted && (tail_queued || !same);    // (an exact re-open leaves counted == false)
+        if (!tail_ok) c.tm->have[kTmFinalised] = c.tm->have[kTmScoreStart] = c.tm->have[kTmScored] = false;
+        if (counted && !dev_tail && (rc = mark(c.tm, kTmCounted, c.st))) return rc;
+        hh = *host_out;
+    }
     frisk_b200_fasta* qh = hh;
     if (!same) {
         frisk_internal::IngestSink qsink;                            // planes only: nothing of the query is counted
+        if (bg) qsink.uploaded_mark = c.tm->ev[kTmUploaded];         // with a background the query is the only upload
         bool q_queued = false;
         if (tail_ok)
             qsink.on_complete = [&](frisk_b200_fasta* h, cudaStream_t s2) -> int {
@@ -579,18 +613,19 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
             };
         qsink.counted = false;
         if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, fmt, c.st, &qsink, query_out))) return rc;
+        if (bg) c.tm->have[kTmUploaded] = q_n > 0;
         qh = *query_out;
         // (qsink has no on_range, so `counted` says nothing: a query that was re-opened exactly has a handle without the
         // speculative table the hook used -- detect it by the hook not having run or the open statistics)
         tail_ok = tail_ok && q_queued && frisk_internal::fasta_open_was_streamed(qh);
     }
-    uint64_t h_rec = 0, h_padded = 0, h_stats[3], q_rec = 0, q_padded = 0, q_stats[3];
-    if ((rc = frisk_b200_fasta_info(hh, &h_rec, &h_padded, h_stats))) return rc;
+    uint64_t h_rec = 0, h_padded = 0, h_stats[3] = {}, q_rec = 0, q_padded = 0, q_stats[3];
+    const uint32_t *dhc = nullptr, *dhi = nullptr, *dhl = nullptr, *dqc, *dqi, *dql;
+    if (hh && ((rc = frisk_b200_fasta_info(hh, &h_rec, &h_padded, h_stats)) || (rc = frisk_b200_fasta_planes(hh, &dhc, &dhi, &dhl))))
+        return rc;
     if ((rc = frisk_b200_fasta_info(qh, &q_rec, &q_padded, q_stats))) return rc;
-    const uint32_t *dhc, *dhi, *dhl, *dqc, *dqi, *dql;
-    if ((rc = frisk_b200_fasta_planes(hh, &dhc, &dhi, &dhl))) return rc;
     if ((rc = frisk_b200_fasta_planes(qh, &dqc, &dqi, &dql))) return rc;
-    const int64_t space = (int64_t)h_stats[0] - (int64_t)h_stats[1];
+    const int64_t space = bg ? bg->space : (int64_t)h_stats[0] - (int64_t)h_stats[1];
 
     if (tail_ok) {
         // everything is queued: bring the rows and the [window count, genome space] back, wait, check the capacity
@@ -599,7 +634,7 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
         if ((rc = results(c, rows_cap, r, j, dtab, dscal, h_scal, 16))) return rc;
         const uint64_t n_win = ((const uint64_t*)h_scal)[0];
         if (n_win_out) *n_win_out = n_win;
-        if ((int64_t)((const uint64_t*)h_scal)[1] != space) return FRISK_E_CUDA;   // (cannot happen)
+        if (!bg && (int64_t)((const uint64_t*)h_scal)[1] != space) return FRISK_E_CUDA;   // (cannot happen)
         return n_win > rows_cap ? FRISK_E_CAPACITY : FRISK_OK;
     }
     // windows of the query (F:194-251), into pinned staging -- produced once the tables' finalisation is queued
@@ -628,11 +663,11 @@ int run_fasta_body(RunCall& c, const char* h_text, uint64_t h_n, const char* q_t
     CK(cudaEventRecord(c.cc->join, c.st));                          // the copy stream joins behind the ingest
     CK(cudaStreamWaitEvent(c.cc->copy, c.cc->join, 0));
     return run_tail(c, PeerArgs(), Planes{dhc, dhi, dhl, h_padded}, counted, Planes{dqc, dqi, dql, q_padded}, {}, j, space, dfwd,
-                    &late);
+                    &late, bg ? bg->ig : nullptr);
 }
 
-// frisk_b200_run_fasta, _run_fasta_bgzf, _run_fasta_gzip and _run_2bit
-int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
+// frisk_b200_run_fasta, _run_fasta_bgzf, _run_fasta_gzip, _run_2bit (bg == nullptr) and frisk_b200_background_run
+int run_fasta_any(const struct frisk_b200_background* bg, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
                   int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                   uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                   frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
@@ -643,12 +678,13 @@ int run_fasta_any(const char* h_text, uint64_t h_n, const char* q_text, uint64_t
     int rc = frisk_internal::check_k(kmin, kmax);
     if (rc) return rc;
     if (w < 1 || step < 1) return FRISK_E_INVALID;
+    if (bg && (rc = bg_current(bg))) return rc;
     const Job j{kmin, kmax, mask_host, want_rip, rows_out, status_out, tables_out, valid_kmax_out};
     RunCall c;
     bool threw = false;
     if (!(rc = c.enter(stream, true))) {
         try {
-            rc = run_fasta_body(c, h_text, h_n, q_text, q_n, fmt, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
+            rc = run_fasta_body(c, bg, h_text, h_n, q_text, q_n, fmt, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
         } catch (...) {
             rc = FRISK_E_CAPACITY;
             threw = true;
@@ -730,7 +766,7 @@ int frisk_b200_run_fasta(const char* h_text, uint64_t h_n, const char* q_text, u
                          int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                          uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                          frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_text, h_n, q_text, q_n, frisk_internal::kFmtText, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
+    return run_fasta_any(nullptr, h_text, h_n, q_text, q_n, frisk_internal::kFmtText, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip, rows_cap, rows_out,
                          status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
@@ -738,7 +774,7 @@ int frisk_b200_run_fasta_bgzf(const char* h_gz, uint64_t h_n, const char* q_gz, 
                               int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                               uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                               frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_gz, h_n, q_gz, q_n, frisk_internal::kFmtBgzf, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+    return run_fasta_any(nullptr, h_gz, h_n, q_gz, q_n, frisk_internal::kFmtBgzf, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
                          rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
@@ -746,7 +782,7 @@ int frisk_b200_run_fasta_gzip(const char* h_gz, uint64_t h_n, const char* q_gz, 
                               int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                               uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                               frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_gz, h_n, q_gz, q_n, frisk_internal::kFmtGzip, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+    return run_fasta_any(nullptr, h_gz, h_n, q_gz, q_n, frisk_internal::kFmtGzip, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
                          rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
 }
 
@@ -754,8 +790,79 @@ int frisk_b200_run_2bit(const char* h_2bit, uint64_t h_n, const char* q_2bit, ui
                         int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
                         uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out, frisk_b200_fasta** host_out,
                         frisk_b200_fasta** query_out, void* stream) {
-    return run_fasta_any(h_2bit, h_n, q_2bit, q_n, frisk_internal::kFmt2bit, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
+    return run_fasta_any(nullptr, h_2bit, h_n, q_2bit, q_n, frisk_internal::kFmt2bit, w, step, scaffolds_all, kmin, kmax, mask_host, want_rip,
                          rows_cap, rows_out, status_out, tables_out, valid_kmax_out, n_win_out, host_out, query_out, stream);
+}
+
+int frisk_b200_background_open(const uint64_t* tables, int kmin, int kmax, int64_t genome_space, void* stream,
+                               struct frisk_b200_background** out) {
+    if (!tables || !out || genome_space <= 0) return FRISK_E_INVALID;   // (a space <= 0 is where F:379-437 divides by zero)
+    *out = nullptr;
+    int rc = frisk_internal::check_k(kmin, kmax);
+    if (rc) return rc;
+    if (frisk_b200_device_count() <= 0) return FRISK_E_NO_DEVICE;
+    const cudaStream_t st = (cudaStream_t)stream;
+    struct frisk_b200_background bg{0, kmin, kmax, genome_space, nullptr};
+    uint64_t* dtab = nullptr;
+    // the tables in the 1..kmax layout the IVOM kernels read, orders below kmin zero (they are never read)
+    auto build = [&]() -> int {
+        CK(cudaGetDevice(&bg.dev));
+        const size_t tsz = table_words(kmax), lo = kmin > 1 ? table_words(kmin - 1) : 0;
+        CK(cudaMalloc((void**)&bg.ig, ivom_bytes(kmax)));
+        CK(cudaMalloc((void**)&dtab, tsz * 8));
+        if (lo) CK(cudaMemsetAsync(dtab, 0, lo * 8, st));
+        CK(cudaMemcpyAsync(dtab + lo, tables, (tsz - lo) * 8, cudaMemcpyHostToDevice, st));
+        int rc2 = frisk_b200_genome_ivom(dtab, kmin, kmax, genome_space, bg.ig, stream);
+        if (rc2) return rc2;
+        CK(cudaStreamSynchronize(st));
+        return FRISK_OK;
+    };
+    rc = build();
+    if (rc) cudaStreamSynchronize(st);
+    if (dtab) cudaFree(dtab);
+    struct frisk_b200_background* h = rc ? nullptr : new (std::nothrow) struct frisk_b200_background(bg);
+    if (!h) {
+        if (bg.ig) cudaFree(bg.ig);
+        cudaGetLastError();
+        return rc ? rc : frisk_internal::cuda_fail(cudaErrorMemoryAllocation, "new frisk_b200_background");
+    }
+    *out = h;
+    return FRISK_OK;
+}
+
+int frisk_b200_background_run(const struct frisk_b200_background* bg, const char* q, uint64_t q_n, int format, int w, int step,
+                              int scaffolds_all, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
+                              uint64_t* n_win_out, frisk_b200_fasta** query_out, void* stream) {
+    if (!bg || !q || format < FRISK_FORMAT_TEXT || format > FRISK_FORMAT_2BIT) return FRISK_E_INVALID;
+    frisk_b200_fasta* no_host = nullptr;
+    return run_fasta_any(bg, nullptr, 0, q, q_n, (frisk_internal::TextFormat)format, w, step, scaffolds_all, bg->kmin, bg->kmax, 0,
+                         want_rip, rows_cap, rows_out, status_out, nullptr, nullptr, n_win_out, &no_host, query_out, stream);
+}
+
+int frisk_b200_background_score(const struct frisk_b200_background* bg, const uint32_t* d_codes, const uint32_t* d_inv,
+                                const uint32_t* d_low, uint64_t padded_len, const uint64_t* win_off, const uint32_t* win_len,
+                                uint64_t n_win, uint32_t max_win_len, int want_rip, double* rows_out, uint32_t* status_out,
+                                void* stream) {
+    if (!bg) return FRISK_E_INVALID;
+    const WindowList wins{win_off, win_len, n_win, max_win_len};
+    const Job j{bg->kmin, bg->kmax, 0, want_rip, rows_out, status_out, nullptr, nullptr};
+    int rc = check_plane_run(d_codes && d_inv, padded_len, padded_len, wins, j);
+    if (rc || (rc = bg_current(bg))) return rc;
+    RunCall c;
+    if (!(rc = c.enter(stream, false)))
+        rc = run_tail(c, PeerArgs(), Planes{}, true, Planes{d_codes, d_inv, d_low, padded_len}, wins, j, bg->space, nullptr, nullptr,
+                      bg->ig);
+    return c.leave(rc);
+}
+
+int frisk_b200_background_close(struct frisk_b200_background* bg, void* stream) {
+    if (!bg) return FRISK_OK;
+    int rc = bg_current(bg);
+    if (rc) return rc;
+    CK(cudaStreamSynchronize((cudaStream_t)stream));
+    CK(cudaFree(bg->ig));
+    delete bg;
+    return FRISK_OK;
 }
 
 // Stage times (ms) of the last frisk_b200_run_* call on the current device,

@@ -12,6 +12,7 @@ C call from pinned host buffers used for end-to-end timing.
 from __future__ import annotations
 
 import ctypes as C
+import os
 import sys
 from dataclasses import dataclass, field
 from typing import List, Optional, Sequence, Tuple, Union
@@ -762,6 +763,13 @@ def assemble(query: PackedGenome, host: PackedGenome, wins: WindowList, tables_1
              names: bool = True) -> HotPathResult:
     """``names=False`` leaves the per-row name list empty (``row_scaf`` + ``scaf_names`` carry the same information
     without a Python object per row: millions of rows of a fragmented assembly)."""
+    meta = (host.total_len, host.ex_max(kmax, valid_kmax), host.nn_total)
+    return _assemble_rows(query, wins, _slice_orders(tables_1k, kmin, kmax).copy(), meta, rows, status, kmin, kmax, dump, names)
+
+
+def _assemble_rows(query: PackedGenome, wins: WindowList, tables: np.ndarray, meta, rows: np.ndarray, status: np.ndarray,
+                   kmin: int, kmax: int, dump: Optional[np.ndarray] = None, names: bool = True) -> HotPathResult:
+    """``assemble`` with the background's tables (orders kmin..kmax) and meta given as they are."""
     keep = (status & _lib.ROW_EXCLUDED) == 0
     n_all = len(status)
     if bool(keep.all()):
@@ -781,11 +789,10 @@ def assemble(query: PackedGenome, host: PackedGenome, wins: WindowList, tables_1
         coords[:, 1] = take(wins.stop)
     else:
         coords = np.zeros((0, 2), np.int64)
-    meta = (host.total_len, host.ex_max(kmax, valid_kmax), host.nn_total)
     wt = None
     if dump is not None:
         wt = _slice_orders(take(dump), kmin, kmax)
-    return HotPathResult(kmin, kmax, _slice_orders(tables_1k, kmin, kmax).copy(), meta, names, coords,
+    return HotPathResult(kmin, kmax, tables, meta, names, coords,
                          take(rows), take(status).astype(np.uint32, copy=False), len(wins), idx, scaf.astype(np.int64), wt,
                          scaf_names=list(query.names) if want_names else query.names)
 
@@ -1302,3 +1309,223 @@ class HostOutputs:
         self.status = _alloc((max(n_win, 1),), np.uint32, pinned)
         self.tables = _alloc((_lib.table_size(1, kmax),), np.uint64, pinned)
         self.valid = _alloc((1,), np.uint64, pinned)
+
+
+# ---------------------------------------------------------------------- stored backgrounds (the reference's genome pickle)
+LETTERS = ("A", "T", "G", "C")             # F:70 -- alphabet and table order
+_WORDS = {}
+
+
+def kmer_words(k: int) -> List[str]:
+    """All 4^k words in the reference's dict order (F:253-265): the order of every table here."""
+    if k not in _WORDS:
+        words = [""]
+        for _ in range(k):
+            words = [w + c for w in words for c in LETTERS]
+        _WORDS[k] = words
+    return _WORDS[k]
+
+
+_META_KEYS = ("totalLen", "exMax", "nnTotal")
+
+
+def genome_kmers(tables: np.ndarray, kmin: int, kmax: int, meta) -> list:
+    """The reference's genomeKmers object (F:356-359): one dict per order kmin..kmax (``tables``: those orders
+    concatenated), then ``{'totalLen'}``, ``{'exMax'}``, ``{'nnTotal'}`` -- what it pickles (F:363)."""
+    maps, a = [], 0
+    for k in range(kmin, kmax + 1):
+        maps.append(dict(zip(kmer_words(k), (int(v) for v in tables[a:a + 4 ** k]))))
+        a += 4 ** k
+    maps.extend({key: int(v)} for key, v in zip(_META_KEYS, meta))
+    return maps
+
+
+def genome_kmers_tables(maps, kmin: Optional[int] = None, kmax: Optional[int] = None):
+    """The inverse of ``genome_kmers``: (tables uint64 of orders kmin..kmax, kmin, kmax, meta).  Words are looked up by
+    key, so a pickle written by the reference's Python 2 frisk (keys in py2 hash order) gives the same tables.  kmin /
+    kmax default to the orders the dicts hold.  ValueError, naming the problem, for a missing or extra order, an order
+    without exactly its 4^k words, or a missing meta dict."""
+    if not isinstance(maps, (list, tuple)):
+        raise ValueError("genome k-mer tables: expected a list of dicts, got %s" % type(maps).__name__)
+    meta, orders = {}, {}
+    for d in maps:
+        if not isinstance(d, dict):
+            raise ValueError("genome k-mer tables: an entry is a %s, not a dict" % type(d).__name__)
+        if len(d) == 1 and next(iter(d)) in _META_KEYS:
+            meta.update(d)
+            continue
+        if not d:
+            raise ValueError("genome k-mer tables: an order's table is empty")
+        k = len(next(iter(d)))
+        if k in orders:
+            raise ValueError("genome k-mer tables: order %d appears twice" % k)
+        orders[k] = d
+    missing = [key for key in _META_KEYS if key not in meta]
+    if missing:
+        raise ValueError("genome k-mer tables: the meta dict {'%s'} is missing" % missing[0])
+    if not orders:
+        raise ValueError("genome k-mer tables: no k-mer table")
+    kmin = min(orders) if kmin is None else int(kmin)
+    kmax = max(orders) if kmax is None else int(kmax)
+    want = set(range(kmin, kmax + 1))
+    lost, extra = sorted(want - set(orders)), sorted(set(orders) - want)
+    if lost:
+        raise ValueError("genome k-mer tables: order %d is missing (orders %d..%d expected)" % (lost[0], kmin, kmax))
+    if extra:
+        raise ValueError("genome k-mer tables: order %d is extra (orders %d..%d expected)" % (extra[0], kmin, kmax))
+    tables = np.empty(_lib.table_size(kmin, kmax), np.uint64)
+    a = 0
+    for k in range(kmin, kmax + 1):
+        d = orders[k]
+        if len(d) != 4 ** k:
+            raise ValueError("genome k-mer tables: order %d holds %d words, not 4^%d = %d" % (k, len(d), k, 4 ** k))
+        try:
+            tables[a:a + 4 ** k] = np.fromiter((d[w] for w in kmer_words(k)), dtype=np.uint64, count=4 ** k)
+        except KeyError as e:
+            raise ValueError("genome k-mer tables: order %d lacks the word %s" % (k, e.args[0])) from None
+        a += 4 ** k
+    return tables, kmin, kmax, tuple(int(meta[key]) for key in _META_KEYS)
+
+
+def _kind_of(buf: np.ndarray) -> str:
+    """What a genome buffer is, by its signature: "2bit", "bgzf", "gzip" or "text"."""
+    return "2bit" if is_2bit(buf) else "bgzf" if is_bgzf(buf) else "gzip" if is_gzip(buf) else "text"
+
+
+class Background:
+    """A host genome's background tables resident on one GPU (frisk_b200_background_open): any number of queries are
+    scored against them without the host genome, which is neither read, uploaded nor counted.  ``tables``: uint64, orders
+    kmin..kmax concatenated in the reference's dict order (``HotPathResult.tables``), finalised -- both strands,
+    ``--maskHost`` applied or not when they were counted; ``meta``: (totalLen, exMax, nnTotal).  The genome IVOM table
+    is built once, when the background is opened.  Goes through the C ABI alone (no PyTorch).  Close it, or use it as a
+    context manager."""
+
+    def __init__(self, tables, kmin: int, kmax: int, meta, device="cuda:0"):
+        tab = np.ascontiguousarray(tables, dtype=np.uint64)
+        if not 1 <= kmin <= kmax:
+            raise ValueError("background orders %d..%d" % (kmin, kmax))
+        if kmax > _lib.MAX_K:
+            _lib.check(_lib.E_UNSUPPORTED, "frisk_b200 Background(kmax=%d)" % kmax)
+        if tab.shape != (_lib.table_size(kmin, kmax),):
+            raise ValueError("background tables: %s entries, orders %d..%d need %d"
+                             % (tab.shape, kmin, kmax, _lib.table_size(kmin, kmax)))
+        self.tables, self.kmin, self.kmax, self.meta = tab, int(kmin), int(kmax), tuple(int(x) for x in meta)
+        self.device = device
+        self.genome_space = self.meta[0] - self.meta[2]        # totalLen - nnTotal (F:379)
+        self._h = C.c_void_p()
+        L = _lib.lib()
+        with self._on_device():
+            _lib.check(L.frisk_b200_background_open(_ptr(tab), self.kmin, self.kmax, self.genome_space,
+                                                    _stream_ptr(self.device), C.byref(self._h)), "frisk_b200_background_open")
+
+    @classmethod
+    def from_result(cls, res: HotPathResult, device="cuda:0") -> "Background":
+        """The background of a run (its ``tables`` and ``meta``)."""
+        return cls(res.tables, res.kmin, res.kmax, res.meta, device)
+
+    @classmethod
+    def from_genome_kmers(cls, maps, kmin: Optional[int] = None, kmax: Optional[int] = None, device="cuda:0") -> "Background":
+        """The background of the reference's genomeKmers object -- what ``<host>_kmers_<m>_<k>_genome.p`` holds (F:363),
+        written by this package or by the reference; ``genome_kmers_tables`` says what is refused."""
+        tables, kmin, kmax, meta = genome_kmers_tables(maps, kmin, kmax)
+        return cls(tables, kmin, kmax, meta, device)
+
+    def genome_kmers(self) -> list:
+        """The reference's genomeKmers object of these tables (``from_genome_kmers``' inverse)."""
+        return genome_kmers(self.tables, self.kmin, self.kmax, self.meta)
+
+    def _on_device(self):
+        if _torch_loaded():
+            return _device_ctx(self.device)
+        _lib.check(_lib.lib().frisk_b200_set_device(_device_index(self.device)), "frisk_b200_set_device")
+        return _NULL_CTX
+
+    def _result(self, query: PackedGenome, wins: WindowList, rows, status) -> HotPathResult:
+        return _assemble_rows(query, wins, self.tables.copy(), self.meta, rows, status, self.kmin, self.kmax)
+
+    def run(self, query, kind: Optional[str] = None, w: int = 5000, step: int = 2500, scaffolds_all: bool = False,
+            rip: bool = True, out=None, assemble_result: bool = True):
+        """The windows of ``query`` scored against this background in one C call (frisk_b200_background_run): the query
+        half of ``run_fasta``.  ``query``: a path (``kind`` from ``read_genome_raw``), or the genome's bytes with ``kind``
+        "text", "bgzf", "gzip" or "2bit" (by signature when not given).  ``out``: reusable buffers with ``rows`` and
+        ``status`` (their row capacity is used; ``out.n_win`` is set).  The result's ``tables`` and ``meta`` are the
+        background's."""
+        if kind is None and isinstance(query, (str, os.PathLike)):
+            buf, kind = read_genome_raw(os.fspath(query))
+        else:
+            buf = _as_u8(query)
+            kind = kind or _kind_of(buf)
+        L = _lib.lib()
+        if out is None:
+            n_text = _text_len_hint(buf, kind)                 # a guess, as in run_fasta; FRISK_E_CAPACITY is handled below
+            out = HostOutputs(n_text // step + n_text // 4096 + 64, 0, pinned=_torch_loaded())
+        qh = C.c_void_p()
+        n_win = C.c_uint64(0)
+        with self._on_device():
+            st = _stream_ptr(self.device)
+            rc = L.frisk_b200_background_run(self._h, _ptr(buf), buf.shape[0], _lib.FORMAT[kind], w, step, int(scaffolds_all),
+                                             int(rip), out.rows.shape[0], _ptr(out.rows), _ptr(out.status), C.byref(n_win),
+                                             C.byref(qh), st)
+            try:
+                if rc not in (_lib.OK, _lib.E_CAPACITY):
+                    _lib.check(rc, "frisk_b200_background_run")
+                n = int(n_win.value)
+                query = _genome_from_handle(L, qh, buf, kind != "text") if assemble_result or rc == _lib.E_CAPACITY else None
+                if rc == _lib.E_CAPACITY:
+                    # more windows than rows: the query's planes are on the device, score them into enough rows
+                    c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
+                    _lib.check(L.frisk_b200_fasta_planes(qh, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
+                    out = HostOutputs(n, 0, pinned=_torch_loaded())
+                    self._score(query, (_HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value)),
+                                query.windows(w, step, scaffolds_all), rip, out)
+            finally:
+                if qh:
+                    L.frisk_b200_fasta_close(qh, st)
+        out.n_win = n
+        if not assemble_result:
+            return out
+        wins = query.windows(w, step, scaffolds_all)
+        assert len(wins) == n
+        return self._result(query, wins, out.rows[:n], out.status[:n])
+
+    def run_resident(self, dq: DeviceGenome, w: int = 5000, step: int = 2500, scaffolds_all: bool = False, rip: bool = True,
+                     wins: Optional[WindowList] = None, out=None, assemble_result: bool = True):
+        """``engine.run_resident`` with this background in place of the host genome (frisk_b200_background_score): the
+        windows of planes already on the device, scored in one C call."""
+        query = dq.host
+        if wins is None:
+            wins = query.windows(w, step, scaffolds_all)
+        n = len(wins)
+        if out is None:
+            out = HostOutputs(n, 0, pinned=_torch_loaded() and not isinstance(dq.codes, DevBuf))
+        self._score(query, (dq.codes, dq.inv, dq.low), wins, rip, out)
+        if not assemble_result:
+            return out
+        return self._result(query, wins, out.rows[:n], out.status[:n])
+
+    def _score(self, query: PackedGenome, planes, wins: WindowList, rip: bool, out) -> None:
+        codes, inv, low = planes
+        with self._on_device():
+            _lib.check(_lib.lib().frisk_b200_background_score(
+                self._h, _ptr(codes), _ptr(inv), _ptr(low), query.padded_len, _ptr(wins.off), _ptr(wins.length), len(wins),
+                wins.max_len, int(rip), _ptr(out.rows), _ptr(out.status), _stream_ptr(self.device)),
+                "frisk_b200_background_score")
+
+    def close(self) -> None:
+        if self._h:
+            with self._on_device():
+                _lib.check(_lib.lib().frisk_b200_background_close(self._h, _stream_ptr(self.device)), "frisk_b200_background_close")
+            self._h = C.c_void_p()
+
+    def __enter__(self) -> "Background":
+        return self
+
+    def __exit__(self, *exc) -> bool:
+        self.close()
+        return False
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

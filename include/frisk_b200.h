@@ -496,6 +496,46 @@ int frisk_b200_run_2bit(const char *h_2bit, uint64_t h_n, const char *q_2bit, ui
                         double *rows_out, uint32_t *status_out, uint64_t *tables_out, uint64_t *valid_kmax_out,
                         uint64_t *n_win_out, frisk_b200_fasta **host_out, frisk_b200_fasta **query_out, void *stream);
 
+/* ------------------------------------------------------------------ resident background (frisk_run.cu)
+ *
+ * Scoring queries against background tables the caller already holds -- the reference's genome pickle
+ * (<host>_kmers_<m>_<k>_genome.p, F:363 / F:1437), HotPathResult.tables, the global tables of a multi-GPU run --
+ * without the host genome: no host text is read, uploaded or counted.
+ *
+ * frisk_b200_background_open: `tables` is a HOST array of orders kmin..kmax concatenated (frisk_b200_table_size(kmin,
+ * kmax) entries, the reference's dict order), finalised as the tables of frisk_b200_run_* are (both strands; --maskHost
+ * was applied, or not, when they were counted).  genome_space = totalLen - nnTotal (F:379) of the host genome, > 0.  The
+ * genome IVOM table (frisk_b200_genome_ivom) is built once, into device memory the handle owns, on the current device;
+ * the handle is bound to that device (any call while another one is current: FRISK_E_INVALID).  Argument errors
+ * (NULL tables / out, genome_space <= 0, kmin / kmax as everywhere) are returned before the device is touched.
+ *
+ * frisk_b200_background_run: frisk_b200_run_fasta with the handle in place of the host genome: q (q_n bytes, `format` one
+ * of FRISK_FORMAT_*) is ingested into planes and its windows scored against the handle's table.  rows_out / status_out /
+ * rows_cap / *n_win_out / FRISK_E_CAPACITY / *query_out as there (on FRISK_E_CAPACITY *query_out is valid and
+ * frisk_b200_background_score can run on its planes).  Stage times: ms[1] and ms[2] are -1 (nothing is counted or
+ * finalised), ms[0] is "query uploaded".
+ *
+ * frisk_b200_background_score: frisk_b200_run_resident with the handle in place of the host planes: query planes in
+ * device memory, window list in host memory, rows and status to host memory.
+ *
+ * frisk_b200_background_close: synchronises `stream`, frees the table and the handle (NULL: nothing to do).
+ *
+ * The handle's type is spelled `struct frisk_b200_background`: there is no typedef, because frisk_b200_background is the
+ * name of the background-count function above (struct tags and functions do not collide).
+ */
+struct frisk_b200_background;
+enum { FRISK_FORMAT_TEXT = 0, FRISK_FORMAT_BGZF = 1, FRISK_FORMAT_GZIP = 2, FRISK_FORMAT_2BIT = 3 };
+int frisk_b200_background_open(const uint64_t *tables, int kmin, int kmax, int64_t genome_space, void *stream,
+                               struct frisk_b200_background **out);
+int frisk_b200_background_run(const struct frisk_b200_background *bg, const char *q, uint64_t q_n, int format, int w, int step,
+                              int scaffolds_all, int want_rip, uint64_t rows_cap, double *rows_out, uint32_t *status_out,
+                              uint64_t *n_win_out, frisk_b200_fasta **query_out, void *stream);
+int frisk_b200_background_score(const struct frisk_b200_background *bg, const uint32_t *d_codes, const uint32_t *d_inv,
+                                const uint32_t *d_low, uint64_t padded_len, const uint64_t *win_off, const uint32_t *win_len,
+                                uint64_t n_win, uint32_t max_win_len, int want_rip, double *rows_out, uint32_t *status_out,
+                                void *stream);
+int frisk_b200_background_close(struct frisk_b200_background *bg, void *stream);
+
 /* Stage times (ms since the start of the call) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call
  * on the current device, from CUDA events recorded on the call's own streams: ms[0] planes uploaded, ms[1] background
  * counted, ms[2] tables + genome IVOM finalised (multi-GPU: includes the wait for the peers' counters), ms[3] window
