@@ -16,6 +16,7 @@ OK, E_INVALID, E_UNSUPPORTED, E_CUDA, E_NO_DEVICE, E_CAPACITY, E_FORMAT = 0, -1,
 ROW_KLD_ZERODIV, ROW_GC_ZERODIV, ROW_LOG_DOMAIN, ROW_EXCLUDED = 1, 2, 4, 8
 MAX_K = 12
 MAX_WINDOW = 0x7FFFFFFF
+MAX_BACKGROUNDS = 8                                       # FRISK_B200_MAX_BACKGROUNDS
 FORMAT = {"text": 0, "bgzf": 1, "gzip": 2, "2bit": 3}     # FRISK_FORMAT_*
 
 _p = C.c_void_p
@@ -87,6 +88,9 @@ PROTOTYPES = {
     "frisk_b200_background_open": (_i, [_p, _i, _i, C.c_int64, _p, C.POINTER(C.c_void_p)]),
     "frisk_b200_background_run": (_i, [_p, _p, _u64, _i, _i, _i, _i, _i, _u64, _p, _p, C.POINTER(_u64), C.POINTER(C.c_void_p), _p]),
     "frisk_b200_background_score": (_i, [_p, _p, _p, _p, _u64, _p, _p, _u64, C.c_uint32, _i, _p, _p, _p]),
+    "frisk_b200_background_run_many": (_i, [_p, _i, _p, _u64, _i, _i, _i, _i, _i, _u64, _p, _p, C.POINTER(_u64),
+                                            C.POINTER(C.c_void_p), _p]),
+    "frisk_b200_background_score_many": (_i, [_p, _i, _p, _p, _p, _u64, _p, _p, _u64, C.c_uint32, _i, _p, _p, _p]),
     "frisk_b200_background_close": (_i, [_p, _p]),
     "frisk_b200_last_run_timing": (_i, [C.POINTER(C.c_float), _i, C.POINTER(_i)]),
     "frisk_b200_score_sweep": (_i, [_p, _p, _p, _p, _p, _u64, C.c_uint32, _p, _i, _i, _p, _p, _p]),

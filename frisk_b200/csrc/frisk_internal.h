@@ -164,6 +164,10 @@ inline int rip_orders(int want_rip, int kmin, int kmax) { return want_rip && kmi
 // FRISK_E_UNSUPPORTED, and runs the launcher of p.kind.  n_win_dev (nibble kernel only): the window count in device
 // memory, j.n_win its capacity.
 int score(const WinPlan& p, WinJob j, const unsigned long long* n_win_dev = nullptr);
+// One query against n_bg (1..FRISK_B200_MAX_BACKGROUNDS) backgrounds: jobs[b] is background b's job -- the same planes,
+// windows, orders and stream in all of them, its own ig, rows and status.  The one place that chooses between the fused
+// nibble kernel (score_nibble_many) and one score() per background (frisk_score.cu).
+int score_many(const WinPlan& p, const WinJob* jobs, int n_bg, const unsigned long long* n_win_dev = nullptr);
 // the instantiation of a window kernel template <..., DUMP, ALLK> a plan runs: the table dump and kmin > 1 share the generic
 // <..., DUMP, false> one, the production default (no dump, kmin 1) has its own
 #define FRISK_WIN_INSTANCE(p, kern, ...)                                                                      \
@@ -253,6 +257,9 @@ int score_direct(const WinPlan& p, const WinJob& j);
 // scratch before its launch (frisk_nibble.cu); the hand-over reads j.ig itself.
 LaunchShape nibble_shape(const WinPlan& p, int K);
 int score_nibble(const WinPlan& p, const WinJob& j, const unsigned long long* n_win_dev = nullptr);
+// the same for n_bg backgrounds (jobs as for score_many, j.rip already reduced): counts every window once and gathers
+// each background's genome-IVOM entries in one launch; every background's hand-over reads the one set of marks
+int score_nibble_many(const WinPlan& p, const WinJob* jobs, int n_bg, const unsigned long long* n_win_dev);
 // the k sweep (BASELINE config C3): rows of kmax' = 1..8, kmin 1, from one pass over every window; ig / rows / status are
 // HOST arrays of 8 device pointers
 int score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off, const uint32_t* win_len,

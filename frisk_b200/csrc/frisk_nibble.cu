@@ -85,25 +85,48 @@ template <typename MT> __device__ __forceinline__ MT top_bits(int n) {       // 
 // from ONE pass over the window: the counts of every order are there after the marginalisation, so the SWEEP
 // instantiation evaluates all K scores -- kmax' <= K-2 by walking that order's bins (coalesced genome-IVOM reads),
 // K-1 and K per position with weights 1/c -- and writes K rows per window.
+// The MANY instantiation (frisk_b200_background_run_many / _score_many) uses the same arrays for up to 8 backgrounds:
+// ig[0] is the first of n_bg (K+1)-mer pair tables that follow one another, background b's at ig[0] + b * 2 * 4^(K+1);
+// rows[b] / status[b] are its output block.
 struct NibSweep {
     const unsigned long long* n_win_dev;   // nullable: the number of windows lives in device memory (frisk_b200_run_fasta builds
                                            // its window list on the device); the n_win argument is then the capacity
     const double2* ig[8];             // genome IVOM table of kmax' = i + 1
     double* rows[8];
     uint32_t* status[8];
+    int n_bg;
 };
+static_assert(FRISK_B200_MAX_BACKGROUNDS <= 8, "NibSweep holds 8 backgrounds");
+
+// Backgrounds scored per pass of P3 in the MANY instantiation: each adds two fp64 accumulators per thread, and the
+// kernel must keep 4 CTAs of 256 threads (64 registers) without spilling.  Further groups re-run P3 alone on the same
+// shared-memory tables.  -Xptxas -v (DESIGN section 4): two per pass spill nothing up to PP = 20 but 24 bytes at PP = 32,
+// one spills nothing anywhere; three or four spill at PP = 20 too.
+template <int PP> __host__ __device__ constexpr int bg_group() { return PP <= 20 ? 2 : 1; }
+
+enum NibMode : int { kNibOne = 0, kNibSweep = 1, kNibMany = 2 };
 
 // PP = positions per thread: a thread owns ONE chunk of cs <= PP consecutive positions of the window
 // (cs = the window length spread over the CTA, a multiple of 4), reads the three or four code words and two or three
 // mask words that cover it once, and issues the atomics of its full K-words back to back from registers.
-template <int K, int PP, bool DUMP, bool ALLK, bool SWEEP = false>
+//
+// MODE: kNibOne, the window scores against one genome-IVOM table; kNibSweep and kNibMany, see NibSweep.  (An int in the
+// place of the former `bool SWEEP`, so that the kernel's name is spelled as before.)
+//
+// MANY: one query scored against sw.n_bg backgrounds.  P1 and P2 run once per window; P3 computes each position's window
+// side (c_K, 1 / c_K, I_w, log2 I_w) once and folds in every background's genome-IVOM entry with the expressions and in the
+// order of the one-background P3, so that background b's row is bit for bit the one that instantiation writes.  The
+// hand-over marks go to redo_dst only (they depend on the window alone); rows / status are unused.
+template <int K, int PP, bool DUMP, bool ALLK, int MODE = kNibOne>
 __global__ void __launch_bounds__(kNT, 4)
 score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* __restrict__ inv, const uint32_t* __restrict__ low,
                             const unsigned long long* __restrict__ win_off, const uint32_t* __restrict__ win_len, uint32_t n_win,
                             const double2* __restrict__ pair, int kmin_arg, int want_rip,
                             double* __restrict__ rows, uint32_t* __restrict__ status, uint16_t* __restrict__ dump,
                             uint32_t* redo_dst, const NibSweep sw) {
+    constexpr bool SWEEP = MODE == kNibSweep, MANY = MODE == kNibMany;
     static_assert(!SWEEP || (K == 8 && ALLK && !DUMP), "the sweep instantiation: K = 8, kmin = 1");
+    static_assert(!MANY || (!SWEEP && !DUMP), "the multi-background instantiation: no sweep, no dump");
     using L = NibLayout<K>;
     static_assert(PP % 4 == 0 && PP >= 4 && PP + K - 1 <= 64, "chunk size");
     constexpr int A = L::A, LP = L::LP, NT = kNT, NW = NT / 32;
@@ -244,8 +267,8 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         uint16_t* dmp = DUMP ? dump + (size_t)win * lvl_off(K + 1) : nullptr;
         if (excluded) {
             for (uint32_t i = tid; i < L::ZERO_BYTES / 16u; i += NT) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
-            if (SWEEP) {
-                if (tid < K) {
+            if (SWEEP || MANY) {
+                if (tid < (SWEEP ? K : sw.n_bg)) {
                     sw.status[tid][win] = FRISK_ROW_EXCLUDED;
                     for (int c = 0; c < 5; ++c) sw.rows[tid][(size_t)win * 5 + c] = CUDART_NAN;
                 }
@@ -551,9 +574,9 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         }
 
         // ---- P3: every position scores its own K-mer with weight 1 / (its count) --------------------
-        double s_w = 0.0, s_g = 0.0, s_t = 0.0;
         const double qK2 = ss.q[K - 3], qK1 = ss.q[K - 2], qK = ss.q[K - 1];
-        auto score_one = [&](uint32_t kap, const double2 g) {
+        // the window side of one position: a = I_w / c_K, om = 1 / c_K, lw = log2 I_w
+        auto window_side = [&](uint32_t kap, double& a, double& om, double& lw) {
             const uint2 v = nib64[kap >> 4];
             const uint32_t ws = (kap & 8u) ? v.y : v.x, wo = (kap & 8u) ? v.x : v.y;
             const uint32_t cK = (ws >> ((kap & 7u) * 4u)) & 15u;
@@ -582,13 +605,132 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
             asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(D));
             r = fma(r, fma(-D, r, 1.0), r);
             r = fma(r, fma(-D, r, 1.0), r);
-            double a = num * r;
+            a = num * r;
             a = fma(fma(-D, a, num), r, a);
-            const double iw = a * dc;
-            const double om = dden * r;
+            om = dden * r;
+            lw = log2_series(a * dc);
+        };
+        // warp 0: the row of this window from the CTA sums in ss.red -- four IEEE divisions and two logarithms, one per
+        // LANE instead of one after the other in a single thread (the other seven warps of the CTA wait for this at the
+        // barrier behind it)
+        auto finish_row = [&](double* __restrict__ rws, uint32_t* __restrict__ stw) {
+            double a = 0, bsum = 0, c = 0;
+            for (int w = 0; w < NW; ++w) { a += ss.red[0][w]; bsum += ss.red[1][w]; c += ss.red[2][w]; }
+            double nu = 0.0, de = 1.0;
+            if (lane == 0) { nu = c; de = a; }
+            else if (lane == 1) { nu = (double)n_gc; de = (double)n_up; }                                   // F:136
+            else if (lane == 2) { nu = (double)ss.c2[4]; de = (double)ss.c2[1]; }                          // TA / AT, F:480-483
+            else if (lane == 3) { nu = (double)(ss.c2[12] + ss.c2[6]); de = (double)(ss.c2[3] + ss.c2[9]); }  // (CA+TG) / (AC+GT), F:485-489
+            const double qv = nu / de;
+            const double lgv = log2(lane == 0 ? bsum : a);
+            const double q_gc = __shfl_sync(kFull, qv, 1), q_pi = __shfl_sync(kFull, qv, 2), q_si = __shfl_sync(kFull, qv, 3);
+            const double lg_a = __shfl_sync(kFull, lgv, 1);
+            if (lane == 0) {
+                uint32_t st = 0;
+                double kld = 0.0;                          // the reference returns 0 for a window without kmax-mers
+                if (!(a == 0.0)) {
+                    bool zd = bsum != bsum;                // NaN genome IVOM entry: ZeroDivisionError at F:437
+                    for (int x = kmin; x <= K; ++x) zd |= ((long long)n_up - (long long)(x - 1)) == 0;
+                    if (zd) { st |= FRISK_ROW_KLD_ZERODIV; kld = CUDART_NAN; }
+                    else {
+                        kld = qv + (lgv - lg_a);
+                        if (!(kld == kld) || isinf(kld)) st |= FRISK_ROW_LOG_DOMAIN;
+                    }
+                }
+                double* row = rws + (size_t)win * 5;
+                row[0] = kld;
+                if (n_up == 0) { st |= FRISK_ROW_GC_ZERODIV; row[1] = CUDART_NAN; }
+                else row[1] = q_gc;
+                double pi = CUDART_NAN, si = CUDART_NAN, cri = CUDART_NAN;
+                if (want_rip) {
+                    if (ss.c2[1] > 0) pi = q_pi;
+                    if (ss.c2[3] + ss.c2[9] > 0) si = q_si;
+                    if (pi != 0.0 && si != 0.0) cri = pi - si;         // F:491: 0.0 falsy, NaN truthy
+                }
+                row[2] = pi; row[3] = si; row[4] = cri;
+                stw[win] = st;
+                if (redo_dst != stw) redo_dst[win] = 0;
+            }
+        };
+
+        if constexpr (MANY) {
+            constexpr int kBgGroup = bg_group<PP>();
+            constexpr uint32_t kPairTable = 2u * pow4(K + 1);              // double2 entries of one pair table
+            // sw's arrays by a run-time index, each element named at compile time: a dynamic index into a kernel argument
+            // would copy the whole struct to local memory
+            auto pick = [](auto const (&arr)[8], int i) {
+                auto v = arr[0];
+#pragma unroll
+                for (int k = 1; k < 8; ++k) v = i == k ? arr[k] : v;
+                return v;
+            };
+            // each group of backgrounds walks kk and vm again: vm is read through a shift, and kk is rotated CYCLICALLY
+            // through all PP / 4 rounds (the ones beyond the window's only rotate), so that it is whole again afterwards
+            const int rounds = (int)(cs >> 2);
+            for (int g0 = 0; g0 < sw.n_bg; g0 += kBgGroup) {
+                double s_w = 0.0, s_g[kBgGroup], s_t[kBgGroup];
+#pragma unroll
+                for (int b = 0; b < kBgGroup; ++b) s_g[b] = s_t[b] = 0.0;
+                const double2* const pg = sw.ig[0] + (size_t)g0 * kPairTable;     // this group's first pair table
+#pragma unroll 1
+                for (int r = 0; r < PP / 4; ++r) {
+                    const MT vr = r < rounds ? vm << (4 * r) : MT(0);
+#pragma unroll
+                    for (int j = 0; j < 4; j += 2) {
+                        const uint32_t k0 = kk[j / 2] & 0xffffu, k1 = kk[j / 2] >> 16;
+                        const bool v0 = vr & (MT(1) << (MB - 1 - j)), v1 = vr & (MT(1) << (MB - 2 - j));
+                        if (v0 || v1) {
+                            const uint32_t mu = v0 ? ((k0 << 2) | (k1 & 3u)) : k1;     // as in the one-background P3 below
+                            double a0 = 0.0, om0 = 0.0, l0 = 0.0, a1 = 0.0, om1 = 0.0, l1 = 0.0;
+                            if (v0) { window_side(k0, a0, om0, l0); s_w += a0; }
+                            if (v1) { window_side(k1, a1, om1, l1); s_w += a1; }
+#pragma unroll
+                            for (int b = 0; b < kBgGroup; ++b) {
+                                if (g0 + b < sw.n_bg) {
+                                    double2 e0, e1;
+                                    ldcg_pair(pg + (size_t)b * kPairTable + 2u * mu, e0, e1);
+                                    if (v0) { s_g[b] = fma(e0.x, om0, s_g[b]); s_t[b] = fma(a0, l0 - e0.y, s_t[b]); }
+                                    if (v1) { s_g[b] = fma(e1.x, om1, s_g[b]); s_t[b] = fma(a1, l1 - e1.y, s_t[b]); }
+                                }
+                            }
+                        }
+                    }
+                    const uint32_t w0 = kk[0], w1 = kk[1];
+#pragma unroll
+                    for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];
+                    kk[PP / 2 - 2] = w0;
+                    kk[PP / 2 - 1] = w1;
+                }
+#pragma unroll
+                for (int ofs = 16; ofs; ofs >>= 1) {
+                    s_w += __shfl_xor_sync(kFull, s_w, ofs);
+#pragma unroll
+                    for (int b = 0; b < kBgGroup; ++b) {
+                        s_g[b] += __shfl_xor_sync(kFull, s_g[b], ofs);
+                        s_t[b] += __shfl_xor_sync(kFull, s_t[b], ofs);
+                    }
+                }
+#pragma unroll
+                for (int b = 0; b < kBgGroup; ++b) {
+                    if (g0 + b >= sw.n_bg) break;                              // (uniform over the CTA)
+                    if (lane == 0) { ss.red[0][warp] = s_w; ss.red[1][warp] = s_g[b]; ss.red[2][warp] = s_t[b]; }
+                    __syncthreads();                                       // (4) the last group: everyone is done with the tables
+                    if (b == 0 && g0 + kBgGroup >= sw.n_bg)
+                        for (uint32_t i = tid; i < L::ZERO_BYTES / 16u; i += NT) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
+                    if (warp == 0) finish_row(pick(sw.rows, g0 + b), pick(sw.status, g0 + b));
+                    __syncthreads();                                       // (5) ss.red consumed
+                }
+            }
+            continue;
+        }
+
+        double s_w = 0.0, s_g = 0.0, s_t = 0.0;
+        auto score_one = [&](uint32_t kap, const double2 g) {
+            double a, om, lw;
+            window_side(kap, a, om, lw);
             s_w += a;
             s_g = fma(g.x, om, s_g);                       // a NaN entry (reference: ZeroDivisionError) poisons the sum
-            s_t = fma(a, log2_series(iw) - g.y, s_t);
+            s_t = fma(a, lw - g.y, s_t);
         };
         const int rounds = (int)(cs >> 2);
 #pragma unroll 1
@@ -626,47 +768,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         if (lane == 0) { ss.red[0][warp] = s_w; ss.red[1][warp] = s_g; ss.red[2][warp] = s_t; }
         __syncthreads();                                                   // (4) everyone is done with the tables
         for (uint32_t i = tid; i < L::ZERO_BYTES / 16u; i += NT) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
-        if (warp == 0) {
-            // the row: four IEEE divisions and two logarithms, one per LANE instead of one after the other in a single
-            // thread (the other seven warps of the CTA wait for this at the barrier below)
-            double a = 0, bsum = 0, c = 0;
-            for (int w = 0; w < NW; ++w) { a += ss.red[0][w]; bsum += ss.red[1][w]; c += ss.red[2][w]; }
-            double nu = 0.0, de = 1.0;
-            if (lane == 0) { nu = c; de = a; }
-            else if (lane == 1) { nu = (double)n_gc; de = (double)n_up; }                                   // F:136
-            else if (lane == 2) { nu = (double)ss.c2[4]; de = (double)ss.c2[1]; }                          // TA / AT, F:480-483
-            else if (lane == 3) { nu = (double)(ss.c2[12] + ss.c2[6]); de = (double)(ss.c2[3] + ss.c2[9]); }  // (CA+TG) / (AC+GT), F:485-489
-            const double qv = nu / de;
-            const double lgv = log2(lane == 0 ? bsum : a);
-            const double q_gc = __shfl_sync(kFull, qv, 1), q_pi = __shfl_sync(kFull, qv, 2), q_si = __shfl_sync(kFull, qv, 3);
-            const double lg_a = __shfl_sync(kFull, lgv, 1);
-            if (lane == 0) {
-                uint32_t st = 0;
-                double kld = 0.0;                          // the reference returns 0 for a window without kmax-mers
-                if (!(a == 0.0)) {
-                    bool zd = bsum != bsum;                // NaN genome IVOM entry: ZeroDivisionError at F:437
-                    for (int x = kmin; x <= K; ++x) zd |= ((long long)n_up - (long long)(x - 1)) == 0;
-                    if (zd) { st |= FRISK_ROW_KLD_ZERODIV; kld = CUDART_NAN; }
-                    else {
-                        kld = qv + (lgv - lg_a);
-                        if (!(kld == kld) || isinf(kld)) st |= FRISK_ROW_LOG_DOMAIN;
-                    }
-                }
-                double* row = rows + (size_t)win * 5;
-                row[0] = kld;
-                if (n_up == 0) { st |= FRISK_ROW_GC_ZERODIV; row[1] = CUDART_NAN; }
-                else row[1] = q_gc;
-                double pi = CUDART_NAN, si = CUDART_NAN, cri = CUDART_NAN;
-                if (want_rip) {
-                    if (ss.c2[1] > 0) pi = q_pi;
-                    if (ss.c2[3] + ss.c2[9] > 0) si = q_si;
-                    if (pi != 0.0 && si != 0.0) cri = pi - si;         // F:491: 0.0 falsy, NaN truthy
-                }
-                row[2] = pi; row[3] = si; row[4] = cri;
-                status[win] = st;
-                if (redo_dst != status) redo_dst[win] = 0;
-            }
-        }
+        if (warp == 0) finish_row(rows, status);
         __syncthreads();                                                   // (5) tables zeroed, ss.red consumed
     }
 }
@@ -732,6 +834,58 @@ int frisk_internal::score_nibble(const WinPlan& p, const WinJob& j, const unsign
     return rc;
 }
 
+namespace {
+template <int K>
+const void* nibble_many_fn(const frisk_internal::WinPlan& p) {
+    if (p.allk) {
+        if (p.variant == 8) return (const void*)score_windows_nibble_kernel<K, 8, false, true, kNibMany>;
+        if (p.variant == 20) return (const void*)score_windows_nibble_kernel<K, 20, false, true, kNibMany>;
+        return (const void*)score_windows_nibble_kernel<K, 32, false, true, kNibMany>;
+    }
+    if (p.variant == 8) return (const void*)score_windows_nibble_kernel<K, 8, false, false, kNibMany>;
+    if (p.variant == 20) return (const void*)score_windows_nibble_kernel<K, 20, false, false, kNibMany>;
+    return (const void*)score_windows_nibble_kernel<K, 32, false, false, kNibMany>;
+}
+}  // namespace
+
+// One query, n_bg backgrounds: one pair table per background (stream-ordered scratch, one allocation), one launch of the
+// MANY instantiation, then the hand-over of each background on the one set of marks.
+int frisk_internal::score_nibble_many(const WinPlan& p, const WinJob* jobs, int n_bg, const unsigned long long* n_win_dev) {
+    const WinJob& j = jobs[0];
+    const int K = j.K;
+    const cudaStream_t st = j.st;
+    if ((K != 7 && K != 8) || p.dump || n_bg < 1 || n_bg > FRISK_B200_MAX_BACKGROUNDS) return FRISK_E_UNSUPPORTED;
+    NibSweep sw{};
+    sw.n_win_dev = n_win_dev;
+    sw.n_bg = n_bg;
+    int rc = pool_ready();
+    if (rc) return rc;
+    const uint32_t n_pair = pow4(K + 1);
+    uint4* pair = nullptr;
+    FRISK_CK(cudaMallocAsync((void**)&pair, (size_t)n_pair * 32u * (size_t)n_bg, st));
+    sw.ig[0] = reinterpret_cast<const double2*>(pair);
+    for (int b = 0; b < n_bg && !rc; ++b) {
+        uint4* pb = pair + (size_t)b * n_pair * 2u;
+        (K == 8 ? ivom_pair_kernel<8> : ivom_pair_kernel<7>)<<<n_pair / 256u, 256, 0, st>>>(reinterpret_cast<const uint4*>(jobs[b].ig), pb);
+        const cudaError_t le = cudaGetLastError();
+        if (le != cudaSuccess) rc = cuda_fail(le, "ivom_pair_kernel");
+        sw.rows[b] = jobs[b].rows;
+        sw.status[b] = jobs[b].status;
+    }
+    // the marks always go to scratch: they serve every background's hand-over, and each of those rewrites its own status
+    if (!rc)
+        rc = with_redo_marks(nullptr, j.n_win, n_win_dev != nullptr, st, [&](uint32_t* redo) {
+            const LaunchShape s{K == 8 ? nibble_many_fn<8>(p) : nibble_many_fn<7>(p), kNT, K == 8 ? NibLayout<8>::TOTAL : NibLayout<7>::TOTAL,
+                                true};
+            int rc2 = launch_nibble(s, j, nullptr, redo, sw);
+            for (int b = 0; b < n_bg && !rc2; ++b) rc2 = score_bucket_redo(jobs[b], redo);
+            return rc2;
+        });
+    const cudaError_t e = cudaFreeAsync(pair, st);
+    if (!rc && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync(pair tables)");
+    return rc;
+}
+
 // The k sweep: rows of kmax' = 1..8 (kmin 1) for every window from one pass (see NibSweep).  A window the 4-bit counters
 // cannot hold is handed, for every kmax', to the kernel that serves that kmax' on its own.
 int frisk_internal::score_sweep(const uint32_t* codes, const uint32_t* inv, const uint32_t* low, const uint64_t* win_off,
@@ -744,9 +898,9 @@ int frisk_internal::score_sweep(const uint32_t* codes, const uint32_t* inv, cons
         sw.ig[k] = reinterpret_cast<const double2*>(ig[k]); sw.rows[k] = rows[k]; sw.status[k] = status[k];
     }
     const int pp = window_variant(WinKernel::Nibble, max_len);
-    const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, true>
-                     : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, true>
-                                : (const void*)score_windows_nibble_kernel<8, 32, false, true, true>;
+    const void* fn = pp == 8    ? (const void*)score_windows_nibble_kernel<8, 8, false, true, kNibSweep>
+                     : pp == 20 ? (const void*)score_windows_nibble_kernel<8, 20, false, true, kNibSweep>
+                                : (const void*)score_windows_nibble_kernel<8, 32, false, true, kNibSweep>;
     const WinJob all{codes, inv, low, win_off, win_len, n_win, max_len, nullptr, 1, 8, want_rip, nullptr, nullptr, nullptr, st};
     return with_redo_marks(nullptr, n_win, false, st, [&](uint32_t* redo) {
         int rc = launch_nibble({fn, kNT, NibLayout<8>::TOTAL, true}, all, nullptr, redo, sw);

@@ -184,6 +184,14 @@ struct WindowList {
     uint64_t n;
     uint32_t max_len;
 };
+// The resident backgrounds a run scores against (frisk_b200_background_run / _score and their _many forms): n handles of
+// one kmin / kmax.  Background b's rows and status go to block b, which starts `stride` rows after block b - 1 (0: the
+// window count).
+struct BgSet {
+    const struct frisk_b200_background* const* h;
+    int n;
+    uint64_t stride;
+};
 struct Planes {                  // one genome's planes in device memory
     const uint32_t *codes, *inv, *low;
     uint64_t padded_len;
@@ -207,6 +215,15 @@ int bg_current(const struct frisk_b200_background* bg) {
     return dev == bg->dev ? FRISK_OK : FRISK_E_INVALID;
 }
 
+// The checks of a list of backgrounds, before anything touches a device: 1..FRISK_B200_MAX_BACKGROUNDS handles, none NULL,
+// all of one kmin / kmax (the windows, and which orders are counted, depend on them)
+int check_backgrounds(const struct frisk_b200_background* const* bgs, int n_bg) {
+    if (!bgs || n_bg < 1 || n_bg > FRISK_B200_MAX_BACKGROUNDS) return FRISK_E_INVALID;
+    for (int b = 0; b < n_bg; ++b)
+        if (!bgs[b] || bgs[b]->kmin != bgs[0]->kmin || bgs[b]->kmax != bgs[0]->kmax) return FRISK_E_INVALID;
+    return FRISK_OK;
+}
+
 // The checks of a run from planes, before anything touches a device: the planes are there and padded to whole 128-base
 // tiles, kmin / kmax, and every window lies inside the query planes -- the window list is host memory here, and a window
 // outside the planes would be an illegal-address fault (and a sticky context error) in the window kernel: O(n), ~1 ns
@@ -226,12 +243,17 @@ int check_plane_run(bool planes, uint64_t h_padded_len, uint64_t q_padded_len, c
 // Where the window kernel writes n rows and their status: straight into the caller's buffers when both are page-locked
 // host memory with a device view (40 + 4 bytes per window, posted PCIe writes while it runs, no download behind it; a
 // pageable pointer makes the query itself report an error, which is cleared), else into workspace rows that results downloads.
+// nb blocks of n rows, `stride` rows apart (several backgrounds, BgSet), are laid out the same way in both.
 struct Rows {
     double* rows;
     uint32_t* status;
     bool direct;
+    int nb = 1;
+    uint64_t stride = 0;
 };
-int rows_for(uint64_t n, const Job& j, Rows* r) {
+int rows_for(uint64_t n, const Job& j, Rows* r, int nb = 1, uint64_t stride = 0) {
+    r->nb = nb;
+    r->stride = stride ? stride : n;
     cudaPointerAttributes pa_rows{}, pa_stat{};
     r->direct = cudaPointerGetAttributes(&pa_rows, j.rows) == cudaSuccess && pa_rows.type == cudaMemoryTypeHost &&
                 cudaPointerGetAttributes(&pa_stat, j.status) == cudaSuccess && pa_stat.type == cudaMemoryTypeHost &&
@@ -243,8 +265,9 @@ int rows_for(uint64_t n, const Job& j, Rows* r) {
         return FRISK_OK;
     }
     int rc;
-    if ((rc = ws_get(kWsRows, n * 40, (void**)&r->rows))) return rc;
-    return ws_get(kWsStatus, n * 4, (void**)&r->status);
+    const uint64_t all = (uint64_t)(nb - 1) * r->stride + n;
+    if ((rc = ws_get(kWsRows, all * 40, (void**)&r->rows))) return rc;
+    return ws_get(kWsStatus, all * 4, (void**)&r->status);
 }
 
 // The tables step: the counters in dfwd (this GPU's, or summed over the peers') become the tables (kWsTables) and the
@@ -268,15 +291,17 @@ int queue_tables(RunCall& c, const PeerArgs& peers, const void* dfwd, const Job&
     return FRISK_OK;
 }
 
-// The results step, on the caller's stream: n rows and their status unless the window kernel wrote them through pinned
+// The results step, on the caller's stream: n rows and their status (of each block) unless the window kernel wrote them through pinned
 // views, the tables unless they went back on the copy stream, then `extra` bytes from d_extra (if any); kTmEnd; wait for
 // the caller's stream, then the copy stream.
 int results(RunCall& c, uint64_t n, const Rows& r, const Job& j, const void* dtab, const void* d_extra = nullptr,
             void* h_extra = nullptr, size_t extra = 0) {
-    if (n && !r.direct) {
-        CK(cudaMemcpyAsync(j.rows, r.rows, n * 40, cudaMemcpyDeviceToHost, c.st));
-        CK(cudaMemcpyAsync(j.status, r.status, n * 4, cudaMemcpyDeviceToHost, c.st));
-    }
+    if (n && !r.direct)
+        for (int b = 0; b < r.nb; ++b) {
+            const uint64_t o = (uint64_t)b * r.stride;
+            CK(cudaMemcpyAsync(j.rows + o * 5, r.rows + o * 5, n * 40, cudaMemcpyDeviceToHost, c.st));
+            CK(cudaMemcpyAsync(j.status + o, r.status + o, n * 4, cudaMemcpyDeviceToHost, c.st));
+        }
     const size_t tsz = table_words(j.kmax);
     if (!c.cc && j.tables) CK(cudaMemcpyAsync(j.tables, dtab, tsz * 8, cudaMemcpyDeviceToHost, c.st));
     if (!c.cc && j.valid) CK(cudaMemcpyAsync(j.valid, (const uint64_t*)dtab + tsz, 8, cudaMemcpyDeviceToHost, c.st));
@@ -290,16 +315,30 @@ int results(RunCall& c, uint64_t n, const Rows& r, const Job& j, const void* dta
     return FRISK_OK;
 }
 
+// The window kernels of one query against every background of bgs: job j (its ig, rows and status unused) with background
+// b's genome IVOM table and rows block b (frisk_internal::score_many chooses the kernels)
+int score_backgrounds(const WinPlan& p, frisk_internal::WinJob j, const BgSet& bgs, const Rows& r, const unsigned long long* n_win_dev) {
+    frisk_internal::WinJob jobs[FRISK_B200_MAX_BACKGROUNDS];
+    for (int b = 0; b < bgs.n; ++b) {
+        jobs[b] = j;
+        jobs[b].ig = bgs.h[b]->ig;
+        jobs[b].rows = r.rows + (size_t)b * r.stride * 5;
+        jobs[b].status = r.status + (size_t)b * r.stride;
+    }
+    return frisk_internal::score_many(p, jobs, bgs.n, n_win_dev);
+}
+
 // the window list of frisk_b200_run_fasta's host tail, produced by the caller after the tables' finalisation is queued (the
 // host derives the windows while the device is still counting)
 typedef std::function<int(WindowList* wins)> LateWindows;
 
 // Everything after the planes are on the device (or on their way, on the copy stream): [background count unless
-// `counted`], tables, window list, window kernel, results.  bg_ig (nullable): a resident background's genome IVOM table,
-// which takes the place of the count and the tables step.
+// `counted`], tables, window list, window kernel, results.  bgs (nullable): resident backgrounds, whose genome IVOM
+// tables take the place of the count and the tables step.
 int run_tail(RunCall& c, const PeerArgs& peers, const Planes& h, bool counted, const Planes& q, WindowList wins, const Job& j,
-             int64_t space, void* dfwd, const LateWindows* late = nullptr, const double* bg_ig = nullptr) {
+             int64_t space, void* dfwd, const LateWindows* late = nullptr, const BgSet* bgs = nullptr) {
     const size_t tsz = table_words(j.kmax);
+    const double* bg_ig = bgs ? bgs->h[0]->ig : nullptr;
     void *dtab = nullptr, *dig = (void*)bg_ig, *dwo = nullptr, *dwl = nullptr;
     Rows r{};
     int rc;
@@ -315,7 +354,7 @@ int run_tail(RunCall& c, const PeerArgs& peers, const Planes& h, bool counted, c
             if ((rc2 = ws_get(kWsWinOff, one_block ? wins.n * 12 : wins.n * 8, &dwo))) return rc2;
             if (one_block) dwl = (char*)dwo + wins.n * 8;
             else if ((rc2 = ws_get(kWsWinLen, wins.n * 4, &dwl))) return rc2;
-            if ((rc2 = rows_for(wins.n, j, &r))) return rc2;
+            if ((rc2 = rows_for(wins.n, j, &r, bgs ? bgs->n : 1, bgs ? bgs->stride : 0))) return rc2;
             // the window list rides behind the planes -- but a late one goes on the compute stream: the copy stream is busy
             // bringing the tables back by then, and the window kernel would wait 0.03 ms for its 190 KB behind them
             cudaStream_t up = (c.cc && !late) ? c.cc->copy : c.st;
@@ -349,8 +388,17 @@ int run_tail(RunCall& c, const PeerArgs& peers, const Planes& h, bool counted, c
     if (c.cc) CK(cudaStreamWaitEvent(c.st, c.cc->windows, 0));
     if (wins.n) {
         if ((rc = mark(c.tm, kTmScoreStart, c.st))) return rc;
-        rc = frisk_b200_score(q.codes, q.inv, q.low, (const uint64_t*)dwo, (const uint32_t*)dwl, wins.n, wins.max_len,
-                              (const double*)dig, j.kmin, j.kmax, j.want_rip, r.rows, r.status, nullptr, c.st);
+        if (!bgs || bgs->n == 1) {
+            rc = frisk_b200_score(q.codes, q.inv, q.low, (const uint64_t*)dwo, (const uint32_t*)dwl, wins.n, wins.max_len,
+                                  (const double*)dig, j.kmin, j.kmax, j.want_rip, r.rows, r.status, nullptr, c.st);
+        } else {
+            WinPlan p;
+            rc = frisk_internal::plan_score(j.kmin, j.kmax, wins.max_len, false, &p);
+            if (!rc)
+                rc = score_backgrounds(p, {q.codes, q.inv, q.low, (const uint64_t*)dwo, (const uint32_t*)dwl, wins.n, wins.max_len,
+                                           nullptr, j.kmin, j.kmax, j.want_rip, nullptr, nullptr, nullptr, c.st},
+                                       *bgs, r, nullptr);
+        }
         if (rc) return rc;
         g_trace.stamp("score_queued");
         if ((rc = mark(c.tm, kTmScored, c.st))) return rc;
@@ -501,17 +549,17 @@ int stage_get(int dev, int slot, size_t bytes, void** out) {
 }
 
 // fmt: h_text / q_text are texts, BGZF buffers or gzip members (the last two inflated on the device by the ingest), or .2bit
-// files (decoded on the device into the planes by frisk_twobit.cu).  bg (nullable): a resident background in place of the
-// host genome -- there is no h_text, q_text is ingested as planes only, and bg's genome IVOM table is what the windows are
-// scored against.  That table's source is the one thing the two kinds of call do differently.
-int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n,
+// files (decoded on the device into the planes by frisk_twobit.cu).  bgs (nullable): resident backgrounds in place of the
+// host genome -- there is no h_text, q_text is ingested as planes only, and the backgrounds' genome IVOM tables are what
+// the windows are scored against.  That table's source is the one thing the two kinds of call do differently.
+int run_fasta_body(RunCall& c, const BgSet* bgs, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n,
                    frisk_internal::TextFormat fmt, int w, int step, int scaffolds_all, const Job& j, uint64_t rows_cap,
                    uint64_t* n_win_out, frisk_b200_fasta** host_out, frisk_b200_fasta** query_out) {
     const int kmin = j.kmin, kmax = j.kmax;
     const size_t tsz = table_words(kmax);
     void* dfwd = nullptr;
     int rc;
-    if (!bg) {
+    if (!bgs) {
         if ((rc = ws_get(kWsFwd, (tsz + 1) * 8, &dfwd))) return rc;
         CK(cudaMemsetAsync(dfwd, 0, (tsz + 1) * 8, c.st));
     }
@@ -527,7 +575,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
         return (int)FRISK_OK;
     };
     sink.uploaded_mark = c.tm->ev[kTmUploaded];
-    const bool same = !bg && (!q_text || (q_text == h_text && q_n == h_n));
+    const bool same = !bgs && (!q_text || (q_text == h_text && q_n == h_n));
 
     // ---- the device-only tail: with the nibble kernel (kmax 7, 8; windows <= 8,186 bases) everything behind the ingest is queued
     // from inside the open, before the host has seen the record table -- genome space and window list by frisk_windows.cu,
@@ -544,11 +592,11 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
     Rows r{};
     bool tail_queued = false;
     if (dev_tail) {
-        if (bg) dig = (void*)bg->ig;
+        if (bgs) dig = (void*)bgs->h[0]->ig;
         else if ((rc = ws_get(kWsTables, (tsz + 1) * 8, &dtab)) || (rc = ws_get(kWsIvom, ivom_bytes(kmax), &dig))) return rc;
         if ((rc = ws_get(kWsWinOff, rows_cap * 12, &dwin))) return rc;
         if ((rc = ws_get(kWsScalars, 64, &dscal))) return rc;
-        if ((rc = rows_for(rows_cap, j, &r))) return rc;
+        if ((rc = rows_for(rows_cap, j, &r, bgs ? bgs->n : 1, rows_cap))) return rc;
     }
     unsigned long long* const scal = (unsigned long long*)dscal;
     const uint32_t* win_codes[3] = {nullptr, nullptr, nullptr};      // planes of the genome whose windows are scored
@@ -568,10 +616,10 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
     auto queue_score = [&](cudaStream_t s2) -> int {
         int rc2;
         if ((rc2 = mark(c.tm, kTmScoreStart, s2))) return rc2;
-        rc2 = frisk_internal::score(tail_plan, {win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
-                                                (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound,
-                                                (const double*)dig, kmin, kmax, j.want_rip, r.rows, r.status, nullptr, s2},
-                                    scal);
+        const frisk_internal::WinJob job{win_codes[0], win_codes[1], win_codes[2], (const uint64_t*)dwin,
+                                         (const uint32_t*)((unsigned long long*)dwin + rows_cap), rows_cap, len_bound,
+                                         (const double*)dig, kmin, kmax, j.want_rip, r.rows, r.status, nullptr, s2};
+        rc2 = bgs ? score_backgrounds(tail_plan, job, *bgs, r, scal) : frisk_internal::score(tail_plan, job, scal);
         if (rc2) return rc2;
         tail_queued = true;
         return mark(c.tm, kTmScored, s2);
@@ -588,7 +636,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
     g_trace.stamp("call");
     frisk_b200_fasta* hh = nullptr;
     bool counted = true, tail_ok = dev_tail;
-    if (!bg) {
+    if (!bgs) {
         if ((rc = frisk_internal::fasta_open_planes(h_text, h_n, fmt, c.st, &sink, host_out))) return rc;
         g_trace.stamp("open_returned");
         c.tm->have[kTmUploaded] = h_n > 0;                          // (recorded behind the last text chunk)
@@ -601,7 +649,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
     frisk_b200_fasta* qh = hh;
     if (!same) {
         frisk_internal::IngestSink qsink;                            // planes only: nothing of the query is counted
-        if (bg) qsink.uploaded_mark = c.tm->ev[kTmUploaded];         // with a background the query is the only upload
+        if (bgs) qsink.uploaded_mark = c.tm->ev[kTmUploaded];         // with a background the query is the only upload
         bool q_queued = false;
         if (tail_ok)
             qsink.on_complete = [&](frisk_b200_fasta* h, cudaStream_t s2) -> int {
@@ -613,7 +661,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
             };
         qsink.counted = false;
         if ((rc = frisk_internal::fasta_open_planes(q_text, q_n, fmt, c.st, &qsink, query_out))) return rc;
-        if (bg) c.tm->have[kTmUploaded] = q_n > 0;
+        if (bgs) c.tm->have[kTmUploaded] = q_n > 0;
         qh = *query_out;
         // (qsink has no on_range, so `counted` says nothing: a query that was re-opened exactly has a handle without the
         // speculative table the hook used -- detect it by the hook not having run or the open statistics)
@@ -625,7 +673,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
         return rc;
     if ((rc = frisk_b200_fasta_info(qh, &q_rec, &q_padded, q_stats))) return rc;
     if ((rc = frisk_b200_fasta_planes(qh, &dqc, &dqi, &dql))) return rc;
-    const int64_t space = bg ? bg->space : (int64_t)h_stats[0] - (int64_t)h_stats[1];
+    const int64_t space = bgs ? bgs->h[0]->space : (int64_t)h_stats[0] - (int64_t)h_stats[1];
 
     if (tail_ok) {
         // everything is queued: bring the rows and the [window count, genome space] back, wait, check the capacity
@@ -634,7 +682,7 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
         if ((rc = results(c, rows_cap, r, j, dtab, dscal, h_scal, 16))) return rc;
         const uint64_t n_win = ((const uint64_t*)h_scal)[0];
         if (n_win_out) *n_win_out = n_win;
-        if (!bg && (int64_t)((const uint64_t*)h_scal)[1] != space) return FRISK_E_CUDA;   // (cannot happen)
+        if (!bgs && (int64_t)((const uint64_t*)h_scal)[1] != space) return FRISK_E_CUDA;   // (cannot happen)
         return n_win > rows_cap ? FRISK_E_CAPACITY : FRISK_OK;
     }
     // windows of the query (F:194-251), into pinned staging -- produced once the tables' finalisation is queued
@@ -663,11 +711,11 @@ int run_fasta_body(RunCall& c, const struct frisk_b200_background* bg, const cha
     CK(cudaEventRecord(c.cc->join, c.st));                          // the copy stream joins behind the ingest
     CK(cudaStreamWaitEvent(c.cc->copy, c.cc->join, 0));
     return run_tail(c, PeerArgs(), Planes{dhc, dhi, dhl, h_padded}, counted, Planes{dqc, dqi, dql, q_padded}, {}, j, space, dfwd,
-                    &late, bg ? bg->ig : nullptr);
+                    &late, bgs);
 }
 
-// frisk_b200_run_fasta, _run_fasta_bgzf, _run_fasta_gzip, _run_2bit (bg == nullptr) and frisk_b200_background_run
-int run_fasta_any(const struct frisk_b200_background* bg, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
+// frisk_b200_run_fasta, _run_fasta_bgzf, _run_fasta_gzip, _run_2bit (bgs == nullptr) and frisk_b200_background_run(_many)
+int run_fasta_any(const BgSet* bgs, const char* h_text, uint64_t h_n, const char* q_text, uint64_t q_n, frisk_internal::TextFormat fmt, int w, int step,
                   int scaffolds_all, int kmin, int kmax, int mask_host, int want_rip, uint64_t rows_cap, double* rows_out,
                   uint32_t* status_out, uint64_t* tables_out, uint64_t* valid_kmax_out, uint64_t* n_win_out,
                   frisk_b200_fasta** host_out, frisk_b200_fasta** query_out, void* stream) {
@@ -678,13 +726,14 @@ int run_fasta_any(const struct frisk_b200_background* bg, const char* h_text, ui
     int rc = frisk_internal::check_k(kmin, kmax);
     if (rc) return rc;
     if (w < 1 || step < 1) return FRISK_E_INVALID;
-    if (bg && (rc = bg_current(bg))) return rc;
+    for (int b = 0; bgs && b < bgs->n; ++b)
+        if ((rc = bg_current(bgs->h[b]))) return rc;
     const Job j{kmin, kmax, mask_host, want_rip, rows_out, status_out, tables_out, valid_kmax_out};
     RunCall c;
     bool threw = false;
     if (!(rc = c.enter(stream, true))) {
         try {
-            rc = run_fasta_body(c, bg, h_text, h_n, q_text, q_n, fmt, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
+            rc = run_fasta_body(c, bgs, h_text, h_n, q_text, q_n, fmt, w, step, scaffolds_all, j, rows_cap, n_win_out, host_out, query_out);
         } catch (...) {
             rc = FRISK_E_CAPACITY;
             threw = true;
@@ -833,25 +882,49 @@ int frisk_b200_background_open(const uint64_t* tables, int kmin, int kmax, int64
 int frisk_b200_background_run(const struct frisk_b200_background* bg, const char* q, uint64_t q_n, int format, int w, int step,
                               int scaffolds_all, int want_rip, uint64_t rows_cap, double* rows_out, uint32_t* status_out,
                               uint64_t* n_win_out, frisk_b200_fasta** query_out, void* stream) {
-    if (!bg || !q || format < FRISK_FORMAT_TEXT || format > FRISK_FORMAT_2BIT) return FRISK_E_INVALID;
+    return frisk_b200_background_run_many(&bg, 1, q, q_n, format, w, step, scaffolds_all, want_rip, rows_cap, rows_out, status_out,
+                                          n_win_out, query_out, stream);
+}
+
+int frisk_b200_background_run_many(const struct frisk_b200_background* const* bgs, int n_bg, const char* q, uint64_t q_n,
+                                   int format, int w, int step, int scaffolds_all, int want_rip, uint64_t rows_cap,
+                                   double* rows_out, uint32_t* status_out, uint64_t* n_win_out,
+                                   frisk_b200_fasta** query_out, void* stream) {
+    int rc = check_backgrounds(bgs, n_bg);
+    if (rc) return rc;
+    if (!q || format < FRISK_FORMAT_TEXT || format > FRISK_FORMAT_2BIT) return FRISK_E_INVALID;
+    const BgSet set{bgs, n_bg, rows_cap};
     frisk_b200_fasta* no_host = nullptr;
-    return run_fasta_any(bg, nullptr, 0, q, q_n, (frisk_internal::TextFormat)format, w, step, scaffolds_all, bg->kmin, bg->kmax, 0,
-                         want_rip, rows_cap, rows_out, status_out, nullptr, nullptr, n_win_out, &no_host, query_out, stream);
+    return run_fasta_any(&set, nullptr, 0, q, q_n, (frisk_internal::TextFormat)format, w, step, scaffolds_all, bgs[0]->kmin,
+                         bgs[0]->kmax, 0, want_rip, rows_cap, rows_out, status_out, nullptr, nullptr, n_win_out, &no_host, query_out,
+                         stream);
 }
 
 int frisk_b200_background_score(const struct frisk_b200_background* bg, const uint32_t* d_codes, const uint32_t* d_inv,
                                 const uint32_t* d_low, uint64_t padded_len, const uint64_t* win_off, const uint32_t* win_len,
                                 uint64_t n_win, uint32_t max_win_len, int want_rip, double* rows_out, uint32_t* status_out,
                                 void* stream) {
-    if (!bg) return FRISK_E_INVALID;
+    return frisk_b200_background_score_many(&bg, 1, d_codes, d_inv, d_low, padded_len, win_off, win_len, n_win, max_win_len,
+                                            want_rip, rows_out, status_out, stream);
+}
+
+int frisk_b200_background_score_many(const struct frisk_b200_background* const* bgs, int n_bg, const uint32_t* d_codes,
+                                     const uint32_t* d_inv, const uint32_t* d_low, uint64_t padded_len,
+                                     const uint64_t* win_off, const uint32_t* win_len, uint64_t n_win,
+                                     uint32_t max_win_len, int want_rip, double* rows_out, uint32_t* status_out,
+                                     void* stream) {
+    int rc = check_backgrounds(bgs, n_bg);
+    if (rc) return rc;
     const WindowList wins{win_off, win_len, n_win, max_win_len};
-    const Job j{bg->kmin, bg->kmax, 0, want_rip, rows_out, status_out, nullptr, nullptr};
-    int rc = check_plane_run(d_codes && d_inv, padded_len, padded_len, wins, j);
-    if (rc || (rc = bg_current(bg))) return rc;
+    const Job j{bgs[0]->kmin, bgs[0]->kmax, 0, want_rip, rows_out, status_out, nullptr, nullptr};
+    if ((rc = check_plane_run(d_codes && d_inv, padded_len, padded_len, wins, j))) return rc;
+    for (int b = 0; b < n_bg; ++b)
+        if ((rc = bg_current(bgs[b]))) return rc;
+    const BgSet set{bgs, n_bg, 0};
     RunCall c;
     if (!(rc = c.enter(stream, false)))
-        rc = run_tail(c, PeerArgs(), Planes{}, true, Planes{d_codes, d_inv, d_low, padded_len}, wins, j, bg->space, nullptr, nullptr,
-                      bg->ig);
+        rc = run_tail(c, PeerArgs(), Planes{}, true, Planes{d_codes, d_inv, d_low, padded_len}, wins, j, bgs[0]->space, nullptr,
+                      nullptr, &set);
     return c.leave(rc);
 }
 

@@ -170,6 +170,25 @@ int frisk_internal::score(const WinPlan& p, WinJob j, const unsigned long long* 
     return FRISK_E_UNSUPPORTED;
 }
 
+// Only the nibble kernel has a multi-background instantiation; every other plan scores the same planes and windows once
+// per background, which gives the one-background rows by construction.  One background is the one-background call.
+int frisk_internal::score_many(const WinPlan& p, const WinJob* jobs, int n_bg, const unsigned long long* n_win_dev) {
+    if (n_bg < 1 || n_bg > FRISK_B200_MAX_BACKGROUNDS) return FRISK_E_INVALID;
+    if (n_bg > 1 && p.kind == WinKernel::Nibble && !p.dump) {
+        const WinJob& j = jobs[0];
+        if (j.max_len > FRISK_B200_MAX_WINDOW || j.n_win > 0xffffffffull) return FRISK_E_UNSUPPORTED;
+        WinJob js[FRISK_B200_MAX_BACKGROUNDS];
+        for (int b = 0; b < n_bg; ++b) {
+            js[b] = jobs[b];
+            js[b].rip = rip_orders(js[b].rip, js[b].kmin, js[b].K);
+        }
+        return score_nibble_many(p, js, n_bg, n_win_dev);
+    }
+    int rc = FRISK_OK;
+    for (int b = 0; b < n_bg && !rc; ++b) rc = score(p, jobs[b], n_win_dev);
+    return rc;
+}
+
 extern "C" {
 
 int frisk_b200_score(const uint32_t* d_codes, const uint32_t* d_inv, const uint32_t* d_low, const uint64_t* d_win_off,

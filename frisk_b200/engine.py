@@ -1529,3 +1529,103 @@ class Background:
             self.close()
         except Exception:
             pass
+
+
+# ---------------------------------------------------------------------- one query, several stored backgrounds
+def _check_backgrounds(backgrounds) -> List[Background]:
+    """The backgrounds of one multi-background call: 1..MAX_BACKGROUNDS open handles of one kmin / kmax (the window count
+    and the orders scored depend on them).  ValueError otherwise, before any C call."""
+    bgs = list(backgrounds)
+    if not 1 <= len(bgs) <= _lib.MAX_BACKGROUNDS:
+        raise ValueError("%d backgrounds: one call scores against 1..%d" % (len(bgs), _lib.MAX_BACKGROUNDS))
+    for i, bg in enumerate(bgs):
+        if not isinstance(bg, Background) or not bg._h:
+            raise ValueError("background %d is not an open engine.Background" % i)
+        if (bg.kmin, bg.kmax) != (bgs[0].kmin, bgs[0].kmax):
+            raise ValueError("background %d has orders %d..%d, background 0 has %d..%d: one call needs one kmin / kmax"
+                             % (i, bg.kmin, bg.kmax, bgs[0].kmin, bgs[0].kmax))
+    return bgs
+
+
+def _handles(bgs: List[Background]):
+    return (C.c_void_p * len(bgs))(*[bg._h.value for bg in bgs])
+
+
+def _score_many(bgs: List[Background], query: PackedGenome, planes, wins: WindowList, rip: bool, rows, status) -> None:
+    codes, inv, low = planes
+    with bgs[0]._on_device():
+        _lib.check(_lib.lib().frisk_b200_background_score_many(
+            _handles(bgs), len(bgs), _ptr(codes), _ptr(inv), _ptr(low), query.padded_len, _ptr(wins.off), _ptr(wins.length),
+            len(wins), wins.max_len, int(rip), _ptr(rows), _ptr(status), _stream_ptr(bgs[0].device)),
+            "frisk_b200_background_score_many")
+
+
+def run_backgrounds(backgrounds, query, kind: Optional[str] = None, w: int = 5000, step: int = 2500, scaffolds_all: bool = False,
+                    rip: bool = True, out=None, assemble_result: bool = True):
+    """``query`` scored against every background of ``backgrounds`` (engine.Background, one kmin / kmax, at most 8) in one
+    C call (frisk_b200_background_run_many): the query is read, uploaded and counted once, only the genome-IVOM lookups are
+    made per background.  Result i equals ``backgrounds[i].run(query, kind, w, step, scaffolds_all, rip)``.  ``query`` and
+    ``kind`` as for ``Background.run``.  ``out``: reusable buffers with ``rows`` and ``status`` of n * rows_cap rows for n
+    backgrounds (background b's block at b * rows_cap; ``out.n_win`` is set), returned as they are without
+    ``assemble_result``.  Goes through the C ABI alone (no PyTorch)."""
+    bgs = _check_backgrounds(backgrounds)
+    if kind is None and isinstance(query, (str, os.PathLike)):
+        buf, kind = read_genome_raw(os.fspath(query))
+    else:
+        buf = _as_u8(query)
+        kind = kind or _kind_of(buf)
+    L = _lib.lib()
+    nb = len(bgs)
+    pinned = _torch_loaded()
+    if out is None:
+        n_text = _text_len_hint(buf, kind)                 # a guess, as in Background.run; FRISK_E_CAPACITY is handled below
+        cap = n_text // step + n_text // 4096 + 64
+        out = HostOutputs(nb * cap, 0, pinned=pinned)
+    cap = out.rows.shape[0] // nb
+    rows, status = out.rows, out.status
+    qh = C.c_void_p()
+    n_win = C.c_uint64(0)
+    with bgs[0]._on_device():
+        st = _stream_ptr(bgs[0].device)
+        rc = L.frisk_b200_background_run_many(_handles(bgs), nb, _ptr(buf), buf.shape[0], _lib.FORMAT[kind], w, step,
+                                              int(scaffolds_all), int(rip), cap, _ptr(rows), _ptr(status), C.byref(n_win),
+                                              C.byref(qh), st)
+        try:
+            if rc not in (_lib.OK, _lib.E_CAPACITY):
+                _lib.check(rc, "frisk_b200_background_run_many")
+            n = int(n_win.value)
+            query = _genome_from_handle(L, qh, buf, kind != "text") if assemble_result or rc == _lib.E_CAPACITY else None
+            if rc == _lib.E_CAPACITY:
+                # more windows than rows: the query's planes are on the device, score them into enough rows
+                c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
+                _lib.check(L.frisk_b200_fasta_planes(qh, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
+                cap = max(n, 1)
+                out = HostOutputs(nb * cap, 0, pinned=pinned)
+                rows, status = out.rows, out.status
+                _score_many(bgs, query, (_HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value)),
+                            query.windows(w, step, scaffolds_all), rip, rows, status)
+        finally:
+            if qh:
+                L.frisk_b200_fasta_close(qh, st)
+    out.n_win = n
+    if not assemble_result:
+        return out
+    wins = query.windows(w, step, scaffolds_all)
+    assert len(wins) == n
+    return [bg._result(query, wins, rows[b * cap:b * cap + n], status[b * cap:b * cap + n]) for b, bg in enumerate(bgs)]
+
+
+def run_backgrounds_resident(backgrounds, dq: DeviceGenome, w: int = 5000, step: int = 2500, scaffolds_all: bool = False,
+                             rip: bool = True, wins: Optional[WindowList] = None) -> List[HotPathResult]:
+    """``run_backgrounds`` for planes already on the device (frisk_b200_background_score_many): result i equals
+    ``backgrounds[i].run_resident(dq, w, step, scaffolds_all, rip, wins)``."""
+    bgs = _check_backgrounds(backgrounds)
+    query = dq.host
+    if wins is None:
+        wins = query.windows(w, step, scaffolds_all)
+    n, nb = len(wins), len(bgs)
+    cap = max(n, 1)
+    pinned = _torch_loaded() and not isinstance(dq.codes, DevBuf)
+    rows, status = _alloc((nb * cap, 5), np.float64, pinned), _alloc((nb * cap,), np.uint32, pinned)
+    _score_many(bgs, query, (dq.codes, dq.inv, dq.low), wins, rip, rows, status)
+    return [bg._result(query, wins, rows[b * cap:b * cap + n], status[b * cap:b * cap + n]) for b, bg in enumerate(bgs)]

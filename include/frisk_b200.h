@@ -37,6 +37,7 @@ extern "C" {
 #define FRISK_B200_MAX_K 12              /* largest supported --maxWordSize (K <= 8: shared-memory kernels; 9..12: general path) */
 #define FRISK_B200_FAST_K 8              /* ... served by the tuned shared-memory kernels */
 #define FRISK_B200_MAX_WINDOW 0x7fffffff /* largest window length (<= 65,535: shared-memory kernels; longer: general path) */
+#define FRISK_B200_MAX_BACKGROUNDS 8     /* most backgrounds one frisk_b200_background_run_many / _score_many call scores against */
 
 enum {
     FRISK_OK = 0,
@@ -520,6 +521,15 @@ int frisk_b200_run_2bit(const char *h_2bit, uint64_t h_n, const char *q_2bit, ui
  *
  * frisk_b200_background_close: synchronises `stream`, frees the table and the handle (NULL: nothing to do).
  *
+ * frisk_b200_background_run_many / _score_many: one query against n_bg backgrounds (bgs[0..n_bg-1]) in one call.  The
+ * query is ingested once and every window counted once; only the genome-IVOM lookups are made per background.  Rows and
+ * status are background-major: background b's block starts at row b * rows_cap (_run_many) or b * n_win (_score_many), and
+ * has the layout, and the bits, of the one-background call for that handle.  rows_out / status_out hold n_bg blocks.
+ * Everything else -- FRISK_E_CAPACITY, *query_out, the stage marks (ms[3]: every background's window kernel done) -- is
+ * as in frisk_b200_background_run / _score.  Refused before any device work with FRISK_E_INVALID: n_bg outside
+ * 1..FRISK_B200_MAX_BACKGROUNDS, a NULL list or handle, handles of different kmin / kmax (the window count depends on
+ * them), a handle bound to another device.  n_bg == 1 is the one-background call.
+ *
  * The handle's type is spelled `struct frisk_b200_background`: there is no typedef, because frisk_b200_background is the
  * name of the background-count function above (struct tags and functions do not collide).
  */
@@ -534,6 +544,15 @@ int frisk_b200_background_score(const struct frisk_b200_background *bg, const ui
                                 const uint32_t *d_low, uint64_t padded_len, const uint64_t *win_off, const uint32_t *win_len,
                                 uint64_t n_win, uint32_t max_win_len, int want_rip, double *rows_out, uint32_t *status_out,
                                 void *stream);
+int frisk_b200_background_run_many(const struct frisk_b200_background *const *bgs, int n_bg, const char *q, uint64_t q_n,
+                                   int format, int w, int step, int scaffolds_all, int want_rip, uint64_t rows_cap,
+                                   double *rows_out, uint32_t *status_out, uint64_t *n_win_out,
+                                   frisk_b200_fasta **query_out, void *stream);
+int frisk_b200_background_score_many(const struct frisk_b200_background *const *bgs, int n_bg, const uint32_t *d_codes,
+                                     const uint32_t *d_inv, const uint32_t *d_low, uint64_t padded_len,
+                                     const uint64_t *win_off, const uint32_t *win_len, uint64_t n_win,
+                                     uint32_t max_win_len, int want_rip, double *rows_out, uint32_t *status_out,
+                                     void *stream);
 int frisk_b200_background_close(struct frisk_b200_background *bg, void *stream);
 
 /* Stage times (ms since the start of the call) of the last frisk_b200_run_host / _sparse / _peers / _run_resident call
