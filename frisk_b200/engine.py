@@ -210,16 +210,6 @@ def twobit_records(buf) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
     return name_off, name_len, seq_len
 
 
-def _name_source(L, h, buf: np.ndarray, device_text: bool) -> np.ndarray:
-    """What a handle's name offsets index: the caller's text, or -- a BGZF, gzip or .2bit open, whose text never leaves
-    the device or does not exist -- the handle's buffer of names (copied: it goes with the handle)."""
-    if not device_text:
-        return buf
-    p, n = C.c_void_p(), C.c_uint64(0)
-    _lib.check(L.frisk_b200_fasta_name_text(h, C.byref(p), C.byref(n)), "frisk_b200_fasta_name_text")
-    return np.frombuffer(C.string_at(p.value, n.value), dtype=np.uint8) if n.value else np.zeros(0, np.uint8)
-
-
 def _decode_names(buf: np.ndarray, name_off: np.ndarray, name_len: np.ndarray) -> List[str]:
     """Header tokens -> str.  All name bytes are gathered with one fancy-index (a 1 M-scaffold
     assembly must not pay a numpy slice of a multi-GB buffer per record), then cut up."""
@@ -493,29 +483,10 @@ class DeviceGenome:
     @classmethod
     def _open_native(cls, text, device, kind: str) -> "DeviceGenome":
         _lib.require_device()
-        L = _lib.lib()
-        buf = _as_u8(text)
-        _lib.check(L.frisk_b200_set_device(_device_index(device)), "frisk_b200_set_device")
-        h = C.c_void_p()
-        nrec, padded = C.c_uint64(0), C.c_uint64(0)
-        stats = np.zeros(3, np.uint64)
-        what = _OPENERS[kind]
-        _lib.check(getattr(L, what)(_ptr(buf), buf.shape[0], None, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
-        try:
-            names_buf = _name_source(L, h, buf, kind != "text")
-            R, P = int(nrec.value), int(padded.value)
-            name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
-            seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
-            _lib.check(L.frisk_b200_fasta_records(h, _ptr(name_off), _ptr(name_len), _ptr(seq_len), _ptr(scaf_off)),
-                       "frisk_b200_fasta_records")
-            codes, inv = DevBuf(P // 4), DevBuf(P // 8)
-            low = DevBuf(P // 8) if int(stats[2]) else None
-            _lib.check(L.frisk_b200_fasta_pack(h, _ptr(codes), _ptr(inv), _ptr(low), None), "frisk_b200_fasta_pack")
-        finally:
-            L.frisk_b200_fasta_close(h, None)
-        names = _decode_names(names_buf, name_off, name_len)
-        g = PackedGenome(names, seq_len, scaf_off, P, None, None, None, int(stats[0]), int(stats[1]), int(stats[2]), False)
-        return cls(g, str(device), planes=(codes, inv, low))
+        _lib.check(_lib.lib().frisk_b200_set_device(_device_index(device)), "frisk_b200_set_device")
+        dg = cls._open_on(text, kind, str(device), None, DevBuf)
+        dg.host.names = list(dg.host.names)           # decoded now, so the file's bytes can go
+        return dg
 
     @classmethod
     def from_fasta_bytes(cls, text: Union[bytes, np.ndarray], device="cuda:0") -> "DeviceGenome":
@@ -546,33 +517,29 @@ class DeviceGenome:
     def _open(cls, text, device, kind: str) -> "DeviceGenome":
         import torch
         _lib.require_device()
+        dev = torch.device(device)
+        with torch.cuda.device(dev):
+            return cls._open_on(text, kind, dev, _stream_ptr(dev),
+                                lambda nbytes: torch.empty(nbytes // 4, dtype=torch.int32, device=dev))
+
+    @classmethod
+    def _open_on(cls, text, kind: str, device, stream, alloc) -> "DeviceGenome":
+        """The device open on the current device: ``kind``'s opener on ``stream``, the planes copied out of the handle
+        into ``alloc(nbytes)`` buffers (torch tensors, or DevBuf without PyTorch), the handle closed."""
         L = _lib.lib()
         buf = _as_u8(text)
-        dev = torch.device(device)
+        h = C.c_void_p()
         what = _OPENERS[kind]
-        opener = getattr(L, what)
-        with torch.cuda.device(dev):
-            st = _stream_ptr(dev)
-            h = C.c_void_p()
-            nrec, padded = C.c_uint64(0), C.c_uint64(0)
-            stats = np.zeros(3, np.uint64)
-            _lib.check(opener(_ptr(buf), buf.shape[0], st, C.byref(h), C.byref(nrec), C.byref(padded), _ptr(stats)), what)
-            try:
-                names_buf = _name_source(L, h, buf, kind != "text")
-                R, P = int(nrec.value), int(padded.value)
-                name_off = np.zeros(R, np.uint64); name_len = np.zeros(R, np.uint32)
-                seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
-                _lib.check(L.frisk_b200_fasta_records(h, _ptr(name_off), _ptr(name_len), _ptr(seq_len), _ptr(scaf_off)),
-                           "frisk_b200_fasta_records")
-                codes = torch.empty(P // 16, dtype=torch.int32, device=dev)
-                inv = torch.empty(P // 32, dtype=torch.int32, device=dev)
-                low = torch.empty(P // 32, dtype=torch.int32, device=dev) if int(stats[2]) else None
-                _lib.check(L.frisk_b200_fasta_pack(h, _ptr(codes), _ptr(inv), _ptr(low), st), "frisk_b200_fasta_pack")
-            finally:
-                L.frisk_b200_fasta_close(h, st)
-        names = LazyNames(names_buf, name_off, name_len)
-        g = PackedGenome(names, seq_len, scaf_off, P, None, None, None, int(stats[0]), int(stats[1]), int(stats[2]), False)
-        return cls(g, dev, planes=(codes, inv, low))
+        _lib.check(getattr(L, what)(_ptr(buf), buf.shape[0], stream, C.byref(h), None, None, None), what)
+        try:
+            g = _genome_from_handle(L, h, buf, kind)
+            P = g.padded_len
+            codes, inv = alloc(P // 4), alloc(P // 8)
+            low = alloc(P // 8) if g.n_lower else None
+            _lib.check(L.frisk_b200_fasta_pack(h, _ptr(codes), _ptr(inv), _ptr(low), stream), "frisk_b200_fasta_pack")
+        finally:
+            L.frisk_b200_fasta_close(h, stream)
+        return cls(g, device, planes=(codes, inv, low))
 
     @classmethod
     def from_fasta(cls, path: str, device="cuda:0") -> "DeviceGenome":
@@ -797,6 +764,15 @@ def _assemble_rows(query: PackedGenome, wins: WindowList, tables: np.ndarray, me
                          scaf_names=list(query.names) if want_names else query.names)
 
 
+def _mark(marks, dev) -> None:
+    """A stage mark: a CUDA event recorded on ``dev``'s current stream, appended to ``marks`` (nothing when it is None)."""
+    if marks is not None:
+        import torch
+        ev = torch.cuda.Event(enable_timing=True)
+        ev.record(torch.cuda.current_stream(dev))
+        marks.append(ev)
+
+
 class Pipeline:
     """The device-resident hot path: planes, window list and all work buffers live in HBM; one
     ``enqueue()`` launches background -> [all-reduce] -> finalize -> genome IVOM -> score on the
@@ -851,22 +827,15 @@ class Pipeline:
         import torch
         L = _lib.lib()
         dev = self.device
-
-        def mark():
-            if marks is not None:
-                ev = torch.cuda.Event(enable_timing=True)
-                ev.record(torch.cuda.current_stream(dev))
-                marks.append(ev)
-
         with torch.cuda.device(dev):
             st = _stream_ptr(dev)
             d_fwd = self.peers.local() if self.peers is not None else self.d_fwd
-            mark()                           # a step includes zeroing its counters
+            _mark(marks, dev)                 # a step includes zeroing its counters
             d_fwd.zero_()
             dh = self.dh
             _lib.check(L.frisk_b200_background(_ptr(dh.codes), _ptr(dh.inv), _ptr(dh.low), self.bg_range[0], self.bg_range[1],
                                                self.kmax, int(self.mask_host), _ptr(d_fwd), st), "frisk_b200_background")
-            mark()
+            _mark(marks, dev)
             space = self.genome_space
             if self.peers is not None:      # counters summed from every rank's buffer inside the (one) finalising launch
                 self.peers.finalize_ivom(self.kmin, self.kmax, int(space), self.d_tables, self.d_valid, self.d_ig, st)
@@ -876,7 +845,7 @@ class Pipeline:
                 _lib.check(L.frisk_b200_finalize_ivom(_ptr(self.d_fwd), None, None, 0, 0, 0, self.kmin, self.kmax, int(space),
                                                       _ptr(self.d_tables), _ptr(self.d_valid), _ptr(self.d_ig), st),
                            "frisk_b200_finalize_ivom")
-            mark()
+            _mark(marks, dev)
             n = len(self.wins)
             if n:
                 dq = self.dq
@@ -884,7 +853,7 @@ class Pipeline:
                                               n, self.wins.max_len, _ptr(self.d_ig), self.kmin, self.kmax, int(self.rip),
                                               _ptr(self.d_rows), _ptr(self.d_status), _ptr(self.d_dump), st),
                            "frisk_b200_score")
-            mark()
+            _mark(marks, dev)
 
     def step_from_host(self, out: "HostOutputs") -> "HostOutputs":
         """One end-to-end pass without any allocation: H2D of the (pinned) host planes into the
@@ -952,32 +921,9 @@ def run_sweep(query, kmaxes: Sequence[int] = tuple(range(1, 9)), kmin: int = 1, 
     reference runs ``-m kmin -k k'``).  The count of x-words does not depend on kmax (F:338-351 counts every
     order independently), so ONE background pass at max(kmaxes) serves every k'; per k' only the genome
     IVOM table and the window kernel run.  Returns {k': HotPathResult}."""
-    import torch
-    _lib.require_device()
-    if fused:                                   # kmax' = 1..8, kmin 1: one window kernel for all of them
-        sw = Sweep(query, kmaxes, kmin, w, step, mask_host, scaffolds_all, rip, device)
-        if sw.fused:
-            sw.enqueue()
-            return sw.results()
-        query = sw.dq
-    dq = query if isinstance(query, DeviceGenome) else DeviceGenome(query, device)
-    g = dq.host
-    top = max(kmaxes)
-    d_tables, _ = finalize(background(dq, top, mask_host), top)
-    wins = g.windows(w, step, scaffolds_all)
-    out = {}
-    for k in sorted(set(int(x) for x in kmaxes)):
-        if k < kmin:
-            continue
-        tsz = _lib.table_size(1, k)
-        d_tab_k = d_tables[:tsz]
-        d_ig = genome_ivom(d_tab_k, kmin, k, g.genome_space)
-        d_rows, d_status, _ = score(dq, wins, d_ig, kmin, k, rip)
-        torch.cuda.synchronize(dq.device)
-        tables = d_tab_k.cpu().numpy().view(np.uint64)
-        valid = int(tables[_lib.table_size(1, k - 1) if k > 1 else 0:].sum()) // 2      # both strands were added
-        out[k] = assemble(g, g, wins, tables, valid, d_rows.cpu().numpy(), d_status.cpu().numpy().view(np.uint32), kmin, k)
-    return out
+    sw = Sweep(query, kmaxes, kmin, w, step, mask_host, scaffolds_all, rip, device, fused=fused)
+    sw.enqueue()
+    return sw.results()
 
 
 class Sweep:
@@ -1026,16 +972,9 @@ class Sweep:
         L = _lib.lib()
         dev, g, dq = self.device, self.dq.host, self.dq
         n = len(self.wins)
-
-        def mark():
-            if marks is not None:
-                ev = torch.cuda.Event(enable_timing=True)
-                ev.record(torch.cuda.current_stream(dev))
-                marks.append(ev)
-
         with torch.cuda.device(dev):
             st = _stream_ptr(dev)
-            mark()
+            _mark(marks, dev)
             self.d_fwd.zero_()
             _lib.check(L.frisk_b200_background(_ptr(dq.codes), _ptr(dq.inv), _ptr(dq.low), self.bg_range[0], self.bg_range[1], self.top,
                                                int(self.mask_host), _ptr(self.d_fwd), st), "frisk_b200_background")
@@ -1043,7 +982,7 @@ class Sweep:
                 self.allreduce(self.d_fwd, g.genome_space)
             _lib.check(L.frisk_b200_finalize_tables(_ptr(self.d_fwd), self.top, 1, _ptr(self.d_tables), _ptr(self.d_valid), st),
                        "frisk_b200_finalize_tables")
-            mark()
+            _mark(marks, dev)
             launches = 5                                   # count, reduce, totals, low, symmetrise
             fused = self.fused and n > 0
             for k in self.kmaxes:
@@ -1057,13 +996,13 @@ class Sweep:
                                                   self.wins.max_len, _ptr(self.d_ig[k]), self.kmin, k, int(self.rip),
                                                   _ptr(self.d_rows[k]), _ptr(self.d_status[k]), None, st), "frisk_b200_score")
                 launches += 2 + (1 if k >= 7 else 0)       # kmax 7, 8: + the (usually empty) hand-over launch
-                mark()
+                _mark(marks, dev)
             if fused:                                      # ONE window kernel for all eight kmax' (+ eight empty hand-over launches)
                 _lib.check(L.frisk_b200_score_sweep(_ptr(dq.codes), _ptr(dq.inv), _ptr(dq.low), _ptr(self.d_off), _ptr(self.d_len), n,
                                                     self.wins.max_len, self._ig_ptrs, 8, int(self.rip), self._row_ptrs, self._st_ptrs, st),
                            "frisk_b200_score_sweep")
                 launches += 9
-                mark()
+                _mark(marks, dev)
             self.launches = launches
 
     def checksums(self):
@@ -1174,7 +1113,18 @@ class _HandlePlane:
         return self._p
 
 
-def _genome_from_handle(L, h, buf, device_text: bool = False) -> PackedGenome:
+def _handle_planes(L, h):
+    """The planes of an open frisk_b200_fasta handle, as (codes, inv, low or None)."""
+    c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
+    _lib.check(L.frisk_b200_fasta_planes(h, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
+    return _HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value) if l.value else None
+
+
+def _genome_from_handle(L, h, buf, kind: str = "text") -> PackedGenome:
+    """The record table of an open frisk_b200_fasta handle of ``buf`` (a ``kind`` buffer) as a PackedGenome without host
+    planes: names, lengths, layout and countN statistics.  The name offsets index ``buf`` when it is text; a BGZF, gzip
+    or .2bit open, whose text never leaves the device or does not exist, has them index the handle's buffer of names
+    (copied: it goes with the handle)."""
     nrec, padded = C.c_uint64(0), C.c_uint64(0)
     stats = np.zeros(3, np.uint64)
     _lib.check(L.frisk_b200_fasta_info(h, C.byref(nrec), C.byref(padded), _ptr(stats)), "frisk_b200_fasta_info")
@@ -1183,7 +1133,11 @@ def _genome_from_handle(L, h, buf, device_text: bool = False) -> PackedGenome:
     seq_len = np.zeros(R, np.uint64); scaf_off = np.zeros(R, np.uint64)
     _lib.check(L.frisk_b200_fasta_records(h, _ptr(name_off), _ptr(name_len), _ptr(seq_len), _ptr(scaf_off)),
                "frisk_b200_fasta_records")
-    return PackedGenome(LazyNames(_name_source(L, h, buf, device_text), name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
+    if kind != "text":
+        p, n = C.c_void_p(), C.c_uint64(0)
+        _lib.check(L.frisk_b200_fasta_name_text(h, C.byref(p), C.byref(n)), "frisk_b200_fasta_name_text")
+        buf = np.frombuffer(C.string_at(p.value, n.value), dtype=np.uint8) if n.value else np.zeros(0, np.uint8)
+    return PackedGenome(LazyNames(buf, name_off, name_len), seq_len, scaf_off, int(padded.value), None, None, None,
                         int(stats[0]), int(stats[1]), int(stats[2]), False)
 
 
@@ -1247,6 +1201,14 @@ def _text_len_hint(buf: np.ndarray, kind: str) -> int:
     return buf.shape[0]
 
 
+def _rows_guess(buf: np.ndarray, kind: str, step: int) -> int:
+    """Row capacity of a one-call run: a guess (one window per step of text, one more per 4 KiB for short scaffolds).  A
+    text with more windows comes back with FRISK_E_CAPACITY and is scored in a second stage -- page-locking a far larger
+    buffer "to be safe" would cost more than the run (~0.3 ms per MB)."""
+    n_text = _text_len_hint(buf, kind)
+    return n_text // step + n_text // 4096 + 64
+
+
 def _run_fasta_any(query_text, host_text, kind, device, out, assemble_result, kmin, kmax, w, step, mask_host, scaffolds_all, rip):
     import torch
     _lib.require_device()
@@ -1255,11 +1217,7 @@ def _run_fasta_any(query_text, host_text, kind, device, out, assemble_result, km
     hbuf = _as_u8(host_text) if host_text is not None else qbuf
     dev = torch.device(device)
     if out is None:
-        # rows: a guess (one window per step of text, one more per 4 KiB for short scaffolds); a text with more windows comes
-        # back with FRISK_E_CAPACITY and is scored in a second stage below -- page-locking a far larger buffer "to be safe"
-        # would cost more than the run (~0.3 ms per MB)
-        n_text = _text_len_hint(qbuf, kind)
-        out = HostOutputs(n_text // step + n_text // 4096 + 64, kmax)
+        out = HostOutputs(_rows_guess(qbuf, kind, step), kmax)
     hh, qh = C.c_void_p(), C.c_void_p()
     n_win = C.c_uint64(0)
     what = _RUNNERS[kind]
@@ -1275,16 +1233,12 @@ def _run_fasta_any(query_text, host_text, kind, device, out, assemble_result, km
                 _lib.check(rc, what)
             n = int(n_win.value)
             need_genomes = assemble_result or rc == _lib.E_CAPACITY
-            host = _genome_from_handle(L, hh, hbuf, kind != "text") if need_genomes else None
-            query = (_genome_from_handle(L, qh, qbuf, kind != "text") if qh else host) if need_genomes else None
+            host = _genome_from_handle(L, hh, hbuf, kind) if need_genomes else None
+            query = (_genome_from_handle(L, qh, qbuf, kind) if qh else host) if need_genomes else None
             if rc == _lib.E_CAPACITY:
                 # more windows than the guessed row capacity: the planes are on the device, score them into enough rows
-                def planes(h):
-                    c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
-                    _lib.check(L.frisk_b200_fasta_planes(h, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
-                    return (_HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value) if l.value else None)
-                dh = DeviceGenome(host, dev, planes=planes(hh))
-                dq = DeviceGenome(query, dev, planes=planes(qh)) if qh else dh
+                dh = DeviceGenome(host, dev, planes=_handle_planes(L, hh))
+                dq = DeviceGenome(query, dev, planes=_handle_planes(L, qh)) if qh else dh
                 out = HostOutputs(n, kmax)
                 out = run_resident(dq, dh, kmin=kmin, kmax=kmax, w=w, step=step, mask_host=mask_host,
                                    scaffolds_all=scaffolds_all, rip=rip, out=out, assemble_result=False)
@@ -1392,6 +1346,15 @@ def _kind_of(buf: np.ndarray) -> str:
     return "2bit" if is_2bit(buf) else "bgzf" if is_bgzf(buf) else "gzip" if is_gzip(buf) else "text"
 
 
+def _query_buf(query, kind: Optional[str]) -> Tuple[np.ndarray, str]:
+    """(bytes, kind) of a query: a path (``kind`` from ``read_genome_raw``), or the genome's bytes with ``kind`` as given
+    or by signature."""
+    if kind is None and isinstance(query, (str, os.PathLike)):
+        return read_genome_raw(os.fspath(query))
+    buf = _as_u8(query)
+    return buf, kind or _kind_of(buf)
+
+
 class Background:
     """A host genome's background tables resident on one GPU (frisk_b200_background_open): any number of queries are
     scored against them without the host genome, which is neither read, uploaded nor counted.  ``tables``: uint64, orders
@@ -1445,71 +1408,28 @@ class Background:
 
     def run(self, query, kind: Optional[str] = None, w: int = 5000, step: int = 2500, scaffolds_all: bool = False,
             rip: bool = True, out=None, assemble_result: bool = True):
-        """The windows of ``query`` scored against this background in one C call (frisk_b200_background_run): the query
-        half of ``run_fasta``.  ``query``: a path (``kind`` from ``read_genome_raw``), or the genome's bytes with ``kind``
-        "text", "bgzf", "gzip" or "2bit" (by signature when not given).  ``out``: reusable buffers with ``rows`` and
-        ``status`` (their row capacity is used; ``out.n_win`` is set).  The result's ``tables`` and ``meta`` are the
-        background's."""
-        if kind is None and isinstance(query, (str, os.PathLike)):
-            buf, kind = read_genome_raw(os.fspath(query))
-        else:
-            buf = _as_u8(query)
-            kind = kind or _kind_of(buf)
-        L = _lib.lib()
-        if out is None:
-            n_text = _text_len_hint(buf, kind)                 # a guess, as in run_fasta; FRISK_E_CAPACITY is handled below
-            out = HostOutputs(n_text // step + n_text // 4096 + 64, 0, pinned=_torch_loaded())
-        qh = C.c_void_p()
-        n_win = C.c_uint64(0)
-        with self._on_device():
-            st = _stream_ptr(self.device)
-            rc = L.frisk_b200_background_run(self._h, _ptr(buf), buf.shape[0], _lib.FORMAT[kind], w, step, int(scaffolds_all),
-                                             int(rip), out.rows.shape[0], _ptr(out.rows), _ptr(out.status), C.byref(n_win),
-                                             C.byref(qh), st)
-            try:
-                if rc not in (_lib.OK, _lib.E_CAPACITY):
-                    _lib.check(rc, "frisk_b200_background_run")
-                n = int(n_win.value)
-                query = _genome_from_handle(L, qh, buf, kind != "text") if assemble_result or rc == _lib.E_CAPACITY else None
-                if rc == _lib.E_CAPACITY:
-                    # more windows than rows: the query's planes are on the device, score them into enough rows
-                    c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
-                    _lib.check(L.frisk_b200_fasta_planes(qh, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
-                    out = HostOutputs(n, 0, pinned=_torch_loaded())
-                    self._score(query, (_HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value)),
-                                query.windows(w, step, scaffolds_all), rip, out)
-            finally:
-                if qh:
-                    L.frisk_b200_fasta_close(qh, st)
-        out.n_win = n
-        if not assemble_result:
-            return out
-        wins = query.windows(w, step, scaffolds_all)
-        assert len(wins) == n
-        return self._result(query, wins, out.rows[:n], out.status[:n])
+        """The windows of ``query`` scored against this background in one C call: the query half of ``run_fasta``, and
+        ``run_backgrounds`` with this one background.  ``query``: a path (``kind`` from ``read_genome_raw``), or the
+        genome's bytes with ``kind`` "text", "bgzf", "gzip" or "2bit" (by signature when not given).  ``out``: reusable
+        buffers with ``rows`` and ``status`` (their row capacity is used; ``out.n_win`` is set).  The result's ``tables``
+        and ``meta`` are the background's."""
+        res = _run_backgrounds([self], query, kind, w, step, scaffolds_all, rip, out, assemble_result)
+        return res[0] if assemble_result else res
 
     def run_resident(self, dq: DeviceGenome, w: int = 5000, step: int = 2500, scaffolds_all: bool = False, rip: bool = True,
                      wins: Optional[WindowList] = None, out=None, assemble_result: bool = True):
-        """``engine.run_resident`` with this background in place of the host genome (frisk_b200_background_score): the
-        windows of planes already on the device, scored in one C call."""
+        """``engine.run_resident`` with this background in place of the host genome: the windows of planes already on the
+        device, scored in one C call."""
         query = dq.host
         if wins is None:
             wins = query.windows(w, step, scaffolds_all)
         n = len(wins)
         if out is None:
             out = HostOutputs(n, 0, pinned=_torch_loaded() and not isinstance(dq.codes, DevBuf))
-        self._score(query, (dq.codes, dq.inv, dq.low), wins, rip, out)
+        _score_many([self], query, (dq.codes, dq.inv, dq.low), wins, rip, out.rows, out.status)
         if not assemble_result:
             return out
         return self._result(query, wins, out.rows[:n], out.status[:n])
-
-    def _score(self, query: PackedGenome, planes, wins: WindowList, rip: bool, out) -> None:
-        codes, inv, low = planes
-        with self._on_device():
-            _lib.check(_lib.lib().frisk_b200_background_score(
-                self._h, _ptr(codes), _ptr(inv), _ptr(low), query.padded_len, _ptr(wins.off), _ptr(wins.length), len(wins),
-                wins.max_len, int(rip), _ptr(out.rows), _ptr(out.status), _stream_ptr(self.device)),
-                "frisk_b200_background_score")
 
     def close(self) -> None:
         if self._h:
@@ -1568,42 +1488,35 @@ def run_backgrounds(backgrounds, query, kind: Optional[str] = None, w: int = 500
     ``kind`` as for ``Background.run``.  ``out``: reusable buffers with ``rows`` and ``status`` of n * rows_cap rows for n
     backgrounds (background b's block at b * rows_cap; ``out.n_win`` is set), returned as they are without
     ``assemble_result``.  Goes through the C ABI alone (no PyTorch)."""
-    bgs = _check_backgrounds(backgrounds)
-    if kind is None and isinstance(query, (str, os.PathLike)):
-        buf, kind = read_genome_raw(os.fspath(query))
-    else:
-        buf = _as_u8(query)
-        kind = kind or _kind_of(buf)
+    return _run_backgrounds(_check_backgrounds(backgrounds), query, kind, w, step, scaffolds_all, rip, out, assemble_result)
+
+
+def _run_backgrounds(bgs: List[Background], query, kind, w, step, scaffolds_all, rip, out, assemble_result):
+    """``run_backgrounds`` for ``bgs``, open Backgrounds of one kmin / kmax (``Background.run``: just itself)."""
+    buf, kind = _query_buf(query, kind)
     L = _lib.lib()
     nb = len(bgs)
     pinned = _torch_loaded()
     if out is None:
-        n_text = _text_len_hint(buf, kind)                 # a guess, as in Background.run; FRISK_E_CAPACITY is handled below
-        cap = n_text // step + n_text // 4096 + 64
-        out = HostOutputs(nb * cap, 0, pinned=pinned)
+        out = HostOutputs(nb * _rows_guess(buf, kind, step), 0, pinned=pinned)
     cap = out.rows.shape[0] // nb
-    rows, status = out.rows, out.status
     qh = C.c_void_p()
     n_win = C.c_uint64(0)
     with bgs[0]._on_device():
         st = _stream_ptr(bgs[0].device)
         rc = L.frisk_b200_background_run_many(_handles(bgs), nb, _ptr(buf), buf.shape[0], _lib.FORMAT[kind], w, step,
-                                              int(scaffolds_all), int(rip), cap, _ptr(rows), _ptr(status), C.byref(n_win),
-                                              C.byref(qh), st)
+                                              int(scaffolds_all), int(rip), cap, _ptr(out.rows), _ptr(out.status),
+                                              C.byref(n_win), C.byref(qh), st)
         try:
             if rc not in (_lib.OK, _lib.E_CAPACITY):
                 _lib.check(rc, "frisk_b200_background_run_many")
             n = int(n_win.value)
-            query = _genome_from_handle(L, qh, buf, kind != "text") if assemble_result or rc == _lib.E_CAPACITY else None
+            query = _genome_from_handle(L, qh, buf, kind) if assemble_result or rc == _lib.E_CAPACITY else None
             if rc == _lib.E_CAPACITY:
                 # more windows than rows: the query's planes are on the device, score them into enough rows
-                c, i, l = C.c_void_p(), C.c_void_p(), C.c_void_p()
-                _lib.check(L.frisk_b200_fasta_planes(qh, C.byref(c), C.byref(i), C.byref(l)), "frisk_b200_fasta_planes")
                 cap = max(n, 1)
                 out = HostOutputs(nb * cap, 0, pinned=pinned)
-                rows, status = out.rows, out.status
-                _score_many(bgs, query, (_HandlePlane(c.value), _HandlePlane(i.value), _HandlePlane(l.value)),
-                            query.windows(w, step, scaffolds_all), rip, rows, status)
+                _score_many(bgs, query, _handle_planes(L, qh), query.windows(w, step, scaffolds_all), rip, out.rows, out.status)
         finally:
             if qh:
                 L.frisk_b200_fasta_close(qh, st)
@@ -1612,7 +1525,7 @@ def run_backgrounds(backgrounds, query, kind: Optional[str] = None, w: int = 500
         return out
     wins = query.windows(w, step, scaffolds_all)
     assert len(wins) == n
-    return [bg._result(query, wins, rows[b * cap:b * cap + n], status[b * cap:b * cap + n]) for b, bg in enumerate(bgs)]
+    return [bg._result(query, wins, out.rows[b * cap:b * cap + n], out.status[b * cap:b * cap + n]) for b, bg in enumerate(bgs)]
 
 
 def run_backgrounds_resident(backgrounds, dq: DeviceGenome, w: int = 5000, step: int = 2500, scaffolds_all: bool = False,
