@@ -81,6 +81,29 @@ template <typename MT> __device__ __forceinline__ MT top_bits(int n) {       // 
     return n >= MB ? ~MT(0) : ~(~MT(0) >> n);
 }
 
+// P3 walks a thread's positions in rounds of four on the code words W of P1 (W[0] = the 16 bases from the round's first
+// position, first base on top): the K-mer of position j of the round and the (K+1)-mer of positions j, j + 1 are bit fields
+// of W[0] (2 j + 2 K + 2 <= 32 for j <= 2, K <= 8), and the next round shifts the words by four bases.
+template <int K> __device__ __forceinline__ uint32_t kmer_w(uint32_t w0, int j) { return (w0 << (2 * j)) >> (32 - 2 * K); }
+template <int K> __device__ __forceinline__ uint32_t pair_w(uint32_t w0, int j) { return (w0 << (2 * j)) >> (30 - 2 * K); }
+template <int NA> __device__ __forceinline__ void next_round(uint32_t (&w)[NA]) {
+#pragma unroll
+    for (int j = 0; j + 1 < NA; ++j) w[j] = __funnelshift_l(w[j + 1], w[j], 8);
+    w[NA - 1] <<= 8;
+}
+
+// Shared-memory reads at a 32-bit shared address (base taken once per CTA): register + immediate addressing in SASS
+__device__ __forceinline__ uint2 lds_u2(uint32_t a) {
+    uint2 v;
+    asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a));
+    return v;
+}
+__device__ __forceinline__ double2 lds_d2(uint32_t a) {
+    double2 v;
+    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(a));
+    return v;
+}
+
 // The k sweep of BASELINE config C3 (scores for kmax' = 1..K with kmin = 1, i.e. K reference runs `-m 1 -k k'`, F:1197-1206)
 // from ONE pass over the window: the counts of every order are there after the marginalisation, so the SWEEP
 // instantiation evaluates all K scores -- kmax' <= K-2 by walking that order's bins (coalesced genome-IVOM reads),
@@ -165,12 +188,12 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         const uint32_t p0 = (uint32_t)tid * cs;                          // this thread's first position
 
         // ---- P1: composition + ONE atomic per full K-word, all from registers ----------------------------
-        uint32_t kk[PP / 2];                                             // two K-mer codes per register
+        uint32_t W[NA];                                                  // W[j]: the 16 bases from position 16 j, first base on top
         MT vm = 0;                                                       // position i (bit MB-1-i) holds a full K-word
         {
             int non = 0, gc = 0, nfull = 0;
 #pragma unroll
-            for (int i = 0; i < PP / 2; ++i) kk[i] = 0;
+            for (int j = 0; j < NA; ++j) W[j] = 0;
             if (p0 < len) {
                 const uint32_t r0 = o_lo + p0;
                 uint32_t raw[NA + 1], mraw[NM], lraw[NM];
@@ -180,7 +203,6 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                 for (int j = 0; j < NM; ++j) mraw[j] = __ldg(mw + (r0 >> 5) + j);
 #pragma unroll
                 for (int j = 0; j < NM; ++j) lraw[j] = lw ? __ldg(lw + (r0 >> 5) + j) : 0u;
-                uint32_t W[NA];                                          // W[j]: the 16 bases from position 16 j
                 const uint32_t sc = (r0 & 15u) * 2u, ms = r0 & 31u;
 #pragma unroll
                 for (int j = 0; j < NA; ++j) W[j] = __funnelshift_l(raw[j + 1], raw[j], sc);
@@ -220,7 +242,6 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                         const uint32_t k0 = kmer_at(i), k1 = kmer_at(i + 1);
                         atomicAdd(&nib32[k0 >> 3], 1u << ((k0 & 7u) * 4u));
                         atomicAdd(&nib32[k1 >> 3], 1u << ((k1 & 7u) * 4u));
-                        kk[i >> 1] = k0 | (k1 << 16);
                     }
                 } else {
 #pragma unroll
@@ -228,7 +249,6 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                         if (vm & (MT(1) << (MB - 1 - i))) {
                             const uint32_t kap = kmer_at(i);
                             atomicAdd(&nib32[kap >> 3], 1u << ((kap & 7u) * 4u));
-                            kk[i >> 1] |= kap << (16 * (i & 1));
                         }
                     }
                 }
@@ -500,7 +520,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
                         if (vm & (MT(1) << (MB - 1 - j))) {
-                            const uint32_t kap = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
+                            const uint32_t kap = kmer_w<K>(W[0], j);
                             const double2 gg8 = __ldcg(sw.ig[7] + kap);           // L2 only, as in P3
                             const uint2 v = nib64[kap >> 4];
                             const uint32_t ws = (kap & 8u) ? v.y : v.x, wo = (kap & 8u) ? v.x : v.y;
@@ -518,8 +538,7 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                         }
                     }
                     vm <<= 4;
-#pragma unroll
-                    for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];
+                    next_round(W);
                 }
             }
             if ((uint32_t)tid < n_side) {                                  // a word of exactly 7 bases is an occurrence of its 7-mer too
@@ -575,16 +594,20 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
 
         // ---- P3: every position scores its own K-mer with weight 1 / (its count) --------------------
         const double qK2 = ss.q[K - 3], qK1 = ss.q[K - 2], qK = ss.q[K - 1];
-        // the window side of one position: a = I_w / c_K, om = 1 / c_K, lw = log2 I_w
+        // the window side of one position: a = I_w / c_K, om = 1 / c_K, lw = log2 I_w.  Its two shared-memory reads (the
+        // nibble word, the folded pair) at 32-bit shared addresses from bases taken once
+        const uint32_t s_nib = (uint32_t)__cvta_generic_to_shared(smem);
+        const uint32_t s_pre = s_nib + (L::FOLD_A ? L::OFF_PREA : L::OFF_PRE);
+        constexpr int PRE_SHIFT = 2 * (K - (L::FOLD_A ? A : LP));
         auto window_side = [&](uint32_t kap, double& a, double& om, double& lw) {
-            const uint2 v = nib64[kap >> 4];
+            const uint2 v = lds_u2(s_nib + (kap >> 4) * 8u);
             const uint32_t ws = (kap & 8u) ? v.y : v.x, wo = (kap & 8u) ? v.x : v.y;
             const uint32_t cK = (ws >> ((kap & 7u) * 4u)) & 15u;
             const uint32_t ps = nib_pairs(ws);
-            const uint32_t hs = ps >> ((kap & 4u) * 4u);                   // the quarter of the (K-1)-prefix: two pair sums
-            uint32_t cK1 = (hs & 0xffu) + ((hs >> 8) & 0xffu);
+            // the quarter of the (K-1)-prefix: two pair sums, the low two bytes after the shift
+            uint32_t cK1 = __dp4a(ps >> ((kap & 4u) * 4u), 0x0101u, 0u);
             uint32_t cK2 = __dp4a(ps + nib_pairs(wo), 0x01010101u, 0u);
-            const double2 pp = L::FOLD_A ? preA[kap >> (2 * (K - A))] : pre[kap >> (2 * (K - LP))];
+            const double2 pp = lds_d2(s_pre + (kap >> PRE_SHIFT) * 16u);
             double num = pp.x;
             uint32_t den = (uint32_t)__double2loint(pp.y);
             if (__double2hiint(pp.y)) {                    // rare: a short word of K-1 / K-2 bases lies below this bin
@@ -594,12 +617,13 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                     else cK2 += (code == (kap >> 4));
                 }
             }
-            if (K - 2 >= kmin) { den += cK2 << (2 * (K - 2)); num = fma(qK2, u32_to_double(cK2 * cK2), num); }
-            if (K - 1 >= kmin) { den += cK1 << (2 * (K - 1)); num = fma(qK1, u32_to_double(cK1 * cK1), num); }
+            if (K - 2 >= kmin) { den += cK2 << (2 * (K - 2)); num = fma(qK2, __uint2double_rn(cK2 * cK2), num); }
+            if (K - 1 >= kmin) { den += cK1 << (2 * (K - 1)); num = fma(qK1, __uint2double_rn(cK1 * cK1), num); }
             den += cK << (2 * K);
-            num = fma(qK, u32_to_double(cK * cK), num);
-            // a = I_w / c_K, om = 1 / c_K from ONE reciprocal, of den * c_K (exact product, < 2^37)
-            const double dden = u32_to_double(den), dc = u32_to_double(cK);
+            num = fma(qK, __uint2double_rn(cK * cK), num);
+            // a = I_w / c_K, om = 1 / c_K from ONE reciprocal, of den * c_K (exact product, < 2^37).  The five conversions
+            // as I2F.F64.U32 (exact): measured faster than the 2^52 + v trick of u32_to_double (a MOV and a DADD each)
+            const double dden = __uint2double_rn(den), dc = __uint2double_rn(cK);
             const double D = dden * dc;
             double r;
             asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(D));
@@ -664,23 +688,25 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                 for (int k = 1; k < 8; ++k) v = i == k ? arr[k] : v;
                 return v;
             };
-            // each group of backgrounds walks kk and vm again: vm is read through a shift, and kk is rotated CYCLICALLY
-            // through all PP / 4 rounds (the ones beyond the window's only rotate), so that it is whole again afterwards
+            // each group of backgrounds walks copies of the code words and of vm
             const int rounds = (int)(cs >> 2);
             for (int g0 = 0; g0 < sw.n_bg; g0 += kBgGroup) {
                 double s_w = 0.0, s_g[kBgGroup], s_t[kBgGroup];
 #pragma unroll
                 for (int b = 0; b < kBgGroup; ++b) s_g[b] = s_t[b] = 0.0;
                 const double2* const pg = sw.ig[0] + (size_t)g0 * kPairTable;     // this group's first pair table
+                uint32_t w[NA];
+#pragma unroll
+                for (int j = 0; j < NA; ++j) w[j] = W[j];
+                MT vr = vm;
 #pragma unroll 1
-                for (int r = 0; r < PP / 4; ++r) {
-                    const MT vr = r < rounds ? vm << (4 * r) : MT(0);
+                for (int r = 0; r < rounds; ++r) {
 #pragma unroll
                     for (int j = 0; j < 4; j += 2) {
-                        const uint32_t k0 = kk[j / 2] & 0xffffu, k1 = kk[j / 2] >> 16;
+                        const uint32_t k0 = kmer_w<K>(w[0], j), k1 = kmer_w<K>(w[0], j + 1);
                         const bool v0 = vr & (MT(1) << (MB - 1 - j)), v1 = vr & (MT(1) << (MB - 2 - j));
                         if (v0 || v1) {
-                            const uint32_t mu = v0 ? ((k0 << 2) | (k1 & 3u)) : k1;     // as in the one-background P3 below
+                            const uint32_t mu = v0 ? pair_w<K>(w[0], j) : k1;           // as in the one-background P3 below
                             double a0 = 0.0, om0 = 0.0, l0 = 0.0, a1 = 0.0, om1 = 0.0, l1 = 0.0;
                             if (v0) { window_side(k0, a0, om0, l0); s_w += a0; }
                             if (v1) { window_side(k1, a1, om1, l1); s_w += a1; }
@@ -695,11 +721,8 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
                             }
                         }
                     }
-                    const uint32_t w0 = kk[0], w1 = kk[1];
-#pragma unroll
-                    for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];
-                    kk[PP / 2 - 2] = w0;
-                    kk[PP / 2 - 1] = w1;
+                    vr <<= 4;
+                    next_round(w);
                 }
 #pragma unroll
                 for (int ofs = 16; ofs; ofs >>= 1) {
@@ -735,29 +758,23 @@ score_windows_nibble_kernel(const uint32_t* __restrict__ codes, const uint32_t* 
         const int rounds = (int)(cs >> 2);
 #pragma unroll 1
         for (int r = 0; r < rounds; ++r) {
-            uint32_t kp[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) kp[j] = (kk[j >> 1] >> (16 * (j & 1))) & 0xffffu;
             // positions j and j + 1 fetch both genome-IVOM entries with ONE 32-byte load from the pair table, at the
-            // (K+1)-mer of bases j .. j+K.  Only j + 1 valid: its K-mer with a leading A (the second half is still its
-            // entry).  Only j valid: the first half is used, kp[j + 1] & 3 only keeps mu in range.  L2 only (.cg): the
-            // table never survives in a ~30 KB L1 anyway, and not allocating there measured faster (0.703 -> 0.671 ms on C2)
+            // (K+1)-mer mu of bases j .. j+K.  Only j + 1 valid: mu is its K-mer with a leading A (the second half is still
+            // its entry).  Only j valid: the first half is used.  L2 only (.cg): the table never survives in a ~30 KB L1
+            // anyway, and not allocating there measured faster (0.703 -> 0.671 ms on C2)
 #pragma unroll
             for (int j = 0; j < 4; j += 2) {
                 const bool v0 = vm & (MT(1) << (MB - 1 - j)), v1 = vm & (MT(1) << (MB - 2 - j));
                 if (v0 || v1) {
-                    const uint32_t mu = v0 ? ((kp[j] << 2) | (kp[j + 1] & 3u)) : kp[j + 1];
+                    const uint32_t k1 = kmer_w<K>(W[0], j + 1), mu = v0 ? pair_w<K>(W[0], j) : k1;
                     double2 g0, g1;
                     ldcg_pair(pair + 2u * mu, g0, g1);
-                    if (v0) score_one(kp[j], g0);
-                    if (v1) score_one(kp[j + 1], g1);
+                    if (v0) score_one(mu >> 2, g0);
+                    if (v1) score_one(k1, g1);
                 }
             }
             vm <<= 4;
-#pragma unroll
-            for (int i = 0; i + 2 < PP / 2; ++i) kk[i] = kk[i + 2];         // rotate: the loop body stays one round long
-#pragma unroll
-            for (int i = (PP / 2 > 2 ? PP / 2 - 2 : 0); i < PP / 2; ++i) kk[i] = 0;
+            next_round(W);
         }
 #pragma unroll
         for (int ofs = 16; ofs; ofs >>= 1) {
